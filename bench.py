@@ -2,24 +2,32 @@
 """bench.py — env-steps/s including observation materialisation (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--num-envs E] [--legs all|none|a,b]
+                    [--dump-outputs DIR]
 
 A "step" is one lockstep step of the whole batch: every environment advances one turn and its observation
 (u8[3,11,11] + food, role, status), reward and done are written to HBM. Workload at N = 1: BASELINE.json
 configs[1] — 4,096 lockstep default-grid v1 environments with fused observation output (weak scaling: 4,096 envs
 per GPU, global env ids, no data-path collective).
 
-How the timed region is built (every leg): W (>= 3) untimed warm-up steps; then the K steps are replayed
-`repeats` times back to back so that the window is at least --min-window-ms long (a 20-step launch of 4,096 envs
-is 60 us — one such launch is not a measurement); the launches of one replay are captured in a CUDA graph so the
-host never throttles the queue; the outputs rotate through a ring of buffers larger than twice the L2; the window
-is bracketed by barrier + synchronize on both sides, timed with CUDA events on the launching stream, max over
-ranks. The one collective of the data-parallel run — the 64-byte all-reduce of the episode statistics — is issued
-a few times during the window on a SIDE stream (wab_gym_b200.sharding.AsyncStatsReducer): the compute stream never
-waits for it and nothing is read on the host before the stop event; its latency is reported as `collective_us`.
+How the headline's timed region is built: reset, W (>= 3) untimed warm-up steps, then a pass of K steps run twice
+untimed (eagerly, which loads every kernel it launches, and as the first replay of its CUDA graph), then the graph
+replayed once more, timed: the window holds exactly K steps (--steps), so a long window needs a large K; a small one
+measures launch latency (at 4,096 envs 20 steps are one 59 us launch). A pass whose outputs fit the 126 MB L2 (at
+4,096 envs, up to about 82 steps) rewrites lines the untimed passes have just written, so its stores may stay in the
+L2 inside the window; not measured, and at such K the launch latency bounds the run anyway. The actions
+are drawn from fixed seeds, so the same arguments give the same inputs and the same outputs on every run
+(--dump-outputs DIR writes the outputs of the last timed step). The other legs replay their pass `repeats` times
+back to back until the window is at least --leg-window-ms long, their outputs rotating through a ring of buffers
+larger than twice the L2 (the headline rotates its launches through up to that many). In every leg the graph keeps
+the host from throttling the queue; the window is bracketed by barrier + synchronize on both sides, timed with CUDA
+events on the launching stream, max over ranks. The one collective of the data-parallel run — the 64-byte all-reduce
+of the episode statistics — is issued during the window on a SIDE stream (wab_gym_b200.sharding.AsyncStatsReducer):
+the compute stream never waits for it and nothing is read on the host before the stop event; its latency is
+reported as `collective_us`.
 
 Printed JSON (rank 0, one line):
-  value        configs[1], device-resident: actions already in HBM, K steps per pass executed by the multi-step
-               kernel in launches of <= --fuse steps, every step's outputs written.
+  value        configs[1], device-resident: actions already in HBM, K steps executed by the multi-step kernel in
+               launches of <= --fuse steps, every step's outputs written.
   per_call     the same workload as single-step launches (what a policy in the loop gets), CUDA-graph replayed.
   e2e          the C-ABI host-buffer call (wab_vec_step_host_packed): pinned host actions in, every output in
                pinned host memory when the call returns, stream sync per step.
@@ -67,13 +75,17 @@ def config_dict(n, world):
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=4096)
+    # default: 131,072 timed steps of 4,096 envs, a window of about a quarter of a second on one B200. Other legs read
+    # K too: at this default the e2e leg runs its 20,000-step cap, and --impl reference its 2e8 env-step budget
+    # (about 48,800 steps at 4,096 envs, some 30 s on 16 host cores).
+    ap.add_argument("--steps", type=int, default=131072, help="timed lockstep steps of the headline")
     ap.add_argument("--warmup", type=int, default=64)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--num-envs", type=int, default=4096, help="environments per GPU")
     ap.add_argument("--fuse", type=int, default=256, help="steps per launch of the multi-step kernel")
-    ap.add_argument("--min-window-ms", type=float, default=500.0, help="shortest timed window of the headline leg")
     ap.add_argument("--leg-window-ms", type=float, default=60.0, help="shortest timed window of every other leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the headline's last timed step to DIR/<name>.npy (rank 0)")
     ap.add_argument("--legs", default="all", help="all | none | comma list of " + ",".join(ALL_LEGS))
     ap.add_argument("--cpu-seconds", type=float, default=20.0, help="budget of the cpu_baseline sample")
     ap.add_argument("--seed", type=int, default=0)
@@ -288,8 +300,10 @@ class Ctx:
 
     def timed_window(self, enqueue, launches_per_unit, min_ms, between=None):
         """Time `repeats` replays of one unit (= `launches_per_unit` calls enqueue(j), captured in a CUDA graph)
-        such that the window is >= min_ms. `between(r, repeats)` runs on the host after replay r was enqueued (side-stream
-        work only). Returns (window_ms max over ranks, repeats)."""
+        such that the window is >= min_ms, or exactly one replay when min_ms is None. Before the window the unit runs
+        once eagerly (loads every kernel, settles every allocation) and, captured, replays untimed (min_ms None: once,
+        the first replay uploads the graph; else twice, the calibration). `between(r, repeats)` runs on the host after
+        replay r was enqueued (side-stream work only). Returns (window_ms max over ranks, repeats)."""
         torch = self.torch
         side = torch.cuda.Stream(device=self.dev)
         graph = torch.cuda.CUDAGraph()
@@ -304,10 +318,15 @@ class Ctx:
         torch.cuda.current_stream(self.dev).wait_stream(side)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         torch.cuda.synchronize(self.dev)
-        e0.record(); graph.replay(); graph.replay(); e1.record()          # calibration (also warm-up of the replay)
+        e0.record(); graph.replay()
+        if min_ms is not None:
+            graph.replay()                                              # calibration (also warm-up of the replay)
+        e1.record()
         torch.cuda.synchronize(self.dev)
-        unit_ms = self.max_over_ranks(e0.elapsed_time(e1) / 2.0)
-        repeats = max(1, int(math.ceil(min_ms / max(unit_ms, 1e-4))))
+        repeats = 1
+        if min_ms is not None:
+            unit_ms = self.max_over_ranks(e0.elapsed_time(e1) / 2.0)
+            repeats = max(1, int(math.ceil(min_ms / max(unit_ms, 1e-4))))
         start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         self.barrier()
         try:                                  # keep the GPU busy ~0.2 ms while the host enqueues the first replays
@@ -326,19 +345,23 @@ class Ctx:
         return self.max_over_ranks(start.elapsed_time(stop)), repeats
 
 
-def v1_fused_leg(ctx, n, K, W, T, min_ms, with_collective):
-    """K lockstep steps of n v1 envs per pass through wab_vec_step_many (launches of <= T steps), replayed."""
+def v1_fused_leg(ctx, n, K, W, T, min_ms, with_collective, dump_dir=None):
+    """K lockstep steps of n v1 envs per pass through wab_vec_step_many (launches of <= T steps), replayed until the
+    window is >= min_ms; min_ms None: one pass, exactly K timed steps. dump_dir: see dump_step_outputs."""
     torch = ctx.torch
     from wab_gym_b200 import VecEnv
     from wab_gym_b200.sharding import AsyncStatsReducer
     env = VecEnv(n, seed=ctx.args.seed, device=ctx.dev, env_id_base=ctx.rank * n)
-    # Launches of <= T steps. K >= T: a pass of K steps is cut into chunks of T. K < T: a launch carries m = T // K whole
-    # passes (the K steps replayed m times inside ONE launch of the multi-step kernel, actions differing per pass).
-    m = max(1, T // K) if K < T else 1
+    once = min_ms is None
+    # Launches of <= T steps. K >= T: a pass of K steps is cut into chunks of T. K < T, replayed: a launch carries
+    # m = T // K whole passes (the K steps replayed m times inside ONE launch of the multi-step kernel, actions differing
+    # per pass).
+    m = max(1, T // K) if K < T and not once else 1
     L = m * K if K < T else T                                             # steps per full launch
     chunks = [(s, min(L, m * K - s)) for s in range(0, m * K, L)]         # launches of one unit of m passes
     slots = max(1, int(math.ceil(RING_BYTES / float(L * n * 372))))       # output ring > 2 x L2
-    units = max(1, int(math.ceil(slots / float(len(chunks)))))            # units per graph
+    units = 1 if once else max(1, int(math.ceil(slots / float(len(chunks)))))   # units per graph
+    slots = min(slots, units * len(chunks))                               # one pass: as many buffers as it has launches
     passes = units * m
     ring = [env._alloc(L) for _ in range(slots)]
     gen = torch.Generator(device=ctx.dev).manual_seed(1 + ctx.rank)
@@ -364,6 +387,8 @@ def v1_fused_leg(ctx, n, K, W, T, min_ms, with_collective):
         reducer.submit(env.stats_tensor)                                  # NCCL sets its channels up on first use
         reducer.result()
     window_ms, repeats = ctx.timed_window(enqueue, len(launches), min_ms, between=between if reducer is not None else None)
+    if dump_dir is not None and ctx.rank == 0:
+        dump_step_outputs(dump_dir, ring[(len(launches) - 1) % slots], launches[-1][1] - 1)
     total_steps = repeats * passes * K
     n_launch = repeats * len(launches)
     collective_us = None
@@ -401,11 +426,32 @@ def v1_fused_leg(ctx, n, K, W, T, min_ms, with_collective):
     return {"value": ctx.world * n * total_steps / (window_ms * 1e-3), "unit": "env-steps/s", "window_ms": window_ms,
             "repeats": repeats * passes, "steps_per_pass": K, "steps_per_launch": steps_per_launch, "launches": n_launch,
             "ms_per_step": window_ms / total_steps, "num_envs_per_gpu": n, "global_envs": ctx.world * n,
-            "ring": "%d output buffers of %d MB (ring of %d MB > 2 x L2), rotated per launch" % (
+            "ring": "%d output buffers of %d MB (ring of %d MB; the L2 holds 126 MB), rotated per launch" % (
                 slots, int(L * n * 372 / 1e6), int(slots * L * n * 372 / 1e6)),
             "roofline": roof, "collective_us": collective_us,
             "collectives_in_window": (reducer.submitted - 2) if reducer is not None else 0,
             "episode_stats": stats_all or stats}
+
+
+DUMP_MAX_ENVS = 32768       # x 369 float32 values per env = 48 MB, under the 64 MB a dump may take
+
+
+def dump_step_outputs(path, buf, t):
+    """Write step t of the multi-step output buffer `buf` — what a caller of wab_vec_step_many receives for that step:
+    grids, food, role, status, reward, done, info — as float32 DIR/<name>.npy, for at most DUMP_MAX_ENVS envs (a fixed,
+    seeded sample of them when there are more). env_index.npy (float64) holds the envs' indices."""
+    import numpy as np
+    import torch
+    n = buf["food"].shape[1]
+    idx = np.arange(n)
+    if n > DUMP_MAX_ENVS:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ENVS, replace=False))
+    sel = torch.from_numpy(idx).to(buf["food"].device)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "env_index.npy"), idx.astype(np.float64))
+    for name, v in buf.items():
+        if v is not None:
+            np.save(os.path.join(path, name + ".npy"), v[t].index_select(0, sel).cpu().numpy().astype(np.float32))
 
 
 def v1_percall_leg(ctx, n, K, W, min_ms):
@@ -596,7 +642,7 @@ def run_ours(args):
     want = ALL_LEGS if args.legs == "all" else tuple(x for x in args.legs.split(",") if x in ALL_LEGS)
 
     with ClockSampler(ctx.local_rank) as clocks:
-        main = v1_fused_leg(ctx, n, K, W, T, args.min_window_ms, with_collective=True)
+        main = v1_fused_leg(ctx, n, K, W, T, None, with_collective=True, dump_dir=args.dump_outputs)
         main_window = ctx.last_window
     percall = v1_percall_leg(ctx, n, K, W, args.leg_window_ms)
 
@@ -631,9 +677,8 @@ def run_ours(args):
             "ms_per_step": main["ms_per_step"], "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "u8 grids / int32 rules / u32 Philox (int food counter proven == f64)",
             "data": "synthetic", "config": config_dict(n, ctx.world),
-            "timing": {"mode": "wab_vec_step_many, %g steps per launch (= %g passes of the K steps in one launch of the multi-step "
-                               "kernel), every step's obs/reward/done written; the K steps replayed %d times for a %.0f ms window" % (
-                                   main["steps_per_launch"], main["steps_per_launch"] / K, main["repeats"], main["window_ms"]),
+            "timing": {"mode": "wab_vec_step_many, %g steps per launch, every step's obs/reward/done written; the K = %d steps "
+                               "timed once, a %.3g ms window" % (main["steps_per_launch"], K, main["window_ms"]),
                        "l2": main["ring"] + "; state lives in registers, no reuse between steps",
                        "collective": "64-byte statistics all-reduce on a side stream, %d issued inside the window, none awaited "
                                      "before the stop event" % main["collectives_in_window"]},

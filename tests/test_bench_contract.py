@@ -45,3 +45,38 @@ def test_gpu_arm_line():
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
     cb = d["cpu_baseline"]
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] > 0 and cb["single_thread"]["cores"] == 1
+
+
+@pytest.mark.gpu
+def test_gpu_arm_times_exactly_the_given_steps_and_dumps_reproducible_outputs(tmp_path):
+    import numpy as np
+    import torch
+    from wab_gym_b200 import VecEnv
+    n, K, W = 4096, 40, 3
+    args = ("--steps", str(K), "--warmup", str(W), "--legs", "none", "--skip-e2e", "--skip-cpu")
+    runs = [_run(*args, "--dump-outputs", str(tmp_path / d)) for d in ("a", "b")]
+    for d in runs:      # the envs stepped W warm-up steps, then the K-step pass twice untimed and once timed
+        assert d["steps"] == K and d["episode_stats"]["steps"] == n * (W + 3 * K)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b"))
+    total = 0
+    for name in names:
+        a, b = np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), name
+        total += os.path.getsize(tmp_path / "a" / name)
+    assert total <= 64 << 20
+    # the dumped step recomputed independently: the same seeded envs and actions through single-step launches
+    env = VecEnv(n, seed=0, device="cuda:0")
+    gen = torch.Generator(device="cuda:0").manual_seed(1)
+    actions = torch.randint(0, env.n_actions, (K + W, n), dtype=torch.uint8, device="cuda:0", generator=gen)
+    env.reset()
+    for a in list(actions[K:]) + 3 * list(actions[:K]):
+        obs, reward, done, info = env.step(a)
+    want = {"grids": obs.grids, "food": obs.food, "role": obs.role, "status": obs.status, "reward": reward, "done": done,
+            "info": info["info"]}
+    want = {k: v.cpu().numpy().astype(np.float32) for k, v in want.items()}
+    env.close()
+    assert names == sorted([k + ".npy" for k in want] + ["env_index.npy"])
+    assert np.array_equal(np.load(tmp_path / "a" / "env_index.npy"), np.arange(n, dtype=np.float64))
+    for k, v in want.items():
+        assert np.array_equal(np.load(tmp_path / "a" / (k + ".npy")), v), k

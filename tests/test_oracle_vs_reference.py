@@ -1,5 +1,6 @@
 """Live differential test: C oracle vs the unmodified reference run under oracle/ref_shim.
-Only runs where /root/reference exists (the build container); the GPU box uses tests/golden."""
+The live comparisons run only where the reference sources are present (WAB_REFERENCE_DIR); tests/golden carries the
+reference's behaviour everywhere else."""
 import importlib.util
 import os
 import sys
@@ -12,10 +13,11 @@ from oracle import ref_shim
 from oracle.wab_oracle import OracleEnv
 from tests.util import OPTION_SETS, pick_action
 
-pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not ref_shim.reference_available(), reason="reference sources not present")]
+needs_reference = pytest.mark.skipif(not ref_shim.reference_available(), reason="reference sources not present")
 
 
+@pytest.mark.reference
+@needs_reference
 @pytest.mark.parametrize("name", ["defaults", "six_actions_random_start", "dense", "tiny_bushes"])
 def test_oracle_matches_reference_live(name):
     overrides, greedy = OPTION_SETS[name]
@@ -48,19 +50,24 @@ def test_oracle_matches_reference_live(name):
 
 
 def test_clip_write_through_caps_food_at_one():
-    """SURVEY §7 step 1: eating at full food must give observation food 39 (not 44)."""
+    """SURVEY §7 step 1: eating at full food must give observation food 39 (not 44) and reward 0.1 — what the reference
+    returns, checked against the reference itself where its sources are present."""
     for env_id in range(200):
         orc = OracleEnv(None, seed=99, env_id=env_id)
         if orc.reset()[0][1][5, 5] == 1:
             break
     else:
         pytest.skip("no env starts on a bush")
-    ref = ref_shim.make_env(None, seed=99, env_id=env_id)
-    obs, reward, done, _ = ref.step(4)
-    assert obs[3] == 39 and abs(reward - 0.1) < 1e-12
-    assert orc.step(4)[0][1] == 39
+    obs, reward, done = orc.step(4)
+    assert obs[1] == 39 and abs(reward - 0.1) < 1e-12
+    if ref_shim.reference_available():
+        ref = ref_shim.make_env(None, seed=99, env_id=env_id)
+        obs, reward, done, _ = ref.step(4)
+        assert obs[3] == 39 and abs(reward - 0.1) < 1e-12
 
 
+@pytest.mark.reference
+@needs_reference
 def test_reference_unit_tests_pass_under_shim():
     """The reference's own known-answer tests (wab_env_test.py: PragmaticObsWrapper) run unmodified."""
     import unittest

@@ -60,7 +60,8 @@ VARIANTS = {
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--sizes", default="4096,1048576")
-    ap.add_argument("--steps", type=int, default=256)
+    ap.add_argument("--steps", type=int, default=0,
+                    help="timed steps per size; 0: 2^28 env-steps, 256 to 65,536 steps (as tools/window_steps.sh)")
     ap.add_argument("--variants", default=",".join(VARIANTS))
     ap.add_argument("--lpe", default="")
     args = ap.parse_args()
@@ -81,7 +82,7 @@ def main():
                 if lpe:
                     env["WAB_LPE"] = lpe
                 fuse = 64 if int(size) <= 65536 else 32
-                p = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--num-envs", size, "--steps", str(args.steps),
+                p = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--num-envs", size, "--steps", str(args.steps or min(65536, max(256, (1 << 28) // int(size)))),
                                     "--warmup", "8", "--fuse", str(fuse), "--skip-e2e", "--skip-cpu"],
                                    stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, env=env)
                 try:
