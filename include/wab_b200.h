@@ -164,6 +164,49 @@ int wab_vec_export_state(WabVec *h, int32_t *x, int32_t *y, double *food, int32_
                          int32_t *turn, int64_t *episode, int32_t *n_wolves, int32_t *wolves_xy,
                          uint32_t *bush_mask, int32_t *n_log, int32_t *log_xyc, void *stream);
 
+/* ---- checkpoint / resume / clone. The state of one env is one fixed-size, 16-byte-aligned RECORD (little-endian):
+ *
+ *   byte  0  u32 format        WAB_STATE_FORMAT
+ *         4  u32 flags         bit 0: stale centre bush (the last step ate the bush under the ostrich empty); others 0
+ *         8  u64 fingerprint   wab_vec_state_fingerprint of the handle that saved it
+ *        16  u64 env_id        global id of the env it was saved from
+ *        24  u32 episode       28 u32 turn       32 i32 x        36 i32 y
+ *        40  u32 role          44 u32 status     48 u32 food counter (WAB_FOOD_INT; 0 in F64 mode)
+ *        52  u32 n_wolves      56 f64 food (WAB_FOOD_F64; 0 in INT mode)
+ *        64  u32 bkey[2]       the episode's bush key
+ *        72  u32 n_log         76 u32 0
+ *        80  u32 window[4]     121-bit bush occupancy of the view (specialised kernels; 0 on the generic ones)
+ *        96  u32 wolves[wolf_cap]         x:i16 | y:i16 << 16; slots >= n_wolves are 0
+ *            u32 log_cell[log_cap]        depletion log, same packing; slots >= n_log are 0
+ *            u8  log_count[log_cap]       eats of each logged bush; slots >= n_log are 0
+ *            (0-padded to 4 bytes)
+ *            u32 hist[max_turns + 1]      only with wab_vec_enable_ego: position after turn t for 1 <= t <= turn, else 0
+ *            (0-padded to 16 bytes)
+ *
+ * Equal states give byte-equal records. The Bloom signature of the log and the "something was eaten empty" flag are not
+ * stored: loading rebuilds them from the log. Draws are keyed by the GLOBAL env id of the slot a record is loaded into,
+ * so a record loaded into the slot of its own id continues bit for bit on any shard layout, and one loaded into another
+ * slot is a clone: same world, ostrich, wolves and log, future draws keyed by the new id. */
+#define WAB_STATE_FORMAT 1
+/* Bytes of one record for this handle (depends on wolf_cap, log_cap, max_turns and whether ego is enabled). */
+int64_t wab_vec_state_record_bytes(const WabVec *h);
+/* 64-bit hash of the validated configuration field values, the bush threshold table, the seed, the kernel kind
+ * (wab_vec_kernel_kind) and the ego flag; not of env_id_base or n_envs. Records load only into a matching handle. */
+int wab_vec_state_fingerprint(const WabVec *h, uint64_t *out);
+/* d_slots i32[n] or NULL (= all N envs, n must be N); d_records u8[n][record_bytes], 16-byte aligned. Record r is the state
+ * of slot d_slots[r] (or r). Enqueued on the stream, no synchronisation. */
+int wab_vec_save_state(WabVec *h, const int32_t *d_slots, int64_t n, void *d_records, void *stream);
+/* Record r goes to slot d_slots[r] (NULL = slot r). obs may be all-NULL: state only, no observation written.
+ * Otherwise the observation (and bound features) of EVERY env is written, as after wab_vec_reset with an empty mask.
+ * *d_rejected (device int32) = number of records refused (format, fingerprint, n_wolves > wolf_cap, n_log > log_cap,
+ * role, status, food counter, turn or flags outside what the kernels maintain, slot out of range); when it is non-zero
+ * nothing was written. All-or-nothing without a host synchronisation. With duplicate destination slots one of the
+ * duplicates wins, unspecified which. */
+int wab_vec_load_state(WabVec *h, const void *d_records, const int32_t *d_slots, int64_t n, WabObs obs,
+                       int32_t *d_rejected, void *stream);
+/* Overwrite the accumulated statistics (row 0 = h_in8, every other per-warp row zeroed). */
+int wab_vec_set_stats(WabVec *h, const int64_t *h_in8, void *stream);
+
 int64_t wab_vec_num_envs(const WabVec *h);
 /* Lanes cooperating on one env (1, 4, 8, 16 or 32), chosen at create from the batch size so that a
  * small batch still covers every SM; results do not depend on it. */
@@ -294,12 +337,13 @@ int wab2_reset(Wab2World *h, void *stream);
  * before it acts. */
 int wab2_turn(Wab2World *h, const uint8_t *d_actions, uint8_t *d_planes, int32_t *d_internal, float *d_reward,
               uint8_t *d_done, void *stream);
-/* Hidden state for tests: out9 i32[N][E][9] = type, x, y, table X, table Y, Visible, food, role, status. Synchronises. */
-int wab2_export_state(Wab2World *h, int32_t *out9, int32_t *turn, void *stream);
+/* Hidden state (tests, checkpoints): out9 i32[N][E][9] = type, x, y, table X, table Y, Visible, food, role, status;
+ * turn and episode i32[N] (either may be NULL). Synchronises. */
+int wab2_export_state(Wab2World *h, int32_t *out9, int32_t *turn, int32_t *episode, void *stream);
 /* The inverse of wab2_export_state (tests: the reference's own known-answer worlds, World_tests.py:5-88, are built
- * from explicit positions): in9 i32[N][E][9] in the export layout (the type column must match the handle's entity
- * order: ostriches, wolves, bushes); turn i32[N] or NULL (unchanged). Synchronises. */
-int wab2_import_state(Wab2World *h, const int32_t *in9, const int32_t *turn, void *stream);
+ * from explicit positions; checkpoints): in9 i32[N][E][9] in the export layout (the type column must match the
+ * handle's entity order: ostriches, wolves, bushes); turn, episode i32[N] or NULL (unchanged). Synchronises. */
+int wab2_import_state(Wab2World *h, const int32_t *in9, const int32_t *turn, const int32_t *episode, void *stream);
 /* Which kernel serves this handle: 0 = wab2_turn_kernel (one thread per world), 1 = wab2_grid_turn_kernel (one
  * warp per world with occupancy planes, for worlds every observation window fits once). Results are identical. */
 int wab2_kernel_kind(const Wab2World *h);

@@ -18,6 +18,7 @@ EXPORTS = [
     "wab_vec_reset_host", "wab_vec_stats", "wab_vec_stats_device", "wab_vec_export_state", "wab_vec_num_envs", "wab_vec_lanes_per_env", "wab_vec_step_many_pipelined", "wab_vec_kernel_kind",
     "wab_vec_destroy", "wab_philox_device", "wab_vec_bind_features", "wab_pragmatic_features",
     "wab_vec_flatten_features", "wab_vec_flatten_features_noisy", "wab_sample_categorical", "wab_policy_tail", "wab_vec_enable_ego", "wab_vec_ego_proximities", "wab_vec_flat_dim", "wab_vec_host_block_layout", "wab_vec_step_host_packed", "wab_vec_forget_host_buffers",
+    "wab_vec_state_record_bytes", "wab_vec_state_fingerprint", "wab_vec_save_state", "wab_vec_load_state", "wab_vec_set_stats",
     "wab_policy_affine1_packed_bytes", "wab_policy_affine1_prepare", "wab_policy_affine1", "wab_policy_linear_packed_bytes", "wab_policy_linear_prepare", "wab_policy_trunk", "wab_policy_forward", "wab2_create", "wab2_kernel_kind", "wab2_output_layout", "wab2_reset", "wab2_turn", "wab2_export_state", "wab2_import_state", "wab2_destroy", "wab_last_error", "wab_abi_version",
 ]
 
@@ -63,6 +64,12 @@ def load():
     L.wab_vec_stats.argtypes = [vp, vp, i32, vp]
     L.wab_vec_stats_device.argtypes = [vp, vp, vp]
     L.wab_vec_export_state.argtypes = [vp] * 14
+    L.wab_vec_state_record_bytes.argtypes = [vp]
+    L.wab_vec_state_record_bytes.restype = i64
+    L.wab_vec_state_fingerprint.argtypes = [vp, vp]
+    L.wab_vec_save_state.argtypes = [vp, vp, i64, vp, vp]
+    L.wab_vec_load_state.argtypes = [vp, vp, vp, i64, WabObs, vp, vp]
+    L.wab_vec_set_stats.argtypes = [vp, vp, vp]
     L.wab_vec_num_envs.argtypes = [vp]
     L.wab_vec_num_envs.restype = i64
     L.wab_vec_kernel_kind.argtypes = [vp]
@@ -95,17 +102,17 @@ def load():
     L.wab2_create.argtypes = [vp, i64, u64, u64, i32, ctypes.POINTER(vp)]
     L.wab2_reset.argtypes = [vp, vp]
     L.wab2_turn.argtypes = [vp] * 7
-    L.wab2_export_state.argtypes = [vp] * 4
+    L.wab2_export_state.argtypes = [vp] * 5
     L.wab2_destroy.argtypes = [vp]
     L.wab2_kernel_kind.argtypes = [vp]
     L.wab2_output_layout.argtypes = [vp]
-    L.wab2_import_state.argtypes = [vp] * 4
+    L.wab2_import_state.argtypes = [vp] * 5
     L.wab2_destroy.restype = None
     L.wab_philox_device.argtypes = [vp, ctypes.c_uint32, ctypes.c_uint32, i64, vp, vp]
     L.wab_last_error.restype = ctypes.c_char_p
     L.wab_abi_version.restype = i32
     for name in EXPORTS:
-        if name not in ("wab_vec_num_envs", "wab_vec_lanes_per_env", "wab_vec_step_many_pipelined", "wab_vec_kernel_kind", "wab_vec_flat_dim", "wab_vec_destroy", "wab2_destroy",
+        if name not in ("wab_vec_num_envs", "wab_vec_state_record_bytes", "wab_vec_lanes_per_env", "wab_vec_step_many_pipelined", "wab_vec_kernel_kind", "wab_vec_flat_dim", "wab_vec_destroy", "wab2_destroy",
                         "wab_last_error", "wab_abi_version"):
             getattr(L, name).restype = ctypes.c_int
     _lib = L

@@ -265,7 +265,7 @@ int wab2_turn(Wab2World* h, const uint8_t* d_actions, uint8_t* d_planes, int32_t
     return WAB_OK;
 }
 
-int wab2_export_state(Wab2World* h, int32_t* out9, int32_t* turn, void* stream) {
+int wab2_export_state(Wab2World* h, int32_t* out9, int32_t* turn, int32_t* episode, void* stream) {
     if (!h || !out9) return fail(WAB_E_NULL, "null argument");
     DeviceGuard guard(h->device);
     WAB_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
@@ -275,6 +275,7 @@ int wab2_export_state(Wab2World* h, int32_t* out9, int32_t* turn, void* stream) 
     uint32_t* tr = new uint32_t[n];
     cudaError_t e = cudaMemcpy(ent, h->st.ent, 4 * n * 3 * E, cudaMemcpyDeviceToHost);
     if (e == cudaSuccess) e = cudaMemcpy(tr, h->st.turn, 4 * n, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && episode) e = cudaMemcpy(episode, h->st.episode, 4 * n, cudaMemcpyDeviceToHost);
     if (e == cudaSuccess)
         for (size_t i = 0; i < n; ++i) {
             if (turn) turn[i] = (int32_t)tr[i];
@@ -292,7 +293,7 @@ int wab2_export_state(Wab2World* h, int32_t* out9, int32_t* turn, void* stream) 
     return WAB_OK;
 }
 
-int wab2_import_state(Wab2World* h, const int32_t* in9, const int32_t* turn, void* stream) {
+int wab2_import_state(Wab2World* h, const int32_t* in9, const int32_t* turn, const int32_t* episode, void* stream) {
     if (!h || !in9) return fail(WAB_E_NULL, "null argument");
     DeviceGuard guard(h->device);
     WAB_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
@@ -313,6 +314,7 @@ int wab2_import_state(Wab2World* h, const int32_t* in9, const int32_t* turn, voi
     cudaError_t e = cudaSuccess;
     if (!bad) e = cudaMemcpy(h->st.ent, ent, 4 * n * 3 * E, cudaMemcpyHostToDevice);
     if (!bad && e == cudaSuccess && turn) e = cudaMemcpy(h->st.turn, turn, 4 * n, cudaMemcpyHostToDevice);
+    if (!bad && e == cudaSuccess && episode) e = cudaMemcpy(h->st.episode, episode, 4 * n, cudaMemcpyHostToDevice);
     delete[] ent;
     if (bad) return fail(WAB_E_CONFIG, "wab2_import_state: entity type order or value range does not fit the handle");
     if (e != cudaSuccess) return cuda_fail(e, "wab2_import_state");

@@ -1287,6 +1287,8 @@ struct WabVec {
     int host_mapped;   // -1 unknown, 0 staged copies, 1 kernel writes the pinned host block directly
     const void* m_actions; const void* m_block;        // host buffer pair whose device aliases are cached below
     const uint8_t* m_dactions; uint8_t* m_dblock;
+    uint64_t fp_config;    // fingerprint of config, bush thresholds, seed and kernel kind (wab_state.cuh; ego folded in on query)
+    uint8_t* d_zero_mask;  // u8[N] zeros: a reset that resets nothing re-emits every env's observation (after a state load)
 };
 
 namespace {
@@ -1559,6 +1561,7 @@ int wab_vec_create(const WabConfig* cfg, const uint32_t* bush_thr, int32_t n_bus
     st.wolves = (uint32_t*)(base + o_wolves); st.logcell = (uint32_t*)(base + o_lcell); st.logcnt = base + o_lcnt;
     st.stats = (unsigned long long*)(base + o_stats); st.n = n_envs;
     st.wstats = (unsigned long long*)(base + o_wstats); h->stat_rows = (int64_t)stat_rows;
+    h->fp_config = config_fingerprint(*cfg, bush_thr, n_bush_thr, seed, h->generic);
     *out = h;
     return WAB_OK;
 }
@@ -1569,6 +1572,7 @@ void wab_vec_destroy(WabVec* h) {
     if (h->slab) cudaFree(h->slab);
     if (h->d_hist) cudaFree(h->d_hist);
     if (h->d_thr) cudaFree(h->d_thr);
+    if (h->d_zero_mask) cudaFree(h->d_zero_mask);
     if (h->stage) cudaFree(h->stage);
     if (h->host_graph) cudaGraphExecDestroy(h->host_graph);
     if (h->host_stream) cudaStreamDestroy(h->host_stream);
@@ -2083,4 +2087,5 @@ int wab_philox_device(const uint32_t* d_ctr, uint32_t key0, uint32_t key1, int64
 
 }  // extern "C"
 
+#include "wab_state.cuh"
 #include "wab2_kernels.cuh"

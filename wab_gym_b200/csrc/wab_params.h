@@ -14,6 +14,35 @@ inline void fill_round_keys(Params& P, uint32_t k0, uint32_t k1) {
     for (int r = 0; r < 10; ++r) { P.rk0[r] = k0; P.rk1[r] = k1; k0 += PHILOX_W0; k1 += PHILOX_W1; }
 }
 
+// Fingerprint of what a saved env state depends on (wab_vec_state_fingerprint): every WabConfig field by VALUE (the
+// struct's padding bytes are undefined), the bush threshold table, the seed and the kernel kind. env_id_base and n_envs
+// are left out, so records move between shard layouts.
+inline uint64_t fp_mix(uint64_t h, uint64_t v) {
+    h ^= v + 0x9E3779B97F4A7C15ull + (h << 6) + (h >> 2);
+    h ^= h >> 30; h *= 0xBF58476D1CE4E5B9ull; h ^= h >> 27; h *= 0x94D049BB133111EBull; h ^= h >> 31;
+    return h;
+}
+inline uint64_t fp_f64(double d) { uint64_t v; memcpy(&v, &d, 8); return v; }
+inline uint64_t config_fingerprint(const WabConfig& c, const uint32_t* bush_thr, int32_t n_bush_thr, uint64_t seed, bool generic) {
+    uint64_t h = 0x5741425354415445ull;
+    const int64_t ints[] = {c.abi_version, c.width, c.height, c.max_turns, c.wolf_spawn_margin, c.n_actions,
+                            c.lookout_only, c.restrict_view, c.wolves, c.wolves_can_move, c.god_mode, c.starting_role,
+                            c.food_mode, c.auto_reset, c.food_int_start, c.food_int_inc, c.food_int_max, c.wolf_cap, c.log_cap};
+    for (int64_t v : ints) h = fp_mix(h, (uint64_t)v);
+    for (int a = 0; a < WAB_MAX_ACTIONS; ++a)
+        h = fp_mix(h, (uint64_t)(uint8_t)c.action_dx[a] | (uint64_t)(uint8_t)c.action_dy[a] << 8 | (uint64_t)(uint8_t)c.action_role[a] << 16);
+    h = fp_mix(h, fp_f64(c.food_start)); h = fp_mix(h, fp_f64(c.food_inc));
+    h = fp_mix(h, fp_f64(c.food_dec)); h = fp_mix(h, fp_f64(c.food_obs_scale));
+    for (int k = 0; k < 32; ++k) { h = fp_mix(h, c.spawn_cdf[k]); h = fp_mix(h, c.init_cdf[k]); }
+    h = fp_mix(h, c.thr_keep);
+    for (int k = 0; k < 8; ++k) { uint32_t v; memcpy(&v, &c.reward_table[k], 4); h = fp_mix(h, v); }
+    for (int k = 0; k < 4; ++k) h = fp_mix(h, (uint64_t)c.mask_lookout[k] | (uint64_t)c.mask_gatherer[k] << 32);
+    h = fp_mix(h, (uint64_t)n_bush_thr);
+    for (int32_t k = 0; k < n_bush_thr; ++k) h = fp_mix(h, bush_thr[k]);
+    h = fp_mix(h, seed);
+    return fp_mix(h, generic ? 1u : 0u);
+}
+
 inline int validate_config(const WabConfig* cfg, int32_t n_bush_thr, int64_t n_envs, std::string& err) {
     auto fail = [&err](int code, const char* msg) { err = msg; return code; };
     if (cfg->abi_version != WAB_ABI_VERSION) return fail(WAB_E_CONFIG, "WabConfig.abi_version mismatch");

@@ -99,6 +99,7 @@ class WolvesAndBushesEnv:
             Box(0, 1, (w, h), int), Box(0, 1, (w, h), int), Box(0, 1, (w, h), int),
             Discrete(game_options["turns_to_empty_food"] + 1), Discrete(2), Discrete(3)))
         self._lib = _lib.load()
+        self._seed, self._env_id, self._device = int(seed), int(env_id), int(device)
         cs = self._game.to_struct()
         thr = np.ascontiguousarray(self._game.bush_thr, dtype=np.uint32)
         handle = ctypes.c_void_p()
@@ -169,6 +170,36 @@ class WolvesAndBushesEnv:
             except ImportError:
                 pass
         return image
+
+    # ------------------------------------------------------------------ copy.deepcopy / pickle
+    def __getstate__(self):
+        """Options, keys, the env's state record (wab_vec_save_state) and the last observation: ``copy.deepcopy(env)`` and
+        ``pickle`` give an env that continues exactly like this one under the same actions."""
+        import torch
+        dev = torch.device("cuda", self._device)
+        buf = torch.empty(int(self._lib.wab_vec_state_record_bytes(self._h)), dtype=torch.uint8, device=dev)
+        stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)     # the copy below reads buf on this stream
+        _lib.check(self._lib.wab_vec_save_state(self._h, None, 1, ctypes.c_void_p(buf.data_ptr()), stream))
+        return {"game_options": self.game_options, "seed": self._seed, "env_id": self._env_id, "device": self._device,
+                "record": buf.cpu().numpy(), "grids": self._grids.copy(), "b": {k: v.copy() for k, v in self._b.items()},
+                "reward": self._reward.copy(), "current_turn": self.current_turn}
+
+    def __setstate__(self, state):
+        import torch
+        self.__init__(state["game_options"], seed=state["seed"], env_id=state["env_id"], device=state["device"])
+        dev = torch.device("cuda", self._device)
+        rec = torch.from_numpy(np.ascontiguousarray(state["record"], dtype=np.uint8)).to(dev)
+        rejected = torch.zeros(1, dtype=torch.int32, device=dev)
+        _lib.check(self._lib.wab_vec_load_state(self._h, ctypes.c_void_p(rec.data_ptr()), None, 1, _lib.WabObs(0, 0, 0, 0),
+                                                ctypes.c_void_p(rejected.data_ptr()),
+                                                ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+        if int(rejected.item()):
+            raise ValueError("the pickled env state does not fit these options")
+        self._grids[...] = state["grids"]
+        for k, v in state["b"].items():
+            self._b[k][...] = v
+        self._reward[...] = state["reward"]
+        self.current_turn = state["current_turn"]
 
     def seed(self, seed=None):
         return []

@@ -192,16 +192,20 @@ class Rollout:
         env.reset()
         self.graph = None
         if use_graph:
-            side = torch.cuda.Stream(device=env.device)
-            side.wait_stream(torch.cuda.current_stream(env.device))
-            with torch.cuda.stream(side):
-                for _ in range(3):
-                    self._step_eager()
-                side.synchronize()
-                self.graph = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(self.graph, stream=side):
-                    self._step_eager()
-            torch.cuda.current_stream(env.device).wait_stream(side)
+            self._capture(warmup=3)
+
+    def _capture(self, warmup: int):
+        env = self.env
+        side = torch.cuda.Stream(device=env.device)
+        side.wait_stream(torch.cuda.current_stream(env.device))
+        with torch.cuda.stream(side):
+            for _ in range(warmup):
+                self._step_eager()
+            side.synchronize()
+            self.graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(self.graph, stream=side):
+                self._step_eager()
+        torch.cuda.current_stream(env.device).wait_stream(side)
 
     @torch.no_grad()
     def _step_eager(self):
@@ -258,6 +262,24 @@ class Rollout:
             self.heads[0].copy_(w); self.heads[1].copy_(b)
         if self.affine1_tc is not None:
             self.affine1_tc.refresh()
+
+    def state_dict(self) -> dict:
+        """Environment state (``VecEnv.state_dict``), policy weights, the noise / sampling draw counter and the sampling seed:
+        a rollout resumed from it produces the same actions, values and rewards as one that never stopped."""
+        return {"env": self.env.state_dict(), "policy": {k: v.detach().cpu().clone() for k, v in self.policy.state_dict().items()},
+                "noise_ctr": int(self.noise_ctr.item()), "sample_seed": self.sample_seed}
+
+    def load_state_dict(self, sd: dict):
+        """Resume from ``state_dict()``. Every tensor is loaded in place, so a captured CUDA graph keeps working; a
+        different sampling seed (a kernel argument of the graph) is captured anew, without stepping."""
+        self.env.load_state_dict(sd["env"])
+        self.policy.load_state_dict(sd["policy"])
+        self.refresh_weights()
+        self.noise_ctr.fill_(int(sd["noise_ctr"]))
+        if int(sd["sample_seed"]) != self.sample_seed:
+            self.sample_seed = int(sd["sample_seed"])
+            if self.graph is not None:
+                self._capture(warmup=0)
 
     def step(self):
         if self.graph is not None:

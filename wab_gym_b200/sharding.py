@@ -26,6 +26,52 @@ def shard_range(total_envs: int, rank: int, world_size: int) -> Tuple[int, int]:
     return first, count
 
 
+# ---- checkpoints over shards: pure functions on state dicts (VecEnv.state_dict / VecWorld2.state_dict) ------------------
+# Draws are keyed by the global env id, so a record resumes bit for bit on whichever rank now holds its id.
+
+def merge_state_dicts(sds) -> dict:
+    """One state dict from the state dicts of several shards: records and ids concatenated, statistics summed."""
+    sds = list(sds)
+    if not sds:
+        raise ValueError("nothing to merge")
+    head = sds[0]
+    for sd in sds[1:]:
+        if sd["format"] != head["format"] or int(sd["fingerprint"]) != int(head["fingerprint"]):
+            raise ValueError("state dicts of different formats or fingerprints cannot be merged")
+        if sd["records"].shape[1:] != head["records"].shape[1:]:
+            raise ValueError("state dicts with different record sizes cannot be merged")
+    return {"format": head["format"], "fingerprint": int(head["fingerprint"]),
+            "env_ids": torch.cat([torch.as_tensor(sd["env_ids"], dtype=torch.int64) for sd in sds]),
+            "records": torch.cat([sd["records"] for sd in sds]),
+            "stats": torch.stack([torch.as_tensor(sd["stats"], dtype=torch.int64) for sd in sds]).sum(0)}
+
+
+def select_shard_records(sd: dict, env_id_base: int, num_envs: int, fingerprint: int, record_width: int,
+                         state_format: int = 1) -> torch.Tensor:
+    """The records of global ids ``env_id_base .. env_id_base + num_envs - 1`` in slot order (CPU). Raises ``ValueError``
+    on a format or fingerprint mismatch, a record size that does not fit, and an id of the range that is missing or
+    present more than once."""
+    if sd.get("format") != state_format:
+        raise ValueError("state format %r, expected %d" % (sd.get("format"), state_format))
+    if int(sd["fingerprint"]) != int(fingerprint):
+        raise ValueError("state fingerprint %#x does not match this handle (%#x): different options, seed or kernel family"
+                         % (int(sd["fingerprint"]), int(fingerprint)))
+    records = sd["records"]
+    ids = torch.as_tensor(sd["env_ids"], dtype=torch.int64).reshape(-1)
+    if records.dim() != 2 or records.shape[1] != record_width or records.shape[0] != ids.numel():
+        raise ValueError("records must be [n, %d] with one env id per record" % record_width)
+    sel = (ids >= env_id_base) & (ids < env_id_base + num_envs)
+    local = ids[sel] - env_id_base
+    counts = torch.bincount(local, minlength=num_envs)
+    if bool((counts == 0).any()):
+        missing = (torch.nonzero(counts == 0).reshape(-1)[:4] + env_id_base).tolist()
+        raise ValueError("the state dict has no record for env id(s) %s" % missing)
+    if bool((counts > 1).any()):
+        dup = (torch.nonzero(counts > 1).reshape(-1)[:4] + env_id_base).tolist()
+        raise ValueError("the state dict has more than one record for env id(s) %s" % dup)
+    return records[sel][torch.argsort(local)]
+
+
 def _distributed(group=None) -> bool:
     import torch.distributed as dist
     return dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1

@@ -35,6 +35,19 @@ class ObsBatch(NamedTuple):
     status: torch.Tensor
 
 
+class EnvStates(NamedTuple):
+    """Saved state of n envs (``VecEnv.save_state``): one opaque record per env (layout: ``WAB_STATE_FORMAT`` in
+    ``include/wab_b200.h``), the global id each record was saved from, and the fingerprint of the options, seed and
+    kernel family the records belong to."""
+
+    records: torch.Tensor      # u8[n, record_bytes] on the device
+    env_ids: torch.Tensor      # i64[n] global env ids (CPU)
+    fingerprint: int
+
+
+#: version of the state record layout (WAB_STATE_FORMAT)
+STATE_FORMAT = 1
+
 _raw_stream = getattr(torch._C, "_cuda_getCurrentRawStream", None)   # the current stream's handle without a Stream object
 
 
@@ -84,6 +97,11 @@ class VecEnv:
         if not self.emit_grids and (not self.with_features or self.generic_kernels):
             raise ValueError("emit_grids=False needs features=True and the default 11 x 11 viewport")
         self.flat_dim = int(self.lib.wab_vec_flat_dim(self._h))
+        #: bytes of one env's state record and the fingerprint records must carry to load here (save_state / load_state)
+        self.record_bytes = int(self.lib.wab_vec_state_record_bytes(self._h))
+        fp = ctypes.c_uint64()
+        _lib.check(self.lib.wab_vec_state_fingerprint(self._h, ctypes.byref(fp)))
+        self.fingerprint = int(fp.value)
         self._out = self._alloc(None)
         self._many: Dict[int, dict] = {}
 
@@ -319,6 +337,87 @@ class VecEnv:
         _lib.check(self.lib.wab_vec_export_state(self._h, *(ctypes.c_void_p(st[k].ctypes.data) for k in order),
                                                  self._stream()))
         return st
+
+    # ------------------------------------------------------------------ checkpoint / resume / clone
+    def _local_slots(self, slots) -> torch.Tensor:
+        s = torch.as_tensor(slots, dtype=torch.int64).reshape(-1).cpu()
+        if s.numel() and (int(s.min()) < 0 or int(s.max()) >= self.num_envs):
+            raise ValueError("slots must lie in [0, %d)" % self.num_envs)
+        return s
+
+    def save_state(self, slots=None) -> EnvStates:
+        """The state of every env (or of ``slots``, in that order) as records on the device. Enqueued on the current
+        stream; nothing synchronises."""
+        if slots is None:
+            local, d_slots = torch.arange(self.num_envs, dtype=torch.int64), None
+        else:
+            local = self._local_slots(slots)
+            d_slots = local.to(device=self.device, dtype=torch.int32)
+        records = torch.empty((local.numel(), self.record_bytes), dtype=torch.uint8, device=self.device)
+        _lib.check(self.lib.wab_vec_save_state(self._h, _ptr(d_slots), local.numel(), _ptr(records), self._stream()))
+        return EnvStates(records, local + self.env_id_base, self.fingerprint)
+
+    def load_state(self, states: EnvStates, slots=None) -> ObsBatch:
+        """Write each record of ``states`` into a slot: the slot of its own global id (which must belong to this handle),
+        or ``slots[r]`` — a clone of the saved env whose future draws are keyed by the destination's global id. Every
+        check passes before anything is written; a refused load raises ``ValueError`` and changes nothing. Returns the
+        observation of every env, as ``reset`` with an empty mask would (``last_features`` is updated too). Synchronises
+        once, to read the device-side verdict."""
+        records = states.records
+        if records.dtype != torch.uint8 or records.dim() != 2 or records.shape[1] != self.record_bytes:
+            raise ValueError("records must be uint8 [n, %d] for this handle" % self.record_bytes)
+        if int(states.fingerprint) != self.fingerprint:
+            raise ValueError("state fingerprint %#x does not match this handle (%#x): different options, seed, wolf/log caps, "
+                             "kernel family or ego setting" % (int(states.fingerprint), self.fingerprint))
+        n = records.shape[0]
+        if slots is None:
+            local = torch.as_tensor(states.env_ids, dtype=torch.int64).reshape(-1).cpu() - self.env_id_base
+            if local.numel() != n:
+                raise ValueError("env_ids and records disagree in length")
+            if n and (int(local.min()) < 0 or int(local.max()) >= self.num_envs):
+                raise ValueError("a record's env id is outside this handle's [%d, %d)" %
+                                 (self.env_id_base, self.env_id_base + self.num_envs))
+        else:
+            local = self._local_slots(slots)
+            if local.numel() != n:
+                raise ValueError("slots and records disagree in length")
+        if torch.unique(local).numel() != n:
+            raise ValueError("duplicate destination slots")
+        identity = n == self.num_envs and torch.equal(local, torch.arange(n, dtype=torch.int64))
+        d_slots = None if identity else local.to(device=self.device, dtype=torch.int32)
+        records = records.to(self.device).contiguous()
+        rejected = torch.zeros(1, dtype=torch.int32, device=self.device)
+        b = self._out
+        self._bind(b)
+        _lib.check(self.lib.wab_vec_load_state(self._h, _ptr(records), _ptr(d_slots), n, self._obs_struct(b), _ptr(rejected),
+                                               self._stream()))
+        bad = int(rejected.item())
+        if bad:
+            raise ValueError("%d of %d state records refused (format word, fingerprint, or a wolf count, log length, role, "
+                             "status, food or turn outside what the kernels maintain); nothing was loaded" % (bad, n))
+        return ObsBatch(b["grids"], b["food"], b["role"], b["status"])
+
+    def state_dict(self) -> dict:
+        """Everything a resume needs, on the host (``torch.save`` works): format, fingerprint, global env ids, the records
+        and the 8 statistics totals. ``sharding.merge_state_dicts`` joins the dicts of several shards."""
+        st = self.save_state()
+        stats = self.stats()
+        return {"format": STATE_FORMAT, "fingerprint": st.fingerprint, "env_ids": st.env_ids.clone(),
+                "records": st.records.cpu(), "stats": torch.tensor([stats[k] for k in STAT_NAMES], dtype=torch.int64)}
+
+    def load_state_dict(self, sd: dict) -> ObsBatch:
+        """Resume from ``state_dict()`` output (of this or any other shard layout: the records of this handle's global ids
+        are picked, each exactly once). The statistics totals go to the shard holding env 0 and every other shard starts
+        from zero, so their sum is preserved."""
+        from .sharding import select_shard_records
+        records = select_shard_records(sd, self.env_id_base, self.num_envs, self.fingerprint, self.record_bytes)
+        ids = torch.arange(self.env_id_base, self.env_id_base + self.num_envs, dtype=torch.int64)
+        obs = self.load_state(EnvStates(records, ids, self.fingerprint))
+        stats = np.zeros(8, dtype=np.int64)
+        if self.env_id_base == 0:
+            stats[:] = torch.as_tensor(sd["stats"], dtype=torch.int64).numpy()
+        _lib.check(self.lib.wab_vec_set_stats(self._h, stats.ctypes.data, self._stream()))
+        return obs
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:

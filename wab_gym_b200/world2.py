@@ -9,6 +9,7 @@ entity i in that order, what the reference driver loop does (``Env2Tests.py:46-8
 from __future__ import annotations
 
 import ctypes
+import hashlib
 from typing import Dict, Optional
 
 import numpy as np
@@ -65,6 +66,7 @@ class VecWorld2:
         self.num_envs, self.n_entities = int(num_envs), n_ostriches + n_wolves + n_bushes
         self.n_acting = n_ostriches + n_wolves
         self.R = self.cfg.window_radius
+        self.seed, self.env_id_base = int(seed) & 0xFFFFFFFFFFFFFFFF, int(env_id_base)
         h = ctypes.c_void_p()
         _lib.check(self.lib.wab2_create(ctypes.byref(self.cfg), self.num_envs, int(seed) & 0xFFFFFFFFFFFFFFFF, int(env_id_base),
                                         self.device.index, ctypes.byref(h)))
@@ -121,19 +123,47 @@ class VecWorld2:
     def kernel_name(self) -> str:
         return "wab2_grid_turn_kernel (warp per world)" if self.lib.wab2_kernel_kind(self._h) else "wab2_turn_kernel (thread per world)"
 
-    def export_state(self):
+    def export_state(self, episode: Optional[np.ndarray] = None):
+        """(state9 i32[N, E, 9], turn i32[N]); ``episode`` (i32[N], optional) receives each world's episode counter."""
         out = np.zeros((self.num_envs, self.n_entities, 9), dtype=np.int32)
         turn = np.zeros(self.num_envs, dtype=np.int32)
-        _lib.check(self.lib.wab2_export_state(self._h, out.ctypes.data, turn.ctypes.data, self._stream()))
+        ep = None if episode is None else episode.ctypes.data
+        _lib.check(self.lib.wab2_export_state(self._h, out.ctypes.data, turn.ctypes.data, ep, self._stream()))
         return out, turn
 
-    def import_state(self, state9: np.ndarray, turn: Optional[np.ndarray] = None):
-        """Inverse of ``export_state`` (tests): ``state9`` i32[N, E, 9] = type, x, y, table X, table Y, Visible, food, role, status."""
+    def import_state(self, state9: np.ndarray, turn: Optional[np.ndarray] = None, episode: Optional[np.ndarray] = None):
+        """Inverse of ``export_state`` (tests, checkpoints): ``state9`` i32[N, E, 9] = type, x, y, table X, table Y, Visible,
+        food, role, status; ``turn`` and ``episode`` i32[N] or None (unchanged)."""
         st = np.ascontiguousarray(state9, dtype=np.int32)
         if st.shape != (self.num_envs, self.n_entities, 9):
             raise ValueError("state9 must have shape (num_envs, n_entities, 9)")
         tn = None if turn is None else np.ascontiguousarray(turn, dtype=np.int32)
-        _lib.check(self.lib.wab2_import_state(self._h, st.ctypes.data, None if tn is None else tn.ctypes.data, self._stream()))
+        ep = None if episode is None else np.ascontiguousarray(episode, dtype=np.int32)
+        _lib.check(self.lib.wab2_import_state(self._h, st.ctypes.data, None if tn is None else tn.ctypes.data,
+                                              None if ep is None else ep.ctypes.data, self._stream()))
+
+    @property
+    def fingerprint(self) -> int:
+        """64-bit hash of the configuration fields and the seed: a checkpoint loads only into a matching handle."""
+        fields = [getattr(self.cfg, name) for name, _ in Wab2ConfigStruct._fields_] + [self.seed]
+        digest = hashlib.blake2b(np.asarray(fields, dtype=np.int64).tobytes(), digest_size=8).digest()
+        return int.from_bytes(digest, "little")
+
+    def state_dict(self) -> dict:
+        """Every world's state on the host (synchronises): one int32 record per world = turn, episode, then the
+        ``export_state`` rows; same dict shape as ``VecEnv.state_dict`` (``sharding.merge_state_dicts`` applies)."""
+        episode = np.zeros(self.num_envs, dtype=np.int32)
+        st, turn = self.export_state(episode)
+        records = np.concatenate([turn[:, None], episode[:, None], st.reshape(self.num_envs, -1)], axis=1)
+        return {"format": 1, "fingerprint": self.fingerprint, "records": torch.from_numpy(records),
+                "env_ids": torch.arange(self.env_id_base, self.env_id_base + self.num_envs, dtype=torch.int64),
+                "stats": torch.zeros(8, dtype=torch.int64)}
+
+    def load_state_dict(self, sd: dict):
+        """Resume from ``state_dict()`` output of any shard layout: the worlds of this handle's global ids, each exactly once."""
+        from .sharding import select_shard_records
+        rec = select_shard_records(sd, self.env_id_base, self.num_envs, self.fingerprint, 2 + 9 * self.n_entities).numpy()
+        self.import_state(rec[:, 2:].reshape(self.num_envs, self.n_entities, 9), rec[:, 0], rec[:, 1])
 
     def close(self):
         if getattr(self, "_h", None):
