@@ -298,6 +298,37 @@ int wab_policy_forward(WabVec *h, const uint8_t *d_features, int64_t n_rows, con
                        const uint64_t *d_counter, uint8_t *d_actions, float *d_value, float *d_probs, float *d_logp,
                        float *d_z3, void *stream);
 
+/* The backward pass of Policy.forward for training (actor_critic.py:128-169) on the tensor cores. For T = n_steps steps of
+ * N = n_envs environments, rows t N + n in step-major order:
+ *   d_features u8[T][N][28] (as wab_vec_flatten_features), d_counters int64[T] (the *d_counter each step's
+ *   wab_policy_forward saw), d_actions u8[T N], d_g_logp / d_g_value f32[T N] (upstream gradients of the sampled
+ *   action's log-probability and of the value).
+ * Writes d_grad f32 = the gradient of sum_rows g_logp log pi(a | x) + g_value V(x) in
+ * torch.nn.utils.parameters_to_vector(policy.parameters()) order: affine1.weight [128][flat_dim], affine1.bias [128],
+ * affine2.weight [150][128], affine2.bias [150], affine3.weight [128][150], affine3.bias [128], action_head.weight [A][128],
+ * action_head.bias [A], value_head.weight [1][128], value_head.bias [1].
+ * x is the input the forward saw: row n of step t under counter d_counters[t] (the noise key is the row within its step,
+ * as wab_vec_flatten_features_noisy / wab_policy_forward key it). The forward is recomputed with wab_policy_forward's
+ * arithmetic: d_logp / d_value f32[T N] (each may be NULL) receive the recomputed log pi(a | x) and V(x), bit-identical
+ * to what wab_policy_forward returned for the same inputs. d_rows int32[...] / d_n_rows int64[1] (both NULL: every row)
+ * restrict the work to the first *d_n_rows entries of d_rows (d_rows must hold that many); the count is read on the device,
+ * so the call never synchronises, and is clamped to [0, T N]. Rows left out contribute nothing, as do listed entries
+ * outside [0, T N) and rows with zero upstream gradients.
+ * d_packed1..3, d_bias1..3, hidden2 (150), d_w_heads / d_b_heads (stacked as for wab_policy_forward) as for
+ * wab_policy_forward; d_packed2t = wab_policy_linear_prepare(affine2.weight^T f32[128][150], 128, 150), d_packed3t =
+ * wab_policy_linear_prepare(affine3.weight^T f32[150][128], 150, 128). d_scratch: at least
+ * wab_policy_backward_scratch_bytes(h) bytes, 16-byte aligned, contents irrelevant. Equal inputs give bit-identical
+ * d_grad (fixed-order reductions, no atomics). WAB_E_NULL for a missing pointer, WAB_E_CONFIG for misalignment or too
+ * small a scratch, WAB_E_UNSUPPORTED beyond 8 actions, for hidden2 != 150 or flat_dim > 512. */
+int64_t wab_policy_backward_scratch_bytes(const WabVec *h);
+int wab_policy_backward(WabVec *h, const uint8_t *d_features, int64_t n_steps, int64_t n_envs, const uint64_t *d_counters,
+                        const uint8_t *d_actions, const float *d_g_logp, const float *d_g_value, const int32_t *d_rows,
+                        const int64_t *d_n_rows, const void *d_packed1, const float *d_bias1, const void *d_packed2,
+                        const float *d_bias2, int32_t hidden2, const void *d_packed3, const float *d_bias3,
+                        const void *d_packed2t, const void *d_packed3t, const float *d_w_heads, const float *d_b_heads,
+                        int32_t n_actions, float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi,
+                        void *d_scratch, int64_t scratch_bytes, float *d_grad, float *d_logp, float *d_value, void *stream);
+
 /* The tail of the reference's Policy.forward + select_action (actor_critic.py:84-97, :108-125) for n_rows rows in one
  * pass, fp32: d_z3 f32[n_rows][128] is the PRE-activation output of affine3; x = clamp(leaky_relu(z3), lo, hi);
  * logits = W[0..A) x + b, value = W[A] x + b[A] (d_w_heads f32[A + 1][128] = action_head.weight stacked on

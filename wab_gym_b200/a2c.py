@@ -18,15 +18,21 @@ reference computes ``nan`` there and poisons its weights); such episodes are lef
 
 ``mode="horizon"`` keeps the fixed-horizon variant of round 1 (returns restart at episode boundaries, the unfinished
 tail is bootstrapped with the critic) — a different estimator, not the reference's update.
+
+``tensor_cores=True`` trains on this library's kernels: collection is ``wab_policy_forward`` (one tcgen05 launch per step,
+keyed sampling), the loss is the same torch code on the recorded log-probabilities and values as leaves, and the backward
+pass is ``wab_policy_backward``, which recomputes the forward from the 28 feature bytes of every step instead of keeping
+autograd's activations (62 bytes per env-step instead of about 5.5 KB). It serves the reference's network only.
 """
 from __future__ import annotations
 
+import copy
 from typing import Dict, Tuple
 
 import torch
 import torch.nn.functional as F
 
-from .policy import Policy
+from .policy import Policy, PolicyTrainTC
 from .vec_env import VecEnv
 
 
@@ -61,9 +67,26 @@ def episodic_actor_critic_loss(log_probs: torch.Tensor, values: torch.Tensor, re
                                       "mean_length": (length * usable).sum() / usable.sum().clamp(min=1)}
 
 
+def horizon_actor_critic_loss(log_probs: torch.Tensor, values: torch.Tensor, rewards: torch.Tensor, dones: torch.Tensor,
+                              bootstrap: torch.Tensor, gamma: float, eps: float) -> Tuple[torch.Tensor, Dict[str, torch.Tensor]]:
+    """The fixed-horizon loss of ``mode="horizon"``: returns restart at done, the tail is bootstrapped with ``bootstrap``."""
+    T, N = rewards.shape
+    with torch.no_grad():
+        running = bootstrap
+        returns = torch.empty(T, N, device=rewards.device)
+        for t in range(T - 1, -1, -1):                                       # R = r + gamma * R, restarted at done
+            running = rewards[t] + gamma * running * (~dones[t]).float()
+            returns[t] = running
+        returns = (returns - returns.mean()) / (returns.std() + eps)
+    advantage = returns - values.detach()
+    policy_loss = -(log_probs * advantage).sum(0).mean()
+    value_loss = F.smooth_l1_loss(values, returns, reduction="none").sum(0).mean()
+    return policy_loss + value_loss, {"policy_loss": policy_loss.detach(), "value_loss": value_loss.detach()}
+
+
 class A2CTrainer:
     def __init__(self, env: VecEnv, policy: Policy = None, horizon: int = None, gamma: float = 0.99, lr: float = 3e-2,
-                 noise: bool = True, mode: str = "episodic"):
+                 noise: bool = True, mode: str = "episodic", tensor_cores: bool = False):
         if not env.with_features:
             raise ValueError("A2CTrainer needs VecEnv(features=True)")
         if mode not in ("episodic", "horizon"):
@@ -75,7 +98,89 @@ class A2CTrainer:
         self.eps = torch.finfo(torch.float32).eps                                # :104
         self._flat = torch.empty(env.num_envs, env.flat_dim, dtype=torch.float32, device=env.device)
         self._ctr = torch.zeros(1, dtype=torch.int64, device=env.device)
+        self.tensor_cores = bool(tensor_cores)
+        self.sample_seed = int(torch.initial_seed()) & (2 ** 63 - 1)
+        if self.tensor_cores:
+            self._init_tensor_cores()
         env.reset()
+
+    def _init_tensor_cores(self):
+        env, p, T, N = self.env, self.policy, self.horizon, self.env.num_envs
+        if any(prm.dtype != torch.float32 for prm in p.parameters()):
+            raise ValueError("tensor_cores=True trains an fp32 policy")
+        shapes = [(m.in_features, m.out_features) for m in (p.affine1, p.affine2, p.affine3, p.value_head)]
+        if shapes != [(env.flat_dim, 128), (128, 150), (150, 128), (128, 1)] or p.action_head.in_features != 128 or \
+                not 1 <= p.action_head.out_features <= 8:
+            raise ValueError("tensor_cores=True is built for the reference's network: flat_dim -> 128 -> 150 -> 128 -> {A <= 8, 1}")
+        self._tc = PolicyTrainTC(env, p)
+        dev = env.device
+        self.last_batch = {"features": torch.empty(T, N, 28, dtype=torch.uint8, device=dev),
+                           "counters": torch.empty(T, dtype=torch.int64, device=dev),
+                           "actions": torch.empty(T, N, dtype=torch.uint8, device=dev),
+                           "logp": torch.empty(T, N, device=dev), "value": torch.empty(T, N, device=dev),
+                           "reward": torch.empty(T, N, device=dev), "done": torch.empty(T, N, dtype=torch.bool, device=dev)}
+        self._grad = torch.empty(self._tc.n_params, device=dev)
+        self._rows = torch.empty(T * N + 1, dtype=torch.int32, device=dev)
+        self._iota = torch.arange(T * N, dtype=torch.int32, device=dev)
+        self._boot_actions = torch.empty(N, dtype=torch.uint8, device=dev)
+
+    def _sample_tc(self, features: torch.Tensor, actions: torch.Tensor, value: torch.Tensor, logp=None):
+        self._ctr += 1
+        self._tc.forward_sample(features, self._tc.heads, actions, value=value, logp=logp, noise_scale=0.01 if self.noise else 0.0,
+                                counter=self._ctr, seed=self.sample_seed)
+
+    def _train_iteration_tc(self) -> Dict[str, torch.Tensor]:
+        env, T, b = self.env, self.horizon, self.last_batch
+        if self.mode == "episodic":
+            env.reset()
+        for t in range(T):                                                       # :179-189, Policy.forward + select_action
+            b["features"][t].copy_(env.last_features)
+            self._sample_tc(b["features"][t], b["actions"][t], b["value"][t], b["logp"][t])
+            b["counters"][t:t + 1].copy_(self._ctr)
+            _, reward, done, _ = env.step(b["actions"][t])
+            b["reward"][t].copy_(reward)
+            b["done"][t].copy_(done)
+        log_probs, values = b["logp"].clone().requires_grad_(), b["value"].clone().requires_grad_()
+        if self.mode == "episodic":
+            loss, info = episodic_actor_critic_loss(log_probs, values, b["reward"], b["done"], self.gamma, self.eps)
+        else:
+            bootstrap = torch.empty(env.num_envs, device=env.device)
+            self._sample_tc(env.last_features, self._boot_actions, bootstrap)
+            loss, info = horizon_actor_critic_loss(log_probs, values, b["reward"], b["done"], bootstrap, self.gamma, self.eps)
+        g_logp, g_value = torch.autograd.grad(loss, [log_probs, values])
+        b["g_logp"], b["g_value"] = g_logp, g_value
+        # the rows with an upstream gradient, compacted on the device (no host synchronisation): after an env's first
+        # done the episodic loss has none
+        active = ((g_logp != 0) | (g_value != 0)).reshape(-1)
+        pos = torch.cumsum(active, 0, dtype=torch.int32) - 1
+        self._rows.scatter_(0, torch.where(active, pos, active.numel()).long(), self._iota)
+        n_rows = active.sum(dtype=torch.int64).reshape(1)
+        self._tc.backward(b["features"], b["counters"], b["actions"], g_logp, g_value, out=self._grad, rows=self._rows,
+                          n_rows=n_rows, noise_scale=0.01 if self.noise else 0.0)
+        off = 0
+        for prm in self.policy.parameters():                                     # .grad = views of the flat gradient
+            prm.grad = self._grad[off:off + prm.numel()].view_as(prm)
+            off += prm.numel()
+        self.optimizer.step()
+        self._tc.refresh()
+        info.update({"loss": loss.detach(), "mean_reward": b["reward"].mean()})
+        return info
+
+    def state_dict(self) -> dict:
+        """Environment state (``VecEnv.state_dict``), policy, Adam state, noise counter and sampling seed. With
+        ``tensor_cores=True`` (keyed sampling, deterministic gradients) a trainer resumed from it continues bit-exactly."""
+        return {"env": self.env.state_dict(), "policy": {k: v.detach().cpu().clone() for k, v in self.policy.state_dict().items()},
+                "optimizer": copy.deepcopy(self.optimizer.state_dict()), "noise_ctr": int(self._ctr.item()),
+                "sample_seed": self.sample_seed}
+
+    def load_state_dict(self, sd: dict):
+        self.env.load_state_dict(sd["env"])
+        self.policy.load_state_dict(sd["policy"])
+        self.optimizer.load_state_dict(sd["optimizer"])
+        self._ctr.fill_(int(sd["noise_ctr"]))
+        self.sample_seed = int(sd["sample_seed"])
+        if self.tensor_cores:
+            self._tc.refresh()
 
     def _observe(self) -> torch.Tensor:
         # gym.spaces.flatten (:188) + np.random.rand(...) / 100 (:189): the keyed kernel the rollout uses
@@ -84,6 +189,8 @@ class A2CTrainer:
         return self._flat.clone()        # autograd keeps a reference to the policy input of every step
 
     def train_iteration(self) -> Dict[str, torch.Tensor]:
+        if self.tensor_cores:
+            return self._train_iteration_tc()
         env, T = self.env, self.horizon
         if self.mode == "episodic":
             env.reset()                                                          # every env starts an episode (:179)
@@ -104,17 +211,7 @@ class A2CTrainer:
         else:
             with torch.no_grad():
                 _, bootstrap = self.policy(self._observe())                      # critic value of the unfinished tail
-                running = bootstrap.squeeze(1)
-                returns = torch.empty(T, env.num_envs, device=env.device)
-                for t in range(T - 1, -1, -1):                                   # R = r + gamma * R, restarted at done
-                    running = rewards[t] + self.gamma * running * (~dones[t]).float()
-                    returns[t] = running
-                returns = (returns - returns.mean()) / (returns.std() + self.eps)
-            advantage = returns - values.detach()
-            policy_loss = -(log_probs * advantage).sum(0).mean()
-            value_loss = F.smooth_l1_loss(values, returns, reduction="none").sum(0).mean()
-            loss = policy_loss + value_loss
-            info = {"policy_loss": policy_loss.detach(), "value_loss": value_loss.detach()}
+            loss, info = horizon_actor_critic_loss(log_probs, values, rewards, dones, bootstrap.squeeze(1), self.gamma, self.eps)
         self.optimizer.zero_grad(set_to_none=True)                               # :159
         loss.backward()                                                          # :165
         self.optimizer.step()

@@ -1033,6 +1033,7 @@ __global__ void __launch_bounds__(256) wab_flatten_noisy_kernel(const __grid_con
 
 }  // namespace
 #include "wab_policy_tc.cuh"
+#include "wab_policy_bwd.cuh"
 namespace {
 
 // The tail of the reference's Policy.forward and select_action in one pass (actor_critic.py:84-97, :108-125): from the
@@ -2054,6 +2055,68 @@ int wab_policy_tail(const float* d_z3, int32_t hidden, const float* d_w_heads, c
     wab_policy_tail_kernel<128><<<grid, 256, 0, (cudaStream_t)stream>>>(
         P, d_z3, d_w_heads, d_b_heads, n_rows, n_actions, leaky_slope, clamp_lo, clamp_hi,
         reinterpret_cast<const unsigned long long*>(d_counter), d_actions, d_value, d_probs, d_logp);
+    WAB_CUDA(cudaGetLastError());
+    return WAB_OK;
+}
+
+static int backward_grid(int device) {
+    int n_sm = 148;
+    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device);
+    return n_sm;
+}
+
+int64_t wab_policy_backward_scratch_bytes(const WabVec* h) {
+    return h ? (int64_t)backward_grid(h->device) * BP_BLOCK * (int64_t)sizeof(float) : 0;
+}
+
+int wab_policy_backward(WabVec* h, const uint8_t* d_features, int64_t n_steps, int64_t n_envs, const uint64_t* d_counters,
+                        const uint8_t* d_actions, const float* d_g_logp, const float* d_g_value, const int32_t* d_rows,
+                        const int64_t* d_n_rows, const void* d_packed1, const float* d_bias1, const void* d_packed2,
+                        const float* d_bias2, int32_t hidden2, const void* d_packed3, const float* d_bias3,
+                        const void* d_packed2t, const void* d_packed3t, const float* d_w_heads, const float* d_b_heads,
+                        int32_t n_actions, float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi,
+                        void* d_scratch, int64_t scratch_bytes, float* d_grad, float* d_logp, float* d_value, void* stream) {
+    if (!h || !d_features || !d_counters || !d_actions || !d_g_logp || !d_g_value || !d_packed1 || !d_bias1 || !d_packed2 ||
+        !d_bias2 || !d_packed3 || !d_bias3 || !d_packed2t || !d_packed3t || !d_w_heads || !d_b_heads || !d_scratch || !d_grad)
+        return fail(WAB_E_NULL, "null argument");
+    if ((d_rows == nullptr) != (d_n_rows == nullptr)) return fail(WAB_E_NULL, "d_rows and d_n_rows go together");
+    if (hidden2 != 150) return fail(WAB_E_UNSUPPORTED, "wab_policy_backward is built for the reference's trunk 128 -> 150 -> 128 (actor_critic.py:59-61)");
+    if (n_actions < 1 || n_actions > 8) return fail(WAB_E_UNSUPPORTED, "wab_policy_backward: at most 8 actions");
+    const int dim = wab_vec_flat_dim(h);
+    if (dim > TC_CHUNKS * TC_KC) return fail(WAB_E_UNSUPPORTED, "wab_policy_backward: the input is at most 512 columns wide");
+    if (n_steps < 0 || n_envs < 0 || n_steps * n_envs > INT32_MAX) return fail(WAB_E_CONFIG, "wab_policy_backward: 0 <= T N < 2^31 rows");
+    if (((uintptr_t)d_packed1 & 15u) != 0 || ((uintptr_t)d_packed2 & 15u) != 0 || ((uintptr_t)d_packed3 & 15u) != 0 ||
+        ((uintptr_t)d_packed2t & 15u) != 0 || ((uintptr_t)d_packed3t & 15u) != 0 || ((uintptr_t)d_scratch & 15u) != 0 ||
+        ((uintptr_t)d_features & 3u) != 0 || ((uintptr_t)d_counters & 7u) != 0 || ((uintptr_t)d_n_rows & 7u) != 0 ||
+        ((uintptr_t)d_rows & 3u) != 0 || ((uintptr_t)d_grad & 3u) != 0 || ((uintptr_t)d_g_logp & 3u) != 0 ||
+        ((uintptr_t)d_g_value & 3u) != 0 || ((uintptr_t)d_logp & 3u) != 0 || ((uintptr_t)d_value & 3u) != 0)
+        return fail(WAB_E_CONFIG, "the packed weights and d_scratch must be 16-byte aligned, d_counters and d_n_rows 8-byte, "
+                                  "d_features, d_rows and the float arrays 4-byte");
+    if (scratch_bytes < wab_policy_backward_scratch_bytes(h)) return fail(WAB_E_CONFIG, "d_scratch is smaller than wab_policy_backward_scratch_bytes");
+    DeviceGuard guard(h->device);
+    static bool attr_set[64] = {false};
+    if (h->device < 64 && !attr_set[h->device]) {
+        WAB_CUDA(cudaFuncSetAttribute(wab_policy_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_SMEM_TOTAL));
+        attr_set[h->device] = true;
+    }
+    BackwardArgs B;
+    memset(&B, 0, sizeof(B));
+    B.features = d_features; B.n_envs = n_envs > 0 ? n_envs : 1; B.n_rows = n_steps * n_envs;
+    B.counters = reinterpret_cast<const unsigned long long*>(d_counters);
+    B.actions = d_actions; B.g_logp = d_g_logp; B.g_value = d_g_value;
+    B.rows = d_rows; B.d_count = reinterpret_cast<const long long*>(d_n_rows);
+    B.w1 = reinterpret_cast<const uint4*>(d_packed1); B.b1 = d_bias1; B.w2 = reinterpret_cast<const uint4*>(d_packed2); B.b2 = d_bias2;
+    B.w3 = reinterpret_cast<const uint4*>(d_packed3); B.b3 = d_bias3;
+    B.w2t = reinterpret_cast<const uint4*>(d_packed2t); B.w3t = reinterpret_cast<const uint4*>(d_packed3t);
+    B.w_heads = d_w_heads; B.b_heads = d_b_heads; B.n_actions = n_actions; B.noise_scale = noise_scale; B.slope = leaky_slope;
+    B.clamp_lo = clamp_lo; B.clamp_hi = clamp_hi; B.scratch = reinterpret_cast<float*>(d_scratch);
+    B.logp_out = d_logp; B.value_out = d_value;
+    const int grid = backward_grid(h->device);
+    wab_policy_bwd_kernel<<<grid, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(h->P, (int)h->cfg.food_obs_scale + 1, B);
+    WAB_CUDA(cudaGetLastError());
+    const int64_t total = 128LL * dim + 128 + 150 * 128 + 150 + 128 * 150 + 128 + (int64_t)(n_actions + 1) * 129;
+    wab_policy_bwd_reduce_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        reinterpret_cast<const float*>(d_scratch), grid, dim, n_actions, d_grad);
     WAB_CUDA(cudaGetLastError());
     return WAB_OK;
 }

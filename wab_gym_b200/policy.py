@@ -153,6 +153,69 @@ class PolicyTrunkTC(Affine1TC):
         return actions
 
 
+class PolicyTrainTC(PolicyTrunkTC):
+    """The backward pass of ``Policy.forward`` on the tensor cores (``wab_policy_backward``): from what a rollout with
+    ``forward_sample`` recorded — features u8[T, N, 28], the noise counter of each step int64[T], actions u8[T, N] — and
+    upstream gradients ``g_logp``, ``g_value`` f32[T, N] of the sampled actions' log-probabilities and of the values, the
+    gradient of ``sum g_logp * log pi(a | x) + g_value * V(x)`` with respect to every parameter of the policy, as one flat
+    f32 buffer in ``parameters_to_vector(policy.parameters())`` order. The forward is recomputed from the feature bytes
+    (the policy input is regenerated, never stored), so training keeps 62 bytes per env-step instead of autograd's
+    activations. ``refresh()`` after an optimiser step re-packs the weights, the transposed ones included."""
+
+    def __init__(self, env: VecEnv, policy: "Policy"):
+        lib = _lib.load()
+        self.packed2t = torch.empty(int(lib.wab_policy_linear_packed_bytes(128, 150)), dtype=torch.uint8, device=env.device)
+        self.packed3t = torch.empty(int(lib.wab_policy_linear_packed_bytes(150, 128)), dtype=torch.uint8, device=env.device)
+        self.scratch = torch.empty(int(lib.wab_policy_backward_scratch_bytes(env._h)), dtype=torch.uint8, device=env.device)
+        self.heads = None
+        super().__init__(env, policy)
+        if policy.action_head.weight.shape[0] > 8 or policy.action_head.in_features != 128 or policy.value_head.in_features != 128:
+            raise ValueError("PolicyTrainTC is built for the reference's heads: 128 -> {A <= 8, 1}")
+        self.n_params = sum(p.numel() for p in policy.parameters())
+
+    @torch.no_grad()
+    def refresh(self):
+        super().refresh()
+        p = self.policy
+        w2t, w3t = p.affine2.weight.detach().float().t().contiguous(), p.affine3.weight.detach().float().t().contiguous()
+        _lib.check(self.lib.wab_policy_linear_prepare(_ptr(w2t), 128, 150, _ptr(self.packed2t), self._stream()))
+        _lib.check(self.lib.wab_policy_linear_prepare(_ptr(w3t), 150, 128, _ptr(self.packed3t), self._stream()))
+        w, b = stacked_heads(p)
+        if self.heads is None:
+            self.heads = (w, b)
+        else:
+            self.heads[0].copy_(w); self.heads[1].copy_(b)
+
+    def backward(self, features: torch.Tensor, counters: torch.Tensor, actions: torch.Tensor, g_logp: torch.Tensor,
+                 g_value: torch.Tensor, out: Optional[torch.Tensor] = None, rows: Optional[torch.Tensor] = None,
+                 n_rows: Optional[torch.Tensor] = None, noise_scale: float = 0.01, slope: float = 0.01,
+                 logp: Optional[torch.Tensor] = None, value: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Returns the flat gradient (``out`` f32[n_params] if given). ``rows`` int32 / ``n_rows`` int64[1] on the device:
+        only the first ``n_rows`` listed rows (indices into the T * N rows) are computed; ``logp`` / ``value`` f32[T, N]
+        receive the recomputed log-probabilities and values of those rows."""
+        T, N = actions.shape
+        if tuple(features.shape) != (T, N, 28) or features.dtype != torch.uint8 or not features.is_contiguous():
+            raise ValueError("features must be a contiguous uint8 [T, N, 28] tensor")
+        for name, t in (("g_logp", g_logp), ("g_value", g_value)):
+            if t.dtype != torch.float32 or tuple(t.shape) != (T, N) or not t.is_contiguous():
+                raise ValueError("%s must be a contiguous float32 [T, N] tensor" % name)
+        if counters.dtype != torch.int64 or counters.numel() != T or actions.dtype != torch.uint8 or not actions.is_contiguous():
+            raise ValueError("counters must be int64[T], actions a contiguous uint8 [T, N] tensor")
+        if (rows is None) != (n_rows is None) or (rows is not None and (rows.dtype != torch.int32 or n_rows.dtype != torch.int64)):
+            raise ValueError("rows (int32) and n_rows (int64[1]) go together")
+        if out is None:
+            out = torch.empty(self.n_params, dtype=torch.float32, device=self.env.device)
+        if out.dtype != torch.float32 or out.numel() != self.n_params or not out.is_contiguous():
+            raise ValueError("out must be a contiguous float32 tensor of n_params elements")
+        w, b = self.heads
+        _lib.check(self.lib.wab_policy_backward(
+            self.env._h, _ptr(features), T, N, _ptr(counters), _ptr(actions), _ptr(g_logp), _ptr(g_value), _ptr(rows), _ptr(n_rows),
+            _ptr(self.packed), _ptr(self.bias), _ptr(self.packed2), _ptr(self.bias2), 150, _ptr(self.packed3), _ptr(self.bias3),
+            _ptr(self.packed2t), _ptr(self.packed3t), _ptr(w), _ptr(b), w.shape[0] - 1, float(noise_scale), float(slope), -4.0, 4.0,
+            _ptr(self.scratch), self.scratch.numel(), _ptr(out), _ptr(logp), _ptr(value), self._stream()))
+        return out
+
+
 class Rollout:
     """N-environment rollout with every tensor resident on the device.
 
