@@ -329,6 +329,31 @@ int wab_policy_backward(WabVec *h, const uint8_t *d_features, int64_t n_steps, i
                         int32_t n_actions, float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi,
                         void *d_scratch, int64_t scratch_bytes, float *d_grad, float *d_logp, float *d_value, void *stream);
 
+/* PPO's clipped objective through the same backward pass, in one launch per minibatch. Arguments as for
+ * wab_policy_backward, except that the upstream gradients are formed on the device from d_logp_old, d_advantage and
+ * d_target f32[T N] (the log-probability the action was sampled with, the advantage A, the value target R). d_grad
+ * receives the gradient of sum over the listed rows of
+ *   l = -policy_weight * min(r A, clip(r, 1 - clip_eps, 1 + clip_eps) A) + value_weight * (V - R)^2 / 2
+ *       - entropy_weight * H,
+ *   r = exp(log pi(a | x) - logp_old),   H = -sum_o p_o log p_o,
+ * with log pi(a | x), V(x) and p recomputed under the current weights (bit-identical to wab_policy_forward's). So
+ * g_logp = -policy_weight A r, or 0 where the clip is active (A > 0 and r > 1 + clip_eps, or A < 0 and r < 1 - clip_eps),
+ * g_value = value_weight (V - R), and the entropy term adds entropy_weight p_o (log p_o + H) to d logit_o. With the
+ * per-row means of a minibatch of M rows, pass weights divided by M. d_logp, d_value and d_entropy f32[T N] (each may be
+ * NULL) receive the new log pi(a | x), V(x) and H of the listed rows. WAB_E_NULL for a missing d_logp_old, d_advantage or
+ * d_target; WAB_E_CONFIG for clip_eps <= 0 or NaN (+inf disables clipping) or a non-finite weight; otherwise as
+ * wab_policy_backward. */
+int wab_policy_ppo_backward(WabVec *h, const uint8_t *d_features, int64_t n_steps, int64_t n_envs,
+                            const uint64_t *d_counters, const uint8_t *d_actions, const float *d_logp_old,
+                            const float *d_advantage, const float *d_target, const int32_t *d_rows, const int64_t *d_n_rows,
+                            const void *d_packed1, const float *d_bias1, const void *d_packed2, const float *d_bias2,
+                            int32_t hidden2, const void *d_packed3, const float *d_bias3, const void *d_packed2t,
+                            const void *d_packed3t, const float *d_w_heads, const float *d_b_heads, int32_t n_actions,
+                            float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi, float clip_eps,
+                            float policy_weight, float value_weight, float entropy_weight, void *d_scratch,
+                            int64_t scratch_bytes, float *d_grad, float *d_logp, float *d_value, float *d_entropy,
+                            void *stream);
+
 /* The tail of the reference's Policy.forward + select_action (actor_critic.py:84-97, :108-125) for n_rows rows in one
  * pass, fp32: d_z3 f32[n_rows][128] is the PRE-activation output of affine3; x = clamp(leaky_relu(z3), lo, hi);
  * logits = W[0..A) x + b, value = W[A] x + b[A] (d_w_heads f32[A + 1][128] = action_head.weight stacked on

@@ -129,17 +129,23 @@ class A2CTrainer:
         self._tc.forward_sample(features, self._tc.heads, actions, value=value, logp=logp, noise_scale=0.01 if self.noise else 0.0,
                                 counter=self._ctr, seed=self.sample_seed)
 
-    def _train_iteration_tc(self) -> Dict[str, torch.Tensor]:
-        env, T, b = self.env, self.horizon, self.last_batch
-        if self.mode == "episodic":
-            env.reset()
-        for t in range(T):                                                       # :179-189, Policy.forward + select_action
+    def _collect_tc(self):
+        """``horizon`` steps from the current state into ``last_batch`` (features, counters, actions, logp, value, reward,
+        done), one ``wab_policy_forward`` launch per step."""
+        env, b = self.env, self.last_batch
+        for t in range(self.horizon):                                            # :179-189, Policy.forward + select_action
             b["features"][t].copy_(env.last_features)
             self._sample_tc(b["features"][t], b["actions"][t], b["value"][t], b["logp"][t])
             b["counters"][t:t + 1].copy_(self._ctr)
             _, reward, done, _ = env.step(b["actions"][t])
             b["reward"][t].copy_(reward)
             b["done"][t].copy_(done)
+
+    def _train_iteration_tc(self) -> Dict[str, torch.Tensor]:
+        env, T, b = self.env, self.horizon, self.last_batch
+        if self.mode == "episodic":
+            env.reset()
+        self._collect_tc()
         log_probs, values = b["logp"].clone().requires_grad_(), b["value"].clone().requires_grad_()
         if self.mode == "episodic":
             loss, info = episodic_actor_critic_loss(log_probs, values, b["reward"], b["done"], self.gamma, self.eps)

@@ -18,6 +18,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <cmath>
 #include <new>
 #include <string>
 #include <type_traits>
@@ -2069,35 +2070,41 @@ int64_t wab_policy_backward_scratch_bytes(const WabVec* h) {
     return h ? (int64_t)backward_grid(h->device) * BP_BLOCK * (int64_t)sizeof(float) : 0;
 }
 
-int wab_policy_backward(WabVec* h, const uint8_t* d_features, int64_t n_steps, int64_t n_envs, const uint64_t* d_counters,
-                        const uint8_t* d_actions, const float* d_g_logp, const float* d_g_value, const int32_t* d_rows,
-                        const int64_t* d_n_rows, const void* d_packed1, const float* d_bias1, const void* d_packed2,
-                        const float* d_bias2, int32_t hidden2, const void* d_packed3, const float* d_bias3,
-                        const void* d_packed2t, const void* d_packed3t, const float* d_w_heads, const float* d_b_heads,
-                        int32_t n_actions, float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi,
-                        void* d_scratch, int64_t scratch_bytes, float* d_grad, float* d_logp, float* d_value, void* stream) {
-    if (!h || !d_features || !d_counters || !d_actions || !d_g_logp || !d_g_value || !d_packed1 || !d_bias1 || !d_packed2 ||
+// wab_policy_backward and wab_policy_ppo_backward: the checks they share, then the backward kernel (the PPO one when
+// `ppo` is given) and the reduction. `d_g_logp` / `d_g_value` are wab_policy_backward's, checked by the caller.
+static int policy_backward_launch(const char* who, WabVec* h, const uint8_t* d_features, int64_t n_steps, int64_t n_envs,
+                                  const uint64_t* d_counters, const uint8_t* d_actions, const float* d_g_logp,
+                                  const float* d_g_value, const PpoArgs* ppo, const int32_t* d_rows, const int64_t* d_n_rows,
+                                  const void* d_packed1, const float* d_bias1, const void* d_packed2, const float* d_bias2,
+                                  int32_t hidden2, const void* d_packed3, const float* d_bias3, const void* d_packed2t,
+                                  const void* d_packed3t, const float* d_w_heads, const float* d_b_heads, int32_t n_actions,
+                                  float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi, void* d_scratch,
+                                  int64_t scratch_bytes, float* d_grad, float* d_logp, float* d_value, void* stream) {
+    if (!h || !d_features || !d_counters || !d_actions || !d_packed1 || !d_bias1 || !d_packed2 ||
         !d_bias2 || !d_packed3 || !d_bias3 || !d_packed2t || !d_packed3t || !d_w_heads || !d_b_heads || !d_scratch || !d_grad)
         return fail(WAB_E_NULL, "null argument");
     if ((d_rows == nullptr) != (d_n_rows == nullptr)) return fail(WAB_E_NULL, "d_rows and d_n_rows go together");
-    if (hidden2 != 150) return fail(WAB_E_UNSUPPORTED, "wab_policy_backward is built for the reference's trunk 128 -> 150 -> 128 (actor_critic.py:59-61)");
-    if (n_actions < 1 || n_actions > 8) return fail(WAB_E_UNSUPPORTED, "wab_policy_backward: at most 8 actions");
+    if (hidden2 != 150) return fail(WAB_E_UNSUPPORTED, std::string(who) + " is built for the reference's trunk 128 -> 150 -> 128 (actor_critic.py:59-61)");
+    if (n_actions < 1 || n_actions > 8) return fail(WAB_E_UNSUPPORTED, std::string(who) + ": at most 8 actions");
     const int dim = wab_vec_flat_dim(h);
-    if (dim > TC_CHUNKS * TC_KC) return fail(WAB_E_UNSUPPORTED, "wab_policy_backward: the input is at most 512 columns wide");
-    if (n_steps < 0 || n_envs < 0 || n_steps * n_envs > INT32_MAX) return fail(WAB_E_CONFIG, "wab_policy_backward: 0 <= T N < 2^31 rows");
+    if (dim > TC_CHUNKS * TC_KC) return fail(WAB_E_UNSUPPORTED, std::string(who) + ": the input is at most 512 columns wide");
+    if (n_steps < 0 || n_envs < 0 || n_steps * n_envs > INT32_MAX) return fail(WAB_E_CONFIG, std::string(who) + ": 0 <= T N < 2^31 rows");
     if (((uintptr_t)d_packed1 & 15u) != 0 || ((uintptr_t)d_packed2 & 15u) != 0 || ((uintptr_t)d_packed3 & 15u) != 0 ||
         ((uintptr_t)d_packed2t & 15u) != 0 || ((uintptr_t)d_packed3t & 15u) != 0 || ((uintptr_t)d_scratch & 15u) != 0 ||
         ((uintptr_t)d_features & 3u) != 0 || ((uintptr_t)d_counters & 7u) != 0 || ((uintptr_t)d_n_rows & 7u) != 0 ||
         ((uintptr_t)d_rows & 3u) != 0 || ((uintptr_t)d_grad & 3u) != 0 || ((uintptr_t)d_g_logp & 3u) != 0 ||
-        ((uintptr_t)d_g_value & 3u) != 0 || ((uintptr_t)d_logp & 3u) != 0 || ((uintptr_t)d_value & 3u) != 0)
+        ((uintptr_t)d_g_value & 3u) != 0 || ((uintptr_t)d_logp & 3u) != 0 || ((uintptr_t)d_value & 3u) != 0 ||
+        (ppo && (((uintptr_t)ppo->logp_old & 3u) != 0 || ((uintptr_t)ppo->advantage & 3u) != 0 ||
+                 ((uintptr_t)ppo->target & 3u) != 0 || ((uintptr_t)ppo->entropy_out & 3u) != 0)))
         return fail(WAB_E_CONFIG, "the packed weights and d_scratch must be 16-byte aligned, d_counters and d_n_rows 8-byte, "
                                   "d_features, d_rows and the float arrays 4-byte");
     if (scratch_bytes < wab_policy_backward_scratch_bytes(h)) return fail(WAB_E_CONFIG, "d_scratch is smaller than wab_policy_backward_scratch_bytes");
     DeviceGuard guard(h->device);
-    static bool attr_set[64] = {false};
-    if (h->device < 64 && !attr_set[h->device]) {
-        WAB_CUDA(cudaFuncSetAttribute(wab_policy_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_SMEM_TOTAL));
-        attr_set[h->device] = true;
+    static bool attr_set[2][64] = {{false}};
+    if (h->device < 64 && !attr_set[ppo ? 1 : 0][h->device]) {
+        if (ppo) WAB_CUDA(cudaFuncSetAttribute(wab_policy_ppo_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_SMEM_TOTAL));
+        else WAB_CUDA(cudaFuncSetAttribute(wab_policy_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_SMEM_TOTAL));
+        attr_set[ppo ? 1 : 0][h->device] = true;
     }
     BackwardArgs B;
     memset(&B, 0, sizeof(B));
@@ -2112,13 +2119,52 @@ int wab_policy_backward(WabVec* h, const uint8_t* d_features, int64_t n_steps, i
     B.clamp_lo = clamp_lo; B.clamp_hi = clamp_hi; B.scratch = reinterpret_cast<float*>(d_scratch);
     B.logp_out = d_logp; B.value_out = d_value;
     const int grid = backward_grid(h->device);
-    wab_policy_bwd_kernel<<<grid, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(h->P, (int)h->cfg.food_obs_scale + 1, B);
+    if (ppo) wab_policy_ppo_bwd_kernel<<<grid, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(h->P, (int)h->cfg.food_obs_scale + 1, B, *ppo);
+    else wab_policy_bwd_kernel<<<grid, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(h->P, (int)h->cfg.food_obs_scale + 1, B);
     WAB_CUDA(cudaGetLastError());
     const int64_t total = 128LL * dim + 128 + 150 * 128 + 150 + 128 * 150 + 128 + (int64_t)(n_actions + 1) * 129;
     wab_policy_bwd_reduce_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const float*>(d_scratch), grid, dim, n_actions, d_grad);
     WAB_CUDA(cudaGetLastError());
     return WAB_OK;
+}
+
+int wab_policy_backward(WabVec* h, const uint8_t* d_features, int64_t n_steps, int64_t n_envs, const uint64_t* d_counters,
+                        const uint8_t* d_actions, const float* d_g_logp, const float* d_g_value, const int32_t* d_rows,
+                        const int64_t* d_n_rows, const void* d_packed1, const float* d_bias1, const void* d_packed2,
+                        const float* d_bias2, int32_t hidden2, const void* d_packed3, const float* d_bias3,
+                        const void* d_packed2t, const void* d_packed3t, const float* d_w_heads, const float* d_b_heads,
+                        int32_t n_actions, float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi,
+                        void* d_scratch, int64_t scratch_bytes, float* d_grad, float* d_logp, float* d_value, void* stream) {
+    if (!d_g_logp || !d_g_value) return fail(WAB_E_NULL, "null argument");
+    return policy_backward_launch("wab_policy_backward", h, d_features, n_steps, n_envs, d_counters, d_actions, d_g_logp,
+                                  d_g_value, nullptr, d_rows, d_n_rows, d_packed1, d_bias1, d_packed2, d_bias2, hidden2,
+                                  d_packed3, d_bias3, d_packed2t, d_packed3t, d_w_heads, d_b_heads, n_actions, noise_scale,
+                                  leaky_slope, clamp_lo, clamp_hi, d_scratch, scratch_bytes, d_grad, d_logp, d_value, stream);
+}
+
+int wab_policy_ppo_backward(WabVec* h, const uint8_t* d_features, int64_t n_steps, int64_t n_envs, const uint64_t* d_counters,
+                            const uint8_t* d_actions, const float* d_logp_old, const float* d_advantage, const float* d_target,
+                            const int32_t* d_rows, const int64_t* d_n_rows, const void* d_packed1, const float* d_bias1,
+                            const void* d_packed2, const float* d_bias2, int32_t hidden2, const void* d_packed3,
+                            const float* d_bias3, const void* d_packed2t, const void* d_packed3t, const float* d_w_heads,
+                            const float* d_b_heads, int32_t n_actions, float noise_scale, float leaky_slope, float clamp_lo,
+                            float clamp_hi, float clip_eps, float policy_weight, float value_weight, float entropy_weight,
+                            void* d_scratch, int64_t scratch_bytes, float* d_grad, float* d_logp, float* d_value,
+                            float* d_entropy, void* stream) {
+    if (!d_logp_old || !d_advantage || !d_target) return fail(WAB_E_NULL, "null argument");
+    if (!(clip_eps > 0.f)) return fail(WAB_E_CONFIG, "wab_policy_ppo_backward: clip_eps must be > 0 (+inf disables clipping)");
+    if (!std::isfinite(policy_weight) || !std::isfinite(value_weight) || !std::isfinite(entropy_weight))
+        return fail(WAB_E_CONFIG, "wab_policy_ppo_backward: the loss weights must be finite");
+    PpoArgs Q;
+    memset(&Q, 0, sizeof(Q));
+    Q.logp_old = d_logp_old; Q.advantage = d_advantage; Q.target = d_target;
+    Q.clip_eps = clip_eps; Q.w_policy = policy_weight; Q.w_value = value_weight; Q.w_entropy = entropy_weight;
+    Q.entropy_out = d_entropy;
+    return policy_backward_launch("wab_policy_ppo_backward", h, d_features, n_steps, n_envs, d_counters, d_actions, nullptr,
+                                  nullptr, &Q, d_rows, d_n_rows, d_packed1, d_bias1, d_packed2, d_bias2, hidden2, d_packed3,
+                                  d_bias3, d_packed2t, d_packed3t, d_w_heads, d_b_heads, n_actions, noise_scale, leaky_slope,
+                                  clamp_lo, clamp_hi, d_scratch, scratch_bytes, d_grad, d_logp, d_value, stream);
 }
 
 int wab_sample_categorical(const void* d_probs, int32_t probs_bf16, int64_t n, int32_t n_actions, uint64_t seed,

@@ -215,6 +215,43 @@ class PolicyTrainTC(PolicyTrunkTC):
             _ptr(self.scratch), self.scratch.numel(), _ptr(out), _ptr(logp), _ptr(value), self._stream()))
         return out
 
+    def ppo_backward(self, features: torch.Tensor, counters: torch.Tensor, actions: torch.Tensor, logp_old: torch.Tensor,
+                     advantage: torch.Tensor, target: torch.Tensor, rows: Optional[torch.Tensor], n_rows: Optional[torch.Tensor],
+                     clip_eps: float, policy_weight: float, value_weight: float, entropy_weight: float,
+                     out: Optional[torch.Tensor] = None, logp: Optional[torch.Tensor] = None, value: Optional[torch.Tensor] = None,
+                     entropy: Optional[torch.Tensor] = None, noise_scale: float = 0.01, slope: float = 0.01) -> torch.Tensor:
+        """PPO's clipped objective in the same pass (``wab_policy_ppo_backward``): the gradient of the sum over the listed rows
+        of ``-policy_weight * min(r A, clip(r, 1 - clip_eps, 1 + clip_eps) A) + value_weight * (V - R)^2 / 2
+        - entropy_weight * H`` with ``r = exp(log pi(a | x) - logp_old)``, ``A = advantage``, ``R = target`` (f32[T, N]) and
+        log pi, V, H under the current weights. ``rows`` / ``n_rows`` as for ``backward`` (a minibatch); ``logp``, ``value``,
+        ``entropy`` f32[T, N] receive the new log-probabilities, values and entropies of the listed rows."""
+        T, N = actions.shape
+        if tuple(features.shape) != (T, N, 28) or features.dtype != torch.uint8 or not features.is_contiguous():
+            raise ValueError("features must be a contiguous uint8 [T, N, 28] tensor")
+        for name, t in (("logp_old", logp_old), ("advantage", advantage), ("target", target)):
+            if t.dtype != torch.float32 or tuple(t.shape) != (T, N) or not t.is_contiguous():
+                raise ValueError("%s must be a contiguous float32 [T, N] tensor" % name)
+        for name, t in (("logp", logp), ("value", value), ("entropy", entropy)):
+            if t is not None and (t.dtype != torch.float32 or tuple(t.shape) != (T, N) or not t.is_contiguous()):
+                raise ValueError("%s must be a contiguous float32 [T, N] tensor" % name)
+        if counters.dtype != torch.int64 or counters.numel() != T or actions.dtype != torch.uint8 or not actions.is_contiguous():
+            raise ValueError("counters must be int64[T], actions a contiguous uint8 [T, N] tensor")
+        if (rows is None) != (n_rows is None) or (rows is not None and (rows.dtype != torch.int32 or n_rows.dtype != torch.int64)):
+            raise ValueError("rows (int32) and n_rows (int64[1]) go together")
+        if out is None:
+            out = torch.empty(self.n_params, dtype=torch.float32, device=self.env.device)
+        if out.dtype != torch.float32 or out.numel() != self.n_params or not out.is_contiguous():
+            raise ValueError("out must be a contiguous float32 tensor of n_params elements")
+        w, b = self.heads
+        _lib.check(self.lib.wab_policy_ppo_backward(
+            self.env._h, _ptr(features), T, N, _ptr(counters), _ptr(actions), _ptr(logp_old), _ptr(advantage), _ptr(target),
+            _ptr(rows), _ptr(n_rows), _ptr(self.packed), _ptr(self.bias), _ptr(self.packed2), _ptr(self.bias2), 150,
+            _ptr(self.packed3), _ptr(self.bias3), _ptr(self.packed2t), _ptr(self.packed3t), _ptr(w), _ptr(b), w.shape[0] - 1,
+            float(noise_scale), float(slope), -4.0, 4.0, float(clip_eps), float(policy_weight), float(value_weight),
+            float(entropy_weight), _ptr(self.scratch), self.scratch.numel(), _ptr(out), _ptr(logp), _ptr(value), _ptr(entropy),
+            self._stream()))
+        return out
+
 
 class Rollout:
     """N-environment rollout with every tensor resident on the device.
