@@ -240,14 +240,23 @@ int wab_vec_flatten_features(WabVec *h, const uint8_t *d_features, int64_t n_row
 int wab_vec_flat_dim(const WabVec *h);
 /* The policy input of actor_critic.py:188-189 in one pass: the same one-hot rows plus noise_scale * U[0,1) per element
  * (the reference adds np.random.rand(...) / 100), written as f32 (out_bf16 = 0) or bf16 (1). The draws are keyed by
- * the handle's seed, the element index and the 64-bit value at d_counter (device memory, may be NULL = 0), which
- * the caller advances between calls — so a captured CUDA graph gets fresh noise on every replay. */
+ * the handle's seed, the element's column, its row's GLOBAL env id (env_id_base + row) and the 64-bit value at
+ * d_counter (device memory, may be NULL = 0), which the caller advances between calls — so a captured CUDA graph gets
+ * fresh noise on every replay.
+ *
+ * Keying contract of the policy entry points: every one that takes a WabVec handle (wab_vec_flatten_features_noisy,
+ * wab_policy_affine1, wab_policy_trunk, wab_policy_forward, wab_policy_backward, wab_policy_ppo_backward) keys its noise
+ * and its action samples by the global env id env_id_base + row (the row within its step for the backward passes), so
+ * a shard [first, first + count) draws exactly what the unsharded batch draws for rows first .. first + count - 1;
+ * outputs stay indexed by the local row. The two handle-less calls, wab_sample_categorical and wab_policy_tail, know no
+ * shard and key by the local row. */
 int wab_vec_flatten_features_noisy(WabVec *h, const uint8_t *d_features, int64_t n_rows, void *d_out,
                                    int32_t out_bf16, float noise_scale, const uint64_t *d_counter, void *stream);
 
 /* Categorical(probs).sample() of the reference's select_action (actor_critic.py:117-120) for n rows of n_actions <= 8
  * probabilities (f32, or bf16 when probs_bf16 = 1), one u8 action per row, on the device: inverse CDF on one
- * uniform per row keyed by (seed, row, *d_counter) — d_counter as in wab_vec_flatten_features_noisy. */
+ * uniform per row keyed by (seed, row, *d_counter) — d_counter as in wab_vec_flatten_features_noisy; row is the LOCAL
+ * row (no handle, no shard). */
 int wab_sample_categorical(const void *d_probs, int32_t probs_bf16, int64_t n, int32_t n_actions, uint64_t seed,
                            const uint64_t *d_counter, uint8_t *d_actions, void *stream);
 
@@ -289,7 +298,7 @@ int wab_policy_trunk(WabVec *h, const uint8_t *d_features, int64_t n_rows, const
 
 /* Policy.forward + select_action (actor_critic.py:84-97, :108-125) for n_rows environments as ONE kernel: wab_policy_trunk
  * followed, in the same launch, by what wab_policy_tail does (x = clamp(leaky_relu(z3), lo, hi), both heads, softmax, one
- * action per row by inverse CDF on a uniform keyed by (sample_seed, row, *d_counter)). Arguments as for those two calls;
+ * action per row by inverse CDF on a uniform keyed by (sample_seed, env_id_base + row, *d_counter)). Arguments as for those two calls;
  * d_value, d_probs, d_logp and d_z3 may be NULL. */
 int wab_policy_forward(WabVec *h, const uint8_t *d_features, int64_t n_rows, const void *d_packed1, const float *d_bias1,
                        const void *d_packed2, const float *d_bias2, int32_t hidden2, const void *d_packed3,
@@ -307,8 +316,8 @@ int wab_policy_forward(WabVec *h, const uint8_t *d_features, int64_t n_rows, con
  * torch.nn.utils.parameters_to_vector(policy.parameters()) order: affine1.weight [128][flat_dim], affine1.bias [128],
  * affine2.weight [150][128], affine2.bias [150], affine3.weight [128][150], affine3.bias [128], action_head.weight [A][128],
  * action_head.bias [A], value_head.weight [1][128], value_head.bias [1].
- * x is the input the forward saw: row n of step t under counter d_counters[t] (the noise key is the row within its step,
- * as wab_vec_flatten_features_noisy / wab_policy_forward key it). The forward is recomputed with wab_policy_forward's
+ * x is the input the forward saw: row n of step t under counter d_counters[t] (the noise key is the global env id
+ * env_id_base + n, as wab_vec_flatten_features_noisy / wab_policy_forward key it). The forward is recomputed with wab_policy_forward's
  * arithmetic: d_logp / d_value f32[T N] (each may be NULL) receive the recomputed log pi(a | x) and V(x), bit-identical
  * to what wab_policy_forward returned for the same inputs. d_rows int32[...] / d_n_rows int64[1] (both NULL: every row)
  * restrict the work to the first *d_n_rows entries of d_rows (d_rows must hold that many); the count is read on the device,
@@ -354,11 +363,23 @@ int wab_policy_ppo_backward(WabVec *h, const uint8_t *d_features, int64_t n_step
                             int64_t scratch_bytes, float *d_grad, float *d_logp, float *d_value, float *d_entropy,
                             void *stream);
 
+/* Data-parallel training: the cross-rank gradient sum, deterministic and rounded once.
+ * wab_policy_backward_grad_f64 reduces the scratch left by the last wab_policy_backward / wab_policy_ppo_backward with
+ * this d_scratch on this stream into d_grad64 f64[n_params] (same layout as d_grad, the same CTA order, the fp64 sums not
+ * rounded). wab_policy_grad_sum_ranks writes d_grad f32[n] = fp32(sum over r in index order of d_rank_grads[r][i]), the
+ * sum in fp64, for an all-gathered d_rank_grads f64[n_ranks][n]. With one rank, sum_ranks(grad_f64) equals
+ * wab_policy_backward's d_grad bit for bit. WAB_E_NULL for a missing pointer; WAB_E_CONFIG for misalignment (16 bytes
+ * for d_scratch, 8 for the fp64 arrays, 4 for d_grad), too small a scratch, n_ranks < 1 or n < 0; WAB_E_UNSUPPORTED
+ * beyond 8 actions or flat_dim > 512. */
+int wab_policy_backward_grad_f64(WabVec *h, const void *d_scratch, int64_t scratch_bytes, int32_t n_actions,
+                                 double *d_grad64, void *stream);
+int wab_policy_grad_sum_ranks(const double *d_rank_grads, int32_t n_ranks, int64_t n, float *d_grad, void *stream);
+
 /* The tail of the reference's Policy.forward + select_action (actor_critic.py:84-97, :108-125) for n_rows rows in one
  * pass, fp32: d_z3 f32[n_rows][128] is the PRE-activation output of affine3; x = clamp(leaky_relu(z3), lo, hi);
  * logits = W[0..A) x + b, value = W[A] x + b[A] (d_w_heads f32[A + 1][128] = action_head.weight stacked on
  * value_head.weight, d_b_heads f32[A + 1]); probs = softmax(logits); one action per row by inverse CDF on a uniform
- * keyed by (seed, row, *d_counter). Outputs: d_actions u8[n_rows]; d_value f32[n_rows], d_probs f32[n_rows][A],
+ * keyed by (seed, row, *d_counter), row the LOCAL row (no handle, no shard). Outputs: d_actions u8[n_rows]; d_value f32[n_rows], d_probs f32[n_rows][A],
  * d_logp f32[n_rows] (log-probability of the sampled action) — each may be NULL. */
 int wab_policy_tail(const float *d_z3, int32_t hidden, const float *d_w_heads, const float *d_b_heads, int64_t n_rows,
                     int32_t n_actions, float leaky_slope, float clamp_lo, float clamp_hi, uint64_t seed,

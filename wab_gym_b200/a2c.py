@@ -23,15 +23,30 @@ tail is bootstrapped with the critic) — a different estimator, not the referen
 keyed sampling), the loss is the same torch code on the recorded log-probabilities and values as leaves, and the backward
 pass is ``wab_policy_backward``, which recomputes the forward from the 28 feature bytes of every step instead of keeping
 autograd's activations (62 bytes per env-step instead of about 5.5 KB). It serves the reference's network only.
+
+Data-parallel training (``group``, a ``torch.distributed`` process group; ``tensor_cores=True`` only): each rank holds one
+contiguous shard of global env ids, ``VecEnv(count, env_id_base=first)`` with ``sharding.shard_range``. Construction
+checks on every rank that the shards tile ``[0, total)`` in rank order and that the trainers agree (options fingerprint,
+horizon, hyper-parameters, action count), then broadcasts rank 0's weights and sampling seed. The policy's draws are
+keyed by the global env id, so collection is invariant to the world size: rank r records exactly rows
+``[first_r, first_r + count_r)`` of a single-process run with the same weights. Every cross-rank sum (the gradient, the
+normalisation statistics of horizon mode and of PPO) is an all-gather followed by a sum in rank order in fp64 on every
+rank, so every rank holds bit-identical weights after every step. Training is deterministic for a fixed shard layout and
+resumes bit for bit on it; it is NOT bit-exact across world sizes (the tensor-core weight gradient rounds per 128-row
+tile in fp32, and the tiles hold other rows under another layout; PPO's minibatches depend on the layout). A checkpoint
+merged with ``sharding.merge_trainer_state_dicts`` resumes on any layout, a single process included, and its next
+collected batch equals the uninterrupted run's. Returned diagnostics describe this rank's rows, except ``grad_norm``
+(PPO), which is global.
 """
 from __future__ import annotations
 
 import copy
-from typing import Dict, Tuple
+from typing import Dict, Optional, Tuple
 
 import torch
 import torch.nn.functional as F
 
+from . import sharding
 from .policy import Policy, PolicyTrainTC
 from .vec_env import VecEnv
 
@@ -67,9 +82,8 @@ def episodic_actor_critic_loss(log_probs: torch.Tensor, values: torch.Tensor, re
                                       "mean_length": (length * usable).sum() / usable.sum().clamp(min=1)}
 
 
-def horizon_actor_critic_loss(log_probs: torch.Tensor, values: torch.Tensor, rewards: torch.Tensor, dones: torch.Tensor,
-                              bootstrap: torch.Tensor, gamma: float, eps: float) -> Tuple[torch.Tensor, Dict[str, torch.Tensor]]:
-    """The fixed-horizon loss of ``mode="horizon"``: returns restart at done, the tail is bootstrapped with ``bootstrap``."""
+def horizon_returns(rewards: torch.Tensor, dones: torch.Tensor, bootstrap: torch.Tensor, gamma: float) -> torch.Tensor:
+    """Discounted returns over [T, N] tensors, restarted at done, the tail bootstrapped with ``bootstrap`` f32[N]."""
     T, N = rewards.shape
     with torch.no_grad():
         running = bootstrap
@@ -77,16 +91,36 @@ def horizon_actor_critic_loss(log_probs: torch.Tensor, values: torch.Tensor, rew
         for t in range(T - 1, -1, -1):                                       # R = r + gamma * R, restarted at done
             running = rewards[t] + gamma * running * (~dones[t]).float()
             returns[t] = running
-        returns = (returns - returns.mean()) / (returns.std() + eps)
+    return returns
+
+
+def horizon_actor_critic_loss(log_probs: torch.Tensor, values: torch.Tensor, rewards: torch.Tensor, dones: torch.Tensor,
+                              bootstrap: torch.Tensor, gamma: float, eps: float, mean: Optional[torch.Tensor] = None,
+                              std: Optional[torch.Tensor] = None,
+                              total_envs: Optional[int] = None) -> Tuple[torch.Tensor, Dict[str, torch.Tensor]]:
+    """The fixed-horizon loss of ``mode="horizon"``: returns restart at done, the tail is bootstrapped with ``bootstrap``.
+    The returns are normalised by their mean and unbiased std over this batch, or by ``mean`` / ``std`` when given (those
+    of a data-parallel run's whole batch); the mean over environments divides by ``total_envs`` when given (the run's
+    environment count, so that the ranks' losses add up to the whole batch's)."""
+    returns = horizon_returns(rewards, dones, bootstrap, gamma)
+    with torch.no_grad():
+        if mean is None:
+            returns = (returns - returns.mean()) / (returns.std() + eps)
+        else:
+            returns = (returns - mean) / (std + eps)
     advantage = returns - values.detach()
-    policy_loss = -(log_probs * advantage).sum(0).mean()
-    value_loss = F.smooth_l1_loss(values, returns, reduction="none").sum(0).mean()
+    if total_envs is None:
+        policy_loss = -(log_probs * advantage).sum(0).mean()
+        value_loss = F.smooth_l1_loss(values, returns, reduction="none").sum(0).mean()
+    else:
+        policy_loss = -(log_probs * advantage).sum() / total_envs
+        value_loss = F.smooth_l1_loss(values, returns, reduction="none").sum() / total_envs
     return policy_loss + value_loss, {"policy_loss": policy_loss.detach(), "value_loss": value_loss.detach()}
 
 
 class A2CTrainer:
     def __init__(self, env: VecEnv, policy: Policy = None, horizon: int = None, gamma: float = 0.99, lr: float = 3e-2,
-                 noise: bool = True, mode: str = "episodic", tensor_cores: bool = False):
+                 noise: bool = True, mode: str = "episodic", tensor_cores: bool = False, group=None):
         if not env.with_features:
             raise ValueError("A2CTrainer needs VecEnv(features=True)")
         if mode not in ("episodic", "horizon"):
@@ -100,9 +134,47 @@ class A2CTrainer:
         self._ctr = torch.zeros(1, dtype=torch.int64, device=env.device)
         self.tensor_cores = bool(tensor_cores)
         self.sample_seed = int(torch.initial_seed()) & (2 ** 63 - 1)
+        self.group = group if sharding._distributed(group) else None
+        if self.group is not None and not self.tensor_cores:
+            raise ValueError("data-parallel training (a group of more than one rank) needs tensor_cores=True")
         if self.tensor_cores:
             self._init_tensor_cores()
         env.reset()
+        if self.group is not None:
+            self._join_group()
+
+    def _signature(self) -> tuple:
+        """What every rank of a data-parallel run must agree on."""
+        return (self.env.fingerprint, self.env.n_actions, self.horizon, self.mode, self.gamma, bool(self.noise),
+                float(self.optimizer.param_groups[0]["lr"]))
+
+    def _join_group(self):
+        """Validate the shard layout and the trainers on every rank (one host synchronisation), then take rank 0's
+        weights and sampling seed."""
+        import torch.distributed as dist
+        world, env = dist.get_world_size(self.group), self.env
+        infos = [None] * world
+        dist.all_gather_object(infos, (env.env_id_base, env.num_envs, self._signature()), group=self.group)
+        self.total_envs = sharding.check_trainer_shards(infos)
+        self._shard_counts = [int(c) for _, c, _ in infos]
+        src = dist.get_global_rank(self.group, 0)
+        with torch.no_grad():
+            for prm in self.policy.parameters():
+                dist.broadcast(prm.data, src, group=self.group)
+        seed = torch.tensor([self.sample_seed], dtype=torch.int64, device=env.device)
+        dist.broadcast(seed, src, group=self.group)
+        self.sample_seed = int(seed.item())
+        self._tc.refresh()
+        self._grad64 = torch.empty(self._tc.n_params, dtype=torch.float64, device=env.device)
+        self._gathered = torch.empty(world, self._tc.n_params, dtype=torch.float64, device=env.device)
+
+    def _sum_grad_over_ranks(self):
+        """The gradient of the last backward pass summed over the ranks into ``_grad``: fp64 per rank, all-gathered,
+        summed in rank order and rounded once."""
+        import torch.distributed as dist
+        self._tc.grad_f64(self._grad64)
+        dist.all_gather(list(self._gathered.unbind(0)), self._grad64, group=self.group)
+        self._tc.grad_sum_ranks(self._gathered, self._grad)
 
     def _init_tensor_cores(self):
         env, p, T, N = self.env, self.policy, self.horizon, self.env.num_envs
@@ -152,7 +224,12 @@ class A2CTrainer:
         else:
             bootstrap = torch.empty(env.num_envs, device=env.device)
             self._sample_tc(env.last_features, self._boot_actions, bootstrap)
-            loss, info = horizon_actor_critic_loss(log_probs, values, b["reward"], b["done"], bootstrap, self.gamma, self.eps)
+            stats = {}
+            if self.group is not None:                                           # normalised over the whole batch
+                mean, std = sharding.global_mean_std(horizon_returns(b["reward"], b["done"], bootstrap, self.gamma), self.group)
+                stats = {"mean": mean, "std": std, "total_envs": self.total_envs}
+            loss, info = horizon_actor_critic_loss(log_probs, values, b["reward"], b["done"], bootstrap, self.gamma, self.eps,
+                                                   **stats)
         g_logp, g_value = torch.autograd.grad(loss, [log_probs, values])
         b["g_logp"], b["g_value"] = g_logp, g_value
         # the rows with an upstream gradient, compacted on the device (no host synchronisation): after an env's first
@@ -163,6 +240,8 @@ class A2CTrainer:
         n_rows = active.sum(dtype=torch.int64).reshape(1)
         self._tc.backward(b["features"], b["counters"], b["actions"], g_logp, g_value, out=self._grad, rows=self._rows,
                           n_rows=n_rows, noise_scale=0.01 if self.noise else 0.0)
+        if self.group is not None:
+            self._sum_grad_over_ranks()
         off = 0
         for prm in self.policy.parameters():                                     # .grad = views of the flat gradient
             prm.grad = self._grad[off:off + prm.numel()].view_as(prm)
@@ -174,7 +253,9 @@ class A2CTrainer:
 
     def state_dict(self) -> dict:
         """Environment state (``VecEnv.state_dict``), policy, Adam state, noise counter and sampling seed. With
-        ``tensor_cores=True`` (keyed sampling, deterministic gradients) a trainer resumed from it continues bit-exactly."""
+        ``tensor_cores=True`` (keyed sampling, deterministic gradients) a trainer resumed from it continues bit-exactly.
+        In a data-parallel run the env part is this rank's shard; ``sharding.merge_trainer_state_dicts`` joins the ranks'
+        dicts, and ``load_state_dict`` takes a merged dict of any layout."""
         return {"env": self.env.state_dict(), "policy": {k: v.detach().cpu().clone() for k, v in self.policy.state_dict().items()},
                 "optimizer": copy.deepcopy(self.optimizer.state_dict()), "noise_ctr": int(self._ctr.item()),
                 "sample_seed": self.sample_seed}

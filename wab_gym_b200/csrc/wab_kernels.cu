@@ -977,7 +977,8 @@ __global__ void wab_flatten_kernel(const __grid_constant__ Params P, const uint8
 // and a column is a table lookup (feature index, value) -> one compare — no division, no per-element branching (the
 // first version spent 64 us on the 32,768 x 449 matrix, 7x its memory time, on 64-bit index arithmetic). One Philox
 // call feeds four columns of a lane; the 64-bit draw counter lives in device memory so a captured graph gets fresh
-// noise on every replay. BF16 = 0: f32 output, 1: bf16 output.
+// noise on every replay. The key is the global env id (env_id_base + row), so a shard draws what the unsharded batch
+// draws for the same envs. BF16 = 0: f32 output, 1: bf16 output.
 constexpr int FLAT_MAX_DIM = 2 * (2 * 4 * (MAX_DISTANCE + 1) + 4 * 11) + 2 + 256 + 2 + 3 + CELLS;
 __device__ __forceinline__ uint32_t flat_descriptor(int k, int food_dim) {     // fi : 8 | value : 8 | view-mask column : 1
     for (int species = 0; species < 2; ++species) {
@@ -1014,8 +1015,9 @@ __global__ void __launch_bounds__(256) wab_flatten_noisy_kernel(const __grid_con
         uint32_t w[4] = {0u, 0u, 0u, 0u};
         int it = 0;
         for (int k = lane; k < dim; k += 32, ++it) {
+            const uint64_t g = P.env_id_base + (uint64_t)row;      // the noise key: the row's global env id
             if (noisy && (it & 3) == 0)
-                philox(P, (uint32_t)row, (uint32_t)(row >> 32) ^ ((uint32_t)(it >> 2) << 24) ^ ((uint32_t)lane << 16), (uint32_t)ctr,
+                philox(P, (uint32_t)g, (uint32_t)(g >> 32) ^ ((uint32_t)(it >> 2) << 24) ^ ((uint32_t)lane << 16), (uint32_t)ctr,
                        (uint32_t)(ctr >> 32) ^ 0x464C4154u, w);
             const uint32_t d = desc[k];
             float v;
@@ -1043,6 +1045,7 @@ namespace {
 // log-probability. One warp per row: each lane holds HID / 32 activations, the n_actions + 1 dot products are warp
 // sums. fp32 throughout. Replaces eleven library launches (clamp, two skinny GEMMs that cuBLAS runs as 17 us gemv-style
 // kernels at 32,768 rows, their bias adds, softmax, sampling, copies) with one pass over the 16 MB activation matrix.
+// wab_policy_tail takes no handle, so it knows no shard: its draws are keyed by the local row.
 template <int HID>
 __global__ void __launch_bounds__(256) wab_policy_tail_kernel(const __grid_constant__ Params P, const float* __restrict__ z3,
                                                               const float* __restrict__ w_heads, const float* __restrict__ b_heads,
@@ -1112,7 +1115,8 @@ __global__ void __launch_bounds__(256) wab_policy_tail_kernel(const __grid_const
 }
 
 // Categorical(probs).sample() of actor_critic.py:117-120 for n rows of up to 8 probabilities: inverse CDF on one keyed
-// uniform per row (rows share a Philox call four at a time). BF16 = 1: probs are bf16.
+// uniform per row (rows share a Philox call four at a time), keyed by the local row (wab_sample_categorical takes no
+// handle, so it knows no shard). BF16 = 1: probs are bf16.
 template <int BF16>
 __global__ void wab_sample_kernel(const __grid_constant__ Params P, const void* __restrict__ probs, int64_t n, int n_actions,
                                   const unsigned long long* __restrict__ d_counter, uint8_t* __restrict__ actions) {
@@ -2070,6 +2074,11 @@ int64_t wab_policy_backward_scratch_bytes(const WabVec* h) {
     return h ? (int64_t)backward_grid(h->device) * BP_BLOCK * (int64_t)sizeof(float) : 0;
 }
 
+// parameters of the reference's Policy with a `dim`-wide input and `n_actions` actions (the flat gradient's length)
+static int64_t policy_n_params(int dim, int n_actions) {
+    return 128LL * dim + 128 + 150 * 128 + 150 + 128 * 150 + 128 + (int64_t)(n_actions + 1) * 129;
+}
+
 // wab_policy_backward and wab_policy_ppo_backward: the checks they share, then the backward kernel (the PPO one when
 // `ppo` is given) and the reduction. `d_g_logp` / `d_g_value` are wab_policy_backward's, checked by the caller.
 static int policy_backward_launch(const char* who, WabVec* h, const uint8_t* d_features, int64_t n_steps, int64_t n_envs,
@@ -2122,8 +2131,8 @@ static int policy_backward_launch(const char* who, WabVec* h, const uint8_t* d_f
     if (ppo) wab_policy_ppo_bwd_kernel<<<grid, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(h->P, (int)h->cfg.food_obs_scale + 1, B, *ppo);
     else wab_policy_bwd_kernel<<<grid, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(h->P, (int)h->cfg.food_obs_scale + 1, B);
     WAB_CUDA(cudaGetLastError());
-    const int64_t total = 128LL * dim + 128 + 150 * 128 + 150 + 128 * 150 + 128 + (int64_t)(n_actions + 1) * 129;
-    wab_policy_bwd_reduce_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+    const int64_t total = policy_n_params(dim, n_actions);
+    wab_policy_bwd_reduce_kernel<float><<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const float*>(d_scratch), grid, dim, n_actions, d_grad);
     WAB_CUDA(cudaGetLastError());
     return WAB_OK;
@@ -2165,6 +2174,35 @@ int wab_policy_ppo_backward(WabVec* h, const uint8_t* d_features, int64_t n_step
                                   nullptr, &Q, d_rows, d_n_rows, d_packed1, d_bias1, d_packed2, d_bias2, hidden2, d_packed3,
                                   d_bias3, d_packed2t, d_packed3t, d_w_heads, d_b_heads, n_actions, noise_scale, leaky_slope,
                                   clamp_lo, clamp_hi, d_scratch, scratch_bytes, d_grad, d_logp, d_value, stream);
+}
+
+int wab_policy_backward_grad_f64(WabVec* h, const void* d_scratch, int64_t scratch_bytes, int32_t n_actions, double* d_grad64,
+                                 void* stream) {
+    if (!h || !d_scratch || !d_grad64) return fail(WAB_E_NULL, "null argument");
+    if (n_actions < 1 || n_actions > 8) return fail(WAB_E_UNSUPPORTED, "wab_policy_backward_grad_f64: at most 8 actions");
+    const int dim = wab_vec_flat_dim(h);
+    if (dim > TC_CHUNKS * TC_KC) return fail(WAB_E_UNSUPPORTED, "wab_policy_backward_grad_f64: the input is at most 512 columns wide");
+    if (((uintptr_t)d_scratch & 15u) != 0 || ((uintptr_t)d_grad64 & 7u) != 0)
+        return fail(WAB_E_CONFIG, "d_scratch must be 16-byte aligned, d_grad64 8-byte");
+    if (scratch_bytes < wab_policy_backward_scratch_bytes(h)) return fail(WAB_E_CONFIG, "d_scratch is smaller than wab_policy_backward_scratch_bytes");
+    DeviceGuard guard(h->device);
+    const int64_t total = policy_n_params(dim, n_actions);
+    wab_policy_bwd_reduce_kernel<double><<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        reinterpret_cast<const float*>(d_scratch), backward_grid(h->device), dim, n_actions, d_grad64);
+    WAB_CUDA(cudaGetLastError());
+    return WAB_OK;
+}
+
+int wab_policy_grad_sum_ranks(const double* d_rank_grads, int32_t n_ranks, int64_t n, float* d_grad, void* stream) {
+    if (!d_rank_grads || !d_grad) return fail(WAB_E_NULL, "null argument");
+    if (n_ranks < 1) return fail(WAB_E_CONFIG, "wab_policy_grad_sum_ranks: n_ranks must be >= 1");
+    if (n < 0) return fail(WAB_E_CONFIG, "wab_policy_grad_sum_ranks: n must be >= 0");
+    if (((uintptr_t)d_rank_grads & 7u) != 0 || ((uintptr_t)d_grad & 3u) != 0)
+        return fail(WAB_E_CONFIG, "d_rank_grads must be 8-byte aligned, d_grad 4-byte");
+    if (n == 0) return WAB_OK;
+    wab_policy_grad_sum_ranks_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(d_rank_grads, n_ranks, n, d_grad);
+    WAB_CUDA(cudaGetLastError());
+    return WAB_OK;
 }
 
 int wab_sample_categorical(const void* d_probs, int32_t probs_bf16, int64_t n, int32_t n_actions, uint64_t seed,

@@ -111,8 +111,10 @@ wab_policy_ppo_bwd_kernel(const __grid_constant__ Params P, int food_dim, const 
 }
 
 // the per-CTA partial sums -> the flat gradient in parameters_to_vector(Policy.parameters()) order, summed over the CTAs
-// in index order in fp64
-__global__ void wab_policy_bwd_reduce_kernel(const float* __restrict__ scratch, int n_blocks, int dim, int n_actions, float* __restrict__ grad) {
+// in index order in fp64. G = float rounds once (wab_policy_backward); G = double keeps the fp64 sum
+// (wab_policy_backward_grad_f64, for a cross-rank sum that rounds once at its end)
+template <typename G>
+__global__ void wab_policy_bwd_reduce_kernel(const float* __restrict__ scratch, int n_blocks, int dim, int n_actions, G* __restrict__ grad) {
     const int64_t n1 = 128LL * dim, o_b1 = n1, o_w2 = o_b1 + 128, o_b2 = o_w2 + 150 * 128, o_w3 = o_b2 + 150, o_b3 = o_w3 + 128 * 150,
                   o_wa = o_b3 + 128, o_ba = o_wa + (int64_t)n_actions * 128, o_wv = o_ba + n_actions, o_bv = o_wv + 128, total = o_bv + 1;
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -133,7 +135,16 @@ __global__ void wab_policy_bwd_reduce_kernel(const float* __restrict__ scratch, 
     else off = BP_BH + n_actions;
     double s = 0.0;
     for (int b = 0; b < n_blocks; ++b) s += (double)scratch[(size_t)b * BP_BLOCK + off];
-    grad[e] = (float)s;
+    grad[e] = (G)s;
+}
+
+// d_grad[i] = fp32(sum over r = 0 .. n_ranks - 1 of d_rank_grads[r][i]), the sum in fp64 in rank order
+__global__ void wab_policy_grad_sum_ranks_kernel(const double* __restrict__ rank_grads, int n_ranks, int64_t n, float* __restrict__ grad) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    double s = 0.0;
+    for (int r = 0; r < n_ranks; ++r) s += rank_grads[(size_t)r * n + i];
+    grad[i] = (float)s;
 }
 
 }  // namespace

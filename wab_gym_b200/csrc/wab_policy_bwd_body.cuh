@@ -204,7 +204,7 @@
         const bool valid = flat >= 0 && flat < B.n_rows;                    // a listed row outside [0, T N) contributes nothing
         if (!valid) flat = 0;
         const int64_t step = flat / B.n_envs;
-        const uint32_t krow = (uint32_t)(flat - step * B.n_envs);           // the noise key: the row within its step
+        const uint32_t krow = (uint32_t)(P.env_id_base + (uint64_t)(flat - step * B.n_envs));   // the noise key: the global env id
         const unsigned long long ctr = B.counters[step];
         // ---- the tile's one-hot bit vectors (as wab_affine1_tc_kernel)
         if (tid >= 128) {

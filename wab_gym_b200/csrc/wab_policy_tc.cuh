@@ -241,11 +241,12 @@ wab_affine1_tc_kernel(const __grid_constant__ Params P, const uint8_t* __restric
         // as wab_flatten_noisy_kernel computes it; parts o (one-hot), n0, n1 (the noise x - o in two bf16 terms)
         float x[4][8];
         const int jb = 16 * (c & 1) + 8 * h;              // this thread's lanes j = jb .. jb + 7 of the chunk's Philox calls
+        const uint64_t g = P.env_id_base + (uint64_t)row; // the noise key: the row's global env id
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
             uint32_t w[4] = {0u, 0u, 0u, 0u};
             if (noisy)
-                philox(P, (uint32_t)row, (uint32_t)(row >> 32) ^ ((uint32_t)(c >> 1) << 24) ^ ((uint32_t)(jb + e) << 16), (uint32_t)ctr,
+                philox(P, (uint32_t)g, (uint32_t)(g >> 32) ^ ((uint32_t)(c >> 1) << 24) ^ ((uint32_t)(jb + e) << 16), (uint32_t)ctr,
                        (uint32_t)(ctr >> 32) ^ 0x464C4154u, w);
 #pragma unroll
             for (int s = 0; s < 4; ++s) x[s][e] = scale * (float)(w[s] >> 8);
@@ -476,7 +477,8 @@ wab_affine1_tc_kernel(const __grid_constant__ Params P, const uint8_t* __restric
                 float ex[8], tot = 0.f;
 #pragma unroll
                 for (int o = 0; o < 8; ++o) { ex[o] = o < A ? expf(acc[o] - mx) : 0.f; tot += ex[o]; }   // F.softmax, :96
-                uint32_t c0 = (uint32_t)(row >> 2), c1 = (uint32_t)(row >> 34), c2 = (uint32_t)ctr, c3 = (uint32_t)(ctr >> 32) ^ 0x53414D50u;
+                const uint64_t g = P.env_id_base + (uint64_t)row;        // the sampling key: the row's global env id
+                uint32_t c0 = (uint32_t)(g >> 2), c1 = (uint32_t)(g >> 34), c2 = (uint32_t)ctr, c3 = (uint32_t)(ctr >> 32) ^ 0x53414D50u;
 #pragma unroll
                 for (int rd = 0; rd < 10; ++rd) {                         // Philox4x32-10 under the sampling seed's round keys
                     const uint64_t p0 = (uint64_t)PHILOX_M0 * c0, p1 = (uint64_t)PHILOX_M1 * c2;
@@ -484,7 +486,7 @@ wab_affine1_tc_kernel(const __grid_constant__ Params P, const uint8_t* __restric
                     c1 = (uint32_t)p1; c3 = (uint32_t)p0; c0 = n0; c2 = n2;
                 }
                 const uint32_t wd[4] = {c0, c1, c2, c3};
-                const float u = (float)(pick4(wd, (uint32_t)row & 3u) >> 8) * (1.0f / 16777216.0f);
+                const float u = (float)(pick4(wd, (uint32_t)g & 3u) >> 8) * (1.0f / 16777216.0f);
                 const float target = u * tot;
                 float cum = 0.f, p_pick = 0.f;
                 int pick = A - 1;

@@ -252,6 +252,30 @@ class PolicyTrainTC(PolicyTrunkTC):
             self._stream()))
         return out
 
+    def grad_f64(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The gradient of the last ``backward`` / ``ppo_backward`` on this stream as f64[n_params]: the same fixed-order
+        fp64 sum over the CTAs, not rounded (``wab_policy_backward_grad_f64``). For a cross-rank sum that rounds once."""
+        if out is None:
+            out = torch.empty(self.n_params, dtype=torch.float64, device=self.env.device)
+        if out.dtype != torch.float64 or out.numel() != self.n_params or not out.is_contiguous():
+            raise ValueError("out must be a contiguous float64 tensor of n_params elements")
+        _lib.check(self.lib.wab_policy_backward_grad_f64(self.env._h, _ptr(self.scratch), self.scratch.numel(),
+                                                         self.heads[0].shape[0] - 1, _ptr(out), self._stream()))
+        return out
+
+    def grad_sum_ranks(self, rank_grads: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """fp32 of the fp64 sum over ranks, in rank order, of ``rank_grads`` f64[W, n_params] (``wab_policy_grad_sum_ranks``)."""
+        if rank_grads.dtype != torch.float64 or rank_grads.dim() != 2 or rank_grads.shape[1] != self.n_params or \
+                not rank_grads.is_contiguous():
+            raise ValueError("rank_grads must be a contiguous float64 [W, n_params] tensor")
+        if out is None:
+            out = torch.empty(self.n_params, dtype=torch.float32, device=self.env.device)
+        if out.dtype != torch.float32 or out.numel() != self.n_params or not out.is_contiguous():
+            raise ValueError("out must be a contiguous float32 tensor of n_params elements")
+        _lib.check(self.lib.wab_policy_grad_sum_ranks(_ptr(rank_grads), rank_grads.shape[0], self.n_params, _ptr(out),
+                                                      self._stream()))
+        return out
+
 
 class Rollout:
     """N-environment rollout with every tensor resident on the device.

@@ -20,6 +20,7 @@ from typing import Dict, Tuple
 
 import torch
 
+from . import sharding
 from .a2c import A2CTrainer
 from .policy import Policy
 from .vec_env import VecEnv
@@ -62,6 +63,12 @@ def ppo_loss(logp_new: torch.Tensor, value_new: torch.Tensor, entropy: torch.Ten
     return loss, info
 
 
+def _perm_seed(sample_seed: int, iteration: int, epoch: int, env_id_base=None) -> int:
+    """The seed of an epoch's minibatch permutation. A rank of a data-parallel run (``env_id_base`` given) folds its
+    first env id in, so that ranks shuffle differently; a single process keeps ``_seed(sample_seed, iteration, epoch)``."""
+    return _seed(sample_seed, iteration, epoch) if env_id_base is None else _seed(sample_seed, iteration, epoch, env_id_base)
+
+
 def _seed(*xs: int) -> int:
     """A 63-bit generator seed from integers (splitmix64 folded over them)."""
     h = 0x9E3779B97F4A7C15
@@ -80,22 +87,34 @@ class PPOTrainer(A2CTrainer):
     of the last observation as bootstrap, normalise the advantages over the batch, then ``epochs`` passes over a fresh
     permutation of the T N rows (``torch.Generator`` seeded by (sampling seed, iteration, epoch)), cut into
     ``minibatches`` contiguous slices. Each slice is one ``wab_policy_ppo_backward`` with the weights divided by its row
-    count (the minibatch mean of ``ppo_loss``), a global-norm clip to ``max_grad_norm`` and an Adam step."""
+    count (the minibatch mean of ``ppo_loss``), a global-norm clip to ``max_grad_norm`` and an Adam step.
+
+    With ``group`` (see ``a2c``'s module docstring) each rank runs GAE on its own envs, normalises the advantages by the
+    mean and unbiased std of the whole batch, and permutes its own rows with ``env_id_base`` folded into the seed; every
+    rank cuts its permutation into ``minibatches`` slices, and minibatch k's weights are divided by its row count summed
+    over the ranks. After each ``wab_policy_ppo_backward`` the gradient is summed over the ranks (fp64, rank order, one
+    rounding) before the clip and Adam, so the weights stay bit-identical on every rank. The returned diagnostics are
+    this rank's rows, except ``grad_norm``, which is the global gradient's."""
 
     def __init__(self, env: VecEnv, policy: Policy = None, horizon: int = 64, epochs: int = 4, minibatches: int = 4,
                  gamma: float = 0.99, lam: float = 0.95, clip_eps: float = 0.2, vf_coef: float = 0.5, ent_coef: float = 0.01,
-                 lr: float = 3e-4, max_grad_norm: float = 0.5, noise: bool = True):
+                 lr: float = 3e-4, max_grad_norm: float = 0.5, noise: bool = True, group=None):
         if epochs < 1 or minibatches < 1 or int(horizon) * env.num_envs < minibatches:
             raise ValueError("PPOTrainer needs epochs >= 1 and 1 <= minibatches <= horizon * num_envs")
         if not clip_eps > 0 or not max_grad_norm > 0:
             raise ValueError("clip_eps and max_grad_norm must be > 0")
-        super().__init__(env, policy, horizon=horizon, gamma=gamma, lr=lr, noise=noise, mode="horizon", tensor_cores=True)
         self.epochs, self.minibatches, self.lam = int(epochs), int(minibatches), float(lam)
         self.clip_eps, self.vf_coef, self.ent_coef, self.max_grad_norm = float(clip_eps), float(vf_coef), float(ent_coef), float(max_grad_norm)
+        super().__init__(env, policy, horizon=horizon, gamma=gamma, lr=lr, noise=noise, mode="horizon", tensor_cores=True,
+                         group=group)
         self.iteration = 0
         T, N, dev = self.horizon, env.num_envs, env.device
         rows = T * N
-        self._bounds = [k * rows // self.minibatches for k in range(self.minibatches + 1)]
+        self._bounds = sharding.minibatch_bounds(rows, self.minibatches)
+        # the row count each minibatch's weights are divided by: this rank's, or the sum over the ranks (known from
+        # construction, so no synchronisation)
+        self._global_counts = ([self._bounds[k + 1] - self._bounds[k] for k in range(self.minibatches)] if self.group is None
+                               else sharding.global_minibatch_counts([T * c for c in self._shard_counts], self.minibatches))
         self._counts = torch.tensor([self._bounds[k + 1] - self._bounds[k] for k in range(self.minibatches)], dtype=torch.int64, device=dev)
         self._new = {k: torch.empty(T, N, device=dev) for k in ("logp", "value", "entropy")}   # the kernel's per-row outputs
         self._perm = torch.empty(rows, dtype=torch.int32, device=dev)                          # this epoch's row order
@@ -107,6 +126,10 @@ class PPOTrainer(A2CTrainer):
             prm.grad = self._grad[off:off + prm.numel()].view_as(prm)
             off += prm.numel()
 
+    def _signature(self) -> tuple:
+        return super()._signature() + (self.epochs, self.minibatches, self.lam, self.clip_eps, self.vf_coef, self.ent_coef,
+                                       self.max_grad_norm)
+
     def train_iteration(self) -> Dict[str, torch.Tensor]:
         """One PPO iteration. Returns device tensors: per minibatch (in order, ``epochs * minibatches`` entries) the
         ``ppo_loss`` diagnostics of its rows from the kernel's outputs and the gradient norm before clipping; the mean
@@ -117,23 +140,29 @@ class PPOTrainer(A2CTrainer):
         self._sample_tc(env.last_features, self._boot_actions, b["bootstrap"])
         adv, ret = gae(b["reward"], b["done"], b["value"], b["bootstrap"], self.gamma, self.lam)
         b["target"].copy_(ret)
-        torch.sub(adv, adv.mean(), out=b["advantage"])                       # normalised once over the whole batch
-        b["advantage"].div_(adv.std() + 1e-8)
+        if self.group is None:
+            mean, std = adv.mean(), adv.std()
+        else:
+            mean, std = sharding.global_mean_std(adv, self.group)
+        torch.sub(adv, mean, out=b["advantage"])                             # normalised once over the whole batch
+        b["advantage"].div_(std + 1e-8)
         del adv, ret
         flat = {k: b[k].view(-1) for k in ("logp", "advantage", "target")}
         new = {k: v.view(-1) for k, v in self._new.items()}
         stats = []
         for epoch in range(self.epochs):
             gen = torch.Generator(device=env.device)
-            gen.manual_seed(_seed(self.sample_seed, self.iteration, epoch))
+            gen.manual_seed(_perm_seed(self.sample_seed, self.iteration, epoch, None if self.group is None else env.env_id_base))
             torch.randperm(self._perm.numel(), generator=gen, out=self._perm)
             for k in range(self.minibatches):
                 rows = self._perm[self._bounds[k]:self._bounds[k + 1]]
-                m = float(rows.numel())
+                m = float(self._global_counts[k])
                 self._tc.ppo_backward(b["features"], b["counters"], b["actions"], b["logp"], b["advantage"], b["target"], rows,
                                       self._counts[k:k + 1], self.clip_eps, 1.0 / m, self.vf_coef / m, self.ent_coef / m,
                                       out=self._grad, logp=self._new["logp"], value=self._new["value"],
                                       entropy=self._new["entropy"], noise_scale=noise)
+                if self.group is not None:
+                    self._sum_grad_over_ranks()
                 norm = torch.linalg.vector_norm(self._grad)
                 self._grad.mul_(torch.clamp(self.max_grad_norm / (norm + 1e-6), max=1.0))
                 self.optimizer.step()

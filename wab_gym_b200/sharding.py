@@ -72,6 +72,94 @@ def select_shard_records(sd: dict, env_id_base: int, num_envs: int, fingerprint:
     return records[sel][torch.argsort(local)]
 
 
+def merge_trainer_state_dicts(sds) -> dict:
+    """One trainer state dict (``A2CTrainer`` / ``PPOTrainer.state_dict``) from those of the ranks of a data-parallel run:
+    the env parts merged with ``merge_state_dicts``, the shared parts (policy, Adam state, noise counter, sampling seed,
+    iteration) taken once. Raises ``ValueError`` unless the shared parts are bit-equal on every rank."""
+    sds = list(sds)
+    if not sds:
+        raise ValueError("nothing to merge")
+    head = sds[0]
+    for i, sd in enumerate(sds[1:], 1):
+        if set(sd) != set(head):
+            raise ValueError("trainer state dict %d has other keys than the first" % i)
+        for key in head:
+            if key != "env" and not _bit_equal(sd[key], head[key]):
+                raise ValueError("trainer state dict %d differs from the first in %r: not one data-parallel run" % (i, key))
+    out = {k: v for k, v in head.items() if k != "env"}
+    out["env"] = merge_state_dicts([sd["env"] for sd in sds])
+    return out
+
+
+def _bit_equal(a, b) -> bool:
+    if isinstance(a, torch.Tensor) or isinstance(b, torch.Tensor):
+        return (isinstance(a, torch.Tensor) and isinstance(b, torch.Tensor) and a.dtype == b.dtype and a.shape == b.shape
+                and torch.equal(a.cpu().view(-1).view(torch.uint8), b.cpu().view(-1).view(torch.uint8)))
+    if isinstance(a, dict):
+        return isinstance(b, dict) and set(a) == set(b) and all(_bit_equal(a[k], b[k]) for k in a)
+    if isinstance(a, (list, tuple)):
+        return type(a) is type(b) and len(a) == len(b) and all(_bit_equal(x, y) for x, y in zip(a, b))
+    return type(a) is type(b) and a == b
+
+
+# ---- data-parallel training: the host-side arithmetic of the trainers' `group` argument ---------------------------------
+
+def check_trainer_shards(infos) -> int:
+    """``infos``: per rank in rank order, ``(env_id_base, num_envs, signature)``. Returns the total env count; raises
+    ``ValueError`` unless the shards tile ``[0, total)`` contiguously in rank order and every signature (fingerprint,
+    horizon, hyper-parameters, ...) equals rank 0's."""
+    infos = list(infos)
+    nxt = 0
+    for r, (first, count, sig) in enumerate(infos):
+        if int(first) != nxt or int(count) < 1:
+            raise ValueError("rank %d holds envs [%d, %d), expected a non-empty shard starting at %d: the shards must tile "
+                             "[0, total) contiguously in rank order" % (r, int(first), int(first) + int(count), nxt))
+        nxt += int(count)
+        if sig != infos[0][2]:
+            raise ValueError("rank %d's trainer differs from rank 0's (%r vs %r)" % (r, sig, infos[0][2]))
+    return nxt
+
+
+def minibatch_bounds(rows: int, minibatches: int):
+    """Row offsets of the ``minibatches`` contiguous slices of a permutation of ``rows`` rows (``PPOTrainer``)."""
+    return [k * rows // minibatches for k in range(minibatches + 1)]
+
+
+def global_minibatch_counts(rows_per_rank, minibatches: int):
+    """Rows of minibatch k summed over the ranks: what each rank divides minibatch k's per-row weights by."""
+    out = [0] * minibatches
+    for rows in rows_per_rank:
+        b = minibatch_bounds(int(rows), minibatches)
+        for k in range(minibatches):
+            out[k] += b[k + 1] - b[k]
+    return out
+
+
+def rank_order_sum(t: torch.Tensor, group=None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """The sum of ``t`` over the ranks of ``group``, added in rank order: an all-gather, then the same additions on every
+    rank, so every rank gets the same bits whatever the collective's algorithm. ``out`` [world, *t.shape] is the
+    gather buffer (allocated when not given)."""
+    import torch.distributed as dist
+    world = dist.get_world_size(group)
+    if out is None:
+        out = torch.empty((world,) + tuple(t.shape), dtype=t.dtype, device=t.device)
+    dist.all_gather(list(out.unbind(0)), t.contiguous(), group=group)
+    s = out[0].clone()
+    for r in range(1, world):
+        s += out[r]
+    return s
+
+
+def global_mean_std(x: torch.Tensor, group=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Mean and unbiased standard deviation of ``x`` over every rank's elements (device scalars of x's dtype): fp64 sum
+    and count, then the fp64 sum of squared deviations from that mean, each summed over the ranks in rank order."""
+    x64 = x.detach().reshape(-1).double()
+    sc = rank_order_sum(torch.stack([x64.sum(), torch.full((), float(x64.numel()), dtype=torch.float64, device=x.device)]), group)
+    mean = sc[0] / sc[1]
+    ss = rank_order_sum(((x64 - mean) ** 2).sum().reshape(1), group)[0]
+    return mean.to(x.dtype), (ss / (sc[1] - 1.0)).sqrt().to(x.dtype)
+
+
 def _distributed(group=None) -> bool:
     import torch.distributed as dist
     return dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
