@@ -21,7 +21,6 @@ VARIANTS = {
     "mb5": ["-DWAB_MIN_BLOCKS_LPE1=5"],
     "mb8": ["-DWAB_MIN_BLOCKS_LPE1=8"],
     "mb7": ["-DWAB_MIN_BLOCKS_LPE1=7"],
-    "eat_rare": ["-DWAB_EAT_RARE"],
     "cta64": ["-DWAB_THREADS_LPE1=64"],
     "cta32": ["-DWAB_THREADS_LPE1=32"],
     "cta256": ["-DWAB_THREADS_LPE1=256"],
@@ -40,11 +39,6 @@ VARIANTS = {
     "s2s2mb5": ["-DWAB_SLIDE_UNROLL=2", "-DWAB_SPAWN_UNROLL=2", "-DWAB_MIN_BLOCKS_LPE1=5"],
     "s3s3mb5": ["-DWAB_SLIDE_UNROLL=3", "-DWAB_SPAWN_UNROLL=3", "-DWAB_MIN_BLOCKS_LPE1=5"],
     "s6s6mb4": ["-DWAB_SLIDE_UNROLL=6", "-DWAB_SPAWN_UNROLL=6", "-DWAB_MIN_BLOCKS_LPE1=4"],
-    "x_nospawn": ["-DWAB_EXP_NOSPAWN"],
-    "x_noslide": ["-DWAB_EXP_NOSLIDE"],
-    "x_nostore": ["-DWAB_EXP_NOSTORE"],
-    "x_noemit": ["-DWAB_EXP_NOEMIT"],
-    "x_nothing": ["-DWAB_EXP_NOSPAWN", "-DWAB_EXP_NOSLIDE", "-DWAB_EXP_NOEMIT"],
     "t32": ["-DWAB_THREADS_LPEN=32"],
     "t128": ["-DWAB_THREADS_LPEN=128"],
     "lpen5": ["-DWAB_MIN_BLOCKS_LPEN=5"],

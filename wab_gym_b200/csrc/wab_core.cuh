@@ -239,16 +239,6 @@ WAB_HD_RARE uint32_t bush_word_rare(uint32_t c0, uint32_t kb, uint32_t key, uint
 WAB_HD uint32_t bush_word(const Params& P, const Env& E, int32_t x, int32_t y) {
     return bush_word_rare(pack_xy(x >> 1, y >> 1) ^ E.bk_a, E.bk_b, P.rk2[0], bush_lane(x, y));
 }
-// The same draw with both calls unrolled in line, for the eat path: rare per env (5 % of steps) but taken by some
-// lane of a 32-env warp on 82 % of its steps, where the rolled out-of-line version costs three times the instructions.
-WAB_HD uint32_t bush_word_inline(const Params& P, const Env& E, int32_t x, int32_t y) {
-    const uint32_t c0 = pack_xy(x >> 1, y >> 1) ^ E.bk_a, lane = bush_lane(x, y);
-    uint32_t p[2], q[2];
-    philox2(P, c0, E.bk_b, p);
-    philox2(P, c0, ~E.bk_b, q);
-    const uint32_t sel = half_sel(lane & 1u);
-    return (half_of((lane & 2u) ? p[1] : p[0], sel) << 16) | half_of((lane & 2u) ? q[1] : q[0], sel);
-}
 WAB_HD uint32_t cell_sig(uint32_t cell) { return 1u << ((cell * 0x9E3779B1u) >> 27); }
 // log slot of a cell, or -1. The signature answers "never eaten here" without touching memory; the
 // search runs newest-first because repeated eats hit the most recent entry.
@@ -425,94 +415,6 @@ WAB_HD void slide_window(const Params& P, Env& E, const Slots& S, int32_t dx, in
     }
 }
 
-// ---- the same reveal as independent pieces (chunked kernel, wab_kernels.cu): the keys of the 12 cells a move reveals
-// depend on the position only, so the six block draws of a step can be made ahead of time by any lane.
-struct RevealGeo { bool along_y; int32_t fixed, vmax, vb0, top; uint32_t fb, sel0, sel1; };
-WAB_HD RevealGeo reveal_geo(int32_t x, int32_t y, int32_t dx, int32_t dy) {   // (x, y) = position AFTER the move
-    RevealGeo g;
-    g.along_y = (dx != 0);
-    g.fixed = g.along_y ? x + HALF * dx : y + HALF * dy;
-    g.vmax = (g.along_y ? y : x) + HALF;
-    g.vb0 = (g.vmax - 10) >> 1;
-    g.fb = (uint32_t)g.fixed & 1u;
-    g.top = g.vmax - 2 * g.vb0 + 1;
-    g.sel0 = half_sel(g.along_y ? g.fb : 0u); g.sel1 = half_sel(g.along_y ? g.fb : 1u);
-    return g;
-}
-// block b of the line: its two cells at bits top - 2b and top - 2b - 1 of the result; bit 31 = a half-word tie
-WAB_HD uint32_t reveal_block(const Params& P, const RevealGeo& g, uint32_t ka, uint32_t kb, int b) {
-    uint32_t p[2];
-    const uint32_t c0 = (g.along_y ? pack_xy(g.fixed >> 1, g.vb0 + b) : pack_xy(g.vb0 + b, g.fixed >> 1)) ^ ka;
-    philox2(P, c0, kb, p);
-    const uint32_t t_hi = P.thr_bush1 >> 16;
-    const uint32_t h0 = half_of((g.along_y || !g.fb) ? p[0] : p[1], g.sel0);
-    const uint32_t h1 = half_of((g.along_y || g.fb) ? p[1] : p[0], g.sel1);
-    const uint32_t bit = 1u << (g.top - 2 * b);
-    return (h0 > t_hi ? bit : 0u) | (h1 > t_hi ? (bit >> 1) : 0u) | ((h0 == t_hi || h1 == t_hi) ? 0x80000000u : 0u);
-}
-WAB_HD uint32_t reveal_block_exact(const Params& P, const RevealGeo& g, uint32_t ka, uint32_t kb, int b) {   // full 32-bit draws
-    const uint32_t c0 = (g.along_y ? pack_xy(g.fixed >> 1, g.vb0 + b) : pack_xy(g.vb0 + b, g.fixed >> 1)) ^ ka;
-    uint32_t acc = 0;
-    WAB_ROLLED
-    for (uint32_t e = 0; e < 2u; ++e) {
-        const uint32_t lane = g.along_y ? (g.fb | (e << 1)) : (e | (g.fb << 1));
-        if (bush_word_rare(c0, kb, P.rk2[0], lane) >= P.thr_bush1) acc |= 1u << (g.top - 2 * b - (int32_t)e);
-    }
-    return acc;
-}
-// slide_window with the six block words of this move already drawn: `pre` = their OR (bit 31 = tie somewhere)
-template <int LPE>
-WAB_HD void slide_window_pre(const Params& P, Env& E, const Slots& S, int32_t dx, int32_t dy, uint32_t pre, const Coop<LPE>& coop) {
-    if (dy > 0) {
-        E.m[0] &= ~ColMask<10, 0>::v; E.m[1] &= ~ColMask<10, 1>::v; E.m[2] &= ~ColMask<10, 2>::v; E.m[3] &= ~ColMask<10, 3>::v;
-    }
-    if (dy < 0) {
-        E.m[0] &= ~ColMask<0, 0>::v; E.m[1] &= ~ColMask<0, 1>::v; E.m[2] &= ~ColMask<0, 2>::v; E.m[3] &= ~ColMask<0, 3>::v;
-    }
-    const int32_t s = 11 * dx + dy;
-    shl128(E.m, (uint32_t)(s > 0 ? s : 0));
-    shr128(E.m, (uint32_t)(s < 0 ? -s : 0));
-    E.m[3] &= TOP_WORD_MASK;
-    uint32_t acc = 0;
-    if (P.n_bush_thr > 0) {
-        acc = pre;
-        if (acc >> 31) {            // a 2^-16 tie in one of the twelve half-words: settle the line on the full draws
-            const RevealGeo g = reveal_geo(E.x, E.y, dx, dy);
-            acc = 0;
-            WAB_ROLLED
-            for (int b = (int)coop.sub; b < 6; b += LPE) acc |= reveal_block_exact(P, g, E.bk_a, E.bk_b, b);
-            acc = group_or(coop, acc);
-        }
-        acc &= 0xFFEu;
-        if (E.dep) {                // something was eaten empty this episode: revealed cells consult the log
-            const bool along_y = dx != 0;
-            const int32_t fixed = along_y ? E.x + HALF * dx : E.y + HALF * dy, vmax = (along_y ? E.y : E.x) + HALF;
-            uint32_t bits = acc;
-            WAB_ROLLED
-            while (bits) {
-#if defined(__CUDA_ARCH__)
-                const int k = __ffs((int)bits) - 1;
-#else
-                const int k = __builtin_ctz(bits);
-#endif
-                bits &= bits - 1u;
-                const int32_t v = vmax - (k - 1);
-                if (!(along_y ? bush_alive(P, E, S, fixed, v) : bush_alive(P, E, S, v, fixed))) acc &= ~(1u << k);
-            }
-        }
-    }
-    const uint32_t line = acc >> 1;
-    if (dx != 0) {
-        E.m[0] |= (dx > 0) ? line : 0u;
-        E.m[3] |= (dx < 0) ? (line << 14) : 0u;
-    } else {
-        uint32_t t[4];
-        spread11(line, t);
-        shl128(t, dy < 0 ? 10u : 0u);
-        E.m[0] |= t[0]; E.m[1] |= t[1]; E.m[2] |= t[2]; E.m[3] |= t[3];
-    }
-}
-
 // ring cell j (oracle/keyed_rng.py ring_index) -> offset from the ostrich
 WAB_HD void ring_offset(int j, int32_t& dx, int32_t& dy) {
     int bx, by;
@@ -545,11 +447,8 @@ WAB_HD void wolf_plane(const Env& E, const Slots& S, uint32_t wm[4]) {
 
 // One step of one environment: wab_env.py:250-342 up to (not including) auto-reset and the
 // observation stores. `F64` selects the reference's fp64 food arithmetic.
-// PRE: the caller may hand in the step's bush draws (`pre_line`, see slide_window_pre) and its spawn draw made ahead of
-// time (`pre_ok` says whether they are valid for this env: they are not after a reset inside the chunk they were made for).
-template <bool F64, int LPE, bool PRE>
-WAB_HD void env_step_impl(const Params& P, Env& E, const Slots& S, uint32_t action, StepOut& O, const Coop<LPE>& coop,
-                          bool pre_ok, uint32_t pre_line, uint64_t pre_spawn) {
+template <bool F64, int LPE>
+WAB_HD void env_step(const Params& P, Env& E, const Slots& S, uint32_t action, StepOut& O, const Coop<LPE>& coop) {
     // ---- :251-258 action
     O.bad_action = (action >= (uint32_t)P.n_actions) ? 1u : 0u;
     const uint32_t code = O.bad_action ? 0x05u /* dx=0, dy=0, keep */ : (uint32_t)(P.act_tbl >> (8 * action)) & 0xFFu;
@@ -561,12 +460,7 @@ WAB_HD void env_step_impl(const Params& P, Env& E, const Slots& S, uint32_t acti
     O.overflow = 0;
 
     // ---- :259 generate_bushes for the newly visible line
-#ifndef WAB_EXP_NOSLIDE
-    if (dx != 0 || dy != 0) {
-        if (PRE && pre_ok) slide_window_pre<LPE>(P, E, S, dx, dy, pre_line, coop);
-        else slide_window<LPE>(P, E, S, dx, dy, coop);
-    }
-#endif
+    if (dx != 0 || dy != 0) slide_window<LPE>(P, E, S, dx, dy, coop);
 
     // ---- :262-264 despawn (keep iff U > chance). rank = ordinal among earlier wolves on the cell.
     if (E.nw) {
@@ -652,11 +546,7 @@ WAB_HD void env_step_impl(const Params& P, Env& E, const Slots& S, uint32_t acti
         } else {
             eats = 1u; O.overflow = 1u;            // counted, never silent (WAB_STAT_OVERFLOWS)
         }
-#ifdef WAB_EAT_FULLWORD   /* tuning A/B only: both Philox2x32 calls of the cell in line, then the full compare */
-        const uint32_t still = alive_after(P, bush_word_inline(P, E, E.x, E.y), eats);
-#else
         const uint32_t still = eaten_bush_alive(P, E, E.x, E.y, eats);
-#endif
         if (!still) { E.m[1] &= ~(1u << 28); E.dep = 1u; E.stale = 1u; }
     }
 
@@ -670,9 +560,8 @@ WAB_HD void env_step_impl(const Params& P, Env& E, const Slots& S, uint32_t acti
     }
 
     // ---- :325-326 spawn_wolves on the 48 ring cells around the moved ostrich: one binomial-first draw
-#ifndef WAB_EXP_NOSPAWN   /* tuning experiments only (tools/tune.py): results are WRONG with these defined */
     if (P.wolves) {
-        const uint64_t v = (PRE && pre_ok) ? pre_spawn : binomial_draw(P, E.env_id, E.episode, SITE_SPAWN, E.turn);
+        const uint64_t v = binomial_draw(P, E.env_id, E.episode, SITE_SPAWN, E.turn);
         if (v >= P.spawn_cdf[0]) {                 // rare (2.4 % of steps): at least one wolf appears
             uint32_t chosen[4];
             binomial_choose(P, E.env_id, E.episode, SITE_SPAWN, E.turn, RING, v, chosen);
@@ -699,7 +588,6 @@ WAB_HD void env_step_impl(const Params& P, Env& E, const Slots& S, uint32_t acti
             }
         }
     }
-#endif
     // ---- :328-340 reward, done
     uint32_t outcome;
     if (E.status == 0u) outcome = (E.turn >= (uint32_t)P.max_turns) ? 1u : 0u;
@@ -713,10 +601,6 @@ WAB_HD void env_step_impl(const Params& P, Env& E, const Slots& S, uint32_t acti
     O.food_obs = food_observation(P, E, F64);
     O.role = E.role;
     O.status = E.status;
-}
-template <bool F64, int LPE>
-WAB_HD void env_step(const Params& P, Env& E, const Slots& S, uint32_t action, StepOut& O, const Coop<LPE>& coop) {
-    env_step_impl<F64, LPE, false>(P, E, S, action, O, coop, false, 0u, 0ull);
 }
 
 // ------------------------------------------------------------------ reset pieces (wab_env.py:231-248)

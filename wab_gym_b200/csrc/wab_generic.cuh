@@ -146,7 +146,7 @@ __device__ __forceinline__ void gen_emit(const GenGeo& g, const GenSmem& sm, uin
         sm.stream[w] = v;
     }
     __syncwarp();
-    stream_flush<false, false>(sm.stream, nullptr, grids + (first_byte - off), off, off + 3 * g.WH, lane);
+    stream_flush<false>(sm.stream, nullptr, grids + (first_byte - off), off, off + 3 * g.WH, lane);
     __syncwarp();
 }
 

@@ -187,21 +187,7 @@ __device__ __forceinline__ void stream_put(uint32_t* stream, int bit0, bool last
     if (nown > 12) stream[fw + 12] = 0u;
 }
 
-// 256-bit global stores (st.global.v8.b32, new with sm_100: SASS STG.E.EF.ENL2.256): a lane turns 32 stream bits into 32
-// bytes and issues ONE store — half the store instructions, loop iterations and stream loads of the 16-byte version.
-// Measured SLOWER on B200 (same box, bench.py legs, profiles/r2p_ab_wide_stores.txt): 131,072 envs 1.116e10 -> 1.035e10
-// env-steps/s, 1M envs 1.200e10 -> 1.167e10, v2 config 3 3.21e8 -> 2.98e8 world turns/s, 4,096 envs 1.974e9 -> 1.924e9 —
-// so the default stays the 16-byte store (STG.E.EF.128); -DWAB_WIDE_STORES=1 builds this version (bit-identical outputs:
-// the whole GPU suite passes with it).
-#ifndef WAB_WIDE_STORES
-#define WAB_WIDE_STORES 0
-#endif
-constexpr bool kWideStores = WAB_WIDE_STORES != 0;
-constexpr int kObsAlign = kWideStores ? 32 : 16;     // the store grid the warp's bit stream is aligned to
-__device__ __forceinline__ void st_cs_256(void* p, uint2 a, uint2 b, uint2 c, uint2 d) {
-    asm volatile("st.global.cs.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "r"(a.x), "r"(a.y), "r"(b.x), "r"(b.y),
-                 "r"(c.x), "r"(c.y), "r"(d.x), "r"(d.y) : "memory");
-}
+constexpr int kObsAlign = 16;     // the store grid the warp's bit stream is aligned to
 // byte offset of an output address inside its store-grid cell (the address minus this is kObsAlign-aligned)
 __device__ __forceinline__ int obs_align_off(const uint8_t* p) { return (int)(reinterpret_cast<uintptr_t>(p) & (uintptr_t)(kObsAlign - 1)); }
 
@@ -209,49 +195,24 @@ __device__ __forceinline__ int obs_align_off(const uint8_t* p) { return (int)(re
 // `lut` = 256 x uint2 in shared memory: byte value -> its 8 bits as 8 bytes (built once per CTA).
 // USE_LUT = false expands with two multiplies per 8 bytes instead (the lanes-per-env kernels: few chunks per step, and no
 // table means no CTA barrier anywhere in a single-step launch).
-// `lane` / STRIDE: the flushing thread's index among STRIDE cooperating threads (a warp: 32; a whole CTA: its size).
-template <bool USE_LUT = true, bool WIDE = kWideStores, int STRIDE = 32>
+// `lane`: the flushing lane of the warp.
+template <bool USE_LUT = true>
 __device__ __forceinline__ void stream_flush(const uint32_t* stream, const uint2* lut, uint8_t* gA, int off, int end,
                                              int lane, bool lut_built = true) {
-    constexpr int SH = WIDE ? 5 : 4, CH = 1 << SH;               // chunk = one store of CH bytes
+    constexpr int SH = 4, CH = 1 << SH;                          // chunk = one 16-byte store
     const int c_lo = (off + CH - 1) >> SH, c_hi = end >> SH;     // chunks entirely inside [off, end)
-    if (WIDE) {
+    const uint16_t* hs = reinterpret_cast<const uint16_t*>(stream);
 #pragma unroll kFlushUnroll
-        for (int c = c_lo + lane; c < c_hi; c += STRIDE) {
-            const uint32_t w = stream[c];
-            uint2 q0, q1, q2, q3;
-            if (USE_LUT && lut_built) {
-                q0 = lut[w & 0xFFu]; q1 = lut[(w >> 8) & 0xFFu]; q2 = lut[(w >> 16) & 0xFFu]; q3 = lut[w >> 24];
-            } else {
-                q0 = make_uint2(nibble_to_bytes(w & 15u), nibble_to_bytes((w >> 4) & 15u));
-                q1 = make_uint2(nibble_to_bytes((w >> 8) & 15u), nibble_to_bytes((w >> 12) & 15u));
-                q2 = make_uint2(nibble_to_bytes((w >> 16) & 15u), nibble_to_bytes((w >> 20) & 15u));
-                q3 = make_uint2(nibble_to_bytes((w >> 24) & 15u), nibble_to_bytes(w >> 28));
-            }
-#ifndef WAB_EXP_NOSTORE
-            st_cs_256(gA + 32 * c, q0, q1, q2, q3);
-#else
-            if (q0.x == 0xdeadbeefu) gA[0] = (uint8_t)q3.y;
-#endif
+    for (int c = c_lo + lane; c < c_hi; c += 32) {
+        const uint32_t h = hs[c];
+        uint2 lo, hi;
+        if (USE_LUT && lut_built) {
+            lo = lut[h & 0xFFu]; hi = lut[h >> 8];
+        } else {
+            lo = make_uint2(nibble_to_bytes(h & 15u), nibble_to_bytes((h >> 4) & 15u));
+            hi = make_uint2(nibble_to_bytes((h >> 8) & 15u), nibble_to_bytes(h >> 12));
         }
-    } else {
-        const uint16_t* hs = reinterpret_cast<const uint16_t*>(stream);
-#pragma unroll kFlushUnroll
-        for (int c = c_lo + lane; c < c_hi; c += STRIDE) {
-            const uint32_t h = hs[c];
-            uint2 lo, hi;
-            if (USE_LUT && lut_built) {
-                lo = lut[h & 0xFFu]; hi = lut[h >> 8];
-            } else {
-                lo = make_uint2(nibble_to_bytes(h & 15u), nibble_to_bytes((h >> 4) & 15u));
-                hi = make_uint2(nibble_to_bytes((h >> 8) & 15u), nibble_to_bytes(h >> 12));
-            }
-#ifndef WAB_EXP_NOSTORE
-            __stcs(reinterpret_cast<uint4*>(gA) + c, make_uint4(lo.x, lo.y, hi.x, hi.y));
-#else
-            if (lo.x == 0xdeadbeefu) gA[0] = (uint8_t)hi.y;
-#endif
-        }
+        __stcs(reinterpret_cast<uint4*>(gA) + c, make_uint4(lo.x, lo.y, hi.x, hi.y));
     }
     if (lane < CH) {                                              // ragged head and tail, one byte per lane
         const int head_end = min(c_lo << SH, end);
@@ -439,9 +400,7 @@ wab_step_kernel(const __grid_constant__ Params P, const StatePtrs st, const uint
             write_scalars(out, o, O);
             if (out.features) write_features(out.features, o, O);
         }
-#ifndef WAB_EXP_NOEMIT
         if (out.grids) emit_obs<LPE>(stream, lut, c, out.grids, first_byte, O.wm, O.bm, lut_built);   // null: features-only stepping
-#endif
     }
     if (c.writer) store_env<F64>(st, c.idx, E, wolves_s, EPB);
     uint32_t cnt[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
@@ -454,258 +413,6 @@ wab_step_kernel(const __grid_constant__ Params P, const StatePtrs st, const uint
         cnt[WAB_STAT_EATS] = (uint32_t)acc_misc & 0xFFFFu;
         cnt[WAB_STAT_BAD_ACTIONS] = (uint32_t)(acc_misc >> 16) & 0xFFFFu;
         cnt[WAB_STAT_OVERFLOWS] = (uint32_t)(acc_misc >> 32) & 0xFFFFu;
-    }
-    flush_stats(st.wstats, cnt);
-}
-
-// ---- the multi-step kernel of the lanes-per-env geometries, chunked over time -------------------------------------
-// A group of LPE lanes owns one env. Run step by step (wab_step_kernel above), a small batch is bound by the length
-// of one step's dependent instruction chain: ~770 instructions per warp-step at < 2 warps per scheduler. But only a
-// small part of a step depends on the previous one. For a chunk of LPE consecutive steps:
-//   phase 1 (parallel over the lanes of a group, one step each): the actions of the chunk are known, so the ostrich's
-//     path is a prefix sum; the cells each move reveals are keyed by position only and the spawn draw by (episode, turn)
-//     only — the 6 x LPE bush-block draws of the chunk are spread over the group's lanes and every lane makes the spawn
-//     draw of "its" step. All of it assumes that the episode does not end inside the chunk.
-//   phase 2 (sequential, the group's lanes in lock step): the rules of wab_core.cuh with the draws handed in; after an
-//     episode end the rest of the chunk falls back to drawing in place (pre_ok = false). Each step's planes and
-//     scalars are parked in shared memory.
-//   phase 3 (parallel again): lane (env, s) puts step s of its env into the bit stream of that step and writes its
-//     scalars; the warp then flushes the LPE streams.
-// Results are identical to wab_step_kernel's (same functions, same draws); WAB_CHUNK=0 selects the step-by-step kernel.
-template <int LPE> struct ChunkGeo {
-    static constexpr int EPW = 32 / LPE;
-    static constexpr int SW = WarpStream<EPW>::WORDS;      // stream words of one step of the warp's envs
-    static constexpr int RES = 12;                         // words parked per (env, step)
-    static constexpr int WARP_WORDS = LPE * SW + 32 * RES + 3 * 32;   // streams, results, line / position / move per (env, step)
-};
-
-template <bool F64, int LPE>
-__global__ void __launch_bounds__(Geo<LPE>::THREADS, 1)
-wab_step_chunk_kernel(const __grid_constant__ Params P, const StatePtrs st, const uint8_t* __restrict__ actions,
-                      const int n_steps, const OutPtrs out) {
-    extern __shared__ uint32_t smem[];
-    constexpr int EPB = Geo<LPE>::EPB, EPW = Geo<LPE>::EPW, SW = ChunkGeo<LPE>::SW, RES = ChunkGeo<LPE>::RES;
-    const int64_t n = st.n;
-    const Ctx c = make_ctx<LPE>(n);
-    uint32_t* wolves_s = smem + c.env_local;                                   // [wolf_cap][EPB]
-    uint32_t* wbase = smem + P.wolf_cap * EPB + (threadIdx.x >> 5) * ChunkGeo<LPE>::WARP_WORDS;
-    uint32_t* streams = wbase;                         // [LPE][SW]
-    uint32_t* res = streams + LPE * SW;                // [EPW][LPE][RES]
-    uint32_t* lines = res + 32 * RES;                  // [EPW][LPE]  OR of the step's six reveal_block words
-    uint32_t* spos = lines + 32;                       // [EPW][LPE]  position after the step, if no episode ends before it
-    uint32_t* smove = spos + 32;                       // [EPW][LPE]  the step's move code
-    pdl_launch_dependents();
-    pdl_wait();
-    Coop<LPE> coop;
-    coop.sub = (uint32_t)c.sub;
-    coop.gmask = LPE == 32 ? FULL : (((1u << (LPE & 31)) - 1u) << (c.lane - c.sub));
-    const int gfirst = c.lane - c.sub, me = c.slot * LPE + c.sub;
-    Env E;
-    Slots S;
-    S.wolves = wolves_s; S.wstride = EPB;
-    S.logcell = st.logcell + (c.active ? c.idx : 0); S.logcnt = st.logcnt + (c.active ? c.idx : 0); S.lstride = n;
-    if (c.active) load_env<F64>(P, st, c.idx, E, wolves_s, EPB);
-    else { E = Env(); }
-    unsigned long long acc_outcome = 0ull, acc_misc = 0ull;
-    for (int t0 = 0; t0 < n_steps; t0 += LPE) {
-        const int Sn = min(LPE, n_steps - t0);
-        // ---------------- phase 1: lane `sub` prepares step t0 + sub of its env
-        uint32_t a_mine = 0xFFu;
-        if (c.active && c.sub < Sn) a_mine = actions[(int64_t)(t0 + c.sub) * n + c.idx];
-        const uint32_t code = a_mine >= (uint32_t)P.n_actions ? 0x05u : (uint32_t)(P.act_tbl >> (8 * a_mine)) & 0xFFu;
-        int32_t px = (int32_t)(code & 3u) - 1, py = (int32_t)((code >> 2) & 3u) - 1;
-#pragma unroll
-        for (int d = 1; d < LPE; d <<= 1) {             // inclusive prefix sum of the moves over the group
-            const int32_t ux = __shfl_up_sync(FULL, px, d, LPE), uy = __shfl_up_sync(FULL, py, d, LPE);
-            if (c.sub >= d) { px += ux; py += uy; }
-        }
-        lines[me] = 0u;
-        spos[me] = pack_xy(E.x + px, E.y + py);
-        smove[me] = code;
-        uint64_t v_mine = 0ull;
-        if (c.active && c.sub < Sn && P.wolves) v_mine = binomial_draw(P, E.env_id, E.episode, SITE_SPAWN, E.turn + (uint32_t)c.sub + 1u);
-        __syncwarp();
-        if (c.active && P.n_bush_thr > 0) {
-            for (int j = c.sub; j < 6 * Sn; j += LPE) {  // bush-block draw j = (step, block) of the chunk
-                const int sj = j / 6, b = j - 6 * sj, at = c.slot * LPE + sj;
-                const uint32_t mj = smove[at];
-                const int32_t jdx = (int32_t)(mj & 3u) - 1, jdy = (int32_t)((mj >> 2) & 3u) - 1;
-                if (jdx != 0 || jdy != 0) {
-                    const uint32_t pj = spos[at];
-                    const RevealGeo g = reveal_geo(unpack_x(pj), unpack_y(pj), jdx, jdy);
-                    atomicOr(lines + at, reveal_block(P, g, E.bk_a, E.bk_b, b));
-                }
-            }
-        }
-        __syncwarp();
-        // ---------------- phase 2: the rules, step by step
-        bool spec_ok = true;
-        for (int s2 = 0; s2 < Sn; ++s2) {
-            StepOut O;
-            bool need_reset = false;
-            const uint32_t a = __shfl_sync(FULL, a_mine, gfirst + s2);
-            const uint64_t v = ((uint64_t)__shfl_sync(FULL, (uint32_t)(v_mine >> 32), gfirst + s2) << 32) |
-                               (uint64_t)__shfl_sync(FULL, (uint32_t)v_mine, gfirst + s2);
-            const uint32_t line = lines[c.slot * LPE + s2];
-            if (c.active) {
-                env_step_impl<F64, LPE, true>(P, E, S, a, O, coop, spec_ok, line, v);
-                if (st.hist && c.writer && E.turn < (uint32_t)st.hist_len) st.hist[(int64_t)E.turn * n + c.idx] = pack_xy(E.x, E.y);
-                need_reset = O.done && P.auto_reset;
-                acc_outcome += 1ull << (16u * O.outcome);
-                acc_misc += (unsigned long long)O.ate | ((unsigned long long)O.bad_action << 16);
-            } else {
-                O = StepOut();
-            }
-            if (__any_sync(FULL, need_reset)) {
-                warp_reset<F64, LPE>(P, E, S, need_reset, c.lane, O.wm, O.bm, O.overflow);
-                if (need_reset) {
-                    O.food_obs = food_observation(P, E, F64);
-                    O.role = E.role; O.status = E.status;
-                    spec_ok = false;               // the draws made ahead belonged to the episode that just ended
-                }
-            }
-            apply_view_mask(P, O.role, O.wm, O.bm);
-            if (c.writer) {
-                acc_misc += (unsigned long long)O.overflow << 32;
-                uint4* r = reinterpret_cast<uint4*>(res + (c.slot * LPE + s2) * RES);
-                r[0] = make_uint4(O.wm[0], O.wm[1], O.wm[2], O.wm[3]);
-                r[1] = make_uint4(O.bm[0], O.bm[1], O.bm[2], O.bm[3]);
-                r[2] = make_uint4(O.food_obs | (O.role << 8) | (O.status << 16) | (O.done << 24), O.info, __float_as_uint(O.reward), 0u);
-            }
-        }
-        __syncwarp();
-        // ---------------- phase 3: lane (env, s) publishes step t0 + s of its env
-        {
-            const int s3 = c.sub;
-            if (s3 < Sn) {
-                const int64_t fb3 = ((int64_t)(t0 + s3) * n + c.warp_first) * OBS_BYTES;
-                const int off3 = (int)(fb3 & 15);
-                const uint4* r = reinterpret_cast<const uint4*>(res + me * RES);
-                const uint4 w4 = r[0], b4 = r[1], sc = r[2];
-                const uint32_t wm[4] = {w4.x, w4.y, w4.z, w4.w}, bm[4] = {b4.x, b4.y, b4.z, b4.w};
-                if (out.grids) stream_put(streams + s3 * SW, off3 + OBS_BYTES * c.slot, c.slot == EPW - 1, off3 + EPW * OBS_BYTES, wm, bm, c.active);
-                if (c.active) {
-                    const int64_t o3 = (int64_t)(t0 + s3) * n + c.idx;
-                    out.food[o3] = (uint8_t)(sc.x & 0xFFu);
-                    out.role[o3] = (uint8_t)((sc.x >> 8) & 0xFFu);
-                    out.status[o3] = (uint8_t)((sc.x >> 16) & 0xFFu);
-                    if (out.reward) out.reward[o3] = __uint_as_float(sc.z);
-                    if (out.done) out.done[o3] = (uint8_t)(sc.x >> 24);
-                    if (out.info) out.info[o3] = (uint8_t)sc.y;
-                    if (out.features) {
-                        StepOut O3;
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) { O3.wm[k] = wm[k]; O3.bm[k] = bm[k]; }
-                        O3.food_obs = sc.x & 0xFFu; O3.role = (sc.x >> 8) & 0xFFu; O3.status = (sc.x >> 16) & 0xFFu;
-                        write_features(out.features, o3, O3);
-                    }
-                }
-            }
-            __syncwarp();
-#pragma unroll 1
-            for (int sf = 0; sf < (out.grids ? Sn : 0); ++sf) {
-                const int64_t fbs = ((int64_t)(t0 + sf) * n + c.warp_first) * OBS_BYTES;
-                const int offs = (int)(fbs & 15);
-                stream_flush<false, false>(streams + sf * SW, nullptr, out.grids + (fbs - offs), offs, offs + OBS_BYTES * c.n_valid, c.lane);
-            }
-            __syncwarp();
-        }
-    }
-    if (c.writer) store_env<F64>(st, c.idx, E, wolves_s, EPB);
-    uint32_t cnt[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
-    if (c.writer) {
-        const uint32_t fin = (uint32_t)(acc_outcome >> 16) & 0xFFFFu, sta = (uint32_t)(acc_outcome >> 32) & 0xFFFFu,
-                       kil = (uint32_t)(acc_outcome >> 48) & 0xFFFFu;
-        cnt[WAB_STAT_EPISODES] = fin + sta + kil;
-        cnt[WAB_STAT_STEPS] = (uint32_t)n_steps;
-        cnt[WAB_STAT_FINISHED] = fin; cnt[WAB_STAT_STARVED] = sta; cnt[WAB_STAT_KILLED] = kil;
-        cnt[WAB_STAT_EATS] = (uint32_t)acc_misc & 0xFFFFu;
-        cnt[WAB_STAT_BAD_ACTIONS] = (uint32_t)(acc_misc >> 16) & 0xFFFFu;
-        cnt[WAB_STAT_OVERFLOWS] = (uint32_t)(acc_misc >> 32) & 0xFFFFu;
-    }
-    flush_stats(st.wstats, cnt);
-}
-
-// ---- single-step kernel for the mapped host path: 8 lanes per env, 16 envs per CTA, CTA-wide emission ----------------
-// wab_vec_step_host_packed lets the kernel write the caller's pinned host block directly, so the step's compute time sits
-// in front of a PCIe-bound burst of stores. The thread-per-env kernel only issues whole 16-byte stores (its warps own
-// 16-byte-aligned slabs) but needs ~8 us for one step of a small batch; the lanes-per-env kernels need ~2.5 us, but
-// their warps own 4 x 363 bytes at arbitrary alignment and finish with up to 30 single-byte stores each — a separate PCIe
-// write per byte. Sixteen consecutive envs are 5,808 bytes = 363 x 16: a CTA of 128 threads (8 lanes per env) builds ONE
-// bit stream for its 16 envs and every store it issues is a full, aligned 16-byte one (a batch that is not a multiple of
-// 16 pays single bytes at its very end only). One CTA barrier per step — acceptable for a single-step launch.
-// Measured (profiles/r1f_e2e_paths.txt, round 2): bit-identical, but the host step does not wait for the compute —
-// 4,096 envs 50.0 -> 52.8 us, 16,384 envs 142 -> 158 us, only 1,024 envs gain (27.7 -> 26.8 us) — so it is opt-in
-// (WAB_HOST_MAPPED=3) and the thread-per-env kernel stays the default of the mapped path.
-constexpr int kCta16Envs = 16, kCta16Threads = 128;
-constexpr int kCta16Stream = (kCta16Envs * OBS_BYTES + 31 + 31) / 32 + 1;
-
-template <bool F64>
-__global__ void __launch_bounds__(kCta16Threads)
-wab_step_cta16_kernel(const __grid_constant__ Params P, const StatePtrs st, const uint8_t* __restrict__ actions, const OutPtrs out) {
-    extern __shared__ uint32_t smem[];
-    constexpr int LPE = 8, EPB = kCta16Envs;
-    const int64_t n = st.n;
-    Ctx c;
-    c.lane = threadIdx.x & 31; c.sub = c.lane % LPE; c.slot = c.lane / LPE;
-    c.env_local = threadIdx.x / LPE;
-    c.idx = (int64_t)blockIdx.x * EPB + c.env_local;
-    c.warp_first = c.idx - c.slot;
-    c.active = c.idx < n; c.writer = c.active && c.sub == 0;
-    c.n_valid = 0;
-    uint32_t* wolves_s = smem + c.env_local;                                  // [wolf_cap][EPB]
-    uint32_t* stream = smem + P.wolf_cap * EPB;                               // one bit stream for the CTA's 16 envs
-    pdl_launch_dependents();
-    pdl_wait();
-    Coop<LPE> coop;
-    coop.sub = (uint32_t)c.sub;
-    coop.gmask = ((1u << LPE) - 1u) << (c.lane - c.sub);
-    Env E;
-    Slots S;
-    S.wolves = wolves_s; S.wstride = EPB;
-    S.logcell = st.logcell + (c.active ? c.idx : 0); S.logcnt = st.logcnt + (c.active ? c.idx : 0); S.lstride = n;
-    if (c.active) load_env<F64>(P, st, c.idx, E, wolves_s, EPB);
-    else { E = Env(); }
-    StepOut O;
-    bool need_reset = false;
-    uint32_t cnt[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
-    if (c.active) {
-        env_step<F64, LPE>(P, E, S, (uint32_t)actions[c.idx], O, coop);
-        if (st.hist && c.writer && E.turn < (uint32_t)st.hist_len) st.hist[(int64_t)E.turn * n + c.idx] = pack_xy(E.x, E.y);
-        need_reset = O.done && P.auto_reset;
-    } else {
-        O = StepOut();
-    }
-    if (c.writer) {
-        cnt[WAB_STAT_STEPS] = 1u;
-        cnt[WAB_STAT_EPISODES] = O.outcome != 0u; cnt[WAB_STAT_FINISHED] = O.outcome == 1u;
-        cnt[WAB_STAT_STARVED] = O.outcome == 2u; cnt[WAB_STAT_KILLED] = O.outcome == 3u;
-        cnt[WAB_STAT_EATS] = O.ate; cnt[WAB_STAT_BAD_ACTIONS] = O.bad_action;
-    }
-    if (__any_sync(FULL, need_reset)) {
-        warp_reset<F64, LPE>(P, E, S, need_reset, c.lane, O.wm, O.bm, O.overflow);
-        if (need_reset) {
-            O.food_obs = food_observation(P, E, F64);
-            O.role = E.role; O.status = E.status;
-        }
-    }
-    apply_view_mask(P, O.role, O.wm, O.bm);
-    if (c.writer) {
-        cnt[WAB_STAT_OVERFLOWS] = O.overflow;
-        write_scalars(out, c.idx, O);
-        if (out.features) write_features(out.features, c.idx, O);
-        store_env<F64>(st, c.idx, E, wolves_s, EPB);
-    }
-    if (out.grids) {
-        const int64_t first_byte = (int64_t)blockIdx.x * EPB * OBS_BYTES;
-        const int off = obs_align_off(out.grids + first_byte);
-        const int64_t left = n - (int64_t)blockIdx.x * EPB;
-        const int n_valid = (int)(left < EPB ? left : EPB);
-        if (c.sub == 0)
-            stream_put(stream, off + OBS_BYTES * c.env_local, c.env_local == EPB - 1, off + EPB * OBS_BYTES, O.wm, O.bm, c.active);
-        __syncthreads();
-        stream_flush<false, kWideStores, kCta16Threads>(stream, nullptr, out.grids + (first_byte - off), off, off + OBS_BYTES * n_valid,
-                                                        (int)threadIdx.x);
     }
     flush_stats(st.wstats, cnt);
 }
@@ -872,9 +579,7 @@ wab_step_pipe_kernel(const __grid_constant__ Params P, const StatePtrs st, const
                 write_scalars(out, o, O);
                 if (out.features) write_features(out.features, o, O);
             }
-#ifndef WAB_EXP_NOEMIT
             if (out.grids) stream_flush<false>(stream, nullptr, out.grids + (first_byte - off), off, off + OBS_BYTES * n_valid, lane);
-#endif
             __syncwarp();
         }
     }
@@ -1331,28 +1036,16 @@ void launch_pdl(void (*kern)(KArgs...), unsigned grid, unsigned block, size_t sm
     cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 
-// The time-chunked kernel is opt-in (WAB_CHUNK=1): bit-identical, but measured no faster than the step-by-step kernel at
-// 4,096 envs (1.77e9 vs 1.79e9 env-steps/s; profiles/r2e_*): the draws it makes ahead are ~15 % of a step's instructions,
-// and parking / re-reading every step's planes costs about as much.
-bool chunk_enabled() { const char* e = getenv("WAB_CHUNK"); return e && atoi(e) != 0; }
 // // WAB_PIPE: 0 = never, 1 (default) = where it pays (see launch_step_t), 2 = always (tests, A/B runs).
 int pipe_mode() { const char* e = getenv("WAB_PIPE"); return e ? atoi(e) : 1; }
 bool use_pipeline(const WabVec* h, int lpe, int T) {
-    if (h->generic || lpe <= 1 || T < 4 || pipe_mode() == 0 || (chunk_enabled() && (lpe == 8 || lpe == 16))) return false;
+    if (h->generic || lpe <= 1 || T < 4 || pipe_mode() == 0) return false;
     const int64_t epw = 32 / lpe, rule_warps = (h->n + epw - 1) / epw;
     return pipe_mode() == 2 || rule_warps <= 8 * (int64_t)h->n_sm;
 }
 template <bool F64, int LPE>
 void launch_step_t(const WabVec* h, const uint8_t* a, int T, const OutPtrs& out, cudaStream_t s) {
     const unsigned grid = (unsigned)((h->n + Geo<LPE>::EPB - 1) / Geo<LPE>::EPB);
-    if constexpr (LPE == 8 || LPE == 16) {
-        if (chunk_enabled() && T > 1) {          // the time-chunked kernel (a single step has nothing to run ahead of)
-            const size_t smem = sizeof(uint32_t) * ((size_t)h->P.wolf_cap * Geo<LPE>::EPB +
-                                                    (size_t)(Geo<LPE>::THREADS / 32) * ChunkGeo<LPE>::WARP_WORDS);
-            launch_pdl(wab_step_chunk_kernel<F64, LPE>, grid, Geo<LPE>::THREADS, smem, s, h->P, h->st, a, T, out);
-            return;
-        }
-    }
     if constexpr (LPE > 1) {
         // two-warp pipeline (rules in one warp, publication in the other) while the batch leaves issue slots free: up to
         // 8 rule warps per SM. Same-box A/B (profiles/r2j_pipe_ab.txt): 4,096 envs at LPE 8 (6.9 rule warps per SM)
@@ -1544,10 +1237,8 @@ int wab_vec_create(const WabConfig* cfg, const uint32_t* bush_thr, int32_t n_bus
         const size_t threads = lpe == 1 ? (size_t)WAB_THREADS_LPE1 : (size_t)WAB_THREADS_LPEN, epb = threads / lpe;
         return (n + epb - 1) / epb * (threads / 32);
     };
-    const size_t cta16_rows = (n + kCta16Envs - 1) / kCta16Envs * (kCta16Threads / 32);   // the mapped host path's kernel
-    size_t stat_rows = h->generic ? (n + GEN_WARPS - 1) / GEN_WARPS * GEN_WARPS
-                                  : (warps_of(1) > warps_of((size_t)h->lpe) ? warps_of(1) : warps_of((size_t)h->lpe));
-    if (!h->generic && cta16_rows > stat_rows) stat_rows = cta16_rows;
+    const size_t stat_rows = h->generic ? (n + GEN_WARPS - 1) / GEN_WARPS * GEN_WARPS
+                                        : (warps_of(1) > warps_of((size_t)h->lpe) ? warps_of(1) : warps_of((size_t)h->lpe));
     const size_t o_wstats = o; o = align_up(o + 64 * stat_rows, 256);
     cudaError_t e = cudaMalloc(&h->slab, o);
     if (e != cudaSuccess) { delete h; return cuda_fail(e, "cudaMalloc(state)"); }
@@ -1675,11 +1366,11 @@ int wab_vec_step_host_packed(WabVec* h, const uint8_t* h_actions, uint8_t* h_blo
     // thread-per-env kernel — whose warps own 16-byte-aligned slabs, so every store is a full 16-byte one — reads the
     // actions from, and streams its outputs into, the caller's pinned (hence device-mapped) host buffers; no staging
     // copy, and the transfer overlaps the step. Measured (profiles/r1_e2e_paths.txt): 52.7 vs 60.2 us per step at
-    // 4,096 envs; the copy engine wins from 32k envs up. WAB_HOST_MAPPED=0/1/2/3 forces staged / mapped / mapped with
-    // the thread-per-env kernel.
+    // 4,096 envs; the copy engine wins from 32k envs up. WAB_HOST_MAPPED=0 forces the staged path, any other value the
+    // mapped one.
     if (h->host_mapped < 0) {
         const char* e = getenv("WAB_HOST_MAPPED");
-        h->host_mapped = e ? atoi(e) : (h->n <= 16384 ? 2 : 0);
+        h->host_mapped = e ? atoi(e) != 0 : h->n <= 16384;
     }
     if (h->host_mapped) {
         if (h->m_actions != h_actions || h->m_block != h_block) {      // resolve the device aliases once per buffer pair
@@ -1698,17 +1389,7 @@ int wab_vec_step_host_packed(WabVec* h, const uint8_t* h_actions, uint8_t* h_blo
         if (h->m_dblock) {
             uint8_t* m = h->m_dblock - L.grids;                        // block offsets are relative to L.grids
             WabObs mo{m + L.grids, m + L.food, m + L.role, m + L.status};
-            if (h->host_mapped == 3 && !h->generic) {          // 16 envs per CTA, every store a full 16-byte one
-                OutPtrs mout{mo.d_grids, mo.d_food, mo.d_role, mo.d_status, (float*)(m + L.reward), m + L.done, m + L.info, h->d_features};
-                const unsigned grid = (unsigned)((h->n + kCta16Envs - 1) / kCta16Envs);
-                const size_t smem = sizeof(uint32_t) * ((size_t)h->P.wolf_cap * kCta16Envs + (size_t)kCta16Stream);
-                if (h->cfg.food_mode == WAB_FOOD_F64)
-                    launch_pdl(wab_step_cta16_kernel<true>, grid, kCta16Threads, smem, s, h->P, h->st, h->m_dactions, mout);
-                else
-                    launch_pdl(wab_step_cta16_kernel<false>, grid, kCta16Threads, smem, s, h->P, h->st, h->m_dactions, mout);
-                WAB_CUDA(cudaGetLastError());
-            } else if (int rc = launch_step(h, 1, h->m_dactions, mo, (float*)(m + L.reward), m + L.done, m + L.info, s,
-                                            h->host_mapped == 2 ? 1 : 0)) return rc;
+            if (int rc = launch_step(h, 1, h->m_dactions, mo, (float*)(m + L.reward), m + L.done, m + L.info, s, 1)) return rc;
             WAB_CUDA(cudaStreamSynchronize(s));
             return WAB_OK;
         }
