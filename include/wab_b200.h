@@ -245,8 +245,8 @@ int wab_vec_flat_dim(const WabVec *h);
  * fresh noise on every replay.
  *
  * Keying contract of the policy entry points: every one that takes a WabVec handle (wab_vec_flatten_features_noisy,
- * wab_policy_affine1, wab_policy_trunk, wab_policy_forward, wab_policy_backward, wab_policy_ppo_backward) keys its noise
- * and its action samples by the global env id env_id_base + row (the row within its step for the backward passes), so
+ * wab_policy_affine1, wab_policy_trunk, wab_policy_forward, wab_policy_backward, wab_policy_ppo_backward,
+ * wab_policy_evaluate, wab_policy_backward_logits) keys its noise and its action samples by the global env id env_id_base + row (the row within its step for the backward passes), so
  * a shard [first, first + count) draws exactly what the unsharded batch draws for rows first .. first + count - 1;
  * outputs stay indexed by the local row. The two handle-less calls, wab_sample_categorical and wab_policy_tail, know no
  * shard and key by the local row. */
@@ -363,10 +363,44 @@ int wab_policy_ppo_backward(WabVec *h, const uint8_t *d_features, int64_t n_step
                             int64_t scratch_bytes, float *d_grad, float *d_logp, float *d_value, float *d_entropy,
                             void *stream);
 
+/* Any loss over the policy's outputs: the recomputed forward and the vector-Jacobian product of (logits, value), so a
+ * caller can write the loss in torch (or anything else) and keep only the outputs per row, never the activations.
+ * Both calls take a LIST of n_rows = M entries: d_rows int32[M] (device; NULL: entry m is row m) with a HOST count, and
+ * entry m = t N + n selects the feature bytes of row n of step t and d_counters[t], as for wab_policy_backward (the noise
+ * key is the global env id env_id_base + n). Their arrays are indexed by the list position m, so a minibatch needs no
+ * [T, N] arrays; an entry may repeat (it then counts once per occurrence, so M may exceed T N). An entry outside
+ * [0, T N) gets NaN logits and value and contributes nothing to the gradient.
+ * wab_policy_evaluate writes d_logits f32[M][A] (the action head's output before the softmax, bias included) and d_value
+ * f32[M]. It recomputes the forward with wab_policy_forward's arithmetic: under the weights a rollout used, d_value equals
+ * what wab_policy_forward returned for that row bit for bit, and log_softmax(d_logits) its log-probabilities to rounding.
+ * wab_policy_backward_logits writes d_grad f32 (layout as wab_policy_backward's) = the gradient of
+ *   sum over m of  sum_o d_g_logits[m][o] logit_o(x_m) + d_g_value[m] V(x_m),
+ * the same pass as wab_policy_backward with d heads taken as given. Its scratch is left as wab_policy_backward's, so
+ * wab_policy_backward_grad_f64 (and wab_policy_grad_sum_ranks over ranks) apply to it. Neither call synchronises.
+ * Arguments otherwise as for wab_policy_backward (wab_policy_evaluate takes no transposed weights; it needs the scratch
+ * of wab_policy_backward_scratch_bytes for the hidden activations of its tiles). Equal inputs give bit-identical outputs.
+ * WAB_E_NULL for a missing pointer (d_rows may be NULL); WAB_E_CONFIG for misalignment, too small a scratch,
+ * n_rows < 0 or a negative or non-finite noise_scale; WAB_E_UNSUPPORTED beyond 8 actions, for hidden2 != 150 or
+ * flat_dim > 512. */
+int wab_policy_evaluate(WabVec *h, const uint8_t *d_features, int64_t n_steps, int64_t n_envs, const uint64_t *d_counters,
+                        const int32_t *d_rows, int64_t n_rows, const void *d_packed1, const float *d_bias1,
+                        const void *d_packed2, const float *d_bias2, int32_t hidden2, const void *d_packed3,
+                        const float *d_bias3, const float *d_w_heads, const float *d_b_heads, int32_t n_actions,
+                        float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi, void *d_scratch,
+                        int64_t scratch_bytes, float *d_logits, float *d_value, void *stream);
+int wab_policy_backward_logits(WabVec *h, const uint8_t *d_features, int64_t n_steps, int64_t n_envs,
+                               const uint64_t *d_counters, const int32_t *d_rows, int64_t n_rows, const float *d_g_logits,
+                               const float *d_g_value, const void *d_packed1, const float *d_bias1, const void *d_packed2,
+                               const float *d_bias2, int32_t hidden2, const void *d_packed3, const float *d_bias3,
+                               const void *d_packed2t, const void *d_packed3t, const float *d_w_heads,
+                               const float *d_b_heads, int32_t n_actions, float noise_scale, float leaky_slope,
+                               float clamp_lo, float clamp_hi, void *d_scratch, int64_t scratch_bytes, float *d_grad,
+                               void *stream);
+
 /* Data-parallel training: the cross-rank gradient sum, deterministic and rounded once.
- * wab_policy_backward_grad_f64 reduces the scratch left by the last wab_policy_backward / wab_policy_ppo_backward with
- * this d_scratch on this stream into d_grad64 f64[n_params] (same layout as d_grad, the same CTA order, the fp64 sums not
- * rounded). wab_policy_grad_sum_ranks writes d_grad f32[n] = fp32(sum over r in index order of d_rank_grads[r][i]), the
+ * wab_policy_backward_grad_f64 reduces the scratch left by the last wab_policy_backward / wab_policy_ppo_backward /
+ * wab_policy_backward_logits with this d_scratch on this stream into d_grad64 f64[n_params] (same layout as d_grad, the
+ * same CTA order, the fp64 sums not rounded). wab_policy_grad_sum_ranks writes d_grad f32[n] = fp32(sum over r in index order of d_rank_grads[r][i]), the
  * sum in fp64, for an all-gathered d_rank_grads f64[n_ranks][n]. With one rank, sum_ranks(grad_f64) equals
  * wab_policy_backward's d_grad bit for bit. WAB_E_NULL for a missing pointer; WAB_E_CONFIG for misalignment (16 bytes
  * for d_scratch, 8 for the fp64 arrays, 4 for d_grad), too small a scratch, n_ranks < 1 or n < 0; WAB_E_UNSUPPORTED

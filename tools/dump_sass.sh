@@ -13,7 +13,8 @@ for f in re.split(r'\n\s*Function : ', txt)[1:]:
     for key, out in (('wab_step_kernelILb0ELi1ELi24E', 'step_lpe1'), ('wab_step_kernelILb0ELi16E', 'step_lpe16'), ('wab2_turn_kernel', 'v2_turn'),
                      ('wab_step_pipe_kernelILb0ELi8E', 'step_pipe_lpe8'), ('wab_affine1_tc_kernelILi2E', 'policy_forward_tcgen05'),
                      ('wab2_grid_turn_kernelILb1ELb0E', 'v2_grid_turn'), ('wab_policy_bwd_kernel', 'policy_backward_tcgen05'),
-                     ('wab_policy_ppo_bwd_kernel', 'policy_ppo_backward_tcgen05')):
+                     ('wab_policy_ppo_bwd_kernel', 'policy_ppo_backward_tcgen05'), ('wab_policy_eval_kernel', 'policy_eval_tcgen05'),
+                     ('wab_policy_logits_bwd_kernel', 'policy_logits_backward_tcgen05')):
         if key in name:
             body = 'Function : ' + f
             # keep the instruction text only: drop the hex encodings (and the encoding-only second line of every instruction)

@@ -1857,6 +1857,99 @@ int wab_policy_ppo_backward(WabVec* h, const uint8_t* d_features, int64_t n_step
                                   clamp_lo, clamp_hi, d_scratch, scratch_bytes, d_grad, d_logp, d_value, stream);
 }
 
+// wab_policy_evaluate and wab_policy_backward_logits: the checks they share, then the list kernel (the evaluation when
+// `d_logits` is given, else the logits backward followed by the reduction). The per-kind arrays are checked by the callers.
+static int policy_list_launch(const char* who, WabVec* h, const uint8_t* d_features, int64_t n_steps, int64_t n_envs,
+                              const uint64_t* d_counters, const int32_t* d_rows, int64_t n_rows, const float* d_g_logits,
+                              const float* d_g_value, const void* d_packed1, const float* d_bias1, const void* d_packed2,
+                              const float* d_bias2, int32_t hidden2, const void* d_packed3, const float* d_bias3,
+                              const void* d_packed2t, const void* d_packed3t, const float* d_w_heads, const float* d_b_heads,
+                              int32_t n_actions, float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi,
+                              void* d_scratch, int64_t scratch_bytes, float* d_grad, float* d_logits, float* d_value,
+                              void* stream) {
+    if (!h || !d_features || !d_counters || !d_packed1 || !d_bias1 || !d_packed2 || !d_bias2 || !d_packed3 || !d_bias3 ||
+        !d_w_heads || !d_b_heads || !d_scratch)
+        return fail(WAB_E_NULL, "null argument");
+    if (hidden2 != 150) return fail(WAB_E_UNSUPPORTED, std::string(who) + " is built for the reference's trunk 128 -> 150 -> 128 (actor_critic.py:59-61)");
+    if (n_actions < 1 || n_actions > 8) return fail(WAB_E_UNSUPPORTED, std::string(who) + ": at most 8 actions");
+    const int dim = wab_vec_flat_dim(h);
+    if (dim > TC_CHUNKS * TC_KC) return fail(WAB_E_UNSUPPORTED, std::string(who) + ": the input is at most 512 columns wide");
+    if (n_steps < 0 || n_envs < 0 || n_steps * n_envs > INT32_MAX) return fail(WAB_E_CONFIG, std::string(who) + ": 0 <= T N < 2^31 rows");
+    if (n_rows < 0) return fail(WAB_E_CONFIG, std::string(who) + ": n_rows must be >= 0");
+    if (!(noise_scale >= 0.f) || !std::isfinite(noise_scale)) return fail(WAB_E_CONFIG, std::string(who) + ": noise_scale must be finite and >= 0");
+    if (((uintptr_t)d_packed1 & 15u) != 0 || ((uintptr_t)d_packed2 & 15u) != 0 || ((uintptr_t)d_packed3 & 15u) != 0 ||
+        ((uintptr_t)d_packed2t & 15u) != 0 || ((uintptr_t)d_packed3t & 15u) != 0 || ((uintptr_t)d_scratch & 15u) != 0 ||
+        ((uintptr_t)d_features & 3u) != 0 || ((uintptr_t)d_counters & 7u) != 0 || ((uintptr_t)d_rows & 3u) != 0 ||
+        ((uintptr_t)d_grad & 3u) != 0 || ((uintptr_t)d_g_logits & 3u) != 0 || ((uintptr_t)d_g_value & 3u) != 0 ||
+        ((uintptr_t)d_logits & 3u) != 0 || ((uintptr_t)d_value & 3u) != 0)
+        return fail(WAB_E_CONFIG, "the packed weights and d_scratch must be 16-byte aligned, d_counters 8-byte, "
+                                  "d_features, d_rows and the float arrays 4-byte");
+    if (scratch_bytes < wab_policy_backward_scratch_bytes(h)) return fail(WAB_E_CONFIG, "d_scratch is smaller than wab_policy_backward_scratch_bytes");
+    const bool eval = d_logits != nullptr;
+    DeviceGuard guard(h->device);
+    static bool attr_set[2][64] = {{false}};
+    if (h->device < 64 && !attr_set[eval ? 1 : 0][h->device]) {
+        if (eval) WAB_CUDA(cudaFuncSetAttribute(wab_policy_eval_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_SMEM_TOTAL));
+        else WAB_CUDA(cudaFuncSetAttribute(wab_policy_logits_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_SMEM_TOTAL));
+        attr_set[eval ? 1 : 0][h->device] = true;
+    }
+    BackwardArgs B;
+    memset(&B, 0, sizeof(B));
+    B.features = d_features; B.n_envs = n_envs > 0 ? n_envs : 1; B.n_rows = n_steps * n_envs;
+    B.counters = reinterpret_cast<const unsigned long long*>(d_counters);
+    B.rows = d_rows;
+    B.w1 = reinterpret_cast<const uint4*>(d_packed1); B.b1 = d_bias1; B.w2 = reinterpret_cast<const uint4*>(d_packed2); B.b2 = d_bias2;
+    B.w3 = reinterpret_cast<const uint4*>(d_packed3); B.b3 = d_bias3;
+    B.w2t = reinterpret_cast<const uint4*>(d_packed2t); B.w3t = reinterpret_cast<const uint4*>(d_packed3t);
+    B.w_heads = d_w_heads; B.b_heads = d_b_heads; B.n_actions = n_actions; B.noise_scale = noise_scale; B.slope = leaky_slope;
+    B.clamp_lo = clamp_lo; B.clamp_hi = clamp_hi; B.scratch = reinterpret_cast<float*>(d_scratch);
+    ListArgs L;
+    memset(&L, 0, sizeof(L));
+    L.n_list = n_rows; L.g_logits = d_g_logits; L.g_value = d_g_value; L.logits_out = d_logits; L.value_out = d_value;
+    const int grid = backward_grid(h->device);
+    if (eval) {
+        wab_policy_eval_kernel<<<grid, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(h->P, (int)h->cfg.food_obs_scale + 1, B, L);
+        WAB_CUDA(cudaGetLastError());
+        return WAB_OK;
+    }
+    wab_policy_logits_bwd_kernel<<<grid, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(h->P, (int)h->cfg.food_obs_scale + 1, B, L);
+    WAB_CUDA(cudaGetLastError());
+    const int64_t total = policy_n_params(dim, n_actions);
+    wab_policy_bwd_reduce_kernel<float><<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        reinterpret_cast<const float*>(d_scratch), grid, dim, n_actions, d_grad);
+    WAB_CUDA(cudaGetLastError());
+    return WAB_OK;
+}
+
+int wab_policy_evaluate(WabVec* h, const uint8_t* d_features, int64_t n_steps, int64_t n_envs, const uint64_t* d_counters,
+                        const int32_t* d_rows, int64_t n_rows, const void* d_packed1, const float* d_bias1,
+                        const void* d_packed2, const float* d_bias2, int32_t hidden2, const void* d_packed3,
+                        const float* d_bias3, const float* d_w_heads, const float* d_b_heads, int32_t n_actions,
+                        float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi, void* d_scratch,
+                        int64_t scratch_bytes, float* d_logits, float* d_value, void* stream) {
+    if (!d_logits || !d_value) return fail(WAB_E_NULL, "null argument");
+    // the evaluation runs no step 3: the transposed weights are never read, the forward's stand in for the checks
+    return policy_list_launch("wab_policy_evaluate", h, d_features, n_steps, n_envs, d_counters, d_rows, n_rows, nullptr,
+                              nullptr, d_packed1, d_bias1, d_packed2, d_bias2, hidden2, d_packed3, d_bias3, d_packed2,
+                              d_packed3, d_w_heads, d_b_heads, n_actions, noise_scale, leaky_slope, clamp_lo, clamp_hi,
+                              d_scratch, scratch_bytes, nullptr, d_logits, d_value, stream);
+}
+
+int wab_policy_backward_logits(WabVec* h, const uint8_t* d_features, int64_t n_steps, int64_t n_envs,
+                               const uint64_t* d_counters, const int32_t* d_rows, int64_t n_rows, const float* d_g_logits,
+                               const float* d_g_value, const void* d_packed1, const float* d_bias1, const void* d_packed2,
+                               const float* d_bias2, int32_t hidden2, const void* d_packed3, const float* d_bias3,
+                               const void* d_packed2t, const void* d_packed3t, const float* d_w_heads,
+                               const float* d_b_heads, int32_t n_actions, float noise_scale, float leaky_slope,
+                               float clamp_lo, float clamp_hi, void* d_scratch, int64_t scratch_bytes, float* d_grad,
+                               void* stream) {
+    if (!d_g_logits || !d_g_value || !d_packed2t || !d_packed3t || !d_grad) return fail(WAB_E_NULL, "null argument");
+    return policy_list_launch("wab_policy_backward_logits", h, d_features, n_steps, n_envs, d_counters, d_rows, n_rows,
+                              d_g_logits, d_g_value, d_packed1, d_bias1, d_packed2, d_bias2, hidden2, d_packed3, d_bias3,
+                              d_packed2t, d_packed3t, d_w_heads, d_b_heads, n_actions, noise_scale, leaky_slope, clamp_lo,
+                              clamp_hi, d_scratch, scratch_bytes, d_grad, nullptr, nullptr, stream);
+}
+
 int wab_policy_backward_grad_f64(WabVec* h, const void* d_scratch, int64_t scratch_bytes, int32_t n_actions, double* d_grad64,
                                  void* stream) {
     if (!h || !d_scratch || !d_grad64) return fail(WAB_E_NULL, "null argument");

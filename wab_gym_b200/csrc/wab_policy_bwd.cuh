@@ -26,6 +26,12 @@
 // H = -sum_o p_o log p_o, with A, R, logp_old read per row. Its upstream gradients are closed forms of what the heads block
 // already holds: g_logp = -w_pi A r (0 where the clip is active), g_value = w_v (V - R), and the entropy adds
 // w_H p_o (log p_o + H) to d logit_o. Everything after the heads is shared.
+//
+// Two more kernels of the same body serve any loss written in torch over (logits, value). They take a LIST of M rows
+// (ListArgs: a host count, B.rows or NULL for row m = m) and index their inputs and outputs by the list position m, so a
+// minibatch needs no [T, N] arrays; a listed entry outside [0, T N) gets NaN outputs and contributes nothing:
+//   wab_policy_eval_kernel        step 1 and the heads only: logits [M][A] (before the softmax, bias included), value [M];
+//   wab_policy_logits_bwd_kernel  the whole pass with d heads read per row (d logits [M][A], d value [M]) in step 2.
 #pragma once
 
 namespace {
@@ -64,6 +70,17 @@ struct PpoArgs {
     float* entropy_out;                      // H per row (optional)
 };
 
+// the list kernels (wab_policy_eval_kernel, wab_policy_logits_bwd_kernel): M = n_list rows, row m = B.rows[m] (B.rows
+// NULL: m); arrays indexed by m. B.d_count, B.actions, B.g_logp, B.g_value, B.logp_out and B.value_out are unused there
+struct ListArgs {
+    long long n_list;                        // M (a host count; may exceed T N when rows repeat)
+    const float* g_logits; const float* g_value;       // upstream d logits [M][A], d value [M] (the logits backward)
+    float* logits_out; float* value_out;     // logits [M][A], value [M] (the evaluation)
+};
+
+// which heads block the body runs (step 2), and whether steps 3 - 5 follow (not for BW_EVAL)
+enum BwKind { BW_A2C, BW_PPO, BW_EVAL, BW_LOGITS };
+
 // element (operand row n, K = tile row k) of a K = 128 operand, canonical K-major layout without swizzle
 __device__ __forceinline__ uint32_t bw_off(int n, int k) { return (uint32_t)((n >> 3) * BW_KROW + (k >> 3) * 128 + (n & 7) * 16 + (k & 7) * 2); }
 __device__ __forceinline__ void bw_st16(uint32_t addr, uint32_t v) { asm volatile("st.shared.u16 [%0], %1;" :: "r"(addr), "h"((unsigned short)v) : "memory"); }
@@ -98,15 +115,35 @@ __device__ __forceinline__ void bw_bias_sum(const float (&g)[CNT], int valid, fl
 
 __global__ void __launch_bounds__(256, 1)
 wab_policy_bwd_kernel(const __grid_constant__ Params P, int food_dim, const __grid_constant__ BackwardArgs B) {
-    constexpr bool PPO = false;
+    constexpr BwKind KIND = BW_A2C;
     const PpoArgs Q{};
+    const ListArgs L{};
 #include "wab_policy_bwd_body.cuh"
 }
 
 __global__ void __launch_bounds__(256, 1)
 wab_policy_ppo_bwd_kernel(const __grid_constant__ Params P, int food_dim, const __grid_constant__ BackwardArgs B,
                           const __grid_constant__ PpoArgs Q) {
-    constexpr bool PPO = true;
+    constexpr BwKind KIND = BW_PPO;
+    const ListArgs L{};
+#include "wab_policy_bwd_body.cuh"
+}
+
+#pragma nv_diag_suppress 128                        // steps 3 - 5 of the body, after the evaluation's `continue`
+__global__ void __launch_bounds__(256, 1)
+wab_policy_eval_kernel(const __grid_constant__ Params P, int food_dim, const __grid_constant__ BackwardArgs B,
+                       const __grid_constant__ ListArgs L) {
+    constexpr BwKind KIND = BW_EVAL;
+    const PpoArgs Q{};
+#include "wab_policy_bwd_body.cuh"
+}
+#pragma nv_diag_default 128
+
+__global__ void __launch_bounds__(256, 1)
+wab_policy_logits_bwd_kernel(const __grid_constant__ Params P, int food_dim, const __grid_constant__ BackwardArgs B,
+                             const __grid_constant__ ListArgs L) {
+    constexpr BwKind KIND = BW_LOGITS;
+    const PpoArgs Q{};
 #include "wab_policy_bwd_body.cuh"
 }
 

@@ -1,7 +1,8 @@
-// wab_policy_bwd_body.cuh — the body of wab_policy_bwd_kernel and wab_policy_ppo_bwd_kernel (wab_policy_bwd.cuh), included
-// inside both. Each kernel declares `constexpr bool PPO`, its parameters P, food_dim, B and a PpoArgs Q; PPO selects the
-// upstream gradients of step 2, and everything else is shared. A fragment rather than a __forceinline__ function: the
-// compiler optimises a device function on its own before inlining it, which changes the code of the existing kernel.
+// wab_policy_bwd_body.cuh — the body of wab_policy_bwd_kernel, wab_policy_ppo_bwd_kernel, wab_policy_eval_kernel and
+// wab_policy_logits_bwd_kernel (wab_policy_bwd.cuh), included inside each. Each kernel declares `constexpr BwKind KIND`,
+// its parameters P, food_dim, B, a PpoArgs Q and a ListArgs L; KIND selects the row list and the heads block of step 2
+// (BW_EVAL stops after it), and everything else is shared. A fragment rather than a __forceinline__ function: the
+// compiler optimises a device function on its own before inlining it, which changes the code of the existing kernels.
     extern __shared__ __align__(1024) uint8_t tc_smem[];
     __shared__ uint32_t tmem_slot;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -15,6 +16,7 @@
     float* red = reinterpret_cast<float*>(tc_smem + BW_SMEM_RED);          // [4 warps][160] bias partial sums
     float* part = B.scratch + (size_t)blockIdx.x * BP_BLOCK;
     const int A = B.n_actions, n_out = A + 1;
+    constexpr bool LIST = KIND == BW_EVAL || KIND == BW_LOGITS;     // rows by list position, a host count
 
     if (warp == 0) {
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"((uint32_t)__cvta_generic_to_shared(&tmem_slot)), "r"(512u) : "memory");
@@ -24,7 +26,8 @@
         asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(s_bar), "r"(1u) : "memory");
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    for (int k = tid; k < BP_PARTIAL; k += 256) part[k] = 0.f;
+    if constexpr (KIND != BW_EVAL)                                          // the evaluation writes no gradient
+        for (int k = tid; k < BP_PARTIAL; k += 256) part[k] = 0.f;
     for (int k = tid; k < 12 * 128; k += 256) {
         const int i = k / 12, o = k - 12 * i;
         wsm[k] = o < n_out ? B.w_heads[o * 128 + i] : 0.f;
@@ -43,8 +46,8 @@
     float* st_h1 = part + BP_H1 + r * 128 + h * 64;                       // this thread's stash: its row, its half
     float* st_h2 = part + BP_H2 + r * 160 + h * 80;
     uint32_t parity = 0;
-    long long count = B.d_count ? *B.d_count : (long long)B.n_rows;
-    count = count < 0 ? 0 : (count > (long long)B.n_rows ? (long long)B.n_rows : count);
+    long long count = LIST ? L.n_list : (B.d_count ? *B.d_count : (long long)B.n_rows);
+    if (!LIST) count = count < 0 ? 0 : (count > (long long)B.n_rows ? (long long)B.n_rows : count);
     const long long n_tiles = (count + TC_TILE_M - 1) / TC_TILE_M;
 
     auto wait_mma = [&]() {
@@ -350,54 +353,70 @@
             if (h == 0) {
 #pragma unroll
                 for (int o = 0; o < 9; ++o) acc[o] = o < n_out ? (partial[(r * 2) * 9 + o] + partial[(r * 2 + 1) * 9 + o]) + B.b_heads[o] : 0.f;
-                float mx = -3.4e38f;
+                if constexpr (LIST) {
+                    if constexpr (KIND == BW_EVAL) {                       // logits and value of listed entry m = slot
+                        if (slot < count) {
+                            const float nan = __int_as_float(0x7FC00000);
 #pragma unroll
-                for (int o = 0; o < 8; ++o) if (o < A) mx = fmaxf(mx, acc[o]);
-                float ex[8], tot = 0.f;
+                            for (int o = 0; o < 8; ++o) if (o < A) L.logits_out[slot * A + o] = valid ? acc[o] : nan;
+                            L.value_out[slot] = valid ? acc[A < 8 ? A : 8] : nan;
+                        }
+                    } else {
 #pragma unroll
-                for (int o = 0; o < 8; ++o) { ex[o] = o < A ? expf(acc[o] - mx) : 0.f; tot += ex[o]; }
-                const int a = valid ? (int)B.actions[flat] : 0;
-                if constexpr (!PPO) {
-                    const float gl = valid ? B.g_logp[flat] : 0.f, gv = valid ? B.g_value[flat] : 0.f;
-                    float p_pick = 0.f;
-#pragma unroll
-                    for (int o = 0; o < 8; ++o) if (o == a) p_pick = ex[o];
-                    if (valid && B.logp_out) B.logp_out[flat] = logf(p_pick / tot);
-                    if (valid && B.value_out) B.value_out[flat] = acc[A < 8 ? A : 8];
-#pragma unroll
-                    for (int o = 0; o < 9; ++o)                                // d log pi_a / d logit_o = 1[o = a] - p_o; d V = g_value
-                        dhs[r * 9 + o] = o < A ? gl * ((o == a ? 1.f : 0.f) - ex[o] / tot) : (o == A ? gv : 0.f);
-                } else {
-                    float p_pick = 0.f;
-#pragma unroll
-                    for (int o = 0; o < 8; ++o) if (o == a) p_pick = ex[o];
-                    const float lp = logf(p_pick / tot), value = acc[A < 8 ? A : 8];   // as the forward (and the branch above)
-                    // log p_o = (z_o - max) - log sum, never log(p_o): an underflowed p_o would make 0 * log 0 a NaN
-                    const float lsum = logf(tot);
-                    float ent = 0.f;
-#pragma unroll
-                    for (int o = 0; o < 8; ++o) if (o < A) ent -= (ex[o] / tot) * ((acc[o] - mx) - lsum);
-                    float gl = 0.f, gv = 0.f, wh = 0.f;
-                    if (valid) {
-                        const float adv = Q.advantage[flat], ratio = expf(lp - Q.logp_old[flat]);
-                        const bool clipped = (adv > 0.f && ratio > 1.f + Q.clip_eps) || (adv < 0.f && ratio < 1.f - Q.clip_eps);
-                        gl = clipped ? 0.f : (-Q.w_policy * adv) * ratio;
-                        gv = Q.w_value * (value - Q.target[flat]);
-                        wh = Q.w_entropy;
-                        if (B.logp_out) B.logp_out[flat] = lp;
-                        if (B.value_out) B.value_out[flat] = value;
-                        if (Q.entropy_out) Q.entropy_out[flat] = ent;
+                        for (int o = 0; o < 9; ++o)                            // d heads as given: d logits, d value
+                            dhs[r * 9 + o] = valid && o < n_out ? (o < A ? L.g_logits[slot * A + o] : L.g_value[slot]) : 0.f;
                     }
+                } else {
+                    float mx = -3.4e38f;
 #pragma unroll
-                    for (int o = 0; o < 9; ++o) {                          // + d(-w_H H) / d logit_o = w_H p_o (log p_o + H)
-                        float d = o < A ? gl * ((o == a ? 1.f : 0.f) - ex[o] / tot) : (o == A ? gv : 0.f);
-                        if (o < A && wh != 0.f) d += wh * ((ex[o] / tot) * (((acc[o] - mx) - lsum) + ent));
-                        dhs[r * 9 + o] = d;
+                    for (int o = 0; o < 8; ++o) if (o < A) mx = fmaxf(mx, acc[o]);
+                    float ex[8], tot = 0.f;
+#pragma unroll
+                    for (int o = 0; o < 8; ++o) { ex[o] = o < A ? expf(acc[o] - mx) : 0.f; tot += ex[o]; }
+                    const int a = valid ? (int)B.actions[flat] : 0;
+                    if constexpr (KIND == BW_A2C) {
+                        const float gl = valid ? B.g_logp[flat] : 0.f, gv = valid ? B.g_value[flat] : 0.f;
+                        float p_pick = 0.f;
+#pragma unroll
+                        for (int o = 0; o < 8; ++o) if (o == a) p_pick = ex[o];
+                        if (valid && B.logp_out) B.logp_out[flat] = logf(p_pick / tot);
+                        if (valid && B.value_out) B.value_out[flat] = acc[A < 8 ? A : 8];
+#pragma unroll
+                        for (int o = 0; o < 9; ++o)                                // d log pi_a / d logit_o = 1[o = a] - p_o; d V = g_value
+                            dhs[r * 9 + o] = o < A ? gl * ((o == a ? 1.f : 0.f) - ex[o] / tot) : (o == A ? gv : 0.f);
+                    } else {
+                        float p_pick = 0.f;
+#pragma unroll
+                        for (int o = 0; o < 8; ++o) if (o == a) p_pick = ex[o];
+                        const float lp = logf(p_pick / tot), value = acc[A < 8 ? A : 8];   // as the forward (and the branch above)
+                        // log p_o = (z_o - max) - log sum, never log(p_o): an underflowed p_o would make 0 * log 0 a NaN
+                        const float lsum = logf(tot);
+                        float ent = 0.f;
+#pragma unroll
+                        for (int o = 0; o < 8; ++o) if (o < A) ent -= (ex[o] / tot) * ((acc[o] - mx) - lsum);
+                        float gl = 0.f, gv = 0.f, wh = 0.f;
+                        if (valid) {
+                            const float adv = Q.advantage[flat], ratio = expf(lp - Q.logp_old[flat]);
+                            const bool clipped = (adv > 0.f && ratio > 1.f + Q.clip_eps) || (adv < 0.f && ratio < 1.f - Q.clip_eps);
+                            gl = clipped ? 0.f : (-Q.w_policy * adv) * ratio;
+                            gv = Q.w_value * (value - Q.target[flat]);
+                            wh = Q.w_entropy;
+                            if (B.logp_out) B.logp_out[flat] = lp;
+                            if (B.value_out) B.value_out[flat] = value;
+                            if (Q.entropy_out) Q.entropy_out[flat] = ent;
+                        }
+#pragma unroll
+                        for (int o = 0; o < 9; ++o) {                          // + d(-w_H H) / d logit_o = w_H p_o (log p_o + H)
+                            float d = o < A ? gl * ((o == a ? 1.f : 0.f) - ex[o] / tot) : (o == A ? gv : 0.f);
+                            if (o < A && wh != 0.f) d += wh * ((ex[o] / tot) * (((acc[o] - mx) - lsum) + ent));
+                            dhs[r * 9 + o] = d;
+                        }
                     }
                 }
             }
             __syncthreads();
         }
+        if constexpr (KIND == BW_EVAL) continue;                           // no gradient: the next tile
         float dh[9];
 #pragma unroll
         for (int o = 0; o < 9; ++o) dh[o] = dhs[r * 9 + o];

@@ -17,6 +17,7 @@ from typing import Dict, Optional
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 from .vec_env import VecEnv, _ptr, _raw_stream
@@ -160,7 +161,9 @@ class PolicyTrainTC(PolicyTrunkTC):
     gradient of ``sum g_logp * log pi(a | x) + g_value * V(x)`` with respect to every parameter of the policy, as one flat
     f32 buffer in ``parameters_to_vector(policy.parameters())`` order. The forward is recomputed from the feature bytes
     (the policy input is regenerated, never stored), so training keeps 62 bytes per env-step instead of autograd's
-    activations. ``refresh()`` after an optimiser step re-packs the weights, the transposed ones included."""
+    activations. ``refresh()`` after an optimiser step re-packs the weights, the transposed ones included.
+
+    ``logits_and_value`` is the same pass behind autograd, for any loss written in torch: it refreshes by itself."""
 
     def __init__(self, env: VecEnv, policy: "Policy"):
         lib = _lib.load()
@@ -185,6 +188,42 @@ class PolicyTrainTC(PolicyTrunkTC):
             self.heads = (w, b)
         else:
             self.heads[0].copy_(w); self.heads[1].copy_(b)
+        self._packed_versions = self._versions()
+
+    def _versions(self) -> tuple:
+        """The identity and version counter of every parameter: any in-place change (an optimiser step, a load) moves one."""
+        return tuple((id(p), p._version) for p in self.policy.parameters())
+
+    def logits_and_value(self, features: torch.Tensor, counters: torch.Tensor, rows: Optional[torch.Tensor] = None,
+                         noise_scale: float = 0.01, slope: float = 0.01):
+        """The policy's outputs for a list of recorded rows, differentiable with respect to ``policy.parameters()``:
+        ``(logits f32[M, A], value f32[M])``, the action head's output before the softmax and the value head's, for the
+        rows ``rows`` int32[M] (indices t * N + n into the T * N rows of ``features`` u8[T, N, 28], each under its step's
+        counter ``counters`` int64[T]; ``None``: all T * N rows in order). Write any loss of them in torch and call
+        ``.backward()``: the gradient comes from one tcgen05 pass that recomputes the forward from the feature bytes
+        (``wab_policy_backward_logits``), so only the outputs are kept per row, never the activations.
+
+        The forward is ``wab_policy_evaluate``: under the weights a rollout used, ``value`` equals what ``forward_sample``
+        returned bit for bit. A listed entry outside [0, T * N) gives NaN and no gradient; a repeated one counts once per
+        occurrence. The packed weights are refreshed when a parameter changed since the last pack (no ``refresh()`` after
+        ``optimizer.step()``), and an in-place change between the forward and the backward raises autograd's version
+        error. Nothing synchronises with the host. Double backward is not supported."""
+        if features.dim() != 3 or features.shape[2] != 28 or features.dtype != torch.uint8 or not features.is_contiguous():
+            raise ValueError("features must be a contiguous uint8 [T, N, 28] tensor")
+        T, N = features.shape[:2]
+        if counters.dtype != torch.int64 or counters.numel() != T or not counters.is_contiguous():
+            raise ValueError("counters must be a contiguous int64 tensor of T elements")
+        if rows is not None and (rows.dtype != torch.int32 or rows.dim() != 1 or not rows.is_contiguous()):
+            raise ValueError("rows must be a contiguous int32 [M] tensor")
+        for name, t in (("features", features), ("counters", counters), ("rows", rows)):
+            if t is not None and t.device != self.env.device:
+                raise ValueError("%s must be on the environment's device" % name)
+        params = list(self.policy.parameters())
+        if any(p.dtype != torch.float32 or p.device != self.env.device for p in params):
+            raise ValueError("the policy's parameters must be float32 on the environment's device")
+        if self._packed_versions != self._versions():
+            self.refresh()
+        return _LogitsAndValue.apply(self, features, counters, rows, float(noise_scale), float(slope), *params)
 
     def backward(self, features: torch.Tensor, counters: torch.Tensor, actions: torch.Tensor, g_logp: torch.Tensor,
                  g_value: torch.Tensor, out: Optional[torch.Tensor] = None, rows: Optional[torch.Tensor] = None,
@@ -275,6 +314,53 @@ class PolicyTrainTC(PolicyTrunkTC):
         _lib.check(self.lib.wab_policy_grad_sum_ranks(_ptr(rank_grads), rank_grads.shape[0], self.n_params, _ptr(out),
                                                       self._stream()))
         return out
+
+
+class _LogitsAndValue(torch.autograd.Function):
+    """``PolicyTrainTC.logits_and_value``: forward ``wab_policy_evaluate``, backward ``wab_policy_backward_logits`` into a
+    fresh flat gradient per call (a buffer reused across calls would alias an accumulated ``.grad``), returned as views in
+    ``parameters_to_vector`` order. The parameters are inputs, saved with the recorded rows, so that autograd checks their
+    versions."""
+
+    @staticmethod
+    def forward(ctx, tc, features, counters, rows, noise_scale, slope, *params):
+        T, N = features.shape[:2]
+        M = T * N if rows is None else rows.numel()
+        w, b = tc.heads
+        A = w.shape[0] - 1
+        logits = torch.empty(M, A, dtype=torch.float32, device=features.device)
+        value = torch.empty(M, dtype=torch.float32, device=features.device)
+        if M > 0:
+            _lib.check(tc.lib.wab_policy_evaluate(
+                tc.env._h, _ptr(features), T, N, _ptr(counters), _ptr(rows), M, _ptr(tc.packed), _ptr(tc.bias),
+                _ptr(tc.packed2), _ptr(tc.bias2), 150, _ptr(tc.packed3), _ptr(tc.bias3), _ptr(w), _ptr(b), A,
+                noise_scale, slope, -4.0, 4.0, _ptr(tc.scratch), tc.scratch.numel(), _ptr(logits), _ptr(value), tc._stream()))
+        ctx.save_for_backward(features, counters, rows, *params)
+        ctx.tc, ctx.noise_scale, ctx.slope, ctx.n_rows = tc, noise_scale, slope, M
+        return logits, value
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_logits, g_value):
+        features, counters, rows, *params = ctx.saved_tensors      # raises if a parameter changed in place since the forward
+        tc, M = ctx.tc, ctx.n_rows
+        T, N = features.shape[:2]
+        grad = torch.zeros(tc.n_params, dtype=torch.float32, device=features.device) if M == 0 else \
+            torch.empty(tc.n_params, dtype=torch.float32, device=features.device)
+        if M > 0:
+            g_logits = g_logits.float().contiguous()
+            g_value = g_value.float().contiguous()
+            w, b = tc.heads
+            _lib.check(tc.lib.wab_policy_backward_logits(
+                tc.env._h, _ptr(features), T, N, _ptr(counters), _ptr(rows), M, _ptr(g_logits), _ptr(g_value),
+                _ptr(tc.packed), _ptr(tc.bias), _ptr(tc.packed2), _ptr(tc.bias2), 150, _ptr(tc.packed3), _ptr(tc.bias3),
+                _ptr(tc.packed2t), _ptr(tc.packed3t), _ptr(w), _ptr(b), w.shape[0] - 1, ctx.noise_scale, ctx.slope, -4.0, 4.0,
+                _ptr(tc.scratch), tc.scratch.numel(), _ptr(grad), tc._stream()))
+        out, off = [], 0
+        for i, p in enumerate(params):
+            out.append(grad[off:off + p.numel()].view_as(p) if ctx.needs_input_grad[6 + i] else None)
+            off += p.numel()
+        return (None, None, None, None, None, None, *out)
 
 
 class Rollout:
