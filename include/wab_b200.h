@@ -245,7 +245,7 @@ int wab_vec_flat_dim(const WabVec *h);
  * fresh noise on every replay.
  *
  * Keying contract of the policy entry points: every one that takes a WabVec handle (wab_vec_flatten_features_noisy,
- * wab_policy_affine1, wab_policy_trunk, wab_policy_forward, wab_policy_backward, wab_policy_ppo_backward,
+ * wab_policy_affine1, wab_policy_trunk, wab_policy_forward, wab_policy_act, wab_policy_backward, wab_policy_ppo_backward,
  * wab_policy_evaluate, wab_policy_backward_logits) keys its noise and its action samples by the global env id env_id_base + row (the row within its step for the backward passes), so
  * a shard [first, first + count) draws exactly what the unsharded batch draws for rows first .. first + count - 1;
  * outputs stay indexed by the local row. The two handle-less calls, wab_sample_categorical and wab_policy_tail, know no
@@ -306,6 +306,19 @@ int wab_policy_forward(WabVec *h, const uint8_t *d_features, int64_t n_rows, con
                        float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi, uint64_t sample_seed,
                        const uint64_t *d_counter, uint8_t *d_actions, float *d_value, float *d_probs, float *d_logp,
                        float *d_z3, void *stream);
+
+/* The greedy (deterministic) action of the same network, for evaluation: wab_policy_forward without sample_seed. The
+ * trunk, clamp, heads and softmax are wab_policy_forward's, and so is the keyed input noise (noise_scale = 0 turns it
+ * off); d_actions[row] is the first index of the largest logit (the action head's output before the softmax, bias
+ * included), so ties go to the lowest index, as torch.argmax does for finite logits. No action sample is drawn.
+ * d_value and d_probs are bit-equal to wab_policy_forward's for the same inputs; d_logp is log(p) of the greedy action,
+ * bit-equal to wab_policy_forward's wherever the sampled action is the greedy one. Arguments, NULL rules, alignment and
+ * return codes as for wab_policy_forward. */
+int wab_policy_act(WabVec *h, const uint8_t *d_features, int64_t n_rows, const void *d_packed1, const float *d_bias1,
+                   const void *d_packed2, const float *d_bias2, int32_t hidden2, const void *d_packed3,
+                   const float *d_bias3, const float *d_w_heads, const float *d_b_heads, int32_t n_actions,
+                   float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi, const uint64_t *d_counter,
+                   uint8_t *d_actions, float *d_value, float *d_probs, float *d_logp, float *d_z3, void *stream);
 
 /* The backward pass of Policy.forward for training (actor_critic.py:128-169) on the tensor cores. For T = n_steps steps of
  * N = n_envs environments, rows t N + n in step-major order:

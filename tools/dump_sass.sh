@@ -11,7 +11,7 @@ txt = open('/tmp/wab_all.sass').read()
 for f in re.split(r'\n\s*Function : ', txt)[1:]:
     name = f.split('\n', 1)[0]
     for key, out in (('wab_step_kernelILb0ELi1ELi24E', 'step_lpe1'), ('wab_step_kernelILb0ELi16E', 'step_lpe16'), ('wab2_turn_kernel', 'v2_turn'),
-                     ('wab_step_pipe_kernelILb0ELi8E', 'step_pipe_lpe8'), ('wab_affine1_tc_kernelILi2E', 'policy_forward_tcgen05'),
+                     ('wab_step_pipe_kernelILb0ELi8E', 'step_pipe_lpe8'), ('wab_affine1_tc_kernelILi2E', 'policy_forward_tcgen05'), ('wab_affine1_tc_kernelILi3E', 'policy_act_tcgen05'),
                      ('wab2_grid_turn_kernelILb1ELb0E', 'v2_grid_turn'), ('wab_policy_bwd_kernel', 'policy_backward_tcgen05'),
                      ('wab_policy_ppo_bwd_kernel', 'policy_ppo_backward_tcgen05'), ('wab_policy_eval_kernel', 'policy_eval_tcgen05'),
                      ('wab_policy_logits_bwd_kernel', 'policy_logits_backward_tcgen05')):

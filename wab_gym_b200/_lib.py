@@ -19,7 +19,7 @@ EXPORTS = [
     "wab_vec_destroy", "wab_philox_device", "wab_vec_bind_features", "wab_pragmatic_features",
     "wab_vec_flatten_features", "wab_vec_flatten_features_noisy", "wab_sample_categorical", "wab_policy_tail", "wab_vec_enable_ego", "wab_vec_ego_proximities", "wab_vec_flat_dim", "wab_vec_host_block_layout", "wab_vec_step_host_packed", "wab_vec_forget_host_buffers",
     "wab_vec_state_record_bytes", "wab_vec_state_fingerprint", "wab_vec_save_state", "wab_vec_load_state", "wab_vec_set_stats",
-    "wab_policy_affine1_packed_bytes", "wab_policy_affine1_prepare", "wab_policy_affine1", "wab_policy_linear_packed_bytes", "wab_policy_linear_prepare", "wab_policy_trunk", "wab_policy_forward", "wab_policy_backward_scratch_bytes", "wab_policy_backward", "wab_policy_ppo_backward", "wab_policy_evaluate", "wab_policy_backward_logits", "wab_policy_backward_grad_f64", "wab_policy_grad_sum_ranks", "wab2_create", "wab2_kernel_kind", "wab2_output_layout", "wab2_reset", "wab2_turn", "wab2_export_state", "wab2_import_state", "wab2_destroy", "wab_last_error", "wab_abi_version",
+    "wab_policy_affine1_packed_bytes", "wab_policy_affine1_prepare", "wab_policy_affine1", "wab_policy_linear_packed_bytes", "wab_policy_linear_prepare", "wab_policy_trunk", "wab_policy_forward", "wab_policy_act", "wab_policy_backward_scratch_bytes", "wab_policy_backward", "wab_policy_ppo_backward", "wab_policy_evaluate", "wab_policy_backward_logits", "wab_policy_backward_grad_f64", "wab_policy_grad_sum_ranks", "wab2_create", "wab2_kernel_kind", "wab2_output_layout", "wab2_reset", "wab2_turn", "wab2_export_state", "wab2_import_state", "wab2_destroy", "wab_last_error", "wab_abi_version",
 ]
 
 
@@ -99,6 +99,8 @@ def load():
     L.wab_policy_trunk.argtypes = [vp, vp, i64, vp, vp, vp, vp, i32, vp, vp, ctypes.c_float, ctypes.c_float, vp, vp, vp]
     L.wab_policy_forward.argtypes = [vp, vp, i64, vp, vp, vp, vp, i32, vp, vp, vp, vp, i32, ctypes.c_float, ctypes.c_float,
                                      ctypes.c_float, ctypes.c_float, u64, vp, vp, vp, vp, vp, vp, vp]
+    L.wab_policy_act.argtypes = [vp, vp, i64, vp, vp, vp, vp, i32, vp, vp, vp, vp, i32, ctypes.c_float, ctypes.c_float,
+                                 ctypes.c_float, ctypes.c_float, vp, vp, vp, vp, vp, vp, vp]
     L.wab_policy_backward_scratch_bytes.argtypes = [vp]
     L.wab_policy_backward_scratch_bytes.restype = i64
     f32 = ctypes.c_float

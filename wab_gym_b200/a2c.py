@@ -47,7 +47,7 @@ import torch
 import torch.nn.functional as F
 
 from . import sharding
-from .policy import Policy, PolicyTrainTC
+from .policy import Policy, PolicyTrainTC, check_reference_network
 from .vec_env import VecEnv
 
 
@@ -178,12 +178,7 @@ class A2CTrainer:
 
     def _init_tensor_cores(self):
         env, p, T, N = self.env, self.policy, self.horizon, self.env.num_envs
-        if any(prm.dtype != torch.float32 for prm in p.parameters()):
-            raise ValueError("tensor_cores=True trains an fp32 policy")
-        shapes = [(m.in_features, m.out_features) for m in (p.affine1, p.affine2, p.affine3, p.value_head)]
-        if shapes != [(env.flat_dim, 128), (128, 150), (150, 128), (128, 1)] or p.action_head.in_features != 128 or \
-                not 1 <= p.action_head.out_features <= 8:
-            raise ValueError("tensor_cores=True is built for the reference's network: flat_dim -> 128 -> 150 -> 128 -> {A <= 8, 1}")
+        check_reference_network(p, env.flat_dim, "tensor_cores=True")
         self._tc = PolicyTrainTC(env, p)
         dev = env.device
         self.last_batch = {"features": torch.empty(T, N, 28, dtype=torch.uint8, device=dev),

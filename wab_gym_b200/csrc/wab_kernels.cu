@@ -1667,7 +1667,7 @@ int wab_policy_linear_prepare(const float* d_weight, int32_t n_out, int32_t n_in
 static int policy_trunk_launch(WabVec* h, const uint8_t* d_features, int64_t n_rows, const void* d_packed1, const float* d_bias1,
                                const void* d_packed2, const float* d_bias2, int32_t hidden2, const void* d_packed3, const float* d_bias3,
                                float noise_scale, float leaky_slope, const uint64_t* d_counter, float* d_z3, void* stream,
-                               const TrunkWeights* tail) {
+                               const TrunkWeights* tail, bool greedy = false) {
     if (!h || !d_features || !d_packed1 || !d_bias1 || !d_packed2 || !d_bias2 || !d_packed3 || !d_bias3 || (!d_z3 && !tail)) return fail(WAB_E_NULL, "null argument");
     if (hidden2 != 150) return fail(WAB_E_UNSUPPORTED, "wab_policy_trunk is built for the reference's trunk 128 -> 150 -> 128 (actor_critic.py:59-61)");
     if (n_rows <= 0) return WAB_OK;
@@ -1680,13 +1680,18 @@ static int policy_trunk_launch(WabVec* h, const uint8_t* d_features, int64_t n_r
     if (h->device < 64 && !attr_set[h->device]) {
         WAB_CUDA(cudaFuncSetAttribute(wab_affine1_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOTAL));
         WAB_CUDA(cudaFuncSetAttribute(wab_affine1_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOTAL));
+        WAB_CUDA(cudaFuncSetAttribute(wab_affine1_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOTAL));
         attr_set[h->device] = true;
     }
     TrunkWeights tw;
     if (tail) tw = *tail; else memset(&tw, 0, sizeof(tw));
     tw.w2 = reinterpret_cast<const uint4*>(d_packed2); tw.b2 = d_bias2; tw.w3 = reinterpret_cast<const uint4*>(d_packed3); tw.b3 = d_bias3; tw.n2 = hidden2;
     const unsigned grid = (unsigned)((n_rows + TC_TILE_M - 1) / TC_TILE_M);
-    if (tail)
+    if (tail && greedy)
+        wab_affine1_tc_kernel<3><<<grid, 256, TC_SMEM_TOTAL, (cudaStream_t)stream>>>(
+            h->P, d_features, n_rows, (int)h->cfg.food_obs_scale + 1, reinterpret_cast<const uint4*>(d_packed1), d_bias1, noise_scale,
+            leaky_slope, reinterpret_cast<const unsigned long long*>(d_counter), d_z3, tw);
+    else if (tail)
         wab_affine1_tc_kernel<2><<<grid, 256, TC_SMEM_TOTAL, (cudaStream_t)stream>>>(
             h->P, d_features, n_rows, (int)h->cfg.food_obs_scale + 1, reinterpret_cast<const uint4*>(d_packed1), d_bias1, noise_scale,
             leaky_slope, reinterpret_cast<const unsigned long long*>(d_counter), d_z3, tw);
@@ -1721,6 +1726,22 @@ int wab_policy_forward(WabVec* h, const uint8_t* d_features, int64_t n_rows, con
     tw.actions = d_actions; tw.value = d_value; tw.probs = d_probs; tw.logp = d_logp;
     return policy_trunk_launch(h, d_features, n_rows, d_packed1, d_bias1, d_packed2, d_bias2, hidden2, d_packed3, d_bias3, noise_scale,
                                leaky_slope, d_counter, d_z3, stream, &tw);
+}
+
+// wab_policy_forward's trunk and tail with the greedy action: the same checks, no sampling seed (MODE 3 reads no round keys)
+int wab_policy_act(WabVec* h, const uint8_t* d_features, int64_t n_rows, const void* d_packed1, const float* d_bias1,
+                   const void* d_packed2, const float* d_bias2, int32_t hidden2, const void* d_packed3, const float* d_bias3,
+                   const float* d_w_heads, const float* d_b_heads, int32_t n_actions, float noise_scale, float leaky_slope,
+                   float clamp_lo, float clamp_hi, const uint64_t* d_counter, uint8_t* d_actions, float* d_value,
+                   float* d_probs, float* d_logp, float* d_z3, void* stream) {
+    if (!d_w_heads || !d_b_heads || !d_actions) return fail(WAB_E_NULL, "null argument");
+    if (n_actions < 1 || n_actions > 8) return fail(WAB_E_CONFIG, "n_actions must be in [1, 8]");
+    TrunkWeights tw;
+    memset(&tw, 0, sizeof(tw));
+    tw.w_heads = d_w_heads; tw.b_heads = d_b_heads; tw.n_actions = n_actions; tw.clamp_lo = clamp_lo; tw.clamp_hi = clamp_hi;
+    tw.actions = d_actions; tw.value = d_value; tw.probs = d_probs; tw.logp = d_logp;
+    return policy_trunk_launch(h, d_features, n_rows, d_packed1, d_bias1, d_packed2, d_bias2, hidden2, d_packed3, d_bias3, noise_scale,
+                               leaky_slope, d_counter, d_z3, stream, &tw, true);
 }
 
 int wab_policy_tail(const float* d_z3, int32_t hidden, const float* d_w_heads, const float* d_b_heads, int64_t n_rows,

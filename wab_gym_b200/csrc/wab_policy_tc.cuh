@@ -162,7 +162,8 @@ struct TrunkWeights {
     int n_actions; float clamp_lo, clamp_hi;
     uint8_t* actions; float* value; float* probs; float* logp;
 };
-// MODE 0: first layer only; 1: the trunk (out = z3); 2: trunk + tail (clamp, both heads, softmax, Categorical sample; out = z3 or null)
+// MODE 0: first layer only; 1: the trunk (out = z3); 2: trunk + tail (clamp, both heads, softmax, Categorical sample; out = z3 or null);
+// 3: MODE 2 with the greedy action (the first index of the largest logit) instead of the sample: no Philox call, the round keys unread
 template <int MODE>
 __global__ void __launch_bounds__(256, 2)
 wab_affine1_tc_kernel(const __grid_constant__ Params P, const uint8_t* __restrict__ features, int64_t rows, int food_dim,
@@ -438,9 +439,10 @@ wab_affine1_tc_kernel(const __grid_constant__ Params P, const uint8_t* __restric
 #pragma unroll
             for (int i = 0; i < 16; ++i) dst[i] = make_float4(z3[4 * i], z3[4 * i + 1], z3[4 * i + 2], z3[4 * i + 3]);
         }
-        if (MODE == 2) {
+        if (MODE >= 2) {
             // ---- the tail: x = clamp(leaky_relu(z3)); the A + 1 head rows as two 64-term partial sums per row (the two threads
             // of a row meet in shared memory — the operand area is free now); softmax; inverse-CDF sample on one keyed uniform
+            // (MODE 2) or the greedy action (MODE 3)
             // head weights transposed and zero-padded to [128][12]: the 9 weights of an input are three 16-byte broadcast loads
             float* wsm = reinterpret_cast<float*>(tc_smem);               // [128][12]
             float* partial = wsm + 12 * 128;                              // [128 rows][2 halves][9]
@@ -477,24 +479,33 @@ wab_affine1_tc_kernel(const __grid_constant__ Params P, const uint8_t* __restric
                 float ex[8], tot = 0.f;
 #pragma unroll
                 for (int o = 0; o < 8; ++o) { ex[o] = o < A ? expf(acc[o] - mx) : 0.f; tot += ex[o]; }   // F.softmax, :96
-                const uint64_t g = P.env_id_base + (uint64_t)row;        // the sampling key: the row's global env id
-                uint32_t c0 = (uint32_t)(g >> 2), c1 = (uint32_t)(g >> 34), c2 = (uint32_t)ctr, c3 = (uint32_t)(ctr >> 32) ^ 0x53414D50u;
-#pragma unroll
-                for (int rd = 0; rd < 10; ++rd) {                         // Philox4x32-10 under the sampling seed's round keys
-                    const uint64_t p0 = (uint64_t)PHILOX_M0 * c0, p1 = (uint64_t)PHILOX_M1 * c2;
-                    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ tw.rk0[rd], n2 = (uint32_t)(p0 >> 32) ^ c3 ^ tw.rk1[rd];
-                    c1 = (uint32_t)p1; c3 = (uint32_t)p0; c0 = n0; c2 = n2;
-                }
-                const uint32_t wd[4] = {c0, c1, c2, c3};
-                const float u = (float)(pick4(wd, (uint32_t)g & 3u) >> 8) * (1.0f / 16777216.0f);
-                const float target = u * tot;
-                float cum = 0.f, p_pick = 0.f;
+                float p_pick = 0.f;
                 int pick = A - 1;
-                bool found = false;
+                if constexpr (MODE == 2) {
+                    const uint64_t g = P.env_id_base + (uint64_t)row;    // the sampling key: the row's global env id
+                    uint32_t c0 = (uint32_t)(g >> 2), c1 = (uint32_t)(g >> 34), c2 = (uint32_t)ctr, c3 = (uint32_t)(ctr >> 32) ^ 0x53414D50u;
 #pragma unroll
-                for (int o = 0; o < 8; ++o) {                             // smallest a with target < e[0] + ... + e[a]
-                    cum += ex[o];
-                    if (!found && o < A && target < cum) { pick = o; found = true; }
+                    for (int rd = 0; rd < 10; ++rd) {                     // Philox4x32-10 under the sampling seed's round keys
+                        const uint64_t p0 = (uint64_t)PHILOX_M0 * c0, p1 = (uint64_t)PHILOX_M1 * c2;
+                        const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ tw.rk0[rd], n2 = (uint32_t)(p0 >> 32) ^ c3 ^ tw.rk1[rd];
+                        c1 = (uint32_t)p1; c3 = (uint32_t)p0; c0 = n0; c2 = n2;
+                    }
+                    const uint32_t wd[4] = {c0, c1, c2, c3};
+                    const float u = (float)(pick4(wd, (uint32_t)g & 3u) >> 8) * (1.0f / 16777216.0f);
+                    const float target = u * tot;
+                    float cum = 0.f;
+                    bool found = false;
+#pragma unroll
+                    for (int o = 0; o < 8; ++o) {                         // smallest a with target < e[0] + ... + e[a]
+                        cum += ex[o];
+                        if (!found && o < A && target < cum) { pick = o; found = true; }
+                    }
+                } else {
+                    // argmax over the LOGITS (two logits may round to one exponential); strict > keeps the lowest index on a tie
+                    float best = acc[0];
+                    pick = 0;
+#pragma unroll
+                    for (int o = 1; o < 8; ++o) if (o < A && acc[o] > best) { best = acc[o]; pick = o; }
                 }
 #pragma unroll
                 for (int o = 0; o < 8; ++o) if (o == pick) p_pick = ex[o];

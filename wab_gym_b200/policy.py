@@ -60,6 +60,18 @@ def policy_tail(policy: "Policy", z3: torch.Tensor, heads: tuple, actions: torch
     return actions
 
 
+def check_reference_network(policy: "Policy", flat_dim: int, who: str) -> None:
+    """What the tensor-core policy kernels serve: the reference's network (``flat_dim -> 128 -> 150 -> 128 -> {A <= 8, 1}``)
+    in fp32. Raises ``ValueError`` naming ``who`` otherwise; reads shapes and dtypes only."""
+    p = policy
+    if any(prm.dtype != torch.float32 for prm in p.parameters()):
+        raise ValueError("%s needs an fp32 policy" % who)
+    shapes = [(m.in_features, m.out_features) for m in (p.affine1, p.affine2, p.affine3, p.value_head)]
+    if shapes != [(flat_dim, 128), (128, 150), (150, 128), (128, 1)] or p.action_head.in_features != 128 or \
+            not 1 <= p.action_head.out_features <= 8:
+        raise ValueError("%s is built for the reference's network: flat_dim -> 128 -> 150 -> 128 -> {A <= 8, 1}" % who)
+
+
 def stacked_heads(policy: "Policy") -> tuple:
     """(action_head.weight stacked on value_head.weight f32[A + 1, 128], the two biases f32[A + 1]) — refresh after an
     optimiser step."""
@@ -151,6 +163,22 @@ class PolicyTrunkTC(Affine1TC):
                                                _ptr(w), _ptr(b), w.shape[0] - 1, float(noise_scale), float(slope), -4.0, 4.0,
                                                int(seed) & (2 ** 64 - 1), _ptr(counter), _ptr(actions), _ptr(value), _ptr(probs),
                                                _ptr(logp), _ptr(z3), self._stream()))
+        return actions
+
+    def forward_greedy(self, features: torch.Tensor, heads: tuple, actions: torch.Tensor, value: Optional[torch.Tensor] = None,
+                       probs: Optional[torch.Tensor] = None, logp: Optional[torch.Tensor] = None, noise_scale: float = 0.01,
+                       counter: Optional[torch.Tensor] = None, z3: Optional[torch.Tensor] = None,
+                       slope: float = 0.01) -> torch.Tensor:
+        """``forward_sample`` with the deterministic action in place of the sample, in ONE launch (``wab_policy_act``):
+        ``actions`` u8[N] = the first index of the largest logit, ``torch.argmax`` of the action head's output. ``value``
+        and ``probs`` are ``forward_sample``'s bit for bit, ``logp`` is the log-probability of the greedy action. The input
+        noise is unchanged (``noise_scale=0``: the argmax of the bare network)."""
+        w, b = heads
+        _lib.check(self.lib.wab_policy_act(self.env._h, _ptr(features), features.shape[0], _ptr(self.packed), _ptr(self.bias),
+                                           _ptr(self.packed2), _ptr(self.bias2), 150, _ptr(self.packed3), _ptr(self.bias3),
+                                           _ptr(w), _ptr(b), w.shape[0] - 1, float(noise_scale), float(slope), -4.0, 4.0,
+                                           _ptr(counter), _ptr(actions), _ptr(value), _ptr(probs), _ptr(logp), _ptr(z3),
+                                           self._stream()))
         return actions
 
 
