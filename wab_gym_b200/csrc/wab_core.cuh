@@ -332,11 +332,55 @@ WAB_HD void spread11(uint32_t v, uint32_t t[4]) {
     t[3] = ((((v >> 9) & 3u) * 0x00100401u) & 0x00400801u) << 3;
 }
 
+// The line of 11 cells a move by (dx, dy) (one of them non-zero) to (E.x, E.y) reveals, and the 6 bush blocks that hold it:
+// slide_window's geometry and block draws for step_draws (slide_window keeps its own copy so that the kernels that do
+// not make their draws first compile to the same code as before; test_two_warp_pipeline_* compare the two).
+struct SlideLine {
+    bool along_y;                 // new row (fixed x) or new column (fixed y)
+    int32_t fixed, vmax, vb0, top;
+    uint32_t fb, sel0, sel1;
+};
+WAB_HD SlideLine slide_line(const Env& E, int32_t dx, int32_t dy) {
+    SlideLine L;
+    L.along_y = (dx != 0);
+    L.fixed = L.along_y ? E.x + HALF * dx : E.y + HALF * dy;
+    L.vmax = (L.along_y ? E.y : E.x) + HALF;              // cell g of the line has coordinate vmax - g
+    L.vb0 = (L.vmax - 10) >> 1;
+    L.fb = (uint32_t)L.fixed & 1u;
+    // The 6 blocks hold 12 cells, g + 1 = top, top - 1, ..., top - 11 with top = 11 or 12: bit g + 1 of `acc`.
+    L.top = L.vmax - 2 * L.vb0 + 1;
+    // a line along y meets word e (cell parity e) at half fb; a line along x meets word fb at half e
+    L.sel0 = half_sel(L.along_y ? L.fb : 0u); L.sel1 = half_sel(L.along_y ? L.fb : 1u);
+    return L;
+}
+// Block b (0..5) of the line: its two cells' hits (high half-word above the threshold's) at bits top - 2b and
+// top - 2b - 1 of `acc`, and whether either high half-word ties with the threshold's.
+WAB_HD void slide_block(const Params& P, const Env& E, const SlideLine& L, int b, uint32_t& acc, uint32_t& tie) {
+    uint32_t p[2];
+    const uint32_t t_hi = P.thr_bush1 >> 16;
+    const uint32_t c0 = (L.along_y ? pack_xy(L.fixed >> 1, L.vb0 + b) : pack_xy(L.vb0 + b, L.fixed >> 1)) ^ E.bk_a;
+    philox2(P, c0, E.bk_b, p);
+    const uint32_t h0 = half_of((L.along_y || !L.fb) ? p[0] : p[1], L.sel0);
+    const uint32_t h1 = half_of((L.along_y || L.fb) ? p[1] : p[0], L.sel1);
+    const uint32_t bit = 1u << (L.top - 2 * b);
+    acc |= (h0 > t_hi ? bit : 0u) | (h1 > t_hi ? (bit >> 1) : 0u);
+    tie |= (h0 == t_hi ? 1u : 0u) | (h1 == t_hi ? 1u : 0u);
+}
+
+// The keyed draws of one step that depend only on the env's state before the step and its action (env_step with DRAWN):
+// this lane's slide blocks and the spawn draw.
+struct StepDraws {
+    uint32_t acc, tie;   // slide_block over this lane's blocks b = sub, sub + LPE, ... < 6
+    uint64_t spawn;      // binomial_draw of SITE_SPAWN at the step's turn
+};
+
 // Slide the window after the ostrich moved by (dx, dy) (one of them non-zero) to (E.x, E.y) and
 // reveal the 11 new cells: generate_bushes, wab_env.py:613-629, for cells without a record; cells
 // seen before get the same draw (keys do not depend on the turn) minus what was eaten.
-template <int LPE>
-WAB_HD void slide_window(const Params& P, Env& E, const Slots& S, int32_t dx, int32_t dy, const Coop<LPE>& coop) {
+// DRAWN: this lane's block draws come in `D` (made before the step's rules) instead of being made here.
+template <int LPE, bool DRAWN = false>
+WAB_HD void slide_window(const Params& P, Env& E, const Slots& S, int32_t dx, int32_t dy, const Coop<LPE>& coop,
+                         const StepDraws* D = nullptr) {
     // drop the column that would wrap into the neighbouring row, then shift by 11*dx + dy
     if (dy > 0) {
         E.m[0] &= ~ColMask<10, 0>::v; E.m[1] &= ~ColMask<10, 1>::v; E.m[2] &= ~ColMask<10, 2>::v; E.m[3] &= ~ColMask<10, 3>::v;
@@ -361,18 +405,22 @@ WAB_HD void slide_window(const Params& P, Env& E, const Slots& S, int32_t dx, in
     const uint32_t sel0 = half_sel(along_y ? fb : 0u), sel1 = half_sel(along_y ? fb : 1u);
     uint32_t acc = 0, tie = 0;
     if (P.n_bush_thr > 0) {
+        if (DRAWN) {
+            acc = D->acc; tie = D->tie;
+        } else {
 #if defined(__CUDA_ARCH__)
 #pragma unroll kSlideUnroll
 #endif
-        for (int b = (int)coop.sub; b < 6; b += LPE) {
-            uint32_t p[2];
-            const uint32_t c0 = (along_y ? pack_xy(fixed >> 1, vb0 + b) : pack_xy(vb0 + b, fixed >> 1)) ^ E.bk_a;
-            philox2(P, c0, E.bk_b, p);
-            const uint32_t h0 = half_of((along_y || !fb) ? p[0] : p[1], sel0);
-            const uint32_t h1 = half_of((along_y || fb) ? p[1] : p[0], sel1);
-            const uint32_t bit = 1u << (top - 2 * b);
-            acc |= (h0 > t_hi ? bit : 0u) | (h1 > t_hi ? (bit >> 1) : 0u);
-            tie |= (h0 == t_hi ? 1u : 0u) | (h1 == t_hi ? 1u : 0u);
+            for (int b = (int)coop.sub; b < 6; b += LPE) {   // slide_block, written out
+                uint32_t p[2];
+                const uint32_t c0 = (along_y ? pack_xy(fixed >> 1, vb0 + b) : pack_xy(vb0 + b, fixed >> 1)) ^ E.bk_a;
+                philox2(P, c0, E.bk_b, p);
+                const uint32_t h0 = half_of((along_y || !fb) ? p[0] : p[1], sel0);
+                const uint32_t h1 = half_of((along_y || fb) ? p[1] : p[0], sel1);
+                const uint32_t bit = 1u << (top - 2 * b);
+                acc |= (h0 > t_hi ? bit : 0u) | (h1 > t_hi ? (bit >> 1) : 0u);
+                tie |= (h0 == t_hi ? 1u : 0u) | (h1 == t_hi ? 1u : 0u);
+            }
         }
         if (tie) {                 // 2^-15 per block: settle this lane's cells on their full 32-bit draws
             acc = 0;
@@ -445,9 +493,33 @@ WAB_HD void wolf_plane(const Env& E, const Slots& S, uint32_t wm[4]) {
     }
 }
 
+// The draws of StepDraws for the step whose action has just moved the ostrich to (E.x, E.y) and advanced E.turn.
+// Straight-line code on every lane — lanes without a block (sub >= 6) draw a harmless duplicate and mask it out — so the
+// independent Philox chains interleave with each other instead of running one after another. (The despawn draws were
+// made here too, wolf k = sub, and measured 6 % slower: they cost a Philox4x32 on every step, wolves or not.)
+template <int LPE>
+WAB_HD StepDraws step_draws(const Params& P, const Env& E, int32_t dx, int32_t dy, const Coop<LPE>& coop) {
+    StepDraws D;
+    D.spawn = binomial_draw(P, E.env_id, E.episode, SITE_SPAWN, E.turn);
+    D.acc = 0u; D.tie = 0u;
+    const SlideLine L = slide_line(E, dx, dy);
+    constexpr int NB = (6 + LPE - 1) / LPE;
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for (int j = 0; j < NB; ++j) {
+        const int b = (int)coop.sub + j * LPE;
+        uint32_t acc = 0u, tie = 0u;
+        slide_block(P, E, L, b < 6 ? b : 5, acc, tie);
+        D.acc |= b < 6 ? acc : 0u; D.tie |= b < 6 ? tie : 0u;
+    }
+    return D;
+}
+
 // One step of one environment: wab_env.py:250-342 up to (not including) auto-reset and the
-// observation stores. `F64` selects the reference's fp64 food arithmetic.
-template <bool F64, int LPE>
+// observation stores. `F64` selects the reference's fp64 food arithmetic. DRAWN makes the step's
+// keyed draws first (step_draws) and hands them to the rules; the results are the same.
+template <bool F64, int LPE, bool DRAWN = false>
 WAB_HD void env_step(const Params& P, Env& E, const Slots& S, uint32_t action, StepOut& O, const Coop<LPE>& coop) {
     // ---- :251-258 action
     O.bad_action = (action >= (uint32_t)P.n_actions) ? 1u : 0u;
@@ -458,9 +530,11 @@ WAB_HD void env_step(const Params& P, Env& E, const Slots& S, uint32_t action, S
     E.x += dx; E.y += dy;                          // :255-256
     if (nrole >= 0) E.role = (uint32_t)nrole;      // :257-258
     O.overflow = 0;
+    StepDraws D;
+    if (DRAWN) D = step_draws<LPE>(P, E, dx, dy, coop);
 
     // ---- :259 generate_bushes for the newly visible line
-    if (dx != 0 || dy != 0) slide_window<LPE>(P, E, S, dx, dy, coop);
+    if (dx != 0 || dy != 0) slide_window<LPE, DRAWN>(P, E, S, dx, dy, coop, &D);
 
     // ---- :262-264 despawn (keep iff U > chance). rank = ordinal among earlier wolves on the cell.
     if (E.nw) {
@@ -561,7 +635,7 @@ WAB_HD void env_step(const Params& P, Env& E, const Slots& S, uint32_t action, S
 
     // ---- :325-326 spawn_wolves on the 48 ring cells around the moved ostrich: one binomial-first draw
     if (P.wolves) {
-        const uint64_t v = binomial_draw(P, E.env_id, E.episode, SITE_SPAWN, E.turn);
+        const uint64_t v = DRAWN ? D.spawn : binomial_draw(P, E.env_id, E.episode, SITE_SPAWN, E.turn);
         if (v >= P.spawn_cdf[0]) {                 // rare (2.4 % of steps): at least one wolf appears
             uint32_t chosen[4];
             binomial_choose(P, E.env_id, E.episode, SITE_SPAWN, E.turn, RING, v, chosen);

@@ -420,11 +420,12 @@ wab_step_kernel(const __grid_constant__ Params P, const StatePtrs st, const uint
 // ---- the multi-step kernel of the lanes-per-env geometries as a two-warp pipeline --------------------------------------
 // A small batch is bound by the length of one step's dependent instruction chain, and a third of that chain is not rules
 // at all: composing the 363-bit strings, expanding them to bytes, the 16-byte stores and the scalar outputs. Here a CTA is
-// one PAIR of warps that owns EPW = 32 / LPE envs: warp 0 runs the rules (exactly the code of wab_step_kernel) and parks
+// one PAIR of warps that owns EPW = 32 / LPE envs: warp 0 runs the rules (wab_step_kernel's, with each step's keyed
+// draws made first as independent chains: step_draws in wab_core.cuh) and parks
 // each step's planes and scalars in a ring of shared-memory slots; warp 1 publishes them — bit stream, byte expansion,
 // stores, scalars, features — while warp 0 is already on the next steps. The two meet only at mbarriers in shared memory
 // (one "full" and one "empty" barrier per ring slot; an arrive never blocks, a wait spins on the barrier's phase parity).
-// Results are identical to wab_step_kernel's (same functions in the same order per env); WAB_PIPE=0 selects that kernel.
+// Results are identical to wab_step_kernel's (the same draws and rules per env); WAB_PIPE=0 selects that kernel.
 template <int LPE> struct PipeGeo {
     static constexpr int EPW = 32 / LPE;
     static constexpr int DEPTH = 4;                        // ring slots, each with a full and an empty mbarrier
@@ -506,7 +507,7 @@ wab_step_pipe_kernel(const __grid_constant__ Params P, const StatePtrs st, const
             ap += n;
             if (c.active && t + 1 < n_steps) a_next = *ap;
             if (c.active) {
-                env_step<F64, LPE>(P, E, S, a, O, coop);
+                env_step<F64, LPE, true>(P, E, S, a, O, coop);
                 if (st.hist && c.writer && E.turn < (uint32_t)st.hist_len) st.hist[(int64_t)E.turn * n + c.idx] = pack_xy(E.x, E.y);
                 need_reset = O.done && P.auto_reset;
                 acc_outcome += 1ull << (16u * O.outcome);
