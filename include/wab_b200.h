@@ -246,7 +246,7 @@ int wab_vec_flat_dim(const WabVec *h);
  *
  * Keying contract of the policy entry points: every one that takes a WabVec handle (wab_vec_flatten_features_noisy,
  * wab_policy_affine1, wab_policy_trunk, wab_policy_forward, wab_policy_act, wab_policy_backward, wab_policy_ppo_backward,
- * wab_policy_evaluate, wab_policy_backward_logits) keys its noise and its action samples by the global env id env_id_base + row (the row within its step for the backward passes), so
+ * wab_policy_evaluate, wab_policy_backward_logits and the population calls) keys its noise and its action samples by the global env id env_id_base + row (the row within its step for the backward passes), so
  * a shard [first, first + count) draws exactly what the unsharded batch draws for rows first .. first + count - 1;
  * outputs stay indexed by the local row. The two handle-less calls, wab_sample_categorical and wab_policy_tail, know no
  * shard and key by the local row. */
@@ -375,6 +375,53 @@ int wab_policy_ppo_backward(WabVec *h, const uint8_t *d_features, int64_t n_step
                             float policy_weight, float value_weight, float entropy_weight, void *d_scratch,
                             int64_t scratch_bytes, float *d_grad, float *d_logp, float *d_value, float *d_entropy,
                             void *stream);
+
+/* A population of P = n_members policies of the reference's network, 1 <= P <= 64, trained side by side on one handle:
+ * member m owns rows [m n, (m + 1) n) of every step, n = member_rows (forward) or n_envs / P (backward), a positive
+ * multiple of 128 (a tile of the kernels never straddles two members). Member m's weights are stacked at fixed strides:
+ * d_packed1 [P][wab_policy_affine1_packed_bytes()], d_packed2 / d_packed3 / d_packed2t / d_packed3t
+ * [P][wab_policy_linear_packed_bytes(..)] of the single-policy layouts, d_bias1 f32[P][128], d_bias2 f32[P][150], d_bias3
+ * f32[P][128], d_w_heads f32[P][A + 1][128], d_b_heads f32[P][A + 1]. Every draw is keyed as for one policy (global env id
+ * env_id_base + row), so with env_id_base = 0 member m's outputs equal, bit for bit, those of the single-policy call with
+ * member m's weights on a handle whose env_id_base is m n.
+ *
+ * wab_policy_forward_population: wab_policy_forward over P n rows, each row under its member's weights. Arguments, NULL
+ * rules and alignment as for wab_policy_forward; WAB_E_CONFIG for P outside [1, 64] or member_rows not a positive
+ * multiple of 128, otherwise as wab_policy_forward.
+ *
+ * wab_policy_ppo_backward_population: wab_policy_ppo_backward for every member in one launch of P x (the single-policy
+ * grid) CTAs. d_rows int32[P][list_len] holds each member's row list as GLOBAL rows t N + n (N = n_envs), d_counts
+ * int64[P] the count of each (read on the device, clamped to [0, min(T N, list_len)]); an entry outside [0, T N) or whose
+ * env is not in the member's block contributes nothing. h_coefs f32[P][4] (host memory, read during the call):
+ * clip_eps, policy_weight, value_weight, entropy_weight of each member, validated as wab_policy_ppo_backward's scalars.
+ * d_logp_old, d_advantage, d_target and the optional d_logp, d_value, d_entropy are f32[T N], indexed by global row.
+ * Member m's tiles go to its CTAs in the order a single-policy launch uses, so row m of d_grad f32[P][stride], stride =
+ * wab_policy_population_grad_stride(h, A) (the parameter count rounded up to 64 floats: with d_grad 256-byte aligned,
+ * each member's row is too), equals member m's wab_policy_ppo_backward gradient bit for bit. d_scratch: at least
+ * wab_policy_backward_population_scratch_bytes(h, P) = P wab_policy_backward_scratch_bytes(h) bytes (0 for P outside
+ * [1, 64]), 16-byte aligned. WAB_E_NULL for a missing d_rows, d_counts, h_coefs or array; WAB_E_CONFIG for P outside
+ * [1, 64], n_envs / P not a positive multiple of 128, list_len < 0, a bad coefficient, misalignment or too small a
+ * scratch; otherwise as wab_policy_ppo_backward. wab_policy_population_grad_stride returns 0 beyond 8 actions. */
+int wab_policy_forward_population(WabVec *h, const uint8_t *d_features, int32_t n_members, int64_t member_rows,
+                                  const void *d_packed1, const float *d_bias1, const void *d_packed2, const float *d_bias2,
+                                  int32_t hidden2, const void *d_packed3, const float *d_bias3, const float *d_w_heads,
+                                  const float *d_b_heads, int32_t n_actions, float noise_scale, float leaky_slope,
+                                  float clamp_lo, float clamp_hi, uint64_t sample_seed, const uint64_t *d_counter,
+                                  uint8_t *d_actions, float *d_value, float *d_probs, float *d_logp, float *d_z3,
+                                  void *stream);
+int64_t wab_policy_backward_population_scratch_bytes(const WabVec *h, int32_t n_members);
+int64_t wab_policy_population_grad_stride(const WabVec *h, int32_t n_actions);
+int wab_policy_ppo_backward_population(WabVec *h, const uint8_t *d_features, int64_t n_steps, int64_t n_envs,
+                                       int32_t n_members, const uint64_t *d_counters, const uint8_t *d_actions,
+                                       const float *d_logp_old, const float *d_advantage, const float *d_target,
+                                       const int32_t *d_rows, int64_t list_len, const int64_t *d_counts,
+                                       const void *d_packed1, const float *d_bias1, const void *d_packed2,
+                                       const float *d_bias2, int32_t hidden2, const void *d_packed3, const float *d_bias3,
+                                       const void *d_packed2t, const void *d_packed3t, const float *d_w_heads,
+                                       const float *d_b_heads, int32_t n_actions, float noise_scale, float leaky_slope,
+                                       float clamp_lo, float clamp_hi, const float *h_coefs, void *d_scratch,
+                                       int64_t scratch_bytes, float *d_grad, float *d_logp, float *d_value,
+                                       float *d_entropy, void *stream);
 
 /* Any loss over the policy's outputs: the recomputed forward and the vector-Jacobian product of (logits, value), so a
  * caller can write the loss in torch (or anything else) and keep only the outputs per row, never the activations.

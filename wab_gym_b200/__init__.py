@@ -5,13 +5,14 @@ Public surface (mirrors ``/root/reference/wab_env.py``):
   * ``WolvesAndBushesEnv``   — single-env gym-style compat class (``reset()``, ``step(a)``)
   * ``VecEnv``               — N lockstep envs on device-resident torch tensors
   * ``Evaluator``            — complete-episode evaluation of a policy, replayable episode by episode
+  * ``PPOPopulation``        — P PPO policies trained side by side on one VecEnv, each bit for bit its standalone run
 
 The compute path is hand-written sm_100a CUDA behind the C ABI of ``include/wab_b200.h``; there is
 no CPU fallback, and importing the env classes fails loudly if the library cannot be loaded.
 """
 from .config import GameConfig, default_game_options  # noqa: F401
 
-__all__ = ["GameConfig", "default_game_options", "VecEnv", "ObsBatch", "WolvesAndBushesEnv", "Evaluator", "EvalResult"]
+__all__ = ["GameConfig", "default_game_options", "VecEnv", "ObsBatch", "WolvesAndBushesEnv", "Evaluator", "EvalResult", "PPOPopulation"]
 
 
 def __getattr__(name):  # lazy: `import wab_gym_b200.config` must work without torch / CUDA
@@ -21,6 +22,9 @@ def __getattr__(name):  # lazy: `import wab_gym_b200.config` must work without t
     if name in ("Evaluator", "EvalResult"):
         from . import evaluate
         return getattr(evaluate, name)
+    if name == "PPOPopulation":
+        from .population import PPOPopulation
+        return PPOPopulation
     if name == "WolvesAndBushesEnv":
         from .env import WolvesAndBushesEnv
         return WolvesAndBushesEnv

@@ -19,7 +19,7 @@ EXPORTS = [
     "wab_vec_destroy", "wab_philox_device", "wab_vec_bind_features", "wab_pragmatic_features",
     "wab_vec_flatten_features", "wab_vec_flatten_features_noisy", "wab_sample_categorical", "wab_policy_tail", "wab_vec_enable_ego", "wab_vec_ego_proximities", "wab_vec_flat_dim", "wab_vec_host_block_layout", "wab_vec_step_host_packed", "wab_vec_forget_host_buffers",
     "wab_vec_state_record_bytes", "wab_vec_state_fingerprint", "wab_vec_save_state", "wab_vec_load_state", "wab_vec_set_stats",
-    "wab_policy_affine1_packed_bytes", "wab_policy_affine1_prepare", "wab_policy_affine1", "wab_policy_linear_packed_bytes", "wab_policy_linear_prepare", "wab_policy_trunk", "wab_policy_forward", "wab_policy_act", "wab_policy_backward_scratch_bytes", "wab_policy_backward", "wab_policy_ppo_backward", "wab_policy_evaluate", "wab_policy_backward_logits", "wab_policy_backward_grad_f64", "wab_policy_grad_sum_ranks", "wab2_create", "wab2_kernel_kind", "wab2_output_layout", "wab2_reset", "wab2_turn", "wab2_export_state", "wab2_import_state", "wab2_destroy", "wab_last_error", "wab_abi_version",
+    "wab_policy_affine1_packed_bytes", "wab_policy_affine1_prepare", "wab_policy_affine1", "wab_policy_linear_packed_bytes", "wab_policy_linear_prepare", "wab_policy_trunk", "wab_policy_forward", "wab_policy_act", "wab_policy_backward_scratch_bytes", "wab_policy_backward", "wab_policy_ppo_backward", "wab_policy_evaluate", "wab_policy_backward_logits", "wab_policy_backward_grad_f64", "wab_policy_grad_sum_ranks", "wab_policy_forward_population", "wab_policy_backward_population_scratch_bytes", "wab_policy_population_grad_stride", "wab_policy_ppo_backward_population", "wab2_create", "wab2_kernel_kind", "wab2_output_layout", "wab2_reset", "wab2_turn", "wab2_export_state", "wab2_import_state", "wab2_destroy", "wab_last_error", "wab_abi_version",
 ]
 
 
@@ -114,6 +114,15 @@ def load():
                                              i32, f32, f32, f32, f32, vp, i64, vp, vp]
     L.wab_policy_backward_grad_f64.argtypes = [vp, vp, i64, i32, vp, vp]
     L.wab_policy_grad_sum_ranks.argtypes = [vp, i32, i64, vp, vp]
+    L.wab_policy_forward_population.argtypes = [vp, vp, i32, i64, vp, vp, vp, vp, i32, vp, vp, vp, vp, i32, f32, f32, f32, f32, u64,
+                                                vp, vp, vp, vp, vp, vp, vp]
+    L.wab_policy_backward_population_scratch_bytes.argtypes = [vp, i32]
+    L.wab_policy_backward_population_scratch_bytes.restype = i64
+    L.wab_policy_population_grad_stride.argtypes = [vp, i32]
+    L.wab_policy_population_grad_stride.restype = i64
+    L.wab_policy_ppo_backward_population.argtypes = [vp, vp, i64, i64, i32, vp, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp, i32,
+                                                     vp, vp, vp, vp, vp, vp, i32, f32, f32, f32, f32, vp, vp, i64, vp, vp, vp, vp,
+                                                     vp]
     L.wab2_create.argtypes = [vp, i64, u64, u64, i32, ctypes.POINTER(vp)]
     L.wab2_reset.argtypes = [vp, vp]
     L.wab2_turn.argtypes = [vp] * 7
@@ -127,7 +136,8 @@ def load():
     L.wab_last_error.restype = ctypes.c_char_p
     L.wab_abi_version.restype = i32
     for name in EXPORTS:
-        if name not in ("wab_vec_num_envs", "wab_vec_state_record_bytes", "wab_policy_backward_scratch_bytes", "wab_vec_lanes_per_env", "wab_vec_step_many_pipelined", "wab_vec_kernel_kind", "wab_vec_flat_dim", "wab_vec_destroy", "wab2_destroy",
+        if name not in ("wab_vec_num_envs", "wab_vec_state_record_bytes", "wab_policy_backward_scratch_bytes", "wab_policy_backward_population_scratch_bytes",
+                        "wab_policy_population_grad_stride", "wab_vec_lanes_per_env", "wab_vec_step_many_pipelined", "wab_vec_kernel_kind", "wab_vec_flat_dim", "wab_vec_destroy", "wab2_destroy",
                         "wab_last_error", "wab_abi_version"):
             getattr(L, name).restype = ctypes.c_int
     _lib = L

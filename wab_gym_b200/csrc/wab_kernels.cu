@@ -1682,13 +1682,18 @@ static int policy_trunk_launch(WabVec* h, const uint8_t* d_features, int64_t n_r
         WAB_CUDA(cudaFuncSetAttribute(wab_affine1_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOTAL));
         WAB_CUDA(cudaFuncSetAttribute(wab_affine1_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOTAL));
         WAB_CUDA(cudaFuncSetAttribute(wab_affine1_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOTAL));
+        WAB_CUDA(cudaFuncSetAttribute(wab_affine1_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOTAL));
         attr_set[h->device] = true;
     }
     TrunkWeights tw;
     if (tail) tw = *tail; else memset(&tw, 0, sizeof(tw));
     tw.w2 = reinterpret_cast<const uint4*>(d_packed2); tw.b2 = d_bias2; tw.w3 = reinterpret_cast<const uint4*>(d_packed3); tw.b3 = d_bias3; tw.n2 = hidden2;
     const unsigned grid = (unsigned)((n_rows + TC_TILE_M - 1) / TC_TILE_M);
-    if (tail && greedy)
+    if (tail && tail->member_rows > 0)
+        wab_affine1_tc_kernel<4><<<grid, 256, TC_SMEM_TOTAL, (cudaStream_t)stream>>>(
+            h->P, d_features, n_rows, (int)h->cfg.food_obs_scale + 1, reinterpret_cast<const uint4*>(d_packed1), d_bias1, noise_scale,
+            leaky_slope, reinterpret_cast<const unsigned long long*>(d_counter), d_z3, tw);
+    else if (tail && greedy)
         wab_affine1_tc_kernel<3><<<grid, 256, TC_SMEM_TOTAL, (cudaStream_t)stream>>>(
             h->P, d_features, n_rows, (int)h->cfg.food_obs_scale + 1, reinterpret_cast<const uint4*>(d_packed1), d_bias1, noise_scale,
             leaky_slope, reinterpret_cast<const unsigned long long*>(d_counter), d_z3, tw);
@@ -1727,6 +1732,27 @@ int wab_policy_forward(WabVec* h, const uint8_t* d_features, int64_t n_rows, con
     tw.actions = d_actions; tw.value = d_value; tw.probs = d_probs; tw.logp = d_logp;
     return policy_trunk_launch(h, d_features, n_rows, d_packed1, d_bias1, d_packed2, d_bias2, hidden2, d_packed3, d_bias3, noise_scale,
                                leaky_slope, d_counter, d_z3, stream, &tw);
+}
+
+int wab_policy_forward_population(WabVec* h, const uint8_t* d_features, int32_t n_members, int64_t member_rows,
+                                  const void* d_packed1, const float* d_bias1, const void* d_packed2, const float* d_bias2,
+                                  int32_t hidden2, const void* d_packed3, const float* d_bias3, const float* d_w_heads,
+                                  const float* d_b_heads, int32_t n_actions, float noise_scale, float leaky_slope, float clamp_lo,
+                                  float clamp_hi, uint64_t sample_seed, const uint64_t* d_counter, uint8_t* d_actions,
+                                  float* d_value, float* d_probs, float* d_logp, float* d_z3, void* stream) {
+    if (!d_w_heads || !d_b_heads || !d_actions) return fail(WAB_E_NULL, "null argument");
+    if (n_actions < 1 || n_actions > 8) return fail(WAB_E_CONFIG, "n_actions must be in [1, 8]");
+    if (n_members < 1 || n_members > 64) return fail(WAB_E_CONFIG, "wab_policy_forward_population: 1 <= n_members <= 64");
+    if (member_rows < TC_TILE_M || member_rows % TC_TILE_M != 0)
+        return fail(WAB_E_CONFIG, "wab_policy_forward_population: member_rows must be a positive multiple of 128");
+    TrunkWeights tw;
+    memset(&tw, 0, sizeof(tw));
+    uint32_t k0 = (uint32_t)sample_seed, k1 = (uint32_t)(sample_seed >> 32);
+    for (int r = 0; r < 10; ++r) { tw.rk0[r] = k0; tw.rk1[r] = k1; k0 += PHILOX_W0; k1 += PHILOX_W1; }
+    tw.w_heads = d_w_heads; tw.b_heads = d_b_heads; tw.n_actions = n_actions; tw.clamp_lo = clamp_lo; tw.clamp_hi = clamp_hi;
+    tw.actions = d_actions; tw.value = d_value; tw.probs = d_probs; tw.logp = d_logp; tw.member_rows = member_rows;
+    return policy_trunk_launch(h, d_features, (int64_t)n_members * member_rows, d_packed1, d_bias1, d_packed2, d_bias2, hidden2,
+                               d_packed3, d_bias3, noise_scale, leaky_slope, d_counter, d_z3, stream, &tw);
 }
 
 // wab_policy_forward's trunk and tail with the greedy action: the same checks, no sampling seed (MODE 3 reads no round keys)
@@ -1782,6 +1808,15 @@ static int64_t policy_n_params(int dim, int n_actions) {
     return 128LL * dim + 128 + 150 * 128 + 150 + 128 * 150 + 128 + (int64_t)(n_actions + 1) * 129;
 }
 
+int64_t wab_policy_backward_population_scratch_bytes(const WabVec* h, int32_t n_members) {
+    return n_members >= 1 && n_members <= 64 ? n_members * wab_policy_backward_scratch_bytes(h) : 0;
+}
+
+int64_t wab_policy_population_grad_stride(const WabVec* h, int32_t n_actions) {
+    if (!h || n_actions < 1 || n_actions > 8) return 0;
+    return (policy_n_params(wab_vec_flat_dim(h), n_actions) + 63) / 64 * 64;
+}
+
 // wab_policy_backward and wab_policy_ppo_backward: the checks they share, then the backward kernel (the PPO one when
 // `ppo` is given) and the reduction. `d_g_logp` / `d_g_value` are wab_policy_backward's, checked by the caller.
 static int policy_backward_launch(const char* who, WabVec* h, const uint8_t* d_features, int64_t n_steps, int64_t n_envs,
@@ -1791,7 +1826,8 @@ static int policy_backward_launch(const char* who, WabVec* h, const uint8_t* d_f
                                   int32_t hidden2, const void* d_packed3, const float* d_bias3, const void* d_packed2t,
                                   const void* d_packed3t, const float* d_w_heads, const float* d_b_heads, int32_t n_actions,
                                   float noise_scale, float leaky_slope, float clamp_lo, float clamp_hi, void* d_scratch,
-                                  int64_t scratch_bytes, float* d_grad, float* d_logp, float* d_value, void* stream) {
+                                  int64_t scratch_bytes, float* d_grad, float* d_logp, float* d_value, void* stream,
+                                  const PopulationArgs* pop = nullptr, int n_members = 1) {
     if (!h || !d_features || !d_counters || !d_actions || !d_packed1 || !d_bias1 || !d_packed2 ||
         !d_bias2 || !d_packed3 || !d_bias3 || !d_packed2t || !d_packed3t || !d_w_heads || !d_b_heads || !d_scratch || !d_grad)
         return fail(WAB_E_NULL, "null argument");
@@ -1810,13 +1846,17 @@ static int policy_backward_launch(const char* who, WabVec* h, const uint8_t* d_f
                  ((uintptr_t)ppo->target & 3u) != 0 || ((uintptr_t)ppo->entropy_out & 3u) != 0)))
         return fail(WAB_E_CONFIG, "the packed weights and d_scratch must be 16-byte aligned, d_counters and d_n_rows 8-byte, "
                                   "d_features, d_rows and the float arrays 4-byte");
-    if (scratch_bytes < wab_policy_backward_scratch_bytes(h)) return fail(WAB_E_CONFIG, "d_scratch is smaller than wab_policy_backward_scratch_bytes");
+    if (scratch_bytes < n_members * wab_policy_backward_scratch_bytes(h))
+        return fail(WAB_E_CONFIG, pop ? "d_scratch is smaller than wab_policy_backward_population_scratch_bytes"
+                                      : "d_scratch is smaller than wab_policy_backward_scratch_bytes");
     DeviceGuard guard(h->device);
-    static bool attr_set[2][64] = {{false}};
-    if (h->device < 64 && !attr_set[ppo ? 1 : 0][h->device]) {
-        if (ppo) WAB_CUDA(cudaFuncSetAttribute(wab_policy_ppo_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_SMEM_TOTAL));
+    static bool attr_set[3][64] = {{false}};
+    const int kind = pop ? 2 : ppo ? 1 : 0;
+    if (h->device < 64 && !attr_set[kind][h->device]) {
+        if (pop) WAB_CUDA(cudaFuncSetAttribute(wab_policy_ppo_bwd_population_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_SMEM_TOTAL));
+        else if (ppo) WAB_CUDA(cudaFuncSetAttribute(wab_policy_ppo_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_SMEM_TOTAL));
         else WAB_CUDA(cudaFuncSetAttribute(wab_policy_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BW_SMEM_TOTAL));
-        attr_set[ppo ? 1 : 0][h->device] = true;
+        attr_set[kind][h->device] = true;
     }
     BackwardArgs B;
     memset(&B, 0, sizeof(B));
@@ -1831,10 +1871,21 @@ static int policy_backward_launch(const char* who, WabVec* h, const uint8_t* d_f
     B.clamp_lo = clamp_lo; B.clamp_hi = clamp_hi; B.scratch = reinterpret_cast<float*>(d_scratch);
     B.logp_out = d_logp; B.value_out = d_value;
     const int grid = backward_grid(h->device);
+    const int64_t total = policy_n_params(dim, n_actions);
+    if (pop) {
+        PopulationArgs G = *pop;
+        G.n_cta = grid;
+        wab_policy_ppo_bwd_population_kernel<<<grid * n_members, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(
+            h->P, (int)h->cfg.food_obs_scale + 1, B, *ppo, G);
+        WAB_CUDA(cudaGetLastError());
+        wab_policy_bwd_reduce_population_kernel<<<dim3((unsigned)((total + 255) / 256), (unsigned)n_members), 256, 0, (cudaStream_t)stream>>>(
+            reinterpret_cast<const float*>(d_scratch), grid, dim, n_actions, (total + 63) / 64 * 64, d_grad);
+        WAB_CUDA(cudaGetLastError());
+        return WAB_OK;
+    }
     if (ppo) wab_policy_ppo_bwd_kernel<<<grid, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(h->P, (int)h->cfg.food_obs_scale + 1, B, *ppo);
     else wab_policy_bwd_kernel<<<grid, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(h->P, (int)h->cfg.food_obs_scale + 1, B);
     WAB_CUDA(cudaGetLastError());
-    const int64_t total = policy_n_params(dim, n_actions);
     wab_policy_bwd_reduce_kernel<float><<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const float*>(d_scratch), grid, dim, n_actions, d_grad);
     WAB_CUDA(cudaGetLastError());
@@ -1877,6 +1928,42 @@ int wab_policy_ppo_backward(WabVec* h, const uint8_t* d_features, int64_t n_step
                                   nullptr, &Q, d_rows, d_n_rows, d_packed1, d_bias1, d_packed2, d_bias2, hidden2, d_packed3,
                                   d_bias3, d_packed2t, d_packed3t, d_w_heads, d_b_heads, n_actions, noise_scale, leaky_slope,
                                   clamp_lo, clamp_hi, d_scratch, scratch_bytes, d_grad, d_logp, d_value, stream);
+}
+
+int wab_policy_ppo_backward_population(WabVec* h, const uint8_t* d_features, int64_t n_steps, int64_t n_envs, int32_t n_members,
+                                       const uint64_t* d_counters, const uint8_t* d_actions, const float* d_logp_old,
+                                       const float* d_advantage, const float* d_target, const int32_t* d_rows, int64_t list_len,
+                                       const int64_t* d_counts, const void* d_packed1, const float* d_bias1,
+                                       const void* d_packed2, const float* d_bias2, int32_t hidden2, const void* d_packed3,
+                                       const float* d_bias3, const void* d_packed2t, const void* d_packed3t,
+                                       const float* d_w_heads, const float* d_b_heads, int32_t n_actions, float noise_scale,
+                                       float leaky_slope, float clamp_lo, float clamp_hi, const float* h_coefs,
+                                       void* d_scratch, int64_t scratch_bytes, float* d_grad, float* d_logp, float* d_value,
+                                       float* d_entropy, void* stream) {
+    if (!d_logp_old || !d_advantage || !d_target || !d_rows || !d_counts || !h_coefs) return fail(WAB_E_NULL, "null argument");
+    if (n_members < 1 || n_members > 64) return fail(WAB_E_CONFIG, "wab_policy_ppo_backward_population: 1 <= n_members <= 64");
+    if (n_envs % n_members != 0 || (n_envs / n_members) % TC_TILE_M != 0 || n_envs == 0)
+        return fail(WAB_E_CONFIG, "wab_policy_ppo_backward_population: n_envs / n_members must be a positive multiple of 128");
+    if (list_len < 0) return fail(WAB_E_CONFIG, "wab_policy_ppo_backward_population: list_len must be >= 0");
+    PopulationArgs G;
+    memset(&G, 0, sizeof(G));
+    for (int m = 0; m < n_members; ++m) {
+        const float* c = h_coefs + 4 * m;
+        if (!(c[0] > 0.f)) return fail(WAB_E_CONFIG, "wab_policy_ppo_backward_population: clip_eps must be > 0 (+inf disables clipping)");
+        if (!std::isfinite(c[1]) || !std::isfinite(c[2]) || !std::isfinite(c[3]))
+            return fail(WAB_E_CONFIG, "wab_policy_ppo_backward_population: the loss weights must be finite");
+        for (int k = 0; k < 4; ++k) G.coef[m][k] = c[k];
+    }
+    G.member_envs = n_envs / n_members; G.list_len = list_len; G.rows = d_rows;
+    G.counts = reinterpret_cast<const long long*>(d_counts);
+    PpoArgs Q;
+    memset(&Q, 0, sizeof(Q));
+    Q.logp_old = d_logp_old; Q.advantage = d_advantage; Q.target = d_target; Q.entropy_out = d_entropy;
+    return policy_backward_launch("wab_policy_ppo_backward_population", h, d_features, n_steps, n_envs, d_counters, d_actions,
+                                  nullptr, nullptr, &Q, d_rows, d_counts, d_packed1, d_bias1, d_packed2, d_bias2, hidden2,
+                                  d_packed3, d_bias3, d_packed2t, d_packed3t, d_w_heads, d_b_heads, n_actions, noise_scale,
+                                  leaky_slope, clamp_lo, clamp_hi, d_scratch, scratch_bytes, d_grad, d_logp, d_value, stream,
+                                  &G, n_members);
 }
 
 // wab_policy_evaluate and wab_policy_backward_logits: the checks they share, then the list kernel (the evaluation when

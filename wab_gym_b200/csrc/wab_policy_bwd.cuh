@@ -78,8 +78,15 @@ struct ListArgs {
     float* logits_out; float* value_out;     // logits [M][A], value [M] (the evaluation)
 };
 
-// which heads block the body runs (step 2), and whether steps 3 - 5 follow (not for BW_EVAL)
-enum BwKind { BW_A2C, BW_PPO, BW_EVAL, BW_LOGITS };
+// which heads block the body runs (step 2), and whether steps 3 - 5 follow (not for BW_EVAL); BW_PPO_POP is BW_PPO for
+// one member of a population (wab_policy_ppo_bwd_population_kernel)
+enum BwKind { BW_A2C, BW_PPO, BW_EVAL, BW_LOGITS, BW_PPO_POP };
+
+// the CTA's member in wab_policy_ppo_bwd_population_kernel; the other kernels declare an unused one
+struct MemberArgs {
+    int member, cta, n_cta;                  // member m = blockIdx.x / n_cta, its local CTA index cta = blockIdx.x % n_cta
+    long long member_envs, list_len;         // n: member m owns envs [m n, (m + 1) n); M: entries of its row list
+};
 
 // element (operand row n, K = tile row k) of a K = 128 operand, canonical K-major layout without swizzle
 __device__ __forceinline__ uint32_t bw_off(int n, int k) { return (uint32_t)((n >> 3) * BW_KROW + (k >> 3) * 128 + (n & 7) * 16 + (k & 7) * 2); }
@@ -118,6 +125,7 @@ wab_policy_bwd_kernel(const __grid_constant__ Params P, int food_dim, const __gr
     constexpr BwKind KIND = BW_A2C;
     const PpoArgs Q{};
     const ListArgs L{};
+    const MemberArgs G{};
 #include "wab_policy_bwd_body.cuh"
 }
 
@@ -126,6 +134,7 @@ wab_policy_ppo_bwd_kernel(const __grid_constant__ Params P, int food_dim, const 
                           const __grid_constant__ PpoArgs Q) {
     constexpr BwKind KIND = BW_PPO;
     const ListArgs L{};
+    const MemberArgs G{};
 #include "wab_policy_bwd_body.cuh"
 }
 
@@ -135,6 +144,7 @@ wab_policy_eval_kernel(const __grid_constant__ Params P, int food_dim, const __g
                        const __grid_constant__ ListArgs L) {
     constexpr BwKind KIND = BW_EVAL;
     const PpoArgs Q{};
+    const MemberArgs G{};
 #include "wab_policy_bwd_body.cuh"
 }
 #pragma nv_diag_default 128
@@ -144,6 +154,35 @@ wab_policy_logits_bwd_kernel(const __grid_constant__ Params P, int food_dim, con
                              const __grid_constant__ ListArgs L) {
     constexpr BwKind KIND = BW_LOGITS;
     const PpoArgs Q{};
+    const MemberArgs G{};
+#include "wab_policy_bwd_body.cuh"
+}
+
+// the population backward: P members of n envs each on ONE grid of P n_cta CTAs (n_cta = the single-policy grid). CTA b
+// serves member m = b / n_cta as local CTA c = b % n_cta and walks tiles c, c + n_cta, ... of m's row list: the tiles a
+// single-policy launch gives its CTA c, into the scratch block b = m n_cta + c, so member m's partial sums are those of
+// its own wab_policy_ppo_bwd_kernel bit for bit. Weights are stacked per member at the packers' strides.
+struct PopulationArgs {
+    int n_cta;
+    long long member_envs, list_len;         // n, M
+    const int32_t* rows; const long long* counts;    // [P][M] global rows t N + n, [P] counts (read on the device)
+    float coef[64][4];                       // clip_eps, w_policy, w_value, w_entropy of each member
+};
+
+__global__ void __launch_bounds__(256, 1)
+wab_policy_ppo_bwd_population_kernel(const __grid_constant__ Params P, int food_dim, const __grid_constant__ BackwardArgs Bs,
+                                     const __grid_constant__ PpoArgs Qs, const __grid_constant__ PopulationArgs Pop) {
+    constexpr BwKind KIND = BW_PPO_POP;
+    const ListArgs L{};
+    const int m = (int)(blockIdx.x / (unsigned)Pop.n_cta);
+    const MemberArgs G{m, (int)blockIdx.x - m * Pop.n_cta, Pop.n_cta, Pop.member_envs, Pop.list_len};
+    const int64_t heads_n = Bs.n_actions + 1;
+    BackwardArgs B = Bs;
+    B.rows = Pop.rows + m * Pop.list_len; B.d_count = Pop.counts + m;
+    B.w1 += m * POP_W1_U4; B.b1 += m * 128; B.w2 += m * POP_LINEAR_U4; B.b2 += m * 150; B.w3 += m * POP_LINEAR_U4;
+    B.b3 += m * 128; B.w2t += m * POP_LINEAR_U4; B.w3t += m * POP_LINEAR_U4; B.w_heads += m * heads_n * 128; B.b_heads += m * heads_n;
+    PpoArgs Q = Qs;
+    Q.clip_eps = Pop.coef[m][0]; Q.w_policy = Pop.coef[m][1]; Q.w_value = Pop.coef[m][2]; Q.w_entropy = Pop.coef[m][3];
 #include "wab_policy_bwd_body.cuh"
 }
 
@@ -173,6 +212,35 @@ __global__ void wab_policy_bwd_reduce_kernel(const float* __restrict__ scratch, 
     double s = 0.0;
     for (int b = 0; b < n_blocks; ++b) s += (double)scratch[(size_t)b * BP_BLOCK + off];
     grad[e] = (G)s;
+}
+
+// wab_policy_bwd_reduce_kernel<float> for each member of a population (blockIdx.y = m): the fp64 sum over m's own n_cta
+// CTAs, in index order, into grad [P][stride]. The element -> partial-sum mapping is restated rather than shared: moved
+// into a device function, it compiles differently inside wab_policy_bwd_reduce_kernel.
+__global__ void wab_policy_bwd_reduce_population_kernel(const float* __restrict__ scratch, int n_cta, int dim, int n_actions,
+                                                        int64_t stride, float* __restrict__ grad) {
+    const int64_t n1 = 128LL * dim, o_b1 = n1, o_w2 = o_b1 + 128, o_b2 = o_w2 + 150 * 128, o_w3 = o_b2 + 150, o_b3 = o_w3 + 128 * 150,
+                  o_wa = o_b3 + 128, o_ba = o_wa + (int64_t)n_actions * 128, o_wv = o_ba + n_actions, o_bv = o_wv + 128, total = o_bv + 1;
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= total) return;
+    int off;
+    if (e < o_b1) {
+        const int j = (int)(e / dim), k = (int)(e - (int64_t)j * dim);
+        const int c = 2 * (k >> 7) + ((k >> 4) & 1), s = (k >> 5) & 3, hh = (k >> 3) & 1, el = k & 7;   // tc_column inverted
+        off = BP_W1 + (c * 128 + j) * 64 + 8 * (4 * hh + s) + el;
+    } else if (e < o_w2) off = BP_B1 + (int)(e - o_b1);
+    else if (e < o_b2) { const int j = (int)((e - o_w2) / 128), i = (int)((e - o_w2) % 128); off = BP_W2T + i * 160 + j; }
+    else if (e < o_w3) off = BP_B2 + (int)(e - o_b2);
+    else if (e < o_b3) { const int j = (int)((e - o_w3) / 150), i = (int)((e - o_w3) % 150); off = BP_W3 + j * 160 + i; }
+    else if (e < o_wa) off = BP_B3 + (int)(e - o_b3);
+    else if (e < o_ba) { const int o = (int)((e - o_wa) / 128), i = (int)((e - o_wa) % 128); off = BP_WH + i * 16 + o; }
+    else if (e < o_wv) off = BP_BH + (int)(e - o_ba);
+    else if (e < o_bv) off = BP_WH + (int)(e - o_wv) * 16 + n_actions;
+    else off = BP_BH + n_actions;
+    const float* member = scratch + (size_t)blockIdx.y * n_cta * BP_BLOCK;
+    double s = 0.0;
+    for (int b = 0; b < n_cta; ++b) s += (double)member[(size_t)b * BP_BLOCK + off];
+    grad[(int64_t)blockIdx.y * stride + e] = (float)s;
 }
 
 // d_grad[i] = fp32(sum over r = 0 .. n_ranks - 1 of d_rank_grads[r][i]), the sum in fp64 in rank order

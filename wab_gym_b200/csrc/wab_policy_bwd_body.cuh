@@ -1,8 +1,9 @@
 // wab_policy_bwd_body.cuh — the body of wab_policy_bwd_kernel, wab_policy_ppo_bwd_kernel, wab_policy_eval_kernel and
-// wab_policy_logits_bwd_kernel (wab_policy_bwd.cuh), included inside each. Each kernel declares `constexpr BwKind KIND`,
-// its parameters P, food_dim, B, a PpoArgs Q and a ListArgs L; KIND selects the row list and the heads block of step 2
-// (BW_EVAL stops after it), and everything else is shared. A fragment rather than a __forceinline__ function: the
-// compiler optimises a device function on its own before inlining it, which changes the code of the existing kernels.
+// wab_policy_logits_bwd_kernel and wab_policy_ppo_bwd_population_kernel (wab_policy_bwd.cuh), included inside each. Each
+// kernel declares `constexpr BwKind KIND`, its parameters P, food_dim, B, a PpoArgs Q, a ListArgs L and a MemberArgs G;
+// KIND selects the row list and the heads block of step 2 (BW_EVAL stops after it), and everything else is shared. A
+// fragment rather than a __forceinline__ function: the compiler optimises a device function on its own before inlining
+// it, which changes the code of the existing kernels.
     extern __shared__ __align__(1024) uint8_t tc_smem[];
     __shared__ uint32_t tmem_slot;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -48,6 +49,7 @@
     uint32_t parity = 0;
     long long count = LIST ? L.n_list : (B.d_count ? *B.d_count : (long long)B.n_rows);
     if (!LIST) count = count < 0 ? 0 : (count > (long long)B.n_rows ? (long long)B.n_rows : count);
+    if constexpr (KIND == BW_PPO_POP) count = count > G.list_len ? G.list_len : count;   // the member's own list only
     const long long n_tiles = (count + TC_TILE_M - 1) / TC_TILE_M;
 
     auto wait_mma = [&]() {
@@ -201,10 +203,12 @@
     };
 
 #pragma unroll 1
-    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    for (long long tile = KIND == BW_PPO_POP ? G.cta : blockIdx.x; tile < n_tiles; tile += KIND == BW_PPO_POP ? G.n_cta : gridDim.x) {
         const long long slot = tile * TC_TILE_M + r;
         int64_t flat = slot < count ? (B.rows ? (int64_t)B.rows[slot] : (int64_t)slot) : -1;
-        const bool valid = flat >= 0 && flat < B.n_rows;                    // a listed row outside [0, T N) contributes nothing
+        bool valid = flat >= 0 && flat < B.n_rows;                          // a listed row outside [0, T N) contributes nothing,
+        if constexpr (KIND == BW_PPO_POP)                                   // nor, in a population, another member's row
+            valid = valid && (flat % B.n_envs) / G.member_envs == G.member;
         if (!valid) flat = 0;
         const int64_t step = flat / B.n_envs;
         const uint32_t krow = (uint32_t)(P.env_id_base + (uint64_t)(flat - step * B.n_envs));   // the noise key: the global env id

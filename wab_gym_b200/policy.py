@@ -344,6 +344,149 @@ class PolicyTrainTC(PolicyTrunkTC):
         return out
 
 
+class PolicyPopulationTC:
+    """P policies of the reference's network on ONE features-enabled ``VecEnv`` of N = P n envs (1 <= P <= 64, n a
+    multiple of 128): member p owns env rows [p n, (p + 1) n), and its weights are packed into row p of stacked buffers
+    (``wab_policy_forward_population``, ``wab_policy_ppo_backward_population``). Each call does for every member what
+    ``PolicyTrainTC`` does for one policy, in one launch, and member p's outputs equal, bit for bit, those of
+    ``PolicyTrainTC`` on ``VecEnv(n, env_id_base=p n)`` (with the same env_id_base shift on this handle). A member is
+    re-packed when one of its parameters changed since its last pack (an optimiser step, a load), as
+    ``PolicyTrainTC.logits_and_value`` does."""
+
+    def __init__(self, env: VecEnv, policies):
+        policies = list(policies)
+        P, N = len(policies), env.num_envs
+        if not 1 <= P <= 64:
+            raise ValueError("a population has 1 to 64 members")
+        if N % P != 0 or (N // P) % 128 != 0:
+            raise ValueError("PolicyPopulationTC needs num_envs = P * n with n a multiple of 128")
+        for p in policies:
+            check_reference_network(p, env.flat_dim, "PolicyPopulationTC")
+        A = policies[0].action_head.out_features
+        if any(p.action_head.out_features != A for p in policies):
+            raise ValueError("every member of a population has the same action count")
+        self.env, self.policies, self.lib = env, policies, _lib.load()
+        self.n_members, self.member_envs, self.n_actions = P, N // P, A
+        self.n_params = sum(prm.numel() for prm in policies[0].parameters())
+        self.grad_stride = int(self.lib.wab_policy_population_grad_stride(env._h, A))
+        dev, lib = env.device, self.lib
+        lin = int(lib.wab_policy_linear_packed_bytes(150, 128))
+        if lin != int(lib.wab_policy_linear_packed_bytes(128, 150)):
+            raise RuntimeError("the stacked layouts assume one packed size for every trunk layer")
+        u8 = dict(dtype=torch.uint8, device=dev)
+        self.packed1 = torch.empty(P, int(lib.wab_policy_affine1_packed_bytes()), **u8)
+        self.packed2, self.packed3, self.packed2t, self.packed3t = (torch.empty(P, lin, **u8) for _ in range(4))
+        self.bias1, self.bias2, self.bias3 = (torch.empty(P, k, device=dev) for k in (128, 150, 128))
+        self.w_heads, self.b_heads = torch.empty(P, A + 1, 128, device=dev), torch.empty(P, A + 1, device=dev)
+        self.scratch = torch.empty(int(lib.wab_policy_backward_population_scratch_bytes(env._h, P)), **u8)
+        self._packed_versions = [None] * P
+        self.refresh()
+
+    def _stream(self):
+        return ctypes.c_void_p(torch.cuda.current_stream(self.env.device).cuda_stream)
+
+    def _versions(self, p: int) -> tuple:
+        return tuple((id(prm), prm._version) for prm in self.policies[p].parameters())
+
+    @torch.no_grad()
+    def refresh(self, members=None):
+        """Re-pack members ``members`` (default: all) into their rows of the stacked buffers."""
+        lib, s = self.lib, self._stream()
+        f = lambda t: t.detach().float().contiguous()
+        for p in range(self.n_members) if members is None else members:
+            pol = self.policies[p]
+            _lib.check(lib.wab_policy_affine1_prepare(_ptr(f(pol.affine1.weight)), self.env.flat_dim, _ptr(self.packed1[p]), s))
+            _lib.check(lib.wab_policy_linear_prepare(_ptr(f(pol.affine2.weight)), 150, 128, _ptr(self.packed2[p]), s))
+            _lib.check(lib.wab_policy_linear_prepare(_ptr(f(pol.affine3.weight)), 128, 150, _ptr(self.packed3[p]), s))
+            _lib.check(lib.wab_policy_linear_prepare(_ptr(f(pol.affine2.weight.t())), 128, 150, _ptr(self.packed2t[p]), s))
+            _lib.check(lib.wab_policy_linear_prepare(_ptr(f(pol.affine3.weight.t())), 150, 128, _ptr(self.packed3t[p]), s))
+            self.bias1[p].copy_(pol.affine1.bias); self.bias2[p].copy_(pol.affine2.bias); self.bias3[p].copy_(pol.affine3.bias)
+            w, b = stacked_heads(pol)
+            self.w_heads[p].copy_(w); self.b_heads[p].copy_(b)
+            self._packed_versions[p] = self._versions(p)
+
+    def _refresh_stale(self):
+        stale = [p for p in range(self.n_members) if self._packed_versions[p] != self._versions(p)]
+        if stale:
+            self.refresh(stale)
+
+    def forward_sample(self, features: torch.Tensor, actions: torch.Tensor, value: Optional[torch.Tensor] = None,
+                       probs: Optional[torch.Tensor] = None, logp: Optional[torch.Tensor] = None, noise_scale: float = 0.01,
+                       counter: Optional[torch.Tensor] = None, seed: int = 0, z3: Optional[torch.Tensor] = None,
+                       slope: float = 0.01) -> torch.Tensor:
+        """``PolicyTrunkTC.forward_sample`` for the N = P n rows of ``features`` u8[N, 28], row r under member r // n's
+        weights, in ONE launch. Fills ``actions`` u8[N] (and ``value`` f32[N], ``probs`` f32[N, A], ``logp`` f32[N],
+        ``z3`` f32[N, 128] when given)."""
+        N, A = self.n_members * self.member_envs, self.n_actions
+        if tuple(features.shape) != (N, 28) or features.dtype != torch.uint8 or not features.is_contiguous():
+            raise ValueError("features must be a contiguous uint8 [P n, 28] tensor")
+        if tuple(actions.shape) != (N,) or actions.dtype != torch.uint8 or not actions.is_contiguous():
+            raise ValueError("actions must be a contiguous uint8 [P n] tensor")
+        for name, t, shape in (("value", value, (N,)), ("probs", probs, (N, A)), ("logp", logp, (N,)), ("z3", z3, (N, 128))):
+            if t is not None and (t.dtype != torch.float32 or tuple(t.shape) != shape or not t.is_contiguous()):
+                raise ValueError("%s must be a contiguous float32 %s tensor" % (name, list(shape)))
+        for name, t in (("features", features), ("actions", actions), ("value", value), ("probs", probs), ("logp", logp),
+                        ("z3", z3), ("counter", counter)):
+            if t is not None and t.device != self.env.device:
+                raise ValueError("%s must be on the environment's device" % name)
+        self._refresh_stale()
+        _lib.check(self.lib.wab_policy_forward_population(
+            self.env._h, _ptr(features), self.n_members, self.member_envs, _ptr(self.packed1), _ptr(self.bias1),
+            _ptr(self.packed2), _ptr(self.bias2), 150, _ptr(self.packed3), _ptr(self.bias3), _ptr(self.w_heads),
+            _ptr(self.b_heads), A, float(noise_scale), float(slope), -4.0, 4.0, int(seed) & (2 ** 64 - 1), _ptr(counter),
+            _ptr(actions), _ptr(value), _ptr(probs), _ptr(logp), _ptr(z3), self._stream()))
+        return actions
+
+    def ppo_backward(self, features: torch.Tensor, counters: torch.Tensor, actions: torch.Tensor, logp_old: torch.Tensor,
+                     advantage: torch.Tensor, target: torch.Tensor, rows: torch.Tensor, counts: torch.Tensor, coefs,
+                     out: Optional[torch.Tensor] = None, logp: Optional[torch.Tensor] = None, value: Optional[torch.Tensor] = None,
+                     entropy: Optional[torch.Tensor] = None, noise_scale: float = 0.01, slope: float = 0.01) -> torch.Tensor:
+        """``PolicyTrainTC.ppo_backward`` for every member in ONE launch. ``rows`` int32[P, M]: member p's row list as
+        GLOBAL rows t N + n (an entry outside [0, T N) or in another member's block contributes nothing); ``counts``
+        int64[P] on the device: member p uses its first ``counts[p]`` entries. ``coefs``: P rows of (clip_eps,
+        policy_weight, value_weight, entropy_weight) on the host. Returns ``out`` f32[P, grad_stride]: row p's first
+        ``n_params`` floats are member p's flat gradient. ``logp``, ``value``, ``entropy`` f32[T, N] as for one policy."""
+        T, N = actions.shape
+        P = self.n_members
+        if N != P * self.member_envs:
+            raise ValueError("actions must be [T, P n]")
+        if tuple(features.shape) != (T, N, 28) or features.dtype != torch.uint8 or not features.is_contiguous():
+            raise ValueError("features must be a contiguous uint8 [T, N, 28] tensor")
+        for name, t in (("logp_old", logp_old), ("advantage", advantage), ("target", target)):
+            if t.dtype != torch.float32 or tuple(t.shape) != (T, N) or not t.is_contiguous():
+                raise ValueError("%s must be a contiguous float32 [T, N] tensor" % name)
+        for name, t in (("logp", logp), ("value", value), ("entropy", entropy)):
+            if t is not None and (t.dtype != torch.float32 or tuple(t.shape) != (T, N) or not t.is_contiguous()):
+                raise ValueError("%s must be a contiguous float32 [T, N] tensor" % name)
+        if counters.dtype != torch.int64 or counters.numel() != T or actions.dtype != torch.uint8 or not actions.is_contiguous():
+            raise ValueError("counters must be int64[T], actions a contiguous uint8 [T, N] tensor")
+        if rows.dtype != torch.int32 or rows.dim() != 2 or rows.shape[0] != P or not rows.is_contiguous():
+            raise ValueError("rows must be a contiguous int32 [P, M] tensor")
+        if counts.dtype != torch.int64 or tuple(counts.shape) != (P,) or not counts.is_contiguous():
+            raise ValueError("counts must be a contiguous int64 [P] tensor")
+        if len(coefs) != P or any(len(row) != 4 for row in coefs):
+            raise ValueError("coefs must hold P rows of (clip_eps, policy_weight, value_weight, entropy_weight)")
+        coef = (ctypes.c_float * (4 * P))(*(float(c) for row in coefs for c in row))
+        if out is None:
+            out = torch.empty(P, self.grad_stride, dtype=torch.float32, device=self.env.device)
+        if out.dtype != torch.float32 or tuple(out.shape) != (P, self.grad_stride) or not out.is_contiguous():
+            raise ValueError("out must be a contiguous float32 [P, grad_stride] tensor")
+        for name, t in (("features", features), ("counters", counters), ("actions", actions), ("logp_old", logp_old),
+                        ("advantage", advantage), ("target", target), ("rows", rows), ("counts", counts), ("out", out),
+                        ("logp", logp), ("value", value), ("entropy", entropy)):
+            if t is not None and t.device != self.env.device:
+                raise ValueError("%s must be on the environment's device" % name)
+        self._refresh_stale()
+        _lib.check(self.lib.wab_policy_ppo_backward_population(
+            self.env._h, _ptr(features), T, N, P, _ptr(counters), _ptr(actions), _ptr(logp_old), _ptr(advantage),
+            _ptr(target), _ptr(rows), rows.shape[1], _ptr(counts), _ptr(self.packed1), _ptr(self.bias1), _ptr(self.packed2),
+            _ptr(self.bias2), 150, _ptr(self.packed3), _ptr(self.bias3), _ptr(self.packed2t), _ptr(self.packed3t),
+            _ptr(self.w_heads), _ptr(self.b_heads), self.n_actions, float(noise_scale), float(slope), -4.0, 4.0,
+            ctypes.cast(coef, ctypes.c_void_p), _ptr(self.scratch), self.scratch.numel(), _ptr(out), _ptr(logp), _ptr(value),
+            _ptr(entropy), self._stream()))
+        return out
+
+
 class _LogitsAndValue(torch.autograd.Function):
     """``PolicyTrainTC.logits_and_value``: forward ``wab_policy_evaluate``, backward ``wab_policy_backward_logits`` into a
     fresh flat gradient per call (a buffer reused across calls would alias an accumulated ``.grad``), returned as views in

@@ -26,20 +26,23 @@ from .policy import Policy
 from .vec_env import VecEnv
 
 
-def gae(rewards: torch.Tensor, dones: torch.Tensor, values: torch.Tensor, bootstrap: torch.Tensor, gamma: float,
-        lam: float) -> Tuple[torch.Tensor, torch.Tensor]:
+def gae(rewards: torch.Tensor, dones: torch.Tensor, values: torch.Tensor, bootstrap: torch.Tensor, gamma,
+        lam: float, gamma_lam=None) -> Tuple[torch.Tensor, torch.Tensor]:
     """Generalised advantage estimation over [T, N] tensors: returns (advantages, returns = advantages + values).
     Step t's successor counts with the mask (1 - done_t): after a done the environment auto-resets, so nothing is
     bootstrapped across the boundary. A v1 episode that ends by ``max_turns`` is treated as terminal too. ``bootstrap``
-    f32[N] is the value of the observation after the last step."""
+    f32[N] is the value of the observation after the last step. Per-column discounts: ``gamma`` f32[N] and
+    ``gamma_lam`` f32[N] (each column's gamma * lam, formed in double and rounded once, as a float gamma and lam are);
+    ``lam`` is then unused."""
     T = rewards.shape[0]
     adv = torch.empty_like(rewards)
     running = torch.zeros_like(bootstrap)
     next_value = bootstrap
+    gl = gamma * lam if gamma_lam is None else gamma_lam
     for t in range(T - 1, -1, -1):
         live = 1.0 - dones[t].to(rewards.dtype)
         delta = rewards[t] + gamma * next_value * live - values[t]
-        running = delta + (gamma * lam) * live * running
+        running = delta + gl * live * running
         adv[t] = running
         next_value = values[t]
     return adv, adv + values
