@@ -246,7 +246,7 @@ int wab_vec_flat_dim(const WabVec *h);
  *
  * Keying contract of the policy entry points: every one that takes a WabVec handle (wab_vec_flatten_features_noisy,
  * wab_policy_affine1, wab_policy_trunk, wab_policy_forward, wab_policy_act, wab_policy_backward, wab_policy_ppo_backward,
- * wab_policy_evaluate, wab_policy_backward_logits and the population calls) keys its noise and its action samples by the global env id env_id_base + row (the row within its step for the backward passes), so
+ * wab_policy_evaluate, wab_policy_backward_logits and the population calls) keys its noise and its action samples by the global env id env_id_base + row (the row within its step for the backward passes; env_id_base + row % n on a handle with replicas, wab_vec_set_replicas), so
  * a shard [first, first + count) draws exactly what the unsharded batch draws for rows first .. first + count - 1;
  * outputs stay indexed by the local row. The two handle-less calls, wab_sample_categorical and wab_policy_tail, know no
  * shard and key by the local row. */
@@ -269,6 +269,17 @@ int wab_sample_categorical(const void *d_probs, int32_t probs_bf16, int64_t n, i
  * without a reset keep only their first max_turns positions. */
 int wab_vec_enable_ego(WabVec *h);
 int wab_vec_ego_proximities(WabVec *h, uint8_t *d_out10, void *stream);
+
+/* Replicas: the handle's N envs become n_replicas copies of n = N / n_replicas envs. Row r takes the global env id
+ * env_id_base + r % n in every draw keyed by the global id: the world draws of the step and reset kernels, the origin id
+ * written by wab_vec_save_state, and the noise and action samples of the policy entry points (the backward passes'
+ * regenerated noise included). So block k of a replicated handle, driven by an action stream, plays exactly what a handle
+ * of n envs at env_id_base plays under that stream: several policies can be scored on the same episodes in one launch.
+ * n_replicas = 1 is the unreplicated handle. Like wab_vec_enable_ego, valid only before the first reset (or load);
+ * WAB_E_CONFIG for n_replicas < 1, a count that does not divide n_envs, n_envs >= 2^32, or a handle already reset. The
+ * state fingerprint is unchanged: a record is valid on either kind of handle, and the slot it is loaded into decides its
+ * ids. */
+int wab_vec_set_replicas(WabVec *h, int64_t n_replicas);
 
 /* The first layer of the reference's Policy on the tensor cores (actor_critic.py:59, :88-90, :188-189), fp32 accuracy:
  * d_out f32[n_rows][128] = leaky_relu(affine1(flatten(obs) + noise_scale * U[0,1))) straight from the 28 feature bytes per
@@ -387,7 +398,9 @@ int wab_policy_ppo_backward(WabVec *h, const uint8_t *d_features, int64_t n_step
  *
  * wab_policy_forward_population: wab_policy_forward over P n rows, each row under its member's weights. Arguments, NULL
  * rules and alignment as for wab_policy_forward; WAB_E_CONFIG for P outside [1, 64] or member_rows not a positive
- * multiple of 128, otherwise as wab_policy_forward.
+ * multiple of 128, otherwise as wab_policy_forward. wab_policy_act_population is the same call with wab_policy_act's
+ * greedy action (no sample_seed), with the same checks and return codes: on a handle with wab_vec_set_replicas(h, P)
+ * every member acts on the same envs, which scores P policies on the same episodes in one launch per step.
  *
  * wab_policy_ppo_backward_population: wab_policy_ppo_backward for every member in one launch of P x (the single-policy
  * grid) CTAs. d_rows int32[P][list_len] holds each member's row list as GLOBAL rows t N + n (N = n_envs), d_counts
@@ -409,6 +422,12 @@ int wab_policy_forward_population(WabVec *h, const uint8_t *d_features, int32_t 
                                   float clamp_lo, float clamp_hi, uint64_t sample_seed, const uint64_t *d_counter,
                                   uint8_t *d_actions, float *d_value, float *d_probs, float *d_logp, float *d_z3,
                                   void *stream);
+int wab_policy_act_population(WabVec *h, const uint8_t *d_features, int32_t n_members, int64_t member_rows,
+                              const void *d_packed1, const float *d_bias1, const void *d_packed2, const float *d_bias2,
+                              int32_t hidden2, const void *d_packed3, const float *d_bias3, const float *d_w_heads,
+                              const float *d_b_heads, int32_t n_actions, float noise_scale, float leaky_slope,
+                              float clamp_lo, float clamp_hi, const uint64_t *d_counter, uint8_t *d_actions,
+                              float *d_value, float *d_probs, float *d_logp, float *d_z3, void *stream);
 int64_t wab_policy_backward_population_scratch_bytes(const WabVec *h, int32_t n_members);
 int64_t wab_policy_population_grad_stride(const WabVec *h, int32_t n_actions);
 int wab_policy_ppo_backward_population(WabVec *h, const uint8_t *d_features, int64_t n_steps, int64_t n_envs,

@@ -123,6 +123,8 @@ class A2CTrainer:
                  noise: bool = True, mode: str = "episodic", tensor_cores: bool = False, group=None):
         if not env.with_features:
             raise ValueError("A2CTrainer needs VecEnv(features=True)")
+        if getattr(env, "replicas", 1) > 1:
+            raise ValueError("the trainers refuse a VecEnv with replicas: its env ids repeat")
         if mode not in ("episodic", "horizon"):
             raise ValueError("mode must be 'episodic' or 'horizon'")
         self.env, self.gamma, self.noise, self.mode = env, float(gamma), noise, mode

@@ -78,7 +78,15 @@ struct Params {
     float reward_table[8];
     uint32_t mask_look[4], mask_gath[4];
     uint64_t env_id_base;
+    uint64_t replica_envs;         // 0, or n of a replicated handle (wab_vec_set_replicas): every block of n rows repeats the ids
 };
+
+// The global env id of `row` (< 2^32: wab_vec_set_replicas refuses larger handles), the key of every draw the handle makes
+// for it: env_id_base + row, or env_id_base + row % n on a replicated handle, whose blocks of n rows are copies of one another.
+WAB_HD uint64_t global_env_id(const Params& P, int64_t row) {
+    if (P.replica_envs) return P.env_id_base + (uint64_t)((uint32_t)row % (uint32_t)P.replica_envs);
+    return P.env_id_base + (uint64_t)row;
+}
 
 // Registers of one environment.
 struct Env {

@@ -191,7 +191,7 @@ __device__ __forceinline__ void gen_load(const Params& P, const StatePtrs& st, i
     E.episode = st.episode[idx]; E.logsig = st.logsig[idx];
     { const uint2 bk = st.bkey[idx]; E.bk_a = bk.x; E.bk_b = bk.y; }
     E.food_f = st.food[idx];
-    E.env_id = (uint32_t)(P.env_id_base + (uint64_t)idx);
+    E.env_id = (uint32_t)global_env_id(P, idx);
     E.m[0] = E.m[1] = E.m[2] = E.m[3] = 0u;
     for (uint32_t k = (uint32_t)lane; k < E.nw; k += 32) wolves[k] = st.wolves[(int64_t)k * st.n + idx];
     __syncwarp();

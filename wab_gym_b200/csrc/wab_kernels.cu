@@ -98,7 +98,7 @@ __device__ __forceinline__ void load_env(const Params& P, const StatePtrs& st, i
     E.logsig = st.logsig[idx];
     { const uint2 bk = st.bkey[idx]; E.bk_a = bk.x; E.bk_b = bk.y; }
     E.food_f = F64 ? st.food[idx] : 0.0;
-    E.env_id = (uint32_t)(P.env_id_base + (uint64_t)idx);
+    E.env_id = (uint32_t)global_env_id(P, idx);
     WAB_ROLLED
     for (uint32_t k = 0; k < E.nw; ++k) wolves_s[k * wstride] = st.wolves[(int64_t)k * st.n + idx];
 }
@@ -720,8 +720,8 @@ __global__ void __launch_bounds__(256) wab_flatten_noisy_kernel(const __grid_con
         const uint32_t* vm = P.restrict_view ? (f[26] == 1 ? P.mask_gath : P.mask_look) : nullptr;
         uint32_t w[4] = {0u, 0u, 0u, 0u};
         int it = 0;
+        const uint64_t g = global_env_id(P, row);                  // the noise key: the row's global env id
         for (int k = lane; k < dim; k += 32, ++it) {
-            const uint64_t g = P.env_id_base + (uint64_t)row;      // the noise key: the row's global env id
             if (noisy && (it & 3) == 0)
                 philox(P, (uint32_t)g, (uint32_t)(g >> 32) ^ ((uint32_t)(it >> 2) << 24) ^ ((uint32_t)lane << 16), (uint32_t)ctr,
                        (uint32_t)(ctr >> 32) ^ 0x464C4154u, w);
@@ -997,6 +997,7 @@ struct WabVec {
     const void* g_actions; void* g_block; const void* g_features;
     bool graph_unsupported;
     int host_mapped;   // -1 unknown, 0 staged copies, 1 kernel writes the pinned host block directly
+    bool started;      // reset or loaded once: the replica layout is fixed from then on
     const void* m_actions; const void* m_block;        // host buffer pair whose device aliases are cached below
     const uint8_t* m_dactions; uint8_t* m_dblock;
     uint64_t fp_config;    // fingerprint of config, bush thresholds, seed and kernel kind (wab_state.cuh; ego folded in on query)
@@ -1286,6 +1287,7 @@ int wab_vec_reset(WabVec* h, const uint8_t* d_mask, WabObs obs, void* stream) {
     if (!h || !obs.d_food || !obs.d_role || !obs.d_status) return fail(WAB_E_NULL, "null argument");
     if (int rc = check_grids(h, obs.d_grids)) return rc;
     DeviceGuard guard(h->device);
+    h->started = true;
     OutPtrs out{obs.d_grids, obs.d_food, obs.d_role, obs.d_status, nullptr, nullptr, nullptr, h->d_features};
     cudaStream_t s = (cudaStream_t)stream;
     if (h->generic) {
@@ -1554,6 +1556,16 @@ int wab_vec_enable_ego(WabVec* h) {
     return WAB_OK;
 }
 
+int wab_vec_set_replicas(WabVec* h, int64_t n_replicas) {
+    if (!h) return fail(WAB_E_NULL, "null argument");
+    if (h->started) return fail(WAB_E_CONFIG, "call wab_vec_set_replicas before the first reset");
+    if (n_replicas < 1 || h->n % n_replicas != 0) return fail(WAB_E_CONFIG, "n_replicas must divide n_envs");
+    if (h->n > (int64_t)UINT32_MAX) return fail(WAB_E_CONFIG, "replicated handles hold fewer than 2^32 envs");
+    h->P.replica_envs = n_replicas == 1 ? 0u : (uint64_t)(h->n / n_replicas);
+    if (h->host_graph) { cudaGraphExecDestroy(h->host_graph); h->host_graph = nullptr; }   // captured with the old Params
+    return WAB_OK;
+}
+
 int wab_vec_ego_proximities(WabVec* h, uint8_t* d_out10, void* stream) {
     if (!h || !d_out10) return fail(WAB_E_NULL, "null argument");
     if (!h->d_hist) return fail(WAB_E_CONFIG, "call wab_vec_enable_ego before the first reset");
@@ -1683,13 +1695,18 @@ static int policy_trunk_launch(WabVec* h, const uint8_t* d_features, int64_t n_r
         WAB_CUDA(cudaFuncSetAttribute(wab_affine1_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOTAL));
         WAB_CUDA(cudaFuncSetAttribute(wab_affine1_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOTAL));
         WAB_CUDA(cudaFuncSetAttribute(wab_affine1_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOTAL));
+        WAB_CUDA(cudaFuncSetAttribute(wab_affine1_tc_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_TOTAL));
         attr_set[h->device] = true;
     }
     TrunkWeights tw;
     if (tail) tw = *tail; else memset(&tw, 0, sizeof(tw));
     tw.w2 = reinterpret_cast<const uint4*>(d_packed2); tw.b2 = d_bias2; tw.w3 = reinterpret_cast<const uint4*>(d_packed3); tw.b3 = d_bias3; tw.n2 = hidden2;
     const unsigned grid = (unsigned)((n_rows + TC_TILE_M - 1) / TC_TILE_M);
-    if (tail && tail->member_rows > 0)
+    if (tail && tail->member_rows > 0 && greedy)
+        wab_affine1_tc_kernel<5><<<grid, 256, TC_SMEM_TOTAL, (cudaStream_t)stream>>>(
+            h->P, d_features, n_rows, (int)h->cfg.food_obs_scale + 1, reinterpret_cast<const uint4*>(d_packed1), d_bias1, noise_scale,
+            leaky_slope, reinterpret_cast<const unsigned long long*>(d_counter), d_z3, tw);
+    else if (tail && tail->member_rows > 0)
         wab_affine1_tc_kernel<4><<<grid, 256, TC_SMEM_TOTAL, (cudaStream_t)stream>>>(
             h->P, d_features, n_rows, (int)h->cfg.food_obs_scale + 1, reinterpret_cast<const uint4*>(d_packed1), d_bias1, noise_scale,
             leaky_slope, reinterpret_cast<const unsigned long long*>(d_counter), d_z3, tw);
@@ -1734,25 +1751,54 @@ int wab_policy_forward(WabVec* h, const uint8_t* d_features, int64_t n_rows, con
                                leaky_slope, d_counter, d_z3, stream, &tw);
 }
 
+// wab_policy_forward_population (sample_seed given) and wab_policy_act_population (greedy, no seed): the checks they share,
+// then MODE 4 or MODE 5 through policy_trunk_launch
+static int policy_population_launch(const char* who, WabVec* h, const uint8_t* d_features, int32_t n_members,
+                                    int64_t member_rows, const void* d_packed1, const float* d_bias1, const void* d_packed2,
+                                    const float* d_bias2, int32_t hidden2, const void* d_packed3, const float* d_bias3,
+                                    const float* d_w_heads, const float* d_b_heads, int32_t n_actions, float noise_scale,
+                                    float leaky_slope, float clamp_lo, float clamp_hi, const uint64_t* sample_seed,
+                                    const uint64_t* d_counter, uint8_t* d_actions, float* d_value, float* d_probs, float* d_logp,
+                                    float* d_z3, void* stream) {
+    if (!d_w_heads || !d_b_heads || !d_actions) return fail(WAB_E_NULL, "null argument");
+    if (n_actions < 1 || n_actions > 8) return fail(WAB_E_CONFIG, "n_actions must be in [1, 8]");
+    if (n_members < 1 || n_members > 64) return fail(WAB_E_CONFIG, std::string(who) + ": 1 <= n_members <= 64");
+    if (member_rows < TC_TILE_M || member_rows % TC_TILE_M != 0)
+        return fail(WAB_E_CONFIG, std::string(who) + ": member_rows must be a positive multiple of 128");
+    TrunkWeights tw;
+    memset(&tw, 0, sizeof(tw));
+    if (sample_seed) {
+        uint32_t k0 = (uint32_t)*sample_seed, k1 = (uint32_t)(*sample_seed >> 32);
+        for (int r = 0; r < 10; ++r) { tw.rk0[r] = k0; tw.rk1[r] = k1; k0 += PHILOX_W0; k1 += PHILOX_W1; }
+    }
+    tw.w_heads = d_w_heads; tw.b_heads = d_b_heads; tw.n_actions = n_actions; tw.clamp_lo = clamp_lo; tw.clamp_hi = clamp_hi;
+    tw.actions = d_actions; tw.value = d_value; tw.probs = d_probs; tw.logp = d_logp; tw.member_rows = member_rows;
+    return policy_trunk_launch(h, d_features, (int64_t)n_members * member_rows, d_packed1, d_bias1, d_packed2, d_bias2, hidden2,
+                               d_packed3, d_bias3, noise_scale, leaky_slope, d_counter, d_z3, stream, &tw, !sample_seed);
+}
+
 int wab_policy_forward_population(WabVec* h, const uint8_t* d_features, int32_t n_members, int64_t member_rows,
                                   const void* d_packed1, const float* d_bias1, const void* d_packed2, const float* d_bias2,
                                   int32_t hidden2, const void* d_packed3, const float* d_bias3, const float* d_w_heads,
                                   const float* d_b_heads, int32_t n_actions, float noise_scale, float leaky_slope, float clamp_lo,
                                   float clamp_hi, uint64_t sample_seed, const uint64_t* d_counter, uint8_t* d_actions,
                                   float* d_value, float* d_probs, float* d_logp, float* d_z3, void* stream) {
-    if (!d_w_heads || !d_b_heads || !d_actions) return fail(WAB_E_NULL, "null argument");
-    if (n_actions < 1 || n_actions > 8) return fail(WAB_E_CONFIG, "n_actions must be in [1, 8]");
-    if (n_members < 1 || n_members > 64) return fail(WAB_E_CONFIG, "wab_policy_forward_population: 1 <= n_members <= 64");
-    if (member_rows < TC_TILE_M || member_rows % TC_TILE_M != 0)
-        return fail(WAB_E_CONFIG, "wab_policy_forward_population: member_rows must be a positive multiple of 128");
-    TrunkWeights tw;
-    memset(&tw, 0, sizeof(tw));
-    uint32_t k0 = (uint32_t)sample_seed, k1 = (uint32_t)(sample_seed >> 32);
-    for (int r = 0; r < 10; ++r) { tw.rk0[r] = k0; tw.rk1[r] = k1; k0 += PHILOX_W0; k1 += PHILOX_W1; }
-    tw.w_heads = d_w_heads; tw.b_heads = d_b_heads; tw.n_actions = n_actions; tw.clamp_lo = clamp_lo; tw.clamp_hi = clamp_hi;
-    tw.actions = d_actions; tw.value = d_value; tw.probs = d_probs; tw.logp = d_logp; tw.member_rows = member_rows;
-    return policy_trunk_launch(h, d_features, (int64_t)n_members * member_rows, d_packed1, d_bias1, d_packed2, d_bias2, hidden2,
-                               d_packed3, d_bias3, noise_scale, leaky_slope, d_counter, d_z3, stream, &tw);
+    return policy_population_launch("wab_policy_forward_population", h, d_features, n_members, member_rows, d_packed1, d_bias1,
+                                    d_packed2, d_bias2, hidden2, d_packed3, d_bias3, d_w_heads, d_b_heads, n_actions, noise_scale,
+                                    leaky_slope, clamp_lo, clamp_hi, &sample_seed, d_counter, d_actions, d_value, d_probs, d_logp,
+                                    d_z3, stream);
+}
+
+int wab_policy_act_population(WabVec* h, const uint8_t* d_features, int32_t n_members, int64_t member_rows,
+                              const void* d_packed1, const float* d_bias1, const void* d_packed2, const float* d_bias2,
+                              int32_t hidden2, const void* d_packed3, const float* d_bias3, const float* d_w_heads,
+                              const float* d_b_heads, int32_t n_actions, float noise_scale, float leaky_slope, float clamp_lo,
+                              float clamp_hi, const uint64_t* d_counter, uint8_t* d_actions, float* d_value, float* d_probs,
+                              float* d_logp, float* d_z3, void* stream) {
+    return policy_population_launch("wab_policy_act_population", h, d_features, n_members, member_rows, d_packed1, d_bias1,
+                                    d_packed2, d_bias2, hidden2, d_packed3, d_bias3, d_w_heads, d_b_heads, n_actions, noise_scale,
+                                    leaky_slope, clamp_lo, clamp_hi, nullptr, d_counter, d_actions, d_value, d_probs, d_logp,
+                                    d_z3, stream);
 }
 
 // wab_policy_forward's trunk and tail with the greedy action: the same checks, no sampling seed (MODE 3 reads no round keys)

@@ -211,7 +211,7 @@
             valid = valid && (flat % B.n_envs) / G.member_envs == G.member;
         if (!valid) flat = 0;
         const int64_t step = flat / B.n_envs;
-        const uint32_t krow = (uint32_t)(P.env_id_base + (uint64_t)(flat - step * B.n_envs));   // the noise key: the global env id
+        const uint32_t krow = (uint32_t)global_env_id(P, flat - step * B.n_envs);   // the noise key: the global env id
         const unsigned long long ctr = B.counters[step];
         // ---- the tile's one-hot bit vectors (as wab_affine1_tc_kernel)
         if (tid >= 128) {

@@ -161,8 +161,9 @@ struct TrunkWeights {
     const float* w_heads; const float* b_heads;   // f32[A + 1][128], f32[A + 1]: action_head stacked on value_head
     int n_actions; float clamp_lo, clamp_hi;
     uint8_t* actions; float* value; float* probs; float* logp;
-    // MODE 4 only — a population of policies (wab_policy_forward_population): rows [m member_rows, (m + 1) member_rows) take
-    // member m's weights, stacked per member at the strides below; member_rows is a multiple of TC_TILE_M
+    // MODES 4 and 5 only — a population of policies (wab_policy_forward_population, wab_policy_act_population): rows
+    // [m member_rows, (m + 1) member_rows) take member m's weights, stacked per member at the strides below; member_rows is
+    // a multiple of TC_TILE_M
     int64_t member_rows;
 };
 // per-member strides of the stacked packed weights, in uint4: wab_policy_affine1_packed_bytes() / 16 and
@@ -171,7 +172,8 @@ struct TrunkWeights {
 constexpr int64_t POP_W1_U4 = (int64_t)TC_CHUNKS * 3 * TC_PART_BYTES / 16, POP_LINEAR_U4 = 3 * 160 * 128 * 2 / 16;
 // MODE 0: first layer only; 1: the trunk (out = z3); 2: trunk + tail (clamp, both heads, softmax, Categorical sample; out = z3 or null);
 // 3: MODE 2 with the greedy action (the first index of the largest logit) instead of the sample: no Philox call, the round keys unread;
-// 4: MODE 2 for a population: the CTA's rows are member row0 / member_rows's, and every weight pointer moves to that member's
+// 4: MODE 2 for a population: the CTA's rows are member row0 / member_rows's, and every weight pointer moves to that member's;
+// 5: MODE 4 with MODE 3's greedy action
 template <int MODE>
 __global__ void __launch_bounds__(256, 2)
 wab_affine1_tc_kernel(const __grid_constant__ Params P, const uint8_t* __restrict__ features, int64_t rows, int food_dim,
@@ -184,7 +186,7 @@ wab_affine1_tc_kernel(const __grid_constant__ Params P, const uint8_t* __restric
     const uint32_t s_a = s_base + TC_SMEM_A, s_b = s_base + TC_SMEM_B, s_bar = s_base + TC_SMEM_BAR;
     uint32_t* rowbits = reinterpret_cast<uint32_t*>(tc_smem + TC_SMEM_BITS);
     const int64_t row0 = (int64_t)blockIdx.x * TC_TILE_M;
-    if constexpr (MODE == 4) {                            // a CTA never straddles two members: member_rows % TC_TILE_M == 0
+    if constexpr (MODE == 4 || MODE == 5) {               // a CTA never straddles two members: member_rows % TC_TILE_M == 0
         const int64_t m = row0 / tw.member_rows, n_out = tw.n_actions + 1;
         wpacked += m * POP_W1_U4; bias += m * TC_N;
         tw.w2 += m * POP_LINEAR_U4; tw.b2 += m * tw.n2; tw.w3 += m * POP_LINEAR_U4; tw.b3 += m * TC_N;
@@ -256,7 +258,7 @@ wab_affine1_tc_kernel(const __grid_constant__ Params P, const uint8_t* __restric
         // as wab_flatten_noisy_kernel computes it; parts o (one-hot), n0, n1 (the noise x - o in two bf16 terms)
         float x[4][8];
         const int jb = 16 * (c & 1) + 8 * h;              // this thread's lanes j = jb .. jb + 7 of the chunk's Philox calls
-        const uint64_t g = P.env_id_base + (uint64_t)row; // the noise key: the row's global env id
+        const uint64_t g = global_env_id(P, row);         // the noise key: the row's global env id
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
             uint32_t w[4] = {0u, 0u, 0u, 0u};
@@ -456,7 +458,7 @@ wab_affine1_tc_kernel(const __grid_constant__ Params P, const uint8_t* __restric
         if (MODE >= 2) {
             // ---- the tail: x = clamp(leaky_relu(z3)); the A + 1 head rows as two 64-term partial sums per row (the two threads
             // of a row meet in shared memory — the operand area is free now); softmax; inverse-CDF sample on one keyed uniform
-            // (MODES 2 and 4) or the greedy action (MODE 3)
+            // (MODES 2 and 4) or the greedy action (MODES 3 and 5)
             // head weights transposed and zero-padded to [128][12]: the 9 weights of an input are three 16-byte broadcast loads
             float* wsm = reinterpret_cast<float*>(tc_smem);               // [128][12]
             float* partial = wsm + 12 * 128;                              // [128 rows][2 halves][9]
@@ -496,7 +498,7 @@ wab_affine1_tc_kernel(const __grid_constant__ Params P, const uint8_t* __restric
                 float p_pick = 0.f;
                 int pick = A - 1;
                 if constexpr (MODE == 2 || MODE == 4) {
-                    const uint64_t g = P.env_id_base + (uint64_t)row;    // the sampling key: the row's global env id
+                    const uint64_t g = global_env_id(P, row);            // the sampling key: the row's global env id
                     uint32_t c0 = (uint32_t)(g >> 2), c1 = (uint32_t)(g >> 34), c2 = (uint32_t)ctr, c3 = (uint32_t)(ctr >> 32) ^ 0x53414D50u;
 #pragma unroll
                     for (int rd = 0; rd < 10; ++rd) {                     // Philox4x32-10 under the sampling seed's round keys

@@ -56,7 +56,7 @@ __global__ void __launch_bounds__(kStateThreads) wab_save_state_kernel(const __g
         uint32_t* r = srec + e * g.sw;
         const uint32_t pos = st.pos[idx], misc = st.misc[idx], nl = st.nlog[idx];
         const uint32_t nw = ((misc >> 11) & 15u) | (((nl >> 9) & 7u) << 4), nlog = nl & 0xFFu, turn = misc >> 16;
-        const uint64_t env_id = P.env_id_base + (uint64_t)idx;
+        const uint64_t env_id = global_env_id(P, idx);
         r[RW_FORMAT] = WAB_STATE_FORMAT; r[RW_FLAGS] = (nl >> 8) & 1u;
         r[RW_FP] = (uint32_t)fp; r[RW_FP + 1] = (uint32_t)(fp >> 32);
         r[RW_ENV_ID] = (uint32_t)env_id; r[RW_ENV_ID + 1] = (uint32_t)(env_id >> 32);
@@ -241,6 +241,7 @@ int wab_vec_load_state(WabVec* h, const void* d_records, const int32_t* d_slots,
         if (int rc = check_grids(h, obs.d_grids)) return rc;
     }
     DeviceGuard guard(h->device);
+    h->started = true;
     cudaStream_t s = (cudaStream_t)stream;
     WAB_CUDA(cudaMemsetAsync(d_rejected, 0, sizeof(int32_t), s));
     if (n > 0) {

@@ -16,15 +16,19 @@ With ``group`` (a ``torch.distributed`` process group) each rank evaluates its c
 (``sharding.shard_range``) and the results are all-gathered in rank order, so every rank returns the same ``EvalResult``.
 Policy draws are keyed by the global env id, so it equals a single-process evaluation of all envs bit for bit, sampled
 evaluation included. Every rank must pass the same weights.
+
+``PopulationEvaluator`` scores P policies at once on ``VecEnv(P n, replicas=P)``: every block of n envs repeats the
+global ids ``env_id_base ..``, so member p plays exactly the episodes ``Evaluator(n)`` plays, in one launch per step for
+all members.
 """
 from __future__ import annotations
 
-from typing import Dict, NamedTuple, Optional
+from typing import Dict, List, NamedTuple, Optional
 
 import torch
 
 from . import sharding
-from .policy import Policy, PolicyTrunkTC, check_reference_network, stacked_heads
+from .policy import Policy, PolicyPopulationTC, PolicyTrunkTC, check_reference_network, stacked_heads
 from .vec_env import VecEnv
 
 
@@ -96,6 +100,8 @@ def check_policy(policy, flat_dim: int) -> None:
 
 
 class Evaluator:
+    _replicas = 1      # PopulationEvaluator: its members' copies of the env block
+
     def __init__(self, num_envs: int, game_options: Optional[dict] = None, seed: int = 0, device="cuda",
                  env_id_base: int = 0, episodes_per_env: int = 1, group=None):
         """``num_envs`` environments with global ids ``env_id_base ..`` (with ``group``: over all ranks together),
@@ -112,7 +118,7 @@ class Evaluator:
                 raise ValueError("Evaluator over %d ranks needs at least one env per rank, got %d envs" % (world, self.num_envs))
             first, count = sharding.shard_range(self.num_envs, dist.get_rank(self.group), world)
         self.env = VecEnv(count, game_options=game_options, device=device, seed=seed, env_id_base=int(env_id_base) + first,
-                          features=True, emit_grids=False)
+                          features=True, emit_grids=False, replicas=self._replicas)
         self.flat_dim, self.n_actions = self.env.flat_dim, self.env.n_actions
         self.max_turns = int(self.env.game_options["max_turns"])
         self.steps = self.episodes_per_env * self.max_turns
@@ -136,6 +142,7 @@ class Evaluator:
         self._count = torch.empty(N, dtype=torch.int64, device=dev)
         self._first = torch.empty(self.episodes_per_env + 1, N, 28, dtype=torch.uint8, device=dev)   # row k: later episodes
         self._cols = torch.arange(N, device=dev)
+        self._slots = torch.arange(N)
         self._policy = self._tc = self._heads = None
 
     def restore(self, policy) -> None:
@@ -154,8 +161,19 @@ class Evaluator:
                 mine.bias.copy_(theirs.bias.detach())
         self._tc.refresh()
         self._heads = stacked_heads(self._policy)
-        self.env.load_state(self._start)
+        self._rewind()
+
+    def _rewind(self) -> None:
+        self.env.load_state(self._start, slots=self._slots)
         self._ctr.zero_()
+
+    def _act(self, greedy: bool, scale: float) -> None:
+        """One step's actions into ``self._actions``: the one launch of the step loop that depends on the policy."""
+        if greedy:
+            self._tc.forward_greedy(self.env.last_features, self._heads, self._actions, noise_scale=scale, counter=self._ctr)
+        else:
+            self._tc.forward_sample(self.env.last_features, self._heads, self._actions, noise_scale=scale, counter=self._ctr,
+                                    seed=self.sample_seed)
 
     @torch.no_grad()
     def play(self, greedy: bool = True, noise: bool = True):
@@ -164,17 +182,13 @@ class Evaluator:
         synchronises with the host."""
         if self._tc is None:
             raise RuntimeError("play() follows restore(policy)")
-        env, tc, k = self.env, self._tc, self.episodes_per_env
+        env, k = self.env, self.episodes_per_env
         scale = 0.01 if noise else 0.0
         self._count.zero_()
         self._first[0].copy_(env.last_features)
         for t in range(self.steps):
             self._ctr += 1
-            if greedy:
-                tc.forward_greedy(env.last_features, self._heads, self._actions, noise_scale=scale, counter=self._ctr)
-            else:
-                tc.forward_sample(env.last_features, self._heads, self._actions, noise_scale=scale, counter=self._ctr,
-                                  seed=self.sample_seed)
+            self._act(greedy, scale)
             _, reward, done, info = env.step(self._actions)
             self._reward[t].copy_(reward)
             self._done[t].copy_(done)
@@ -190,10 +204,7 @@ class Evaluator:
         without. Returns the per-episode results on the host, the same on every rank. ``policy`` (any device) and any
         trainer that owns it are left untouched."""
         self.restore(policy)
-        reward, done, info = self.play(greedy, noise)
-        returns, lengths, outcome, eats = first_episodes(reward, done, info, self.episodes_per_env)
-        first = self._first[:self.episodes_per_env].transpose(0, 1).contiguous()
-        parts = [t.cpu() for t in (returns, lengths, outcome, eats, first)]
+        parts = self._episodes(*self.play(greedy, noise))
         if self.group is not None:
             import torch.distributed as dist
             gathered = [None] * dist.get_world_size(self.group)
@@ -201,5 +212,70 @@ class Evaluator:
             parts = [torch.cat([g[i] for g in gathered]) for i in range(len(parts))]
         return EvalResult(*parts)
 
+    def _episodes(self, reward, done, info):
+        """The five per-episode tensors of ``EvalResult`` of the record ``play`` left, on the host."""
+        returns, lengths, outcome, eats = first_episodes(reward, done, info, self.episodes_per_env)
+        first = self._first[:self.episodes_per_env].transpose(0, 1).contiguous()
+        return [t.cpu() for t in (returns, lengths, outcome, eats, first)]
+
     def close(self):
         self.env.close()
+
+
+class PopulationEvaluator(Evaluator):
+    """P policies scored on the same episodes in one launch per step. It owns ``VecEnv(P n, replicas=P)``: block p of n
+    envs replays the world draws of ``Evaluator(n, ...)``'s envs, member p acts on it through its row block of one
+    ``PolicyPopulationTC`` (``wab_policy_act_population`` or ``wab_policy_forward_population``), and every policy draw
+    is keyed as that evaluator keys it. So ``evaluate(policies)[p]`` equals ``Evaluator(n, game_options, seed, env_id_base,
+    episodes_per_env).evaluate(policies[p])`` bit for bit, and the P results line up episode by episode (common random
+    numbers: what separates close policies such as the members of a population-based training run). ``envs_per_member``
+    = n is a multiple of 128, 1 <= ``members`` <= 64. Data-parallel evaluation (``group``) is not supported."""
+
+    def __init__(self, members: int, envs_per_member: int, game_options: Optional[dict] = None, seed: int = 0,
+                 device="cuda", env_id_base: int = 0, episodes_per_env: int = 1, group=None):
+        P, n = int(members), int(envs_per_member)
+        if group is not None:
+            raise ValueError("PopulationEvaluator is single-process: data-parallel evaluation (group) is not supported")
+        if not 1 <= P <= 64:
+            raise ValueError("a population has 1 to 64 members")
+        if n < 128 or n % 128 != 0:
+            raise ValueError("PopulationEvaluator needs envs_per_member a positive multiple of 128, got %d" % n)
+        self.members, self.envs_per_member, self._replicas = P, n, P
+        super().__init__(P * n, game_options=game_options, seed=seed, device=device, env_id_base=env_id_base,
+                         episodes_per_env=episodes_per_env)
+        self._policies = None
+
+    def restore(self, policies) -> None:
+        """``Evaluator.restore`` for P policies: each one's weights copied into this evaluator's own member and packed."""
+        policies = list(policies)
+        if len(policies) != self.members:
+            raise ValueError("evaluate needs one policy per member (%d), got %d" % (self.members, len(policies)))
+        for pol in policies:
+            check_policy(pol, self.flat_dim)
+        A = policies[0].action_head.out_features
+        if any(pol.action_head.out_features != A for pol in policies):
+            raise ValueError("every member of a population has the same action count")
+        if self._policies is None or self._tc.n_actions != A:
+            with torch.random.fork_rng(devices=[]):                     # the initialisation draws stay off the global RNG
+                self._policies = [Policy(self.flat_dim, A).to(self.env.device) for _ in range(self.members)]
+            self._tc = PolicyPopulationTC(self.env, self._policies)
+        with torch.no_grad():
+            for mine, theirs in zip(self._policies, policies):
+                for a, b in zip(mine.parameters(), theirs.parameters()):
+                    a.copy_(b.detach())
+        self._tc.refresh()
+        self._rewind()
+
+    def _act(self, greedy: bool, scale: float) -> None:
+        # the buffers are this evaluator's own and restore() packed every member: the launch alone
+        self._tc._launch(None if greedy else self.sample_seed, self.env.last_features, self._actions, None, None, None, None,
+                         scale, self._ctr, 0.01)
+
+    def evaluate(self, policies, greedy: bool = True, noise: bool = True) -> List[EvalResult]:
+        """``Evaluator.evaluate`` of every member at once: ``results[p]`` is ``policies[p]``'s ``EvalResult`` over the n
+        envs of block p, whose global ids ``env_id_base ..`` are the same in every block. The policies are only read."""
+        self.restore(policies)
+        parts = self._episodes(*self.play(greedy, noise))
+        P, n = self.members, self.envs_per_member
+        split = [t.view(P, n, *t.shape[1:]) for t in parts]
+        return [EvalResult(*(t[p] for t in split)) for p in range(P)]

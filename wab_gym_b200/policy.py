@@ -417,6 +417,33 @@ class PolicyPopulationTC:
         """``PolicyTrunkTC.forward_sample`` for the N = P n rows of ``features`` u8[N, 28], row r under member r // n's
         weights, in ONE launch. Fills ``actions`` u8[N] (and ``value`` f32[N], ``probs`` f32[N, A], ``logp`` f32[N],
         ``z3`` f32[N, 128] when given)."""
+        self._check_forward(features, actions, value, probs, logp, z3, counter)
+        return self._launch(int(seed), features, actions, value, probs, logp, z3, noise_scale, counter, slope)
+
+    def forward_greedy(self, features: torch.Tensor, actions: torch.Tensor, value: Optional[torch.Tensor] = None,
+                       probs: Optional[torch.Tensor] = None, logp: Optional[torch.Tensor] = None, noise_scale: float = 0.01,
+                       counter: Optional[torch.Tensor] = None, z3: Optional[torch.Tensor] = None,
+                       slope: float = 0.01) -> torch.Tensor:
+        """``PolicyTrunkTC.forward_greedy`` for every member in ONE launch (``wab_policy_act_population``): row r's action is
+        the argmax of member r // n's logits; the arguments and their checks are ``forward_sample``'s, without a seed."""
+        self._check_forward(features, actions, value, probs, logp, z3, counter)
+        return self._launch(None, features, actions, value, probs, logp, z3, noise_scale, counter, slope)
+
+    def _launch(self, seed, features, actions, value, probs, logp, z3, noise_scale, counter, slope):
+        """The launch of ``forward_sample`` (``seed`` given) or ``forward_greedy`` (``seed`` None) without the checks and
+        the re-pack: for a caller that checked its own buffers and packed its members once (``PopulationEvaluator``)."""
+        common = (self.env._h, _ptr(features), self.n_members, self.member_envs, _ptr(self.packed1), _ptr(self.bias1),
+                  _ptr(self.packed2), _ptr(self.bias2), 150, _ptr(self.packed3), _ptr(self.bias3), _ptr(self.w_heads),
+                  _ptr(self.b_heads), self.n_actions, float(noise_scale), float(slope), -4.0, 4.0)
+        outs = (_ptr(counter), _ptr(actions), _ptr(value), _ptr(probs), _ptr(logp), _ptr(z3), self._stream())
+        if seed is None:
+            _lib.check(self.lib.wab_policy_act_population(*common, *outs))
+        else:
+            _lib.check(self.lib.wab_policy_forward_population(*common, seed & (2 ** 64 - 1), *outs))
+        return actions
+
+    def _check_forward(self, features, actions, value, probs, logp, z3, counter):
+        """The argument checks of the forward calls, then a re-pack of the members whose weights changed."""
         N, A = self.n_members * self.member_envs, self.n_actions
         if tuple(features.shape) != (N, 28) or features.dtype != torch.uint8 or not features.is_contiguous():
             raise ValueError("features must be a contiguous uint8 [P n, 28] tensor")
@@ -430,12 +457,6 @@ class PolicyPopulationTC:
             if t is not None and t.device != self.env.device:
                 raise ValueError("%s must be on the environment's device" % name)
         self._refresh_stale()
-        _lib.check(self.lib.wab_policy_forward_population(
-            self.env._h, _ptr(features), self.n_members, self.member_envs, _ptr(self.packed1), _ptr(self.bias1),
-            _ptr(self.packed2), _ptr(self.bias2), 150, _ptr(self.packed3), _ptr(self.bias3), _ptr(self.w_heads),
-            _ptr(self.b_heads), A, float(noise_scale), float(slope), -4.0, 4.0, int(seed) & (2 ** 64 - 1), _ptr(counter),
-            _ptr(actions), _ptr(value), _ptr(probs), _ptr(logp), _ptr(z3), self._stream()))
-        return actions
 
     def ppo_backward(self, features: torch.Tensor, counters: torch.Tensor, actions: torch.Tensor, logp_old: torch.Tensor,
                      advantage: torch.Tensor, target: torch.Tensor, rows: torch.Tensor, counts: torch.Tensor, coefs,

@@ -84,6 +84,8 @@ class PPOPopulation:
             raise ValueError("PPOPopulation needs num_envs = members * n with n a multiple of 128 (got %d envs, %d members)" % (N, P))
         if not env.with_features:
             raise ValueError("PPOPopulation needs VecEnv(features=True)")
+        if getattr(env, "replicas", 1) > 1:
+            raise ValueError("PPOPopulation refuses a VecEnv with replicas: its members own distinct env ids")
         n = N // P
         if epochs < 1 or minibatches < 1 or int(horizon) * n < minibatches:
             raise ValueError("PPOPopulation needs epochs >= 1 and 1 <= minibatches <= horizon * n")
@@ -233,6 +235,18 @@ class PPOPopulation:
         self.iteration = int(sd["iteration"])
         self._set_discounts()
         self._tc.refresh()
+
+    def set_member_hyperparameters(self, p: int, hp: Dict[str, float]):
+        """Member p's hyper-parameters: the keys of ``hp`` replace p's (the others stay), validated as the constructor
+        validates them, and written everywhere they live: the dict, the lr of p's Adam and the GAE discounts. (After
+        ``load_member_state_dict(p, member_state_dict(q))`` p's Adam holds q's lr, so this is the explore step of
+        population-based training.)"""
+        self._member_slots(p)
+        full = member_hyperparameters([{**self.hyperparameters[p], **hp}], 1)[0]
+        self.hyperparameters[p] = full
+        for group in self.optimizers[p].param_groups:
+            group["lr"] = full["lr"]
+        self._set_discounts()
 
     def _member_slots(self, p: int) -> torch.Tensor:
         if not 0 <= p < self.n_members:

@@ -58,7 +58,8 @@ def _ptr(t: Optional[torch.Tensor]):
 class VecEnv:
     def __init__(self, num_envs: int, game_options: Optional[dict] = None, device="cuda", seed: int = 0,
                  env_id_base: int = 0, auto_reset: bool = True, wolf_cap: int = 16, log_cap: Optional[int] = None,
-                 force_f64_food: bool = False, features: bool = False, ego: bool = False, emit_grids: bool = True):
+                 force_f64_food: bool = False, features: bool = False, ego: bool = False, emit_grids: bool = True,
+                 replicas: int = 1):
         self._h = None
         self._bound = None     # feature buffer currently bound in the handle
         self.lib = _lib.load()  # raises if the CUDA library is unavailable — no fallback
@@ -77,6 +78,13 @@ class VecEnv:
         #: specialised kernels, every other odd size up to 31 x 31 (margins 1, 2) on the warp-per-env generic ones
         self.view = (int(self.game_options["width"]), int(self.game_options["height"]))
         self.seed, self.env_id_base = int(seed), int(env_id_base)
+        #: replicas = R > 1: the N envs are R copies of n = N / R envs. Row r has global env id env_id_base + r % n in every
+        #: draw keyed by the global id (world, policy noise and samples), so block k, driven by its own actions, plays what
+        #: VecEnv(n, env_id_base=env_id_base) plays: R policies can be scored on the same episodes side by side. The ids are
+        #: not unique, so state_dict / load_state_dict and load_state without slots refuse such a handle, as do the trainers.
+        self.replicas = int(replicas)
+        if self.replicas < 1 or self.num_envs % self.replicas != 0:
+            raise ValueError("replicas must divide num_envs (got %d envs, %d replicas)" % (self.num_envs, self.replicas))
         cs = self.game.to_struct()
         thr = np.ascontiguousarray(self.game.bush_thr, dtype=np.uint32)
         handle = ctypes.c_void_p()
@@ -84,6 +92,8 @@ class VecEnv:
                                            self.seed & 0xFFFFFFFFFFFFFFFF, self.env_id_base, self.device.index,
                                            ctypes.byref(handle)))
         self._h = handle
+        if self.replicas > 1:
+            _lib.check(self.lib.wab_vec_set_replicas(self._h, self.replicas))
         self.lanes_per_env = int(self.lib.wab_vec_lanes_per_env(self._h))
         self.generic_kernels = bool(self.lib.wab_vec_kernel_kind(self._h))
         self.with_ego = bool(ego)
@@ -347,7 +357,7 @@ class VecEnv:
 
     def save_state(self, slots=None) -> EnvStates:
         """The state of every env (or of ``slots``, in that order) as records on the device. Enqueued on the current
-        stream; nothing synchronises."""
+        stream; nothing synchronises. On a handle with replicas the ids repeat: block k's records carry block 0's ids."""
         if slots is None:
             local, d_slots = torch.arange(self.num_envs, dtype=torch.int64), None
         else:
@@ -355,7 +365,7 @@ class VecEnv:
             d_slots = local.to(device=self.device, dtype=torch.int32)
         records = torch.empty((local.numel(), self.record_bytes), dtype=torch.uint8, device=self.device)
         _lib.check(self.lib.wab_vec_save_state(self._h, _ptr(d_slots), local.numel(), _ptr(records), self._stream()))
-        return EnvStates(records, local + self.env_id_base, self.fingerprint)
+        return EnvStates(records, local % (self.num_envs // self.replicas) + self.env_id_base, self.fingerprint)
 
     def load_state(self, states: EnvStates, slots=None) -> ObsBatch:
         """Write each record of ``states`` into a slot: the slot of its own global id (which must belong to this handle),
@@ -363,6 +373,8 @@ class VecEnv:
         check passes before anything is written; a refused load raises ``ValueError`` and changes nothing. Returns the
         observation of every env, as ``reset`` with an empty mask would (``last_features`` is updated too). Synchronises
         once, to read the device-side verdict."""
+        if slots is None and self.replicas > 1:
+            raise ValueError("a handle with replicas repeats its env ids: load_state needs slots")
         records = states.records
         if records.dtype != torch.uint8 or records.dim() != 2 or records.shape[1] != self.record_bytes:
             raise ValueError("records must be uint8 [n, %d] for this handle" % self.record_bytes)
@@ -400,6 +412,7 @@ class VecEnv:
     def state_dict(self) -> dict:
         """Everything a resume needs, on the host (``torch.save`` works): format, fingerprint, global env ids, the records
         and the 8 statistics totals. ``sharding.merge_state_dicts`` joins the dicts of several shards."""
+        self._refuse_replicas("state_dict")
         st = self.save_state()
         stats = self.stats()
         return {"format": STATE_FORMAT, "fingerprint": st.fingerprint, "env_ids": st.env_ids.clone(),
@@ -409,6 +422,7 @@ class VecEnv:
         """Resume from ``state_dict()`` output (of this or any other shard layout: the records of this handle's global ids
         are picked, each exactly once). The statistics totals go to the shard holding env 0 and every other shard starts
         from zero, so their sum is preserved."""
+        self._refuse_replicas("load_state_dict")
         from .sharding import select_shard_records
         records = select_shard_records(sd, self.env_id_base, self.num_envs, self.fingerprint, self.record_bytes)
         ids = torch.arange(self.env_id_base, self.env_id_base + self.num_envs, dtype=torch.int64)
@@ -418,6 +432,11 @@ class VecEnv:
             stats[:] = torch.as_tensor(sd["stats"], dtype=torch.int64).numpy()
         _lib.check(self.lib.wab_vec_set_stats(self._h, stats.ctypes.data, self._stream()))
         return obs
+
+    def _refuse_replicas(self, what: str):
+        if self.replicas > 1:
+            raise ValueError("%s needs unique env ids; this handle has %d replicas (use save_state / load_state with slots)"
+                             % (what, self.replicas))
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:
