@@ -246,7 +246,7 @@ int wab_vec_flat_dim(const WabVec *h);
  *
  * Keying contract of the policy entry points: every one that takes a WabVec handle (wab_vec_flatten_features_noisy,
  * wab_policy_affine1, wab_policy_trunk, wab_policy_forward, wab_policy_act, wab_policy_backward, wab_policy_ppo_backward,
- * wab_policy_evaluate, wab_policy_backward_logits and the population calls) keys its noise and its action samples by the global env id env_id_base + row (the row within its step for the backward passes; env_id_base + row % n on a handle with replicas, wab_vec_set_replicas), so
+ * wab_policy_evaluate, wab_policy_backward_logits and the population calls) keys its noise and its action samples by the global env id env_id_base + row (the row within its step for the backward passes; env_id_base + row % n on a handle with replicas, wab_vec_set_replicas, and the block's id on a blocked handle, wab_vec_set_blocks), so
  * a shard [first, first + count) draws exactly what the unsharded batch draws for rows first .. first + count - 1;
  * outputs stay indexed by the local row. The two handle-less calls, wab_sample_categorical and wab_policy_tail, know no
  * shard and key by the local row. */
@@ -280,6 +280,16 @@ int wab_vec_ego_proximities(WabVec *h, uint8_t *d_out10, void *stream);
  * state fingerprint is unchanged: a record is valid on either kind of handle, and the slot it is loaded into decides its
  * ids. */
 int wab_vec_set_replicas(WabVec *h, int64_t n_replicas);
+
+/* Blocks: the handle's N envs become n_blocks blocks of c = N / n_blocks envs, and row r = k c + j takes the global env id
+ * env_id_base + k block_stride + j in every draw keyed by the global id (the same sites as for replicas). So block k,
+ * driven by an action stream, plays exactly what a handle of c envs at env_id_base + k block_stride plays: a rank of a
+ * data-parallel population holds every member's shard of ids on one handle. block_stride = 0 is wab_vec_set_replicas(h,
+ * n_blocks); n_blocks = 1 is the plain handle. Valid only before the first reset (or load); WAB_E_CONFIG for n_blocks < 1,
+ * a count that does not divide n_envs, a negative block_stride or 0 < block_stride < N / n_blocks (the blocks' ids would
+ * overlap), a layout whose last id lies 2^32 or more past env_id_base ((n_blocks - 1) block_stride + N / n_blocks > 2^32),
+ * n_envs >= 2^32, or a handle already reset. The state fingerprint is unchanged. */
+int wab_vec_set_blocks(WabVec *h, int64_t n_blocks, int64_t block_stride);
 
 /* The first layer of the reference's Policy on the tensor cores (actor_critic.py:59, :88-90, :188-189), fp32 accuracy:
  * d_out f32[n_rows][128] = leaky_relu(affine1(flatten(obs) + noise_scale * U[0,1))) straight from the 28 feature bytes per
@@ -487,6 +497,16 @@ int wab_policy_backward_logits(WabVec *h, const uint8_t *d_features, int64_t n_s
 int wab_policy_backward_grad_f64(WabVec *h, const void *d_scratch, int64_t scratch_bytes, int32_t n_actions,
                                  double *d_grad64, void *stream);
 int wab_policy_grad_sum_ranks(const double *d_rank_grads, int32_t n_ranks, int64_t n, float *d_grad, void *stream);
+/* wab_policy_backward_grad_f64 for a population: reduces the scratch left by the last wab_policy_ppo_backward_population of
+ * n_members members with this d_scratch on this stream into d_grad64 f64[n_members][stride], stride =
+ * wab_policy_population_grad_stride(h, n_actions), in the same element order as that call's d_grad, the fp64 sums not
+ * rounded; the padding entries of every row are written as 0. With one rank, wab_policy_grad_sum_ranks over n =
+ * n_members stride elements equals wab_policy_ppo_backward_population's d_grad bit for bit on every parameter.
+ * WAB_E_NULL for a missing pointer; WAB_E_CONFIG for n_members outside [1, 64], misalignment (16 bytes for d_scratch, 8
+ * for d_grad64) or a scratch smaller than wab_policy_backward_population_scratch_bytes(h, n_members); WAB_E_UNSUPPORTED
+ * beyond 8 actions or flat_dim > 512. */
+int wab_policy_backward_population_grad_f64(WabVec *h, const void *d_scratch, int64_t scratch_bytes, int32_t n_members,
+                                            int32_t n_actions, double *d_grad64, void *stream);
 
 /* The tail of the reference's Policy.forward + select_action (actor_critic.py:84-97, :108-125) for n_rows rows in one
  * pass, fp32: d_z3 f32[n_rows][128] is the PRE-activation output of affine3; x = clamp(leaky_relu(z3), lo, hi);

@@ -17,9 +17,9 @@ EXPORTS = [
     "wab_vec_create", "wab_vec_reset", "wab_vec_step", "wab_vec_step_many", "wab_vec_step_host",
     "wab_vec_reset_host", "wab_vec_stats", "wab_vec_stats_device", "wab_vec_export_state", "wab_vec_num_envs", "wab_vec_lanes_per_env", "wab_vec_step_many_pipelined", "wab_vec_kernel_kind",
     "wab_vec_destroy", "wab_philox_device", "wab_vec_bind_features", "wab_pragmatic_features",
-    "wab_vec_flatten_features", "wab_vec_flatten_features_noisy", "wab_sample_categorical", "wab_policy_tail", "wab_vec_enable_ego", "wab_vec_set_replicas", "wab_vec_ego_proximities", "wab_vec_flat_dim", "wab_vec_host_block_layout", "wab_vec_step_host_packed", "wab_vec_forget_host_buffers",
+    "wab_vec_flatten_features", "wab_vec_flatten_features_noisy", "wab_sample_categorical", "wab_policy_tail", "wab_vec_enable_ego", "wab_vec_set_replicas", "wab_vec_set_blocks", "wab_vec_ego_proximities", "wab_vec_flat_dim", "wab_vec_host_block_layout", "wab_vec_step_host_packed", "wab_vec_forget_host_buffers",
     "wab_vec_state_record_bytes", "wab_vec_state_fingerprint", "wab_vec_save_state", "wab_vec_load_state", "wab_vec_set_stats",
-    "wab_policy_affine1_packed_bytes", "wab_policy_affine1_prepare", "wab_policy_affine1", "wab_policy_linear_packed_bytes", "wab_policy_linear_prepare", "wab_policy_trunk", "wab_policy_forward", "wab_policy_act", "wab_policy_backward_scratch_bytes", "wab_policy_backward", "wab_policy_ppo_backward", "wab_policy_evaluate", "wab_policy_backward_logits", "wab_policy_backward_grad_f64", "wab_policy_grad_sum_ranks", "wab_policy_forward_population", "wab_policy_act_population", "wab_policy_backward_population_scratch_bytes", "wab_policy_population_grad_stride", "wab_policy_ppo_backward_population", "wab2_create", "wab2_kernel_kind", "wab2_output_layout", "wab2_reset", "wab2_turn", "wab2_export_state", "wab2_import_state", "wab2_destroy", "wab_last_error", "wab_abi_version",
+    "wab_policy_affine1_packed_bytes", "wab_policy_affine1_prepare", "wab_policy_affine1", "wab_policy_linear_packed_bytes", "wab_policy_linear_prepare", "wab_policy_trunk", "wab_policy_forward", "wab_policy_act", "wab_policy_backward_scratch_bytes", "wab_policy_backward", "wab_policy_ppo_backward", "wab_policy_evaluate", "wab_policy_backward_logits", "wab_policy_backward_grad_f64", "wab_policy_grad_sum_ranks", "wab_policy_backward_population_grad_f64", "wab_policy_forward_population", "wab_policy_act_population", "wab_policy_backward_population_scratch_bytes", "wab_policy_population_grad_stride", "wab_policy_ppo_backward_population", "wab2_create", "wab2_kernel_kind", "wab2_output_layout", "wab2_reset", "wab2_turn", "wab2_export_state", "wab2_import_state", "wab2_destroy", "wab_last_error", "wab_abi_version",
 ]
 
 
@@ -87,6 +87,7 @@ def load():
     L.wab_policy_tail.argtypes = [vp, i32, vp, vp, i64, i32, ctypes.c_float, ctypes.c_float, ctypes.c_float, u64, vp, vp, vp, vp, vp, vp]
     L.wab_vec_enable_ego.argtypes = [vp]
     L.wab_vec_set_replicas.argtypes = [vp, i64]
+    L.wab_vec_set_blocks.argtypes = [vp, i64, i64]
     L.wab_vec_ego_proximities.argtypes = [vp, vp, vp]
     L.wab_vec_flat_dim.argtypes = [vp]
     L.wab_vec_flat_dim.restype = i32
@@ -115,6 +116,7 @@ def load():
                                              i32, f32, f32, f32, f32, vp, i64, vp, vp]
     L.wab_policy_backward_grad_f64.argtypes = [vp, vp, i64, i32, vp, vp]
     L.wab_policy_grad_sum_ranks.argtypes = [vp, i32, i64, vp, vp]
+    L.wab_policy_backward_population_grad_f64.argtypes = [vp, vp, i64, i32, i32, vp, vp]
     L.wab_policy_forward_population.argtypes = [vp, vp, i32, i64, vp, vp, vp, vp, i32, vp, vp, vp, vp, i32, f32, f32, f32, f32, u64,
                                                 vp, vp, vp, vp, vp, vp, vp]
     L.wab_policy_act_population.argtypes = [vp, vp, i32, i64, vp, vp, vp, vp, i32, vp, vp, vp, vp, i32, f32, f32, f32, f32,

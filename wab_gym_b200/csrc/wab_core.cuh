@@ -78,13 +78,23 @@ struct Params {
     float reward_table[8];
     uint32_t mask_look[4], mask_gath[4];
     uint64_t env_id_base;
-    uint64_t replica_envs;         // 0, or n of a replicated handle (wab_vec_set_replicas): every block of n rows repeats the ids
+    // a handle cut into blocks of c rows (wab_vec_set_replicas / wab_vec_set_blocks), packed into the 8 bytes the field
+    // replica_envs always took, so that Params keeps its size and every later argument its constant-bank offset:
+    uint32_t replica_envs;         // c, or 0 for a plain handle
+    uint32_t block_delta;          // block_stride - c (mod 2^32): -c for replicas (block_stride 0)
 };
 
-// The global env id of `row` (< 2^32: wab_vec_set_replicas refuses larger handles), the key of every draw the handle makes
-// for it: env_id_base + row, or env_id_base + row % n on a replicated handle, whose blocks of n rows are copies of one another.
+// The global env id of `row` (< 2^32: wab_vec_set_replicas and wab_vec_set_blocks refuse larger handles), the key of every
+// draw the handle makes for it: env_id_base + row, or, on a handle cut into blocks of c rows, env_id_base +
+// (row / c) block_stride + row % c = env_id_base + row + (row / c) (block_stride - c): every block repeats the ids of the
+// first (replicas, block_stride = 0), or block k holds the ids from env_id_base + k block_stride (blocks). The offset is
+// exact in 32 bits (wab_vec_set_blocks refuses a layout whose last id is 2^32 or more past env_id_base). One division and
+// one multiply-add inside the branch, as the remainder of replicas took before; a plain handle runs the code it ran.
 WAB_HD uint64_t global_env_id(const Params& P, int64_t row) {
-    if (P.replica_envs) return P.env_id_base + (uint64_t)((uint32_t)row % (uint32_t)P.replica_envs);
+    if (P.replica_envs) {
+        const uint32_t r = (uint32_t)row;
+        return P.env_id_base + (uint64_t)(r + (r / P.replica_envs) * P.block_delta);
+    }
     return P.env_id_base + (uint64_t)row;
 }
 

@@ -1561,7 +1561,24 @@ int wab_vec_set_replicas(WabVec* h, int64_t n_replicas) {
     if (h->started) return fail(WAB_E_CONFIG, "call wab_vec_set_replicas before the first reset");
     if (n_replicas < 1 || h->n % n_replicas != 0) return fail(WAB_E_CONFIG, "n_replicas must divide n_envs");
     if (h->n > (int64_t)UINT32_MAX) return fail(WAB_E_CONFIG, "replicated handles hold fewer than 2^32 envs");
-    h->P.replica_envs = n_replicas == 1 ? 0u : (uint64_t)(h->n / n_replicas);
+    h->P.replica_envs = n_replicas == 1 ? 0u : (uint32_t)(h->n / n_replicas);
+    h->P.block_delta = 0u - h->P.replica_envs;                                            // block_stride 0
+    if (h->host_graph) { cudaGraphExecDestroy(h->host_graph); h->host_graph = nullptr; }   // captured with the old Params
+    return WAB_OK;
+}
+
+int wab_vec_set_blocks(WabVec* h, int64_t n_blocks, int64_t block_stride) {
+    if (!h) return fail(WAB_E_NULL, "null argument");
+    if (h->started) return fail(WAB_E_CONFIG, "call wab_vec_set_blocks before the first reset");
+    if (n_blocks < 1 || h->n % n_blocks != 0) return fail(WAB_E_CONFIG, "n_blocks must divide n_envs");
+    if (block_stride < 0 || (block_stride > 0 && block_stride < h->n / n_blocks))
+        return fail(WAB_E_CONFIG, "block_stride must be 0 (replicas) or at least n_envs / n_blocks: the blocks' ids would overlap");
+    if (h->n > (int64_t)UINT32_MAX) return fail(WAB_E_CONFIG, "blocked handles hold fewer than 2^32 envs");
+    const int64_t c = h->n / n_blocks;
+    if (block_stride > (int64_t)UINT32_MAX || (n_blocks - 1) * block_stride + c > ((int64_t)1 << 32))
+        return fail(WAB_E_CONFIG, "a blocked handle's ids lie within 2^32 of env_id_base: (n_blocks - 1) block_stride + n_envs / n_blocks <= 2^32");
+    h->P.replica_envs = n_blocks == 1 ? 0u : (uint32_t)c;
+    h->P.block_delta = n_blocks == 1 ? 0u : (uint32_t)block_stride - (uint32_t)c;
     if (h->host_graph) { cudaGraphExecDestroy(h->host_graph); h->host_graph = nullptr; }   // captured with the old Params
     return WAB_OK;
 }
@@ -1924,7 +1941,7 @@ static int policy_backward_launch(const char* who, WabVec* h, const uint8_t* d_f
         wab_policy_ppo_bwd_population_kernel<<<grid * n_members, 256, BW_SMEM_TOTAL, (cudaStream_t)stream>>>(
             h->P, (int)h->cfg.food_obs_scale + 1, B, *ppo, G);
         WAB_CUDA(cudaGetLastError());
-        wab_policy_bwd_reduce_population_kernel<<<dim3((unsigned)((total + 255) / 256), (unsigned)n_members), 256, 0, (cudaStream_t)stream>>>(
+        wab_policy_bwd_reduce_population_kernel<float><<<dim3((unsigned)((total + 255) / 256), (unsigned)n_members), 256, 0, (cudaStream_t)stream>>>(
             reinterpret_cast<const float*>(d_scratch), grid, dim, n_actions, (total + 63) / 64 * 64, d_grad);
         WAB_CUDA(cudaGetLastError());
         return WAB_OK;
@@ -2118,6 +2135,25 @@ int wab_policy_backward_grad_f64(WabVec* h, const void* d_scratch, int64_t scrat
     const int64_t total = policy_n_params(dim, n_actions);
     wab_policy_bwd_reduce_kernel<double><<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const float*>(d_scratch), backward_grid(h->device), dim, n_actions, d_grad64);
+    WAB_CUDA(cudaGetLastError());
+    return WAB_OK;
+}
+
+int wab_policy_backward_population_grad_f64(WabVec* h, const void* d_scratch, int64_t scratch_bytes, int32_t n_members,
+                                            int32_t n_actions, double* d_grad64, void* stream) {
+    if (!h || !d_scratch || !d_grad64) return fail(WAB_E_NULL, "null argument");
+    if (n_members < 1 || n_members > 64) return fail(WAB_E_CONFIG, "wab_policy_backward_population_grad_f64: 1 <= n_members <= 64");
+    if (n_actions < 1 || n_actions > 8) return fail(WAB_E_UNSUPPORTED, "wab_policy_backward_population_grad_f64: at most 8 actions");
+    const int dim = wab_vec_flat_dim(h);
+    if (dim > TC_CHUNKS * TC_KC) return fail(WAB_E_UNSUPPORTED, "wab_policy_backward_population_grad_f64: the input is at most 512 columns wide");
+    if (((uintptr_t)d_scratch & 15u) != 0 || ((uintptr_t)d_grad64 & 7u) != 0)
+        return fail(WAB_E_CONFIG, "d_scratch must be 16-byte aligned, d_grad64 8-byte");
+    if (scratch_bytes < n_members * wab_policy_backward_scratch_bytes(h))
+        return fail(WAB_E_CONFIG, "d_scratch is smaller than wab_policy_backward_population_scratch_bytes");
+    DeviceGuard guard(h->device);
+    const int64_t stride = wab_policy_population_grad_stride(h, n_actions);
+    wab_policy_bwd_reduce_population_kernel<double><<<dim3((unsigned)((stride + 255) / 256), (unsigned)n_members), 256, 0, (cudaStream_t)stream>>>(
+        reinterpret_cast<const float*>(d_scratch), backward_grid(h->device), dim, n_actions, stride, d_grad64);
     WAB_CUDA(cudaGetLastError());
     return WAB_OK;
 }

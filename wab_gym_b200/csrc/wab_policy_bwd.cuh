@@ -214,15 +214,21 @@ __global__ void wab_policy_bwd_reduce_kernel(const float* __restrict__ scratch, 
     grad[e] = (G)s;
 }
 
-// wab_policy_bwd_reduce_kernel<float> for each member of a population (blockIdx.y = m): the fp64 sum over m's own n_cta
-// CTAs, in index order, into grad [P][stride]. The element -> partial-sum mapping is restated rather than shared: moved
-// into a device function, it compiles differently inside wab_policy_bwd_reduce_kernel.
+// wab_policy_bwd_reduce_kernel for each member of a population (blockIdx.y = m): the fp64 sum over m's own n_cta CTAs, in
+// index order, into grad [P][stride]. G = float rounds once (wab_policy_ppo_backward_population); G = double keeps the
+// fp64 sum (wab_policy_backward_population_grad_f64, for a cross-rank sum) and, launched over the whole stride, also
+// writes the padding entries as 0. The element -> partial-sum mapping is restated rather than shared: moved into a
+// device function, it compiles differently inside wab_policy_bwd_reduce_kernel.
+template <typename G>
 __global__ void wab_policy_bwd_reduce_population_kernel(const float* __restrict__ scratch, int n_cta, int dim, int n_actions,
-                                                        int64_t stride, float* __restrict__ grad) {
+                                                        int64_t stride, G* __restrict__ grad) {
     const int64_t n1 = 128LL * dim, o_b1 = n1, o_w2 = o_b1 + 128, o_b2 = o_w2 + 150 * 128, o_w3 = o_b2 + 150, o_b3 = o_w3 + 128 * 150,
                   o_wa = o_b3 + 128, o_ba = o_wa + (int64_t)n_actions * 128, o_wv = o_ba + n_actions, o_bv = o_wv + 128, total = o_bv + 1;
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= total) return;
+    if (e >= total) {
+        if (sizeof(G) == 8 && e < stride) grad[(int64_t)blockIdx.y * stride + e] = (G)0;
+        return;
+    }
     int off;
     if (e < o_b1) {
         const int j = (int)(e / dim), k = (int)(e - (int64_t)j * dim);
@@ -240,7 +246,7 @@ __global__ void wab_policy_bwd_reduce_population_kernel(const float* __restrict_
     const float* member = scratch + (size_t)blockIdx.y * n_cta * BP_BLOCK;
     double s = 0.0;
     for (int b = 0; b < n_cta; ++b) s += (double)member[(size_t)b * BP_BLOCK + off];
-    grad[(int64_t)blockIdx.y * stride + e] = (float)s;
+    grad[(int64_t)blockIdx.y * stride + e] = (G)s;
 }
 
 // d_grad[i] = fp32(sum over r = 0 .. n_ranks - 1 of d_rank_grads[r][i]), the sum in fp64 in rank order

@@ -19,7 +19,8 @@ evaluation included. Every rank must pass the same weights.
 
 ``PopulationEvaluator`` scores P policies at once on ``VecEnv(P n, replicas=P)``: every block of n envs repeats the
 global ids ``env_id_base ..``, so member p plays exactly the episodes ``Evaluator(n)`` plays, in one launch per step for
-all members.
+all members. With ``group`` rank r owns ``VecEnv(P c_r, replicas=P, env_id_base=env_id_base + first_r)``, its shard
+``(first_r, c_r)`` of ``sharding.population_shards(n, W)``, and every rank returns the single-process results bit for bit.
 """
 from __future__ import annotations
 
@@ -113,10 +114,7 @@ class Evaluator:
         first, count = 0, self.num_envs
         if self.group is not None:
             import torch.distributed as dist
-            world = dist.get_world_size(self.group)
-            if self.num_envs < world:             # known on every rank: all of them refuse, none waits for a peer
-                raise ValueError("Evaluator over %d ranks needs at least one env per rank, got %d envs" % (world, self.num_envs))
-            first, count = sharding.shard_range(self.num_envs, dist.get_rank(self.group), world)
+            first, count = self._shard(dist.get_rank(self.group), dist.get_world_size(self.group))
         self.env = VecEnv(count, game_options=game_options, device=device, seed=seed, env_id_base=int(env_id_base) + first,
                           features=True, emit_grids=False, replicas=self._replicas)
         self.flat_dim, self.n_actions = self.env.flat_dim, self.env.n_actions
@@ -144,6 +142,20 @@ class Evaluator:
         self._cols = torch.arange(N, device=dev)
         self._slots = torch.arange(N)
         self._policy = self._tc = self._heads = None
+
+    def _shard(self, rank: int, world: int):
+        """(first global id offset, env count) of this rank's handle. Refusals depend on arguments every rank shares, so
+        all ranks refuse alike and none waits for a peer."""
+        if self.num_envs < world:
+            raise ValueError("Evaluator over %d ranks needs at least one env per rank, got %d envs" % (world, self.num_envs))
+        return sharding.shard_range(self.num_envs, rank, world)
+
+    def _gather(self, parts):
+        """The per-episode tensors of every rank, concatenated in rank order (every rank gets the same)."""
+        import torch.distributed as dist
+        gathered = [None] * dist.get_world_size(self.group)
+        dist.all_gather_object(gathered, parts, group=self.group)
+        return gathered
 
     def restore(self, policy) -> None:
         """Steps 1-3 of ``evaluate``: the start state (one synchronisation), the draw counter, and a copy of ``policy``'s
@@ -206,9 +218,7 @@ class Evaluator:
         self.restore(policy)
         parts = self._episodes(*self.play(greedy, noise))
         if self.group is not None:
-            import torch.distributed as dist
-            gathered = [None] * dist.get_world_size(self.group)
-            dist.all_gather_object(gathered, parts, group=self.group)
+            gathered = self._gather(parts)
             parts = [torch.cat([g[i] for g in gathered]) for i in range(len(parts))]
         return EvalResult(*parts)
 
@@ -229,21 +239,30 @@ class PopulationEvaluator(Evaluator):
     is keyed as that evaluator keys it. So ``evaluate(policies)[p]`` equals ``Evaluator(n, game_options, seed, env_id_base,
     episodes_per_env).evaluate(policies[p])`` bit for bit, and the P results line up episode by episode (common random
     numbers: what separates close policies such as the members of a population-based training run). ``envs_per_member``
-    = n is a multiple of 128, 1 <= ``members`` <= 64. Data-parallel evaluation (``group``) is not supported."""
+    = n is a multiple of 128, 1 <= ``members`` <= 64.
+
+    With ``group`` (W > 1 ranks) rank r owns ``VecEnv(P c_r, replicas=P, env_id_base=env_id_base + first_r)`` for its shard
+    ``(first_r, c_r)`` of ``sharding.population_shards(n, W)`` (each c_r a positive multiple of 128). Member p's per-episode
+    tensors are all-gathered in rank order, so every rank returns the single-process ``results`` bit for bit. Every rank
+    must pass the same policies."""
 
     def __init__(self, members: int, envs_per_member: int, game_options: Optional[dict] = None, seed: int = 0,
                  device="cuda", env_id_base: int = 0, episodes_per_env: int = 1, group=None):
         P, n = int(members), int(envs_per_member)
-        if group is not None:
-            raise ValueError("PopulationEvaluator is single-process: data-parallel evaluation (group) is not supported")
+        group = sharding.process_group(group, "PopulationEvaluator")
         if not 1 <= P <= 64:
             raise ValueError("a population has 1 to 64 members")
         if n < 128 or n % 128 != 0:
             raise ValueError("PopulationEvaluator needs envs_per_member a positive multiple of 128, got %d" % n)
         self.members, self.envs_per_member, self._replicas = P, n, P
         super().__init__(P * n, game_options=game_options, seed=seed, device=device, env_id_base=env_id_base,
-                         episodes_per_env=episodes_per_env)
+                         episodes_per_env=episodes_per_env, group=group)
+        self.shard_envs = self.env.num_envs // P         # c_r: this rank's envs of each member
         self._policies = None
+
+    def _shard(self, rank: int, world: int):
+        first, c = sharding.population_shards(self.envs_per_member, world)[rank]
+        return first, self.members * c
 
     def restore(self, policies) -> None:
         """``Evaluator.restore`` for P policies: each one's weights copied into this evaluator's own member and packed."""
@@ -276,6 +295,10 @@ class PopulationEvaluator(Evaluator):
         envs of block p, whose global ids ``env_id_base ..`` are the same in every block. The policies are only read."""
         self.restore(policies)
         parts = self._episodes(*self.play(greedy, noise))
-        P, n = self.members, self.envs_per_member
-        split = [t.view(P, n, *t.shape[1:]) for t in parts]
+        P = self.members
+        if self.group is None:
+            split = [t.view(P, self.envs_per_member, *t.shape[1:]) for t in parts]
+        else:                                            # member p: its c_r rows of every rank, in rank order
+            gathered = self._gather(parts)
+            split = [torch.cat([g[i].view(P, -1, *g[i].shape[1:]) for g in gathered], dim=1) for i in range(len(parts))]
         return [EvalResult(*(t[p] for t in split)) for p in range(P)]

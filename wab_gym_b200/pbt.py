@@ -57,15 +57,24 @@ class PopulationBasedTraining:
     """Population-based training of ``population`` (a ``PPOPopulation``) scored by ``evaluator`` (a ``PopulationEvaluator``
     with the same member count): see the module docstring. ``greedy`` selects the evaluator's greedy or sampled actions.
     ``history`` holds one dict per ready event: ``iteration``, ``fitness`` (f64[P]), ``ranking``, ``copies`` [(p, q)],
-    ``factors`` {p: {key: factor}} and ``hyperparameters`` (every member's, after the event)."""
+    ``factors`` {p: {key: factor}} and ``hyperparameters`` (every member's, after the event).
+
+    A data-parallel population and evaluator (the same ``group``) work unchanged: every rank holds every member, the
+    evaluator returns the same fitness on every rank, and the keyed draws are the same there, so every rank takes the same
+    decisions and no member state moves between ranks. ``state_dict()`` is then per rank; its ``population`` parts merge
+    with ``sharding.merge_population_state_dicts``."""
 
     def __init__(self, population, evaluator, interval: int = 5, fraction: float = 0.25,
                  perturb: Sequence[str] = ("lr", "ent_coef"), factors: Sequence[float] = (0.8, 1.2), seed: int = 0,
                  greedy: bool = True):
         if population.n_members != evaluator.members:
             raise ValueError("the population has %d members, the evaluator %d" % (population.n_members, evaluator.members))
-        self.population, self.evaluator = population, evaluator
         self._configure(interval, fraction, perturb, factors, seed, greedy)
+        # the group each was built on (None: a single process), read from the instance's own attributes only
+        if vars(population).get("group") is not vars(evaluator).get("group"):
+            raise ValueError("the population and the evaluator must both be single-process or both data-parallel on the same "
+                             "group")
+        self.population, self.evaluator = population, evaluator
         self.history: List[dict] = []
 
     def _configure(self, interval, fraction, perturb, factors, seed, greedy):

@@ -349,7 +349,8 @@ class PolicyPopulationTC:
     multiple of 128): member p owns env rows [p n, (p + 1) n), and its weights are packed into row p of stacked buffers
     (``wab_policy_forward_population``, ``wab_policy_ppo_backward_population``). Each call does for every member what
     ``PolicyTrainTC`` does for one policy, in one launch, and member p's outputs equal, bit for bit, those of
-    ``PolicyTrainTC`` on ``VecEnv(n, env_id_base=p n)`` (with the same env_id_base shift on this handle). A member is
+    ``PolicyTrainTC`` on ``VecEnv(n, env_id_base=p n)`` (with the same env_id_base shift on this handle; on a blocked
+    handle, ``VecEnv(n, env_id_base=`` the block's first id ``)``). A member is
     re-packed when one of its parameters changed since its last pack (an optimiser step, a load), as
     ``PolicyTrainTC.logits_and_value`` does."""
 
@@ -505,6 +506,34 @@ class PolicyPopulationTC:
             _ptr(self.w_heads), _ptr(self.b_heads), self.n_actions, float(noise_scale), float(slope), -4.0, 4.0,
             ctypes.cast(coef, ctypes.c_void_p), _ptr(self.scratch), self.scratch.numel(), _ptr(out), _ptr(logp), _ptr(value),
             _ptr(entropy), self._stream()))
+        return out
+
+    def grad_f64(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The gradient of the last ``ppo_backward`` on this stream as f64[P, grad_stride]: every member's fixed-order fp64
+        sum over its CTAs, not rounded, padding 0 (``wab_policy_backward_population_grad_f64``). For a cross-rank sum that
+        rounds once."""
+        shape = (self.n_members, self.grad_stride)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float64, device=self.env.device)
+        if out.dtype != torch.float64 or tuple(out.shape) != shape or not out.is_contiguous() or out.device != self.env.device:
+            raise ValueError("out must be a contiguous float64 [P, grad_stride] tensor on the environment's device")
+        _lib.check(self.lib.wab_policy_backward_population_grad_f64(self.env._h, _ptr(self.scratch), self.scratch.numel(),
+                                                                    self.n_members, self.n_actions, _ptr(out), self._stream()))
+        return out
+
+    def grad_sum_ranks(self, rank_grads: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """fp32 of the fp64 sum over ranks, in rank order, of ``rank_grads`` f64[W, P, grad_stride] into ``out`` f32[P,
+        grad_stride] (``wab_policy_grad_sum_ranks`` over P grad_stride elements)."""
+        shape = (self.n_members, self.grad_stride)
+        if rank_grads.dtype != torch.float64 or rank_grads.dim() != 3 or tuple(rank_grads.shape[1:]) != shape or \
+                not rank_grads.is_contiguous() or rank_grads.device != self.env.device:
+            raise ValueError("rank_grads must be a contiguous float64 [W, P, grad_stride] tensor on the environment's device")
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float32, device=self.env.device)
+        if out.dtype != torch.float32 or tuple(out.shape) != shape or not out.is_contiguous() or out.device != self.env.device:
+            raise ValueError("out must be a contiguous float32 [P, grad_stride] tensor on the environment's device")
+        _lib.check(self.lib.wab_policy_grad_sum_ranks(_ptr(rank_grads), rank_grads.shape[0], out.numel(), _ptr(out),
+                                                      self._stream()))
         return out
 
 

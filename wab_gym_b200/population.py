@@ -16,7 +16,23 @@ member-local rows (seeded as ``PPOTrainer`` seeds it), translated to each member
 slices. Each slice is ONE ``wab_policy_ppo_backward_population`` launch, then a global-norm clip and an Adam step per
 member. Every per-member statistic (normalisation mean and std, gradient norm, mean reward, diagnostics) is computed on a
 contiguous tensor of that member alone, as ``PPOTrainer`` computes it, so it rounds the same way. Nothing in an iteration
-synchronises with the host. Data-parallel populations (``group``) are not supported.
+synchronises with the host.
+
+Data-parallel populations (``group``, a ``torch.distributed`` process group of W > 1 ranks): every rank holds all P
+members, each on its contiguous shard ``[first_r, first_r + c_r)`` of the member's n envs (``sharding.population_shards``,
+c_r a positive multiple of 128), on ONE handle ``VecEnv(P c_r, env_id_base=B + first_r, blocks=P, block_stride=n)``: row
+p c_r + j is member p's global id ``B + p n + first_r + j``, the id it has in a single-process population whose first id is
+B. Construction all-gathers each rank's layout and signature, checks them on every rank (so a refusal is raised on every
+rank and none is left waiting in a collective), then broadcasts rank 0's policies and sampling seed. Per iteration each
+member does what ``PPOTrainer(group)`` does: advantages normalised by the member's mean and std over all ranks
+(``sharding.global_mean_std_members``: two collectives for all members), one permutation per member seeded with the first
+global id of its shard on this rank, minibatch k's weights divided by its row count summed over the ranks, and after each
+population backward the fp64 gradient of every member (``wab_policy_backward_population_grad_f64``) all-gathered once and
+summed in rank order (``wab_policy_grad_sum_ranks``) before the clip and Adam. So every rank holds bit-identical weights,
+Adam state and hyper-parameters, and member p is bit for bit the 1-member data-parallel population on ids from B + p n.
+Collection is invariant to the world size; training, like that of the data-parallel trainers, is not (``a2c``'s module
+docstring), but ``sharding.merge_population_state_dicts`` of the ranks' ``state_dict()``s resumes on any layout. A group of
+one rank is the single-process population.
 """
 from __future__ import annotations
 
@@ -57,14 +73,17 @@ def member_hyperparameters(hyperparameters, n_members: int) -> List[Dict[str, fl
 
 
 def member_rows(perm: torch.Tensor, n_members: int, member_envs: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Member-local rows t n + j (``perm``, int32[M]) -> each member's global rows t N + p n + j, N = P n: int32[P, M]
-    (written into ``out`` when given, which may be a column slice of a wider buffer)."""
+    """Member-local rows t n + j (``perm``: int32[M], shared by every member, or int32[P, M], one list per member) -> each
+    member's global rows t N + p n + j, N = P n: int32[P, M] (written into ``out`` when given, which may be a column slice
+    of a wider buffer)."""
     n = member_envs
     local = (perm // n) * (n_members * n) + perm % n
+    if local.dim() == 1:
+        local = local[None, :]
     offsets = torch.arange(n_members, dtype=perm.dtype, device=perm.device) * n
     if out is None:
-        return local[None, :] + offsets[:, None]
-    return torch.add(local[None, :], offsets[:, None], out=out)
+        return local + offsets[:, None]
+    return torch.add(local, offsets[:, None], out=out)
 
 
 class PPOPopulation:
@@ -74,32 +93,15 @@ class PPOPopulation:
 
     def __init__(self, env: VecEnv, members: int, hyperparameters=None, policies=None, horizon: int = 64, epochs: int = 4,
                  minibatches: int = 4, noise: bool = True, group=None):
-        # everything PPOTrainer refuses, and a group, before any device work
-        if group is not None:
-            raise ValueError("PPOPopulation is single-process: data-parallel populations (group) are not supported")
-        P, N = int(members), env.num_envs
-        if not 1 <= P <= 64:
-            raise ValueError("a population has 1 to 64 members")
-        if N % P != 0 or (N // P) % 128 != 0:
-            raise ValueError("PPOPopulation needs num_envs = members * n with n a multiple of 128 (got %d envs, %d members)" % (N, P))
-        if not env.with_features:
-            raise ValueError("PPOPopulation needs VecEnv(features=True)")
-        if getattr(env, "replicas", 1) > 1:
-            raise ValueError("PPOPopulation refuses a VecEnv with replicas: its members own distinct env ids")
-        n = N // P
-        if epochs < 1 or minibatches < 1 or int(horizon) * n < minibatches:
-            raise ValueError("PPOPopulation needs epochs >= 1 and 1 <= minibatches <= horizon * n")
-        self.hyperparameters = member_hyperparameters(hyperparameters, P)
+        # everything PPOTrainer refuses before any device work; with a group, on every rank (the layout is checked too)
+        self.group = sharding.process_group(group, "PPOPopulation")
+        if self.group is None:
+            policies = self._validate(env, members, hyperparameters, policies, horizon, epochs, minibatches, True)
+        else:
+            policies = self._join_layout(env, members, hyperparameters, policies, horizon, epochs, minibatches, noise)
+        P, N, n = int(members), env.num_envs, env.num_envs // int(members)
         if policies is None:
             policies = [Policy(env.flat_dim, env.n_actions) for _ in range(P)]
-        policies = list(policies)
-        if len(policies) != P:
-            raise ValueError("policies must hold one Policy per member (%d), got %d" % (P, len(policies)))
-        for pol in policies:
-            check_reference_network(pol, env.flat_dim, "PPOPopulation")
-        if any(pol.action_head.out_features != env.n_actions for pol in policies):
-            raise ValueError("every member's action head must have the environment's %d actions" % env.n_actions)
-
         self.env, self.n_members, self.member_envs = env, P, n
         self.horizon, self.epochs, self.minibatches, self.noise = int(horizon), int(epochs), int(minibatches), noise
         self.policies = [pol.to(env.device) for pol in policies]
@@ -118,8 +120,12 @@ class PPOPopulation:
                            "target": torch.empty(T, N, device=dev)}
         self._boot_actions = torch.empty(N, dtype=torch.uint8, device=dev)
         self._new = {k: torch.empty(T, N, device=dev) for k in ("logp", "value", "entropy")}
-        self._perm = torch.empty(T * n, dtype=torch.int32, device=dev)
+        # one permutation of member-local rows per epoch, shared by the members (single process) or one per member (group)
+        self._perm = torch.empty(T * n if self.group is None else (P, T * n), dtype=torch.int32, device=dev)
         self._bounds = sharding.minibatch_bounds(T * n, self.minibatches)
+        # the row count minibatch k's weights are divided by: this process's, or the sum over the ranks
+        self._global_counts = ([self._bounds[k + 1] - self._bounds[k] for k in range(self.minibatches)] if self.group is None
+                               else sharding.global_minibatch_counts([T * c for c in self._shard_counts], self.minibatches))
         # minibatch k's row lists [P][M_k], M_k rounded up to 64 entries so that each member's gathered rows start 256-byte
         # aligned (a contiguous tensor of its own, like PPOTrainer's); the padding entries are never read by the kernel
         sizes = [self._bounds[k + 1] - self._bounds[k] for k in range(self.minibatches)]
@@ -135,6 +141,95 @@ class PPOPopulation:
             assert off == n_params
         self._set_discounts()
         env.reset()
+        if self.group is not None:
+            self._join_weights()
+
+    def _validate(self, env, members, hyperparameters, policies, horizon, epochs, minibatches, single: bool):
+        """The constructor's refusals (``ValueError``), before any device work. Sets ``hyperparameters``; returns the
+        policies as a list (or None)."""
+        P, N = int(members), env.num_envs
+        if not 1 <= P <= 64:
+            raise ValueError("a population has 1 to 64 members")
+        if N % P != 0 or (N // P) % 128 != 0:
+            raise ValueError("PPOPopulation needs num_envs = members * n with n a multiple of 128 (got %d envs, %d members)" % (N, P))
+        if not env.with_features:
+            raise ValueError("PPOPopulation needs VecEnv(features=True)")
+        if getattr(env, "replicas", 1) > 1:
+            raise ValueError("PPOPopulation refuses a VecEnv with replicas: its members own distinct env ids")
+        n = N // P
+        blocks, stride = getattr(env, "blocks", 1), getattr(env, "block_stride", 0)
+        if single and not (blocks == 1 or (blocks == P and stride == n)):
+            raise ValueError("a single-process PPOPopulation needs a plain VecEnv (or blocks=%d, block_stride=%d: the same ids)"
+                             % (P, n))
+        if epochs < 1 or minibatches < 1 or int(horizon) * n < minibatches:
+            raise ValueError("PPOPopulation needs epochs >= 1 and 1 <= minibatches <= horizon * n")
+        self.hyperparameters = member_hyperparameters(hyperparameters, P)
+        if policies is None:
+            return None
+        policies = list(policies)
+        if len(policies) != P:
+            raise ValueError("policies must hold one Policy per member (%d), got %d" % (P, len(policies)))
+        for pol in policies:
+            check_reference_network(pol, env.flat_dim, "PPOPopulation")
+        if any(pol.action_head.out_features != env.n_actions for pol in policies):
+            raise ValueError("every member's action head must have the environment's %d actions" % env.n_actions)
+        return policies
+
+    def _signature(self, env, members, horizon, epochs, minibatches, noise) -> tuple:
+        """What every rank of a data-parallel population must agree on."""
+        return (int(env.fingerprint), int(env.n_actions), int(members), int(horizon), int(epochs), int(minibatches), bool(noise),
+                tuple(tuple(sorted(hp.items())) for hp in self.hyperparameters))
+
+    def _join_layout(self, env, members, hyperparameters, policies, horizon, epochs, minibatches, noise):
+        """The refusals of a data-parallel population on every rank: this rank's own checks (an exception of any type is a
+        refusal), then one all-gather of every rank's verdict, layout and signature (one host synchronisation), then the
+        layout check. Any refusal raises ``ValueError`` on every rank."""
+        import torch.distributed as dist
+        err, sig, local = None, None, None
+        try:
+            policies = self._validate(env, members, hyperparameters, policies, horizon, epochs, minibatches, False)
+            sig = self._signature(env, members, horizon, epochs, minibatches, noise)
+        except Exception as exc:          # any refusal, of any type, is gathered: no rank skips the collective below
+            local = exc
+            err = str(exc) if isinstance(exc, ValueError) else "%s: %s" % (type(exc).__name__, exc)
+        info = (int(env.env_id_base), int(env.num_envs), int(getattr(env, "blocks", 1)), int(getattr(env, "block_stride", 0)),
+                sig, err)
+        infos = [None] * dist.get_world_size(self.group)
+        dist.all_gather_object(infos, info, group=self.group)
+        for r, i in enumerate(infos):
+            if i[5] is not None:
+                raise ValueError("rank %d refused the population: %s" % (r, i[5])) from local
+        self.first_id, self.total_member_envs = sharding.check_population_shards([i[:5] for i in infos], int(members))
+        self._shard_counts = [int(i[1]) // int(members) for i in infos]
+        return policies
+
+    def _join_weights(self):
+        """Rank 0's policies and sampling seed on every rank, and the buffers of the cross-rank gradient sum."""
+        import torch.distributed as dist
+        dev, world = self.env.device, dist.get_world_size(self.group)
+        src = dist.get_global_rank(self.group, 0)
+        with torch.no_grad():
+            for pol in self.policies:
+                for prm in pol.parameters():
+                    dist.broadcast(prm.data, src, group=self.group)
+        seed = torch.tensor([self.sample_seed], dtype=torch.int64, device=dev)
+        dist.broadcast(seed, src, group=self.group)
+        self.sample_seed = int(seed.item())
+        self._tc.refresh()
+        self._grad64 = torch.empty(self.n_members, self._tc.grad_stride, dtype=torch.float64, device=dev)
+        self._gathered = torch.empty(world, self.n_members, self._tc.grad_stride, dtype=torch.float64, device=dev)
+
+    def _member_first_id(self, p: int) -> int:
+        """The global id of member p's first row on this handle."""
+        return int(self.env.global_ids([p * self.member_envs])[0])
+
+    def _sum_grad_over_ranks(self):
+        """Every member's gradient of the last population backward summed over the ranks into ``_grad``: fp64 per rank,
+        one all-gather of [P, stride], summed in rank order and rounded once."""
+        import torch.distributed as dist
+        self._tc.grad_f64(self._grad64)
+        dist.all_gather(list(self._gathered.unbind(0)), self._grad64, group=self.group)
+        self._tc.grad_sum_ranks(self._gathered, self._grad)
 
     def _set_discounts(self):
         """The per-column gamma and gamma * lam of GAE: member p's values on its n columns (gamma * lam in double, rounded
@@ -176,26 +271,39 @@ class PPOPopulation:
         adv, ret = gae(b["reward"], b["done"], b["value"], b["bootstrap"], self._gamma, None, gamma_lam=self._gamma_lam)
         b["target"].copy_(ret)
         by_member = self._by_member(adv)
-        mean = torch.stack([by_member[p].mean() for p in range(P)])
-        std = torch.stack([by_member[p].std() for p in range(P)])
+        if self.group is None:
+            mean = torch.stack([by_member[p].mean() for p in range(P)])
+            std = torch.stack([by_member[p].std() for p in range(P)])
+        else:
+            mean, std = sharding.global_mean_std_members(by_member, self.group)
         by_member.sub_(mean[:, None, None]).div_((std + 1e-8)[:, None, None])   # normalised once per member's batch
         b["advantage"].view(T, P, n).copy_(by_member.transpose(0, 1))
         del adv, ret, by_member
         flat = {k: b[k].view(-1) for k in ("logp", "advantage", "target")}
         new = {k: v.view(-1) for k, v in self._new.items()}
         stats = [[] for _ in range(P)]
+        first_ids = None if self.group is None else [self._member_first_id(p) for p in range(P)]
         for epoch in range(self.epochs):
-            gen = torch.Generator(device=env.device)
-            gen.manual_seed(_perm_seed(self.sample_seed, self.iteration, epoch))
-            torch.randperm(self._perm.numel(), generator=gen, out=self._perm)
+            if self.group is None:
+                gen = torch.Generator(device=env.device)
+                gen.manual_seed(_perm_seed(self.sample_seed, self.iteration, epoch))
+                torch.randperm(self._perm.numel(), generator=gen, out=self._perm)
+            else:                                        # member p's shard shuffled as its data-parallel trainer would
+                for p in range(P):
+                    gen = torch.Generator(device=env.device)
+                    gen.manual_seed(_perm_seed(self.sample_seed, self.iteration, epoch, first_ids[p]))
+                    torch.randperm(self._perm.shape[1], generator=gen, out=self._perm[p])
             for k in range(self.minibatches):
                 m = self._bounds[k + 1] - self._bounds[k]
                 rows = self._mb_rows[k]
-                member_rows(self._perm[self._bounds[k]:self._bounds[k + 1]], P, n, out=rows[:, :m])
-                coefs = [(hp["clip_eps"], 1.0 / m, hp["vf_coef"] / m, hp["ent_coef"] / m) for hp in hps]
+                member_rows(self._perm[..., self._bounds[k]:self._bounds[k + 1]], P, n, out=rows[:, :m])
+                mg = self._global_counts[k]
+                coefs = [(hp["clip_eps"], 1.0 / mg, hp["vf_coef"] / mg, hp["ent_coef"] / mg) for hp in hps]
                 self._tc.ppo_backward(b["features"], b["counters"], b["actions"], b["logp"], b["advantage"], b["target"],
                                       rows, self._mb_counts[k], coefs, out=self._grad, logp=self._new["logp"],
                                       value=self._new["value"], entropy=self._new["entropy"], noise_scale=noise)
+                if self.group is not None:
+                    self._sum_grad_over_ranks()
                 picked = [t.index_select(0, rows.view(-1)).view(P, -1) for t in (new["logp"], new["value"], new["entropy"],
                                                                                    flat["logp"], flat["advantage"], flat["target"])]
                 for p, hp in enumerate(hps):
@@ -274,12 +382,13 @@ class PPOPopulation:
         counter, sampling seed and iteration are the population's and are not changed."""
         slots = self._member_slots(p)
         ids = torch.as_tensor(sd["env"]["env_ids"], dtype=torch.int64).reshape(-1)
-        own = ids.numel() == slots.numel() and torch.equal(torch.sort(ids).values, slots + self.env.env_id_base)
+        own_ids = self.env.global_ids(slots)             # contiguous: member p's shard of ids on this handle
+        own = ids.numel() == slots.numel() and torch.equal(torch.sort(ids).values, own_ids)
         hp = member_hyperparameters([sd.get("hyperparameters", self.hyperparameters[p])], 1)[0]
         if own:
-            records = sharding.select_shard_records(sd["env"], self.env.env_id_base + p * self.member_envs, self.member_envs,
+            records = sharding.select_shard_records(sd["env"], int(own_ids[0]), self.member_envs,
                                                     self.env.fingerprint, self.env.record_bytes, STATE_FORMAT)
-            self.env.load_state(EnvStates(records, slots + self.env.env_id_base, self.env.fingerprint))
+            self.env.load_state(EnvStates(records, own_ids, self.env.fingerprint))
         self.policies[p].load_state_dict(sd["policy"])
         self.optimizers[p].load_state_dict(sd["optimizer"])
         self.hyperparameters[p] = hp

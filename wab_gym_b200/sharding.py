@@ -9,7 +9,7 @@ are identical for any world size.
 """
 from __future__ import annotations
 
-from typing import Callable, Dict, Optional, Tuple
+from typing import Callable, Dict, List, Optional, Tuple
 
 import torch
 
@@ -24,6 +24,43 @@ def shard_range(total_envs: int, rank: int, world_size: int) -> Tuple[int, int]:
     count = base + (1 if rank < extra else 0)
     first = rank * base + min(rank, extra)
     return first, count
+
+
+def population_shards(member_envs: int, world_size: int) -> List[Tuple[int, int]]:
+    """Every rank's ``(first, c)`` of a data-parallel population whose members have ``member_envs`` = n envs each: rank r
+    holds ids ``[first, first + c)`` of every member (``shard_range``). Raises ``ValueError`` (on every rank alike: it
+    depends on n and the world size only) unless every c is a positive multiple of 128, which the population kernels
+    need."""
+    shards = [shard_range(int(member_envs), r, int(world_size)) for r in range(int(world_size))]
+    bad = [(r, c) for r, (_, c) in enumerate(shards) if c < 128 or c % 128 != 0]
+    if bad:
+        raise ValueError("a data-parallel population needs each rank's share of a member's %d envs to be a positive multiple "
+                         "of 128; over %d ranks rank %d would hold %d" % (int(member_envs), int(world_size), *bad[0]))
+    return shards
+
+
+def blocked_env_ids(rows: torch.Tensor, blocks: int, block_envs: int, block_stride: int, env_id_base: int) -> torch.Tensor:
+    """The global env ids of ``rows`` (int64) on a handle of ``blocks`` blocks of ``block_envs`` rows: ``env_id_base +
+    (row // block_envs) block_stride + row % block_envs`` (``VecEnv(blocks=, block_stride=)``; block_stride 0 repeats the
+    ids, as replicas do; one block is the plain handle)."""
+    rows = torch.as_tensor(rows, dtype=torch.int64)
+    return int(env_id_base) + torch.div(rows, int(block_envs), rounding_mode="floor") * int(block_stride) + rows % int(block_envs)
+
+
+def blocked_env_slots(ids: torch.Tensor, blocks: int, block_envs: int, block_stride: int, env_id_base: int) -> torch.Tensor:
+    """The inverse of ``blocked_env_ids`` for unique ids (block_stride >= block_envs, or one block): the row of every id of
+    ``ids``. Raises ``ValueError`` for an id the handle does not hold."""
+    off = torch.as_tensor(ids, dtype=torch.int64) - int(env_id_base)
+    if int(blocks) == 1:
+        k, j = torch.zeros_like(off), off
+    else:
+        k, j = torch.div(off, int(block_stride), rounding_mode="floor"), off % int(block_stride)
+    bad = (off < 0) | (k >= int(blocks)) | (j >= int(block_envs))
+    if bool(bad.any()):
+        first = int(off[bad][0]) + int(env_id_base)
+        raise ValueError("env id %d is outside this handle's ids (%d blocks of %d from %d, %d apart)"
+                         % (first, int(blocks), int(block_envs), int(env_id_base), int(block_stride)))
+    return k * int(block_envs) + j
 
 
 # ---- checkpoints over shards: pure functions on state dicts (VecEnv.state_dict / VecWorld2.state_dict) ------------------
@@ -76,6 +113,18 @@ def merge_trainer_state_dicts(sds) -> dict:
     """One trainer state dict (``A2CTrainer`` / ``PPOTrainer.state_dict``) from those of the ranks of a data-parallel run:
     the env parts merged with ``merge_state_dicts``, the shared parts (policy, Adam state, noise counter, sampling seed,
     iteration) taken once. Raises ``ValueError`` unless the shared parts are bit-equal on every rank."""
+    return _merge_run_state_dicts(sds)
+
+
+def merge_population_state_dicts(sds) -> dict:
+    """One ``PPOPopulation.state_dict`` from those of the ranks of a data-parallel population: the env parts (each rank's
+    blocked ids of every member) merged with ``merge_state_dicts``, the shared parts (every member's policy, Adam state and
+    hyper-parameters, the noise counter, sampling seed and iteration) taken once. Raises ``ValueError`` unless the shared
+    parts are bit-equal on every rank. The result loads into a population of any layout, a single process included."""
+    return _merge_run_state_dicts(sds)
+
+
+def _merge_run_state_dicts(sds) -> dict:
     sds = list(sds)
     if not sds:
         raise ValueError("nothing to merge")
@@ -120,6 +169,36 @@ def check_trainer_shards(infos) -> int:
     return nxt
 
 
+def check_population_shards(infos, members: int) -> Tuple[int, int]:
+    """``infos``: per rank in rank order, ``(env_id_base, num_envs, blocks, block_stride, signature)`` of a data-parallel
+    population of ``members`` = P. Returns ``(B, n)``: the population's first id (rank 0's env_id_base) and the env count
+    of each member. Raises ``ValueError`` unless every rank holds ``VecEnv(P c_r, env_id_base=B + first_r, blocks=P,
+    block_stride=n)`` with the shards ``[first_r, first_r + c_r)`` tiling ``[0, n)`` in rank order, every c_r a positive
+    multiple of 128, and every signature equal to rank 0's."""
+    infos, P = list(infos), int(members)
+    B = int(infos[0][0])
+    counts = []
+    for r, (base, num, blocks, stride, sig) in enumerate(infos):
+        if int(num) % P != 0 or int(num) // P < 128 or (int(num) // P) % 128 != 0:
+            raise ValueError("rank %d holds %d envs: a data-parallel population of %d members needs %d c envs per rank, c a "
+                             "positive multiple of 128" % (r, int(num), P, P))
+        if int(blocks) != P:
+            raise ValueError("rank %d's VecEnv has %d blocks; a data-parallel population of %d members needs blocks=%d (one "
+                             "per member)" % (r, int(blocks), P, P))
+        counts.append(int(num) // P)
+        if sig != infos[0][4]:
+            raise ValueError("rank %d's population differs from rank 0's (%r vs %r)" % (r, sig, infos[0][4]))
+    n, nxt = sum(counts), 0
+    for r, (base, num, blocks, stride, sig) in enumerate(infos):
+        if int(base) != B + nxt:
+            raise ValueError("rank %d's shard starts at id %d, expected %d: the shards must tile [%d, %d) contiguously in "
+                             "rank order" % (r, int(base), B + nxt, B, B + n))
+        if P > 1 and int(stride) != n:
+            raise ValueError("rank %d's VecEnv has block_stride %d; members of %d envs need block_stride=%d" % (r, int(stride), n, n))
+        nxt += counts[r]
+    return B, n
+
+
 def minibatch_bounds(rows: int, minibatches: int):
     """Row offsets of the ``minibatches`` contiguous slices of a permutation of ``rows`` rows (``PPOTrainer``)."""
     return [k * rows // minibatches for k in range(minibatches + 1)]
@@ -158,6 +237,30 @@ def global_mean_std(x: torch.Tensor, group=None) -> Tuple[torch.Tensor, torch.Te
     mean = sc[0] / sc[1]
     ss = rank_order_sum(((x64 - mean) ** 2).sum().reshape(1), group)[0]
     return mean.to(x.dtype), (ss / (sc[1] - 1.0)).sqrt().to(x.dtype)
+
+
+def global_mean_std_members(x: torch.Tensor, group=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """``global_mean_std`` of every member at once: x [P, ...] holds member p's elements in ``x[p]``. Returns mean and
+    std [P] (x's dtype), each bit-equal to ``global_mean_std(x[p].contiguous(), group)``, with two collectives in all
+    instead of 2 P: the per-member fp64 sums are formed as that call forms them, one member at a time."""
+    P = x.shape[0]
+    x64 = [x[p].detach().reshape(-1).double() for p in range(P)]
+    sc = rank_order_sum(torch.stack([torch.stack([v.sum(), torch.full((), float(v.numel()), dtype=torch.float64, device=x.device)])
+                                     for v in x64]), group)
+    mean = sc[:, 0] / sc[:, 1]
+    ss = rank_order_sum(torch.stack([((v - mean[p]) ** 2).sum() for p, v in enumerate(x64)]), group)
+    return mean.to(x.dtype), (ss / (sc[:, 1] - 1.0)).sqrt().to(x.dtype)
+
+
+def process_group(group, who: str):
+    """The group a population-level object works over: ``None`` for a single process (no group, or a group of one rank),
+    else ``group``. Raises ``ValueError`` for a group given without an initialised ``torch.distributed``."""
+    import torch.distributed as dist
+    if group is None:
+        return None
+    if not (dist.is_available() and dist.is_initialized()):
+        raise ValueError("%s was given a group, but torch.distributed is not initialised" % who)
+    return group if dist.get_world_size(group) > 1 else None
 
 
 def _distributed(group=None) -> bool:

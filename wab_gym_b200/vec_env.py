@@ -59,7 +59,7 @@ class VecEnv:
     def __init__(self, num_envs: int, game_options: Optional[dict] = None, device="cuda", seed: int = 0,
                  env_id_base: int = 0, auto_reset: bool = True, wolf_cap: int = 16, log_cap: Optional[int] = None,
                  force_f64_food: bool = False, features: bool = False, ego: bool = False, emit_grids: bool = True,
-                 replicas: int = 1):
+                 replicas: int = 1, blocks: int = 1, block_stride: int = 0):
         self._h = None
         self._bound = None     # feature buffer currently bound in the handle
         self.lib = _lib.load()  # raises if the CUDA library is unavailable — no fallback
@@ -85,6 +85,19 @@ class VecEnv:
         self.replicas = int(replicas)
         if self.replicas < 1 or self.num_envs % self.replicas != 0:
             raise ValueError("replicas must divide num_envs (got %d envs, %d replicas)" % (self.num_envs, self.replicas))
+        #: blocks = K > 1: the N envs are K blocks of c = N / K envs, and row k c + j has global env id env_id_base +
+        #: k block_stride + j in every draw keyed by the global id, so block k, driven by its own actions, plays what
+        #: VecEnv(c, env_id_base=env_id_base + k block_stride) plays. With block_stride >= c the ids are unique: one handle
+        #: holds a shard of every member of a data-parallel population (ids B + p n + first .. of member p). state_dict,
+        #: load_state_dict and load_state without slots work on the blocked ids (``global_ids`` / ``slots_of_ids``).
+        self.blocks, self.block_stride = int(blocks), int(block_stride)
+        if self.blocks > 1 and self.replicas > 1:
+            raise ValueError("a handle has replicas or blocks, not both")
+        if self.blocks < 1 or self.num_envs % self.blocks != 0:
+            raise ValueError("blocks must divide num_envs (got %d envs, %d blocks)" % (self.num_envs, self.blocks))
+        if self.blocks > 1 and self.block_stride < self.num_envs // self.blocks:
+            raise ValueError("block_stride must be at least num_envs / blocks = %d, or the blocks' ids overlap (got %d)"
+                             % (self.num_envs // self.blocks, self.block_stride))
         cs = self.game.to_struct()
         thr = np.ascontiguousarray(self.game.bush_thr, dtype=np.uint32)
         handle = ctypes.c_void_p()
@@ -94,6 +107,8 @@ class VecEnv:
         self._h = handle
         if self.replicas > 1:
             _lib.check(self.lib.wab_vec_set_replicas(self._h, self.replicas))
+        if self.blocks > 1:
+            _lib.check(self.lib.wab_vec_set_blocks(self._h, self.blocks, self.block_stride))
         self.lanes_per_env = int(self.lib.wab_vec_lanes_per_env(self._h))
         self.generic_kernels = bool(self.lib.wab_vec_kernel_kind(self._h))
         self.with_ego = bool(ego)
@@ -355,9 +370,33 @@ class VecEnv:
             raise ValueError("slots must lie in [0, %d)" % self.num_envs)
         return s
 
+    def _layout(self):
+        """(blocks, envs per block, block_stride) of this handle's id map: (1, N, 0) for a plain handle, (R, N / R, 0) with
+        replicas."""
+        if self.replicas > 1:
+            return self.replicas, self.num_envs // self.replicas, 0
+        if self.blocks > 1:
+            return self.blocks, self.num_envs // self.blocks, self.block_stride
+        return 1, self.num_envs, 0
+
+    def global_ids(self, slots=None) -> torch.Tensor:
+        """The global env id of every slot (or of ``slots``), int64 on the CPU: the key of every draw made for it."""
+        local = torch.arange(self.num_envs, dtype=torch.int64) if slots is None else self._local_slots(slots)
+        from .sharding import blocked_env_ids
+        return blocked_env_ids(local, *self._layout(), self.env_id_base)
+
+    def slots_of_ids(self, env_ids) -> torch.Tensor:
+        """The slot of every global id of ``env_ids`` (int64, CPU). Raises ``ValueError`` for an id this handle does not
+        hold, or on a handle with replicas, whose ids repeat."""
+        self._refuse_replicas("slots_of_ids")
+        from .sharding import blocked_env_slots
+        return blocked_env_slots(torch.as_tensor(env_ids, dtype=torch.int64).reshape(-1).cpu(), *self._layout(),
+                                 self.env_id_base)
+
     def save_state(self, slots=None) -> EnvStates:
         """The state of every env (or of ``slots``, in that order) as records on the device. Enqueued on the current
-        stream; nothing synchronises. On a handle with replicas the ids repeat: block k's records carry block 0's ids."""
+        stream; nothing synchronises. On a handle with replicas the ids repeat: block k's records carry block 0's ids. On a
+        blocked handle they are the blocked ids."""
         if slots is None:
             local, d_slots = torch.arange(self.num_envs, dtype=torch.int64), None
         else:
@@ -365,7 +404,8 @@ class VecEnv:
             d_slots = local.to(device=self.device, dtype=torch.int32)
         records = torch.empty((local.numel(), self.record_bytes), dtype=torch.uint8, device=self.device)
         _lib.check(self.lib.wab_vec_save_state(self._h, _ptr(d_slots), local.numel(), _ptr(records), self._stream()))
-        return EnvStates(records, local % (self.num_envs // self.replicas) + self.env_id_base, self.fingerprint)
+        from .sharding import blocked_env_ids
+        return EnvStates(records, blocked_env_ids(local, *self._layout(), self.env_id_base), self.fingerprint)
 
     def load_state(self, states: EnvStates, slots=None) -> ObsBatch:
         """Write each record of ``states`` into a slot: the slot of its own global id (which must belong to this handle),
@@ -383,12 +423,10 @@ class VecEnv:
                              "kernel family or ego setting" % (int(states.fingerprint), self.fingerprint))
         n = records.shape[0]
         if slots is None:
-            local = torch.as_tensor(states.env_ids, dtype=torch.int64).reshape(-1).cpu() - self.env_id_base
-            if local.numel() != n:
+            ids = torch.as_tensor(states.env_ids, dtype=torch.int64).reshape(-1).cpu()
+            if ids.numel() != n:
                 raise ValueError("env_ids and records disagree in length")
-            if n and (int(local.min()) < 0 or int(local.max()) >= self.num_envs):
-                raise ValueError("a record's env id is outside this handle's [%d, %d)" %
-                                 (self.env_id_base, self.env_id_base + self.num_envs))
+            local = self.slots_of_ids(ids)
         else:
             local = self._local_slots(slots)
             if local.numel() != n:
@@ -420,13 +458,14 @@ class VecEnv:
 
     def load_state_dict(self, sd: dict) -> ObsBatch:
         """Resume from ``state_dict()`` output (of this or any other shard layout: the records of this handle's global ids
-        are picked, each exactly once). The statistics totals go to the shard holding env 0 and every other shard starts
-        from zero, so their sum is preserved."""
+        are picked, each exactly once; on a blocked handle each block's range). The statistics totals go to the shard
+        holding env 0 and every other shard starts from zero, so their sum is preserved."""
         self._refuse_replicas("load_state_dict")
         from .sharding import select_shard_records
-        records = select_shard_records(sd, self.env_id_base, self.num_envs, self.fingerprint, self.record_bytes)
-        ids = torch.arange(self.env_id_base, self.env_id_base + self.num_envs, dtype=torch.int64)
-        obs = self.load_state(EnvStates(records, ids, self.fingerprint))
+        K, c, stride = self._layout()
+        records = torch.cat([select_shard_records(sd, self.env_id_base + k * stride, c, self.fingerprint, self.record_bytes)
+                             for k in range(K)])            # block k: its contiguous id range, in slot order
+        obs = self.load_state(EnvStates(records, self.global_ids(), self.fingerprint))
         stats = np.zeros(8, dtype=np.int64)
         if self.env_id_base == 0:
             stats[:] = torch.as_tensor(sd["stats"], dtype=torch.int64).numpy()
