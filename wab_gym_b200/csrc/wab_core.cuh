@@ -36,6 +36,35 @@
 
 namespace wab {
 
+// ---- cycle probe of the pipeline kernel's rule warp (a separate build: -DWAB_PIPE_CLOCKS, tools/pipe_clocks.py).
+// Lane 0 of each rule warp reads clock64() at the region boundaries of every step and adds the cycles since the previous
+// boundary to its warp's row in shared memory; the first active lane of a warp counts each pass through a rare path
+// (divergent groups that run it one after another count once each). Without the switch the marks compile to nothing.
+enum PipeRegion : int { PC_DRAWS, PC_SLIDE, PC_DEPLOG, PC_DESPAWN, PC_CHASE, PC_EAT, PC_TAIL, PC_RESET, PC_HANDOFF, PC_N };
+enum PipePath : int { PP_STEPS, PP_TIE, PP_DEPLOG, PP_WOLVES, PP_EAT, PP_EAT_HIT, PP_SPAWN, PP_RESET, PP_N };
+#if defined(WAB_PIPE_CLOCKS) && defined(__CUDACC__)
+constexpr int kPcWarps = 8;                     // rule warps per CTA the rows cover (WAB_PIPE_PAIRS <= 8)
+__shared__ unsigned long long pc_cyc[kPcWarps][PC_N + 1];   // [PC_N]: clock of the last boundary
+__shared__ unsigned int pc_cnt[kPcWarps][PP_N];
+__device__ __forceinline__ void pc_mark(int r) {
+    const unsigned long long t = clock64();
+    if ((threadIdx.x & 31) == 0) {
+        unsigned long long* row = pc_cyc[(threadIdx.x >> 5) % kPcWarps];
+        row[r] += t - row[PC_N]; row[PC_N] = t;
+    }
+}
+__device__ __forceinline__ void pc_count(int k) {
+    if ((int)(threadIdx.x & 31) == __ffs((int)__activemask()) - 1) atomicAdd(&pc_cnt[(threadIdx.x >> 5) % kPcWarps][k], 1u);
+}
+#endif
+#if defined(WAB_PIPE_CLOCKS) && defined(__CUDA_ARCH__)
+#define WAB_PC_MARK(r) ::wab::pc_mark(r)
+#define WAB_PC_COUNT(k) ::wab::pc_count(k)
+#else
+#define WAB_PC_MARK(r) ((void)0)
+#define WAB_PC_COUNT(k) ((void)0)
+#endif
+
 constexpr uint32_t PHILOX_M0 = 0xD2511F53u, PHILOX_M1 = 0xCD9E8D57u;
 constexpr uint32_t PHILOX_W0 = 0x9E3779B9u, PHILOX_W1 = 0xBB67AE85u;
 enum : uint32_t { SITE_BUSH = 1, SITE_INIT = 2, SITE_SPAWN = 3, SITE_DESP = 4, SITE_START = 5 };
@@ -385,7 +414,7 @@ WAB_HD void slide_block(const Params& P, const Env& E, const SlideLine& L, int b
     tie |= (h0 == t_hi ? 1u : 0u) | (h1 == t_hi ? 1u : 0u);
 }
 
-// The keyed draws of one step that depend only on the env's state before the step and its action (env_step with DRAWN):
+// The keyed draws of one step that depend only on the env's state before the step and its action (env_step_pipe):
 // this lane's slide blocks and the spawn draw.
 struct StepDraws {
     uint32_t acc, tie;   // slide_block over this lane's blocks b = sub, sub + LPE, ... < 6
@@ -395,10 +424,8 @@ struct StepDraws {
 // Slide the window after the ostrich moved by (dx, dy) (one of them non-zero) to (E.x, E.y) and
 // reveal the 11 new cells: generate_bushes, wab_env.py:613-629, for cells without a record; cells
 // seen before get the same draw (keys do not depend on the turn) minus what was eaten.
-// DRAWN: this lane's block draws come in `D` (made before the step's rules) instead of being made here.
-template <int LPE, bool DRAWN = false>
-WAB_HD void slide_window(const Params& P, Env& E, const Slots& S, int32_t dx, int32_t dy, const Coop<LPE>& coop,
-                         const StepDraws* D = nullptr) {
+template <int LPE>
+WAB_HD void slide_window(const Params& P, Env& E, const Slots& S, int32_t dx, int32_t dy, const Coop<LPE>& coop) {
     // drop the column that would wrap into the neighbouring row, then shift by 11*dx + dy
     if (dy > 0) {
         E.m[0] &= ~ColMask<10, 0>::v; E.m[1] &= ~ColMask<10, 1>::v; E.m[2] &= ~ColMask<10, 2>::v; E.m[3] &= ~ColMask<10, 3>::v;
@@ -423,22 +450,18 @@ WAB_HD void slide_window(const Params& P, Env& E, const Slots& S, int32_t dx, in
     const uint32_t sel0 = half_sel(along_y ? fb : 0u), sel1 = half_sel(along_y ? fb : 1u);
     uint32_t acc = 0, tie = 0;
     if (P.n_bush_thr > 0) {
-        if (DRAWN) {
-            acc = D->acc; tie = D->tie;
-        } else {
 #if defined(__CUDA_ARCH__)
 #pragma unroll kSlideUnroll
 #endif
-            for (int b = (int)coop.sub; b < 6; b += LPE) {   // slide_block, written out
-                uint32_t p[2];
-                const uint32_t c0 = (along_y ? pack_xy(fixed >> 1, vb0 + b) : pack_xy(vb0 + b, fixed >> 1)) ^ E.bk_a;
-                philox2(P, c0, E.bk_b, p);
-                const uint32_t h0 = half_of((along_y || !fb) ? p[0] : p[1], sel0);
-                const uint32_t h1 = half_of((along_y || fb) ? p[1] : p[0], sel1);
-                const uint32_t bit = 1u << (top - 2 * b);
-                acc |= (h0 > t_hi ? bit : 0u) | (h1 > t_hi ? (bit >> 1) : 0u);
-                tie |= (h0 == t_hi ? 1u : 0u) | (h1 == t_hi ? 1u : 0u);
-            }
+        for (int b = (int)coop.sub; b < 6; b += LPE) {   // slide_block, written out
+            uint32_t p[2];
+            const uint32_t c0 = (along_y ? pack_xy(fixed >> 1, vb0 + b) : pack_xy(vb0 + b, fixed >> 1)) ^ E.bk_a;
+            philox2(P, c0, E.bk_b, p);
+            const uint32_t h0 = half_of((along_y || !fb) ? p[0] : p[1], sel0);
+            const uint32_t h1 = half_of((along_y || fb) ? p[1] : p[0], sel1);
+            const uint32_t bit = 1u << (top - 2 * b);
+            acc |= (h0 > t_hi ? bit : 0u) | (h1 > t_hi ? (bit >> 1) : 0u);
+            tie |= (h0 == t_hi ? 1u : 0u) | (h1 == t_hi ? 1u : 0u);
         }
         if (tie) {                 // 2^-15 per block: settle this lane's cells on their full 32-bit draws
             acc = 0;
@@ -535,9 +558,8 @@ WAB_HD StepDraws step_draws(const Params& P, const Env& E, int32_t dx, int32_t d
 }
 
 // One step of one environment: wab_env.py:250-342 up to (not including) auto-reset and the
-// observation stores. `F64` selects the reference's fp64 food arithmetic. DRAWN makes the step's
-// keyed draws first (step_draws) and hands them to the rules; the results are the same.
-template <bool F64, int LPE, bool DRAWN = false>
+// observation stores. `F64` selects the reference's fp64 food arithmetic.
+template <bool F64, int LPE>
 WAB_HD void env_step(const Params& P, Env& E, const Slots& S, uint32_t action, StepOut& O, const Coop<LPE>& coop) {
     // ---- :251-258 action
     O.bad_action = (action >= (uint32_t)P.n_actions) ? 1u : 0u;
@@ -548,11 +570,9 @@ WAB_HD void env_step(const Params& P, Env& E, const Slots& S, uint32_t action, S
     E.x += dx; E.y += dy;                          // :255-256
     if (nrole >= 0) E.role = (uint32_t)nrole;      // :257-258
     O.overflow = 0;
-    StepDraws D;
-    if (DRAWN) D = step_draws<LPE>(P, E, dx, dy, coop);
 
     // ---- :259 generate_bushes for the newly visible line
-    if (dx != 0 || dy != 0) slide_window<LPE, DRAWN>(P, E, S, dx, dy, coop, &D);
+    if (dx != 0 || dy != 0) slide_window<LPE>(P, E, S, dx, dy, coop);
 
     // ---- :262-264 despawn (keep iff U > chance). rank = ordinal among earlier wolves on the cell.
     if (E.nw) {
@@ -653,7 +673,7 @@ WAB_HD void env_step(const Params& P, Env& E, const Slots& S, uint32_t action, S
 
     // ---- :325-326 spawn_wolves on the 48 ring cells around the moved ostrich: one binomial-first draw
     if (P.wolves) {
-        const uint64_t v = DRAWN ? D.spawn : binomial_draw(P, E.env_id, E.episode, SITE_SPAWN, E.turn);
+        const uint64_t v = binomial_draw(P, E.env_id, E.episode, SITE_SPAWN, E.turn);
         if (v >= P.spawn_cdf[0]) {                 // rare (2.4 % of steps): at least one wolf appears
             uint32_t chosen[4];
             binomial_choose(P, E.env_id, E.episode, SITE_SPAWN, E.turn, RING, v, chosen);
@@ -693,6 +713,266 @@ WAB_HD void env_step(const Params& P, Env& E, const Slots& S, uint32_t action, S
     O.food_obs = food_observation(P, E, F64);
     O.role = E.role;
     O.status = E.status;
+}
+
+// OR over the LPE lanes of a group as a butterfly; the whole warp must be converged here (env_step_pipe).
+template <int LPE>
+WAB_HD uint32_t group_or_converged(uint32_t v) {
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+    for (int o = 1; o < LPE; o <<= 1) v |= __shfl_xor_sync(0xFFFFFFFFu, v, o);
+#endif
+    return v;
+}
+// A warp-uniform test: every lane takes the branch if any lane needs it, so the warp never splits on it.
+#if defined(__CUDA_ARCH__)
+#define WAB_ANY(p) __any_sync(0xFFFFFFFFu, (p))
+#else
+#define WAB_ANY(p) (p)
+#endif
+
+// slide_window's settling of a revealed line on full 32-bit draws, for a lane whose blocks had a tie (2^-15 per block).
+template <int LPE>
+WAB_HD uint32_t slide_settle(const Params& P, const Env& E, const SlideLine& L, uint32_t sub) {
+    uint32_t acc = 0u;
+    WAB_ROLLED
+    for (int b = (int)sub; b < 6; b += LPE) {
+        const uint32_t c0 = (L.along_y ? pack_xy(L.fixed >> 1, L.vb0 + b) : pack_xy(L.vb0 + b, L.fixed >> 1)) ^ E.bk_a;
+        WAB_ROLLED
+        for (uint32_t e = 0; e < 2u; ++e) {
+            const uint32_t lane = L.along_y ? (L.fb | (e << 1)) : (e | (L.fb << 1));
+            if (bush_word_rare(c0, E.bk_b, P.rk2[0], lane) >= P.thr_bush1) acc |= 1u << (L.top - 2 * b - (int32_t)e);
+        }
+    }
+    return acc;
+}
+
+// env_step for the pipeline kernel's rule warp, with the same results. Every lane of the warp calls it, converged; lanes
+// whose env does not exist (`active` false, the ragged last warp) step a neutral Env that never eats or spawns and whose
+// results the caller drops. The step's keyed draws are made first (step_draws), and the common step is straight-line code:
+// every env slides (a stay is a shift by 0 and an empty deposit), both deposit forms are computed and selected, and the
+// group's OR of the revealed line is a butterfly. Each rare path (a tie of a revealed block, the depletion log of an env
+// that has eaten a bush empty, wolves, an eat, a spawn) is entered through one warp-uniform test, so the warp never splits
+// on it: inside, each env is predicated as in env_step, and the warp runs the path once whichever of its envs need it.
+template <bool F64, int LPE>
+WAB_HD void env_step_pipe(const Params& P, Env& E, const Slots& S, uint32_t action, StepOut& O, const Coop<LPE>& coop,
+                          bool active) {
+    // ---- :251-258 action
+    O.bad_action = (action >= (uint32_t)P.n_actions) ? 1u : 0u;
+    const uint32_t code = O.bad_action ? 0x05u /* dx=0, dy=0, keep */ : (uint32_t)(P.act_tbl >> (8 * action)) & 0xFFu;
+    const int32_t dx = (int32_t)(code & 3u) - 1, dy = (int32_t)((code >> 2) & 3u) - 1;
+    const int32_t nrole = (int32_t)((code >> 4) & 3u) - 1;
+    E.turn += 1;                                   // :252
+    E.x += dx; E.y += dy;                          // :255-256
+    E.role = nrole >= 0 ? (uint32_t)nrole : E.role;   // :257-258
+    O.overflow = 0;
+    const StepDraws D = step_draws<LPE>(P, E, dx, dy, coop);
+    WAB_PC_MARK(PC_DRAWS);
+
+    // ---- :259 generate_bushes for the newly visible line (slide_window)
+    const uint32_t d0 = dy > 0 ? ColMask<10, 0>::v : dy < 0 ? ColMask<0, 0>::v : 0u;
+    const uint32_t d1 = dy > 0 ? ColMask<10, 1>::v : dy < 0 ? ColMask<0, 1>::v : 0u;
+    const uint32_t d2 = dy > 0 ? ColMask<10, 2>::v : dy < 0 ? ColMask<0, 2>::v : 0u;
+    const uint32_t d3 = dy > 0 ? ColMask<10, 3>::v : dy < 0 ? ColMask<0, 3>::v : 0u;
+    E.m[0] &= ~d0; E.m[1] &= ~d1; E.m[2] &= ~d2; E.m[3] &= ~d3;
+    const int32_t s = 11 * dx + dy;
+    shl128(E.m, (uint32_t)(s > 0 ? s : 0));
+    shr128(E.m, (uint32_t)(s < 0 ? -s : 0));
+    E.m[3] &= TOP_WORD_MASK;
+    const bool reveal = (dx != 0 || dy != 0) && P.n_bush_thr > 0;
+    const SlideLine L = slide_line(E, dx, dy);
+    uint32_t acc = reveal ? D.acc : 0u;
+    const uint32_t tie = reveal ? D.tie : 0u;
+    if (WAB_ANY(tie != 0u)) {
+        WAB_PC_COUNT(PP_TIE);
+        if (tie) acc = slide_settle<LPE>(P, E, L, coop.sub);
+    }
+    acc &= 0xFFEu;                                 // cells g = 0..10
+    WAB_PC_MARK(PC_SLIDE);
+    if (WAB_ANY(E.dep && acc)) {                   // something was eaten empty this episode: revealed cells consult the log
+        WAB_PC_COUNT(PP_DEPLOG);
+        uint32_t bits = E.dep ? acc : 0u;
+        WAB_ROLLED
+        while (bits) {
+#if defined(__CUDA_ARCH__)
+            const int k = __ffs((int)bits) - 1;
+#else
+            const int k = __builtin_ctz(bits);
+#endif
+            bits &= bits - 1u;
+            const int32_t v = L.vmax - (k - 1);
+            if (!(L.along_y ? bush_alive(P, E, S, L.fixed, v) : bush_alive(P, E, S, v, L.fixed))) acc &= ~(1u << k);
+        }
+    }
+    WAB_PC_MARK(PC_DEPLOG);
+    {
+        const uint32_t line = group_or_converged<LPE>(acc >> 1);
+        uint32_t t[4];                             // column j = 0 (dy > 0) or j = 10 (dy < 0): bits 11*g + j
+        spread11(line, t);
+        shl128(t, dy < 0 ? 10u : 0u);
+        const bool along_y = dx != 0;              // row i = 0 (dx > 0) or i = 10 (dx < 0): bits 11*i + g
+        E.m[0] |= along_y ? (dx > 0 ? line : 0u) : t[0];
+        E.m[1] |= along_y ? 0u : t[1];
+        E.m[2] |= along_y ? 0u : t[2];
+        E.m[3] |= along_y ? (dx < 0 ? (line << 14) : 0u) : t[3];   // 110 = 96 + 14
+    }
+    WAB_PC_MARK(PC_SLIDE);
+
+    // ---- :262-264 despawn (keep iff U > chance). rank = ordinal among earlier wolves on the cell.
+    const bool any_wolf = WAB_ANY(E.nw != 0u);
+    if (any_wolf) {
+        WAB_PC_COUNT(PP_WOLVES);
+        if (E.nw) {
+            uint32_t kept = 0;
+            uint64_t keepmask = 0;                         // wolf_cap <= 64
+            WAB_ROLLED
+            for (uint32_t k = 0; k < E.nw; ++k) {
+                const uint32_t p = S.wolves[(int32_t)k * S.wstride];
+                uint32_t rank = 0;
+                WAB_ROLLED
+                for (uint32_t q = 0; q < k; ++q) rank += (S.wolves[(int32_t)q * S.wstride] == p) ? 1u : 0u;
+                uint32_t w[4];
+                philox(P, E.env_id, E.episode, ctr2(SITE_DESP, E.turn, rank >> 2), p, w);
+                if ((uint64_t)pick4(w, rank & 3u) >= P.thr_keep) keepmask |= 1ull << k;
+            }
+            group_sync(coop);                       // every lane of the group has read the slots
+            if (group_leader(coop)) {
+                WAB_ROLLED
+                for (uint32_t k = 0; k < E.nw; ++k)
+                    if ((keepmask >> k) & 1ull) {
+                        S.wolves[(int32_t)kept * S.wstride] = S.wolves[(int32_t)k * S.wstride];
+                        ++kept;
+                    }
+            }
+            group_sync(coop);
+            E.nw = popc32((uint32_t)keepmask) + popc32((uint32_t)(keepmask >> 32));
+        }
+    }
+    WAB_PC_MARK(PC_DESPAWN);
+
+    // ---- :266 the frame the rest of the step reads: bushes with food > 0, ostrich status
+    O.bm[0] = E.m[0]; O.bm[1] = E.m[1]; O.bm[2] = E.m[2]; O.bm[3] = E.m[3];
+    const uint32_t status_pre = E.status;
+
+    // ---- :267-297 wolves chase (ties -> x axis), kill on contact; wolf plane after the move (:289)
+    O.wm[0] = O.wm[1] = O.wm[2] = O.wm[3] = 0u;
+    if (any_wolf) {
+        WAB_ROLLED
+        for (uint32_t k = 0; k < E.nw; ++k) {
+            const uint32_t p = S.wolves[(int32_t)k * S.wstride];
+            int32_t wx = unpack_x(p), wy = unpack_y(p);
+            int32_t ddx = E.x - wx, ddy = E.y - wy;                                  // :59-60
+            if (P.wolves_can_move) {
+                const int32_t ax = ddx < 0 ? -ddx : ddx, ay = ddy < 0 ? -ddy : ddy;
+                const int32_t sx = (ddx > 0) - (ddx < 0), sy = (ddy > 0) - (ddy < 0);
+                wx += (ax >= ay) ? sx : 0;                                           // :278-280
+                wy += (ax < ay) ? sy : 0;                                            // :281-283
+                group_sync(coop);                                                    // all lanes hold the old position
+                if (group_leader(coop)) S.wolves[(int32_t)k * S.wstride] = pack_xy(wx, wy);   // :285-286
+                ddx = E.x - wx; ddy = E.y - wy;
+            }
+            if (ddx == 0 && ddy == 0 && !P.god_mode) E.status = 2u;                  // :292-297
+            if (ddx >= -HALF && ddx <= HALF && ddy >= -HALF && ddy <= HALF)          // :416-427
+                setbit128(O.wm, 11 * (ddx + HALF) + (ddy + HALF), 1u);
+        }
+        if (E.nw && P.wolves_can_move) group_sync(coop);                             // moved positions published to the group
+    }
+    WAB_PC_MARK(PC_CHASE);
+
+    // ---- :300-313 eat (bush and status as of the frame above; role is fresh)
+    O.ate = 0;
+    E.stale = 0u;
+    const bool eat = active && ((O.bm[1] >> 28) & 1u) && (E.role == 1u || P.lookout_only) && status_pre == 0u;   // bit 60 = [5][5]
+    if (WAB_ANY(eat)) {
+        WAB_PC_COUNT(PP_EAT);
+        if (eat) {
+            O.ate = 1u;
+            if (F64) {
+                double f = E.food_f + P.food_inc;                                    // :307-309
+                f = f < 0.0 ? 0.0 : f; f = f > 1.0 ? 1.0 : f;                        // :310
+                E.food_f = f;
+            } else {
+                int32_t f = E.food_i + P.food_int_inc;
+                E.food_i = f > P.food_int_max ? P.food_int_max : f;
+            }
+            // bush.food -= 1 (:312): count the eat; the cell disappears when eats == its first-reveal value
+            const uint32_t cell = pack_xy(E.x, E.y);
+            int32_t l = log_find(E, S, cell);
+            uint32_t eats;
+            if (l >= 0) {
+                WAB_PC_COUNT(PP_EAT_HIT);
+                eats = (uint32_t)S.logcnt[(int64_t)l * S.lstride] + 1u;
+                group_sync(coop);                      // every lane of the group has read the old count
+                if (group_leader(coop)) S.logcnt[(int64_t)l * S.lstride] = (uint8_t)eats;
+                group_sync(coop);
+            } else if (E.nlog < (uint32_t)P.log_cap) {
+                eats = 1u;
+                S.logcell[(int64_t)E.nlog * S.lstride] = cell;
+                S.logcnt[(int64_t)E.nlog * S.lstride] = 1;
+                E.nlog += 1;
+                E.logsig |= cell_sig(cell);
+            } else {
+                eats = 1u; O.overflow = 1u;            // counted, never silent (WAB_STAT_OVERFLOWS)
+            }
+            const uint32_t still = eaten_bush_alive(P, E, E.x, E.y, eats);
+            if (!still) { E.m[1] &= ~(1u << 28); E.dep = 1u; E.stale = 1u; }
+        }
+    }
+    WAB_PC_MARK(PC_EAT);
+
+    // ---- :316-322 hunger, starvation (overrides killed)
+    if (F64) {
+        const double f = E.food_f - P.food_dec;
+        E.status = f <= 0.0 ? 1u : E.status;
+        E.food_f = f <= 0.0 ? 0.0 : f;
+    } else {
+        const int32_t f = E.food_i - 1;
+        E.status = f <= 0 ? 1u : E.status;
+        E.food_i = f <= 0 ? 0 : f;
+    }
+
+    // ---- :325-326 spawn_wolves on the 48 ring cells around the moved ostrich: one binomial-first draw
+    const bool spawn = P.wolves && active && D.spawn >= P.spawn_cdf[0];   // rare (2.4 % of steps): at least one wolf appears
+    if (WAB_ANY(spawn)) {
+        WAB_PC_COUNT(PP_SPAWN);
+        if (spawn) {
+            uint32_t chosen[4];
+            binomial_choose(P, E.env_id, E.episode, SITE_SPAWN, E.turn, RING, D.spawn, chosen);
+            WAB_ROLLED
+            for (int w = 0; w < 2; ++w) {                                         // :571-574, ring order
+                uint32_t bits = w ? chosen[1] : chosen[0];
+                WAB_ROLLED
+                while (bits) {
+#if defined(__CUDA_ARCH__)
+                    const int j = 32 * w + __ffs((int)bits) - 1;
+#else
+                    const int j = 32 * w + __builtin_ctz(bits);
+#endif
+                    bits &= bits - 1u;
+                    int32_t ox, oy;
+                    ring_offset(j, ox, oy);
+                    if (E.nw < (uint32_t)P.wolf_cap) {
+                        S.wolves[(int32_t)E.nw * S.wstride] = pack_xy(E.x + ox, E.y + oy);
+                        E.nw += 1;
+                    } else {
+                        O.overflow = 1u;
+                    }
+                }
+            }
+        }
+    }
+    // ---- :328-340 reward, done
+    const uint32_t outcome = E.status == 0u ? ((E.turn >= (uint32_t)P.max_turns) ? 1u : 0u) : (E.status == 1u ? 2u : 3u);
+    O.outcome = outcome;
+    O.done = outcome != 0u;
+    O.reward = P.reward_table[O.ate * 4u + outcome];
+    O.info = outcome | (O.ate << 2) | (O.bad_action << 3) | (E.status << 4);
+
+    // ---- :342, :387-391, :450-452 scalar observation (fresh)
+    O.food_obs = food_observation(P, E, F64);
+    O.role = E.role;
+    O.status = E.status;
+    WAB_PC_MARK(PC_TAIL);
 }
 
 // ------------------------------------------------------------------ reset pieces (wab_env.py:231-248)

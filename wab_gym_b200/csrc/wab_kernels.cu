@@ -420,8 +420,8 @@ wab_step_kernel(const __grid_constant__ Params P, const StatePtrs st, const uint
 // ---- the multi-step kernel of the lanes-per-env geometries as a two-warp pipeline --------------------------------------
 // A small batch is bound by the length of one step's dependent instruction chain, and a third of that chain is not rules
 // at all: composing the 363-bit strings, expanding them to bytes, the 16-byte stores and the scalar outputs. Here a CTA is
-// one PAIR of warps that owns EPW = 32 / LPE envs: warp 0 runs the rules (wab_step_kernel's, with each step's keyed
-// draws made first as independent chains: step_draws in wab_core.cuh) and parks
+// one PAIR of warps that owns EPW = 32 / LPE envs: warp 0 runs the rules (env_step_pipe in wab_core.cuh: wab_step_kernel's
+// rules with each step's keyed draws made first and the rare paths behind warp-uniform tests) and parks
 // each step's planes and scalars in a ring of shared-memory slots; warp 1 publishes them — bit stream, byte expansion,
 // stores, scalars, features — while warp 0 is already on the next steps. The two meet only at mbarriers in shared memory
 // (one "full" and one "empty" barrier per ring slot; an arrive never blocks, a wait spins on the barrier's phase parity).
@@ -458,6 +458,32 @@ __device__ __forceinline__ void pipe_mbar_wait(uint64_t* b, uint32_t parity) {
                      : "=r"(ok) : "r"(a), "r"(parity) : "memory");
     } while (!ok);
 }
+
+#if defined(WAB_PIPE_CLOCKS)
+// The probe's totals over every rule warp of every launch since the last wab_pipe_clocks_read(clear = 1):
+// [PC_N] cycles by region, then [PP_N] passes through each rare path (PP_STEPS: warp-steps).
+__device__ unsigned long long wab_pipe_clocks_buf[PC_N + PP_N];
+__device__ __forceinline__ void pipe_clocks_begin() {
+    const int w = (threadIdx.x >> 5) % kPcWarps;
+    if ((threadIdx.x & 31) == 0) {
+        for (int r = 0; r < PC_N; ++r) pc_cyc[w][r] = 0ull;
+        for (int k = 0; k < PP_N; ++k) pc_cnt[w][k] = 0u;
+    }
+    __syncwarp();
+    if ((threadIdx.x & 31) == 0) pc_cyc[w][PC_N] = clock64();
+}
+__device__ __forceinline__ void pipe_clocks_flush() {
+    __syncwarp();
+    const int w = (threadIdx.x >> 5) % kPcWarps;
+    if ((threadIdx.x & 31) == 0) {
+        for (int r = 0; r < PC_N; ++r) atomicAdd(&wab_pipe_clocks_buf[r], pc_cyc[w][r]);
+        for (int k = 0; k < PP_N; ++k) atomicAdd(&wab_pipe_clocks_buf[PC_N + k], (unsigned long long)pc_cnt[w][k]);
+    }
+}
+#else
+__device__ __forceinline__ void pipe_clocks_begin() {}
+__device__ __forceinline__ void pipe_clocks_flush() {}
+#endif
 
 template <bool F64, int LPE>
 __global__ void __launch_bounds__(PipeGeo<LPE>::THREADS, 1)
@@ -500,22 +526,20 @@ wab_step_pipe_kernel(const __grid_constant__ Params P, const StatePtrs st, const
         unsigned long long acc_outcome = 0ull, acc_misc = 0ull;
         const uint8_t* ap = actions + (c.active ? c.idx : 0);
         uint32_t a_next = c.active ? *ap : 0u;
+        pipe_clocks_begin();
         for (int t = 0; t < n_steps; ++t) {
+            WAB_PC_COUNT(PP_STEPS);
             StepOut O;
-            bool need_reset = false;
             const uint32_t a = a_next;
             ap += n;
             if (c.active && t + 1 < n_steps) a_next = *ap;
-            if (c.active) {
-                env_step<F64, LPE, true>(P, E, S, a, O, coop);
-                if (st.hist && c.writer && E.turn < (uint32_t)st.hist_len) st.hist[(int64_t)E.turn * n + c.idx] = pack_xy(E.x, E.y);
-                need_reset = O.done && P.auto_reset;
-                acc_outcome += 1ull << (16u * O.outcome);
-                acc_misc += (unsigned long long)O.ate | ((unsigned long long)O.bad_action << 16);
-            } else {
-                O = StepOut();
-            }
+            env_step_pipe<F64, LPE>(P, E, S, a, O, coop, c.active);   // the whole warp, absent envs included
+            if (st.hist && c.writer && E.turn < (uint32_t)st.hist_len) st.hist[(int64_t)E.turn * n + c.idx] = pack_xy(E.x, E.y);
+            const bool need_reset = c.active && O.done && P.auto_reset;
+            acc_outcome += c.active ? 1ull << (16u * O.outcome) : 0ull;
+            acc_misc += c.active ? (unsigned long long)O.ate | ((unsigned long long)O.bad_action << 16) : 0ull;
             if (__any_sync(FULL, need_reset)) {
+                WAB_PC_COUNT(PP_RESET);
                 warp_reset<F64, LPE>(P, E, S, need_reset, c.lane, O.wm, O.bm, O.overflow);
                 if (need_reset) {
                     O.food_obs = food_observation(P, E, F64);
@@ -523,6 +547,7 @@ wab_step_pipe_kernel(const __grid_constant__ Params P, const StatePtrs st, const
                 }
             }
             apply_view_mask(P, O.role, O.wm, O.bm);
+            WAB_PC_MARK(PC_RESET);
             const int s = t & (D - 1);
             __syncwarp();
             if (t >= D) pipe_mbar_wait(empty + s, ((uint32_t)(t / D) - 1u) & 1u);   // the publisher has taken step t - D out of this slot
@@ -536,7 +561,9 @@ wab_step_pipe_kernel(const __grid_constant__ Params P, const StatePtrs st, const
             }
             __syncwarp();
             if (lane == 0) pipe_mbar_arrive(full + s);      // step t is in the slot
+            WAB_PC_MARK(PC_HANDOFF);
         }
+        pipe_clocks_flush();
         if (c.writer) store_env<F64>(st, c.idx, E, wolves_s, EPW);
         uint32_t cnt[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
         if (c.writer) {
@@ -1191,6 +1218,22 @@ extern "C" {
 
 const char* wab_last_error(void) { return g_err.c_str(); }
 int wab_abi_version(void) { return WAB_ABI_VERSION; }
+
+#if defined(WAB_PIPE_CLOCKS)
+// Probe build only (tools/pipe_clocks.py): copy the current device's PC_N + PP_N probe totals to `out`, then zero them
+// if `clear`. Synchronises the device.
+int wab_pipe_clocks_read(unsigned long long* out, int clear) {
+    if (cudaDeviceSynchronize() != cudaSuccess ||
+        cudaMemcpyFromSymbol(out, wab_pipe_clocks_buf, sizeof(wab_pipe_clocks_buf)) != cudaSuccess)
+        return fail(WAB_E_CUDA, "wab_pipe_clocks_read failed");
+    if (clear) {
+        static const unsigned long long zero[PC_N + PP_N] = {};
+        if (cudaMemcpyToSymbol(wab_pipe_clocks_buf, zero, sizeof(zero)) != cudaSuccess)
+            return fail(WAB_E_CUDA, "wab_pipe_clocks_read failed");
+    }
+    return WAB_OK;
+}
+#endif
 
 int wab_vec_create(const WabConfig* cfg, const uint32_t* bush_thr, int32_t n_bush_thr, int64_t n_envs,
                    uint64_t seed, uint64_t env_id_base, int32_t device, WabVec** out) {
